@@ -428,11 +428,11 @@ def bench_multi_gpu(args, cfg_name, cfg, dev, rank, world, ClockSampler, hbm_pea
             pm, dg, ph, every = {}, {}, {}, {}
             for plan in ns_plans:
                 S2.timed(plan, 1)
-                # five steps timed one by one (barrier + synchronize around each, max over ranks); the MEDIAN is reported, so a
+                # --steps steps timed one by one (barrier + synchronize around each, max over ranks); the MEDIAN is reported, so a
                 # single hiccup on one of the N ranks (an allocator refill, a late NCCL channel) does not decide the plan
-                runs = [S2.timed(plan, 1) for _ in range(5)]
+                runs = [S2.timed(plan, 1) for _ in range(args.steps)]
                 every[plan] = [round(r[0], 3) for r in runs]
-                mid = sorted(range(5), key=lambda i: runs[i][0])[2]
+                mid = sorted(range(args.steps), key=lambda i: runs[i][0])[args.steps // 2]
                 pm[plan], r2, ph[plan] = runs[mid]
                 dg[plan] = content_digest(torch, dist, r2, bc, S2.table if plan != "keyshard_rs" else None)
             v2, ok2 = _verify(S2, ns_plans, dg)
@@ -447,7 +447,7 @@ def bench_multi_gpu(args, cfg_name, cfg, dev, rank, world, ClockSampler, hbm_pea
             line["north_star"].append({
                 "workload": name, "scaling": "strong", "reads": S2.n, "bases": S2.L, "k": c2["k"], "n_gpus": world,
                 "plan": b2, "plan_ms": pm, "plan_ms_every_step": every, "ms_per_step": pm[b2], "value": S2.L / pm[b2] / 1e6, "unit": "Gbases/s",
-                "timing": "median of 5 single steps, each bracketed by barrier + synchronize, max over ranks",
+                "timing": f"median of {args.steps} single steps, each bracketed by barrier + synchronize, max over ranks",
                 "phases_ms_rank0": ph[b2], "plan_phases_ms_rank0": ph, "verify": v2,
                 "exchange_rank0": (px.timings() if (px is not None and b2.endswith("/p2p")) else None),
                 "load_imbalance_max_over_mean_slots": float(mx.item()) / (float(own_bases.item()) / world)})

@@ -9,10 +9,12 @@ Inputs are written as tests/golden/<name>.{fa,fq,fa.gz}; for each input the scri
   <name>.table.npz                  non-zero (keys, counts) of the 4 GiB 15mers-counts file + its sha256
   <name>.cov_bs{S}_bc{B}.txt.gz     search-15mers output for several (bin_size, bins)
 The reference has no tests of its own (SURVEY.md §4); these outputs are the pins for oracle/ and
-for the CUDA path.
+for the CUDA path.  `python tests/golden/make_golden.py --config1 [--oracle-drivers]` writes only the
+digests of BASELINE.json config #1 (config1_digests).
 """
 import gzip
 import hashlib
+import json
 import os
 import sys
 import tempfile
@@ -25,6 +27,8 @@ sys.path.insert(0, ROOT)
 from oracle import oracle  # noqa: E402
 
 COV_PARAMS = [(10, 8), (32, 10), (1, 5), (3, 1), (10, 32), (2, 3)]
+CFG1 = "cfg1_100k_5kb_k3"
+CFG1_SOURCES = {False: "reference tools (oracle/_ref)", True: "oracle file drivers (oracle/lrb_oracle.c)"}
 
 
 def rand_seq(rng, n):
@@ -173,7 +177,42 @@ def gz_write(path, data):
         f.write(data)
 
 
+def config1_digests(oracle_drivers=False):
+    """BASELINE.json config #1 in full (100 k reads, 0.5 Gbases, -k 3 -bs 32 -bc 10) is too large to store: keep the size
+    and sha256 of its FASTA and of the three files the tools write for it (<CFG1>.files.json).  The unmodified reference
+    tools write them; only with --oracle-drivers do the oracle's file drivers, which tests/test_oracle_pins.py pins to the
+    tools' files (15mers-counts by sha256 included).  `source` records which."""
+    if not oracle_drivers:
+        assert oracle.ref_available(), "run `make -C oracle ref` first (needs /root/reference), or pass --oracle-drivers"
+    from lrbinner_b200.synth import CONFIGS, SynthSpec, write_fasta
+    cfg = CONFIGS[CFG1]
+    threads = os.cpu_count() or 8
+    with tempfile.TemporaryDirectory(dir=os.environ.get("TMPDIR", "/tmp")) as tmp:
+        fasta = os.path.join(tmp, "cfg1.fa")
+        write_fasta(fasta, SynthSpec(cfg["n_reads"], lengths=cfg["lengths"], errors=cfg["errors"], seed=cfg["seed"]).host_sequences())
+        com, tbl, cov = (os.path.join(tmp, x) for x in ("com_profs", "15mers-counts", "cov_profs"))
+        if oracle_drivers:
+            assert oracle.count_kmers_file(fasta, com, cfg["k"]) == 0
+            assert oracle.count_15mers_file(fasta, tbl) == 0
+            assert oracle.search_15mers_file(tbl, fasta, cov, 32, 10) == 0
+        else:
+            oracle.ref_count_kmers(fasta, com, cfg["k"], threads)
+            oracle.ref_count_15mers(fasta, tbl, threads)
+            oracle.ref_search_15mers(tbl, fasta, cov, 32, 10, threads)
+        files = {name: {"bytes": os.path.getsize(p), "sha256": sha256_file(p)}
+                 for name, p in (("reads.fa", fasta), ("com_profs", com), ("15mers-counts", tbl), ("cov_profs", cov))}
+    source = CFG1_SOURCES[oracle_drivers]
+    rec = {"workload": CFG1, "k": cfg["k"], "bin_size": 32, "bins": 10, "source": source, "files": files}
+    with open(os.path.join(HERE, f"{CFG1}.files.json"), "w") as f:
+        json.dump(rec, f, indent=1)
+        f.write("\n")
+    print(f"{CFG1}: digests of the files written by the {source}", flush=True)
+
+
 def main():
+    if "--config1" in sys.argv:
+        config1_digests(oracle_drivers="--oracle-drivers" in sys.argv)
+        return
     assert oracle.ref_available(), "run `make -C oracle ref` first (needs /root/reference)"
     files = build_inputs()
     for name, txt in files.items():

@@ -31,6 +31,33 @@ def test_kernel_table_gives_every_kernel_its_8d_bytes_and_bound():
     assert rows["k_mirror"]["algorithmic_bytes"] == 2.0 ** 32 and rows["k_mirror"]["launches_per_step"] == 1
 
 
+def test_dump_outputs_is_a_fixed_exact_sample_under_64_mb(tmp_path):
+    """--dump-outputs: the same rows and table entries every run, u32 values exact (the table's above 2^31 too), <= 64 MB at k = 5"""
+    import numpy as np
+    import torch
+    n, P, B = 40000, 512, 10
+    comp = torch.randint(0, 5000, (n, P), dtype=torch.int32)
+    comp[:, 0] = torch.arange(n, dtype=torch.int32)                     # row i carries i
+    hist = comp[:, :B] * 3
+    sums = comp[:, 0] + 7
+    table = torch.from_numpy((np.arange(1 << 22, dtype=np.uint32) * np.uint32(1021)).view(np.int32))   # entry i holds 1021 i < 2^32
+    a = bench.sample_outputs(comp, hist, sums, table)
+    b = bench.sample_outputs(comp, hist, sums, table)
+    assert set(a) == {"comp", "hist", "sums", "table"} and all(np.array_equal(a[x], b[x]) for x in a)
+    rows = a["comp"][:, 0].astype(np.int64)
+    assert len(rows) == bench.DUMP_ROWS and np.all(np.diff(rows) > 0)
+    assert np.array_equal(a["comp"], comp.numpy()[rows]) and np.array_equal(a["hist"], hist.numpy()[rows])
+    assert np.array_equal(a["sums"], sums.numpy()[rows])
+    keys = a["table"] / 1021
+    assert a["table"].dtype == np.float64 and len(keys) == bench.DUMP_KEYS and a["table"].max() > 2 ** 31
+    assert np.array_equal(keys, np.floor(keys)) and np.all(np.diff(keys) > 0)
+    assert sum(x.nbytes for x in a.values()) <= 64 << 20
+    bench.write_outputs(str(tmp_path / "out"), a)
+    for name, x in a.items():
+        y = np.load(tmp_path / "out" / f"{name}.npy")
+        assert y.dtype in (np.float32, np.float64) and np.array_equal(x, y)
+
+
 def test_committed_bench_lines_carry_the_contract_keys():
     """the lines kept under profiles/ (what DESIGN.md quotes) have the keys the contract names"""
     for name in ("r02_bench_n1_final.json", "r02_bench_n2_final.json", "r02_bench_n4_final.json", "r02_bench_n8_final.json"):

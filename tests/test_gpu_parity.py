@@ -772,16 +772,23 @@ def _full_size_properties(name, subsample=200):
     del table, comp, hist
 
 
-def test_config1_full_size_all_three_files_against_the_reference_tools():
-    """BASELINE.json config #1 in full (100 k reads, 0.5 Gbases, -k 3 -bs 32 -bc 10): the UNMODIFIED reference tools
-    (oracle/_ref, built from /root/reference and shipped with the repo) and the drop-ins on the same FASTA; com_profs and
-    cov_profs byte for byte, 15mers-counts by sha256 of the whole 4 GiB file — fused call and the three separate calls."""
+def test_config1_full_size_all_three_files_against_stored_digests():
+    """BASELINE.json config #1 in full (100 k reads, 0.5 Gbases, -k 3 -bs 32 -bc 10): the drop-ins on the config's FASTA
+    leave com_profs, cov_profs and the whole 4 GiB 15mers-counts with the size and sha256 stored in
+    tests/golden/cfg1_100k_5kb_k3.files.json — fused call and the three separate calls.  make_golden.py --config1 writes
+    those digests with the unmodified reference tools, or with --oracle-drivers with the oracle's file drivers, which
+    tests/test_oracle_pins.py pins to the tools' files; `source` says which wrote them."""
     import hashlib
+    import json
     import shutil
     import tempfile
-    if not oracle.ref_available():
-        pytest.skip("oracle/_ref not built (needs /root/reference at build time)")
     cfg = CONFIGS["cfg1_100k_5kb_k3"]
+    with open(os.path.join(GOLDEN, "cfg1_100k_5kb_k3.files.json")) as f:
+        gold = json.load(f)
+    assert gold["source"] in ("reference tools (oracle/_ref)", "oracle file drivers (oracle/lrb_oracle.c)"), gold["source"]
+    assert (gold["k"], gold["bin_size"], gold["bins"]) == (cfg["k"], 32, 10)
+    want = gold["files"]
+    assert want["com_profs"]["bytes"] == cfg["n_reads"] * (32 * 9 + 1) and want["cov_profs"]["bytes"] == cfg["n_reads"] * 90
     base = "/dev/shm" if os.path.isdir("/dev/shm") and shutil.disk_usage("/dev/shm").free > 12 * 2 ** 30 else None
     work = tempfile.mkdtemp(prefix="lrb_cfg1_", dir=base)
     try:
@@ -789,35 +796,26 @@ def test_config1_full_size_all_three_files_against_the_reference_tools():
         fasta = os.path.join(work, "cfg1.fa")
         write_fasta(fasta, spec.host_sequences())
         threads = os.cpu_count() or 8
-        ref = {x: os.path.join(work, "ref_" + x) for x in ("com", "tbl", "cov")}
-        oracle.ref_count_kmers(fasta, ref["com"], cfg["k"], threads)
-        oracle.ref_count_15mers(fasta, ref["tbl"], threads)
-        oracle.ref_search_15mers(ref["tbl"], fasta, ref["cov"], 32, 10, threads)
 
-        def sha(path):
+        def digest(path):
             h = hashlib.sha256()
             with open(path, "rb") as f:
                 for blk in iter(lambda: f.read(1 << 24), b""):
                     h.update(blk)
-            return h.hexdigest()
+            return {"bytes": os.path.getsize(path), "sha256": h.hexdigest()}
 
-        want_tbl = sha(ref["tbl"])
-        os.remove(ref["tbl"])
-        want_com, want_cov = open(ref["com"], "rb").read(), open(ref["cov"], "rb").read()
-        assert len(want_com) == cfg["n_reads"] * (32 * 9 + 1) and len(want_cov) == cfg["n_reads"] * 90
+        assert digest(fasta) == want["reads.fa"]                 # the input the golden digests were taken of
         out = os.path.join(work, "fused")
         runners_utils.run_profile(fasta, out, cfg["k"], 32, 10, threads, write_table=True)
-        assert open(f"{out}/profiles/com_profs", "rb").read() == want_com
-        assert open(f"{out}/profiles/cov_profs", "rb").read() == want_cov
-        assert sha(f"{out}/profiles/15mers-counts") == want_tbl
+        for name in ("com_profs", "cov_profs", "15mers-counts"):
+            assert digest(f"{out}/profiles/{name}") == want[name], ("fused", name, gold["source"])
         shutil.rmtree(out)
         out = os.path.join(work, "three")
         runners_utils.run_kmers(fasta, out, cfg["k"], threads)
         runners_utils.run_15mer_counts(fasta, out, threads)
         runners_utils.run_15mer_vecs(fasta, out, 32, 10, threads)
-        assert open(f"{out}/profiles/com_profs", "rb").read() == want_com
-        assert open(f"{out}/profiles/cov_profs", "rb").read() == want_cov
-        assert sha(f"{out}/profiles/15mers-counts") == want_tbl
+        for name in ("com_profs", "cov_profs", "15mers-counts"):
+            assert digest(f"{out}/profiles/{name}") == want[name], ("three calls", name, gold["source"])
     finally:
         shutil.rmtree(work, ignore_errors=True)
 

@@ -66,6 +66,32 @@ def test_oracle_file_drivers_byte_identical(tmp_path):
         assert open(out, "rb").read() == _gz(os.path.join(GOLDEN, f"g03_edge.com_k{k}.txt.gz"))
 
 
+@pytest.mark.parametrize("name", ["g03_edge.fa", "g06_community.fa"])
+def test_oracle_table_and_search_file_drivers_byte_identical(name, tmp_path):
+    # the whole 15mers-counts file (size + sha256 of the reference's) and search-15mers' text read back from it
+    import hashlib
+    import shutil
+    import tempfile
+    stem = name.split(".")[0]
+    src = os.path.join(GOLDEN, name)
+    gold = np.load(os.path.join(GOLDEN, f"{stem}.table.npz"))
+    base = "/dev/shm" if os.path.isdir("/dev/shm") and shutil.disk_usage("/dev/shm").free > 6 * 2 ** 30 else str(tmp_path)
+    work = tempfile.mkdtemp(prefix="lrb_pins_", dir=base)
+    try:
+        table, cov = os.path.join(work, "15mers-counts"), os.path.join(work, "cov_profs")
+        assert oracle.count_15mers_file(src, table) == 0
+        h = hashlib.sha256()
+        with open(table, "rb") as f:
+            for blk in iter(lambda: f.read(1 << 24), b""):
+                h.update(blk)
+        assert os.path.getsize(table) == int(gold["file_bytes"]) and h.hexdigest() == str(gold["sha256"])
+        for bs, bc in COV_PARAMS:
+            assert oracle.search_15mers_file(table, src, cov, bs, bc) == 0
+            assert open(cov, "rb").read() == _gz(os.path.join(GOLDEN, f"{stem}.cov_bs{bs}_bc{bc}.txt.gz")), (name, bs, bc)
+    finally:
+        shutil.rmtree(work, ignore_errors=True)
+
+
 def test_known_answers_survey_section4():
     # SURVEY.md section 4 probes, observed on the reference binaries
     assert _gz(os.path.join(GOLDEN, "g01_identical25.cov_bs10_bc8.txt.gz")).splitlines()[0] == b"0.000000 1.000000 0.000000 0.000000 0.000000 0.000000 0.000000 0.000000"
