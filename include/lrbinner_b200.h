@@ -109,6 +109,18 @@ int lrb_dev_count(const lrb_reads_view* dev, uint32_t* table, uint64_t blk_lo, u
                   uint32_t key_lo, uint32_t key_hi, void* stream);
 int lrb_dev_mirror(uint32_t* table, void* stream);
 
+/* Abundance spectrum of the table (the reference has no counterpart: it never reads the table as a distribution).
+ * Reads only the bit-15-clear keys in [key_lo, key_hi) — one key per {x, revcomp(x)} pair, 2 GiB for the whole table —
+ * so neither a mirror nor a complete key space is needed (a key-sharded table works as it is).  Accumulates into
+ * spectrum[max_count + 3] u64 (device; the caller zeroes it once):
+ *   spectrum[c]   += keys with T == c, c < max_count     spectrum[max_count]     += keys with T >= max_count
+ *   spectrum[max_count + 1] += sum of T over those keys  spectrum[max_count + 2]  = max(itself, largest T in the range)
+ * so spectra of disjoint key ranges added into one buffer equal the spectrum of their union.  The table is not written.
+ * 2 <= max_count <= LRB_SPECTRUM_MAX_COUNT; an empty key range does nothing. */
+#define LRB_SPECTRUM_MAX_COUNT (1u << 24)
+int lrb_dev_table_spectrum(const uint32_t* table, uint32_t key_lo, uint32_t key_hi, uint32_t max_count, uint64_t* spectrum,
+                           void* stream);
+
 /* Multi-GPU table exchange helpers (the reference has no counterpart: it is single-process; SURVEY.md 8e).
  * lrb_dev_copy2d: pitched device-to-device copy on the copy engines; src may be a peer GPU's table mapped into this
  * process (rows of 2^15 bit-15-clear entries, pitch 2^16 entries).  lrb_dev_add_planes: dst rows (pitched) += the sum of
@@ -289,6 +301,10 @@ void* lrb_pinned_alloc(size_t bytes);
 void lrb_pinned_free(void* p);
 int lrb_ctx_table_load(lrb_ctx* ctx, const char* path);          /* readKmerFile -> HBM */
 int lrb_ctx_table_save(lrb_ctx* ctx, const char* path);          /* HBM -> writeKmerFile format */
+/* lrb_dev_table_spectrum over the whole table of the primary device (complete after lrb_profile_host with a count, a
+ * multi-device call included, or lrb_ctx_table_load) into spectrum_host[max_count + 3]; synchronous.  LRB_EINVAL when the
+ * context holds no table.  The table is left as it is.  No reference counterpart. */
+int lrb_ctx_table_spectrum(lrb_ctx* ctx, uint32_t max_count, uint64_t* spectrum_host);
 
 /* Launch accounting (csrc/prof.cu).  lrb_prof_launches: kernels this library has launched since it was loaded (always
  * counted; bench.py's gpu_launches).  lrb_prof_enable(1) additionally brackets every launch with CUDA events on the stream
@@ -317,6 +333,17 @@ int lrb_write_coverage_npy(const char* path, const uint32_t* hist, const uint32_
                            int threads);
 int lrb_table_write_file(const char* path, const uint32_t* table);  /* u64 2^30, then 2^30 u32 */
 int lrb_table_read_file(const char* path, uint32_t* table);
+/* What a spectrum (lrb_dev_table_spectrum layout) implies for the coverage profile with -bs bin_size -bc bins:
+ * mass[b] = sum over c of c * n_c * [coverage bin of c == b], i.e. the number of windows that land in bin b summed over
+ * all reads, when the table was counted from the same reads that are searched (each canonical pair counted c times
+ * is met by c windows, all binned by c).  Keys at or above max_count add their sum to the last bin.  LRB_EINVAL for
+ * bin_size < 1 or bins outside [1, LRB_MAX_BINS], and when keys at or above max_count exist but
+ * max_count < bin_size * (bins + 1): their bin is then not determined by the spectrum.  No reference counterpart. */
+int lrb_spectrum_bin_mass(const uint64_t* spectrum, uint32_t max_count, long bin_size, int bins, uint64_t* mass);
+/* jellyfish `histo` text of a spectrum: "c n_c\n" for every c in [1, max_count) with n_c > 0, ascending, then
+ * "max_count n_over\n" when keys at or above max_count exist.  Counts are of canonical 15-mers (each {x, revcomp(x)}
+ * pair once).  No reference counterpart. */
+int lrb_write_spectrum_txt(const char* path, const uint64_t* spectrum, uint32_t max_count);
 
 /* canonical k-mer index table of count-kmers (compute_kmer_inds, count-kmers.cpp:38-64); returns P. */
 int lrb_kmer_lut(int k, uint16_t* lut /* 4^k */);
@@ -328,6 +355,9 @@ int lrb_count_kmers(const char* reads_path, const char* out_txt, int k, int thre
 int lrb_count_15mers(const char* reads_path, const char* out_table, int threads);
 int lrb_search_15mers(const char* table_path, const char* reads_path, const char* out_txt, long bin_size, int bins,
                       int threads);
+/* Abundance spectrum of a 15mers-counts file as lrb_write_spectrum_txt text (loaded on device LRB_DEVICE).  Missing or
+ * malformed table file: LRB_EIO / LRB_EFORMAT; no device: LRB_ECUDA.  No reference counterpart. */
+int lrb_table_spectrum(const char* table_path, const char* out_txt, uint32_t max_count);
 /* Fused stage: parse once, keep reads + table in HBM, write com_profs, cov_profs (and 15mers-counts if
  * write_table) into out_dir/profiles/; write_npy additionally emits com_profs.npy / cov_profs.npy. */
 int lrb_profile(const char* reads_path, const char* out_dir, int k, long bin_size, int bins, int threads,

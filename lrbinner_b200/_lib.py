@@ -13,6 +13,7 @@ LRB_OK, LRB_EINVAL, LRB_EIO, LRB_ECUDA, LRB_ENOMEM, LRB_EFORMAT = range(6)
 TABLE_ENTRIES = 1 << 30
 TILE_BLOCKS = 256
 MAX_BINS = 4096
+SPECTRUM_MAX_COUNT = 1 << 24
 
 
 class LrbError(RuntimeError):
@@ -81,6 +82,7 @@ _SIG = {
     "lrb_dev_composition": (C.c_int, [C.POINTER(ReadsView), C.c_int, _P, C.c_uint64, C.c_uint64, _P]),
     "lrb_dev_count": (C.c_int, [C.POINTER(ReadsView), _P, C.c_uint64, C.c_uint64, C.c_uint32, C.c_uint32, _P]),
     "lrb_dev_mirror": (C.c_int, [_P, _P]),
+    "lrb_dev_table_spectrum": (C.c_int, [_P, C.c_uint32, C.c_uint32, C.c_uint32, _P, _P]),
     "lrb_dev_copy2d": (C.c_int, [_P, C.c_uint64, _P, C.c_uint64, C.c_uint64, C.c_uint64, _P]),
     "lrb_dev_add_planes": (C.c_int, [_P, C.c_uint64, _P, C.c_uint64, C.c_int, C.c_uint32, C.c_uint32, _P]),
     "lrb_dev_search": (C.c_int, [C.POINTER(ReadsView), _P, C.c_long, C.c_int, _P, _P, C.c_uint64, C.c_uint64,
@@ -111,6 +113,7 @@ _SIG = {
     "lrb_pinned_free": (None, [_P]),
     "lrb_ctx_table_load": (C.c_int, [_P, C.c_char_p]),
     "lrb_ctx_table_save": (C.c_int, [_P, C.c_char_p]),
+    "lrb_ctx_table_spectrum": (C.c_int, [_P, C.c_uint32, _P]),
     "lrb_prof_launches": (C.c_uint64, []),
     "lrb_prof_enable": (C.c_int, [C.c_int]),
     "lrb_prof_report": (C.c_int, [_P, C.c_size_t]),
@@ -121,10 +124,13 @@ _SIG = {
     "lrb_write_coverage_npy": (C.c_int, [C.c_char_p, _P, _P, C.c_uint64, C.c_int, C.c_int]),
     "lrb_table_write_file": (C.c_int, [C.c_char_p, _P]),
     "lrb_table_read_file": (C.c_int, [C.c_char_p, _P]),
+    "lrb_spectrum_bin_mass": (C.c_int, [_P, C.c_uint32, C.c_long, C.c_int, _P]),
+    "lrb_write_spectrum_txt": (C.c_int, [C.c_char_p, _P, C.c_uint32]),
     "lrb_kmer_lut": (C.c_int, [C.c_int, _P]),
     "lrb_count_kmers": (C.c_int, [C.c_char_p, C.c_char_p, C.c_int, C.c_int]),
     "lrb_count_15mers": (C.c_int, [C.c_char_p, C.c_char_p, C.c_int]),
     "lrb_search_15mers": (C.c_int, [C.c_char_p, C.c_char_p, C.c_char_p, C.c_long, C.c_int, C.c_int]),
+    "lrb_table_spectrum": (C.c_int, [C.c_char_p, C.c_char_p, C.c_uint32]),
     "lrb_profile": (C.c_int, [C.c_char_p, C.c_char_p, C.c_int, C.c_long, C.c_int, C.c_int, C.c_int, C.c_int]),
     "lrb_profile_multi": (C.c_int, [C.c_char_p, C.c_char_p, C.c_int, C.c_long, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int]),
 }

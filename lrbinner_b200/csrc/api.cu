@@ -1048,6 +1048,23 @@ extern "C" int lrb_ctx_table_load(lrb_ctx* c, const char* path) {
     return rc;
 }
 
+extern "C" int lrb_ctx_table_spectrum(lrb_ctx* c, uint32_t max_count, uint64_t* spectrum_host) {
+    if (!c || !spectrum_host) return lrb_set_error(LRB_EINVAL, "lrb_ctx_table_spectrum: null argument");
+    if (max_count < 2 || max_count > LRB_SPECTRUM_MAX_COUNT)
+        return lrb_set_error(LRB_EINVAL, "lrb_ctx_table_spectrum: max_count must be in [2, %u] (got %u)", LRB_SPECTRUM_MAX_COUNT, max_count);
+    if (!c->table_ready) return lrb_set_error(LRB_EINVAL, "lrb_ctx_table_spectrum: no table in this context");
+    CTX_CUDA(cudaSetDevice(c->device));
+    const size_t bytes = sizeof(uint64_t) * ((size_t)max_count + 3);
+    DevBuf spec;
+    int rc = spec.reserve(bytes);
+    if (!rc && cudaMemsetAsync(spec.p, 0, bytes, c->stream) != cudaSuccess) rc = lrb_set_error(LRB_ECUDA, "cudaMemsetAsync failed");
+    if (!rc) rc = lrb_dev_table_spectrum((const uint32_t*)c->table.p, 0, (uint32_t)kTableEntries, max_count, (uint64_t*)spec.p, c->stream);
+    if (!rc && cudaMemcpyAsync(spectrum_host, spec.p, bytes, cudaMemcpyDeviceToHost, c->stream) != cudaSuccess) rc = lrb_set_error(LRB_ECUDA, "D2H failed");
+    if (cudaStreamSynchronize(c->stream) != cudaSuccess && !rc) rc = lrb_set_error(LRB_ECUDA, "spectrum failed: %s", cudaGetErrorString(cudaGetLastError()));
+    spec.release();
+    return rc;
+}
+
 // ---- synthetic reads ---------------------------------------------------------------------------
 namespace {
 
@@ -1189,6 +1206,19 @@ extern "C" int lrb_search_15mers(const char* table_path, const char* reads_path,
     std::vector<uint32_t> hist((size_t)n * bins + 1), sums(n + 1);
     if ((rc = lrb_profile_host(cg.c, rg.r, 0, bin_size, bins, nullptr, hist.data(), sums.data(), nullptr, LRB_PROFILE_USE_LOADED_TABLE))) return rc;
     return lrb_write_coverage_txt(out_txt, hist.data(), sums.data(), n, bins, threads);
+}
+
+extern "C" int lrb_table_spectrum(const char* table_path, const char* out_txt, uint32_t max_count) {
+    if (!table_path || !out_txt) return lrb_set_error(LRB_EINVAL, "lrb_table_spectrum: null path");
+    if (max_count < 2 || max_count > LRB_SPECTRUM_MAX_COUNT)
+        return lrb_set_error(LRB_EINVAL, "max_count must be in [2, %u] (got %u)", LRB_SPECTRUM_MAX_COUNT, max_count);
+    int rc;
+    CtxGuard cg;
+    if ((rc = create_ctx(1, &cg.c))) return rc;
+    if ((rc = lrb_ctx_table_load(cg.c, table_path))) return rc;
+    std::vector<uint64_t> spec((size_t)max_count + 3);
+    if ((rc = lrb_ctx_table_spectrum(cg.c, max_count, spec.data()))) return rc;
+    return lrb_write_spectrum_txt(out_txt, spec.data(), max_count);
 }
 
 extern "C" int lrb_profile_multi(const char* reads_path, const char* out_dir, int k, long bin_size, int bins, int threads,

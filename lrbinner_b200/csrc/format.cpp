@@ -19,6 +19,7 @@
 
 #include "common.h"
 #include "fixed6.h"
+#include "lane_core.cuh"
 
 // ---- error plumbing ----------------------------------------------------------------------------
 static thread_local char t_err[512] = "";
@@ -240,5 +241,38 @@ extern "C" int lrb_table_read_file(const char* path, uint32_t* table) {
         left -= (size_t)r;
     }
     close(fd);
+    return LRB_OK;
+}
+
+// ---- abundance spectrum of the table (lrb_dev_table_spectrum layout: n_c for c < M, then n_over, sum_over, max) ----
+extern "C" int lrb_spectrum_bin_mass(const uint64_t* spectrum, uint32_t max_count, long bin_size, int bins, uint64_t* mass) {
+    if (!spectrum || !mass) return lrb_set_error(LRB_EINVAL, "lrb_spectrum_bin_mass: null argument");
+    if (bin_size < 1) return lrb_set_error(LRB_EINVAL, "lrb_spectrum_bin_mass: bin_size must be >= 1");
+    if (bins < 1 || bins > LRB_MAX_BINS) return lrb_set_error(LRB_EINVAL, "lrb_spectrum_bin_mass: bins must be in [1, %d]", LRB_MAX_BINS);
+    const uint64_t M = max_count;
+    // every count >= S * (B + 1) lands in the last bin; below that the spectrum must resolve the count itself
+    const bool over_determined = bin_size < (long)M && M >= (uint64_t)bin_size * (uint64_t)(bins + 1);
+    if (spectrum[M] > 0 && !over_determined)
+        return lrb_set_error(LRB_EINVAL, "lrb_spectrum_bin_mass: %llu keys counted >= max_count %u, which is below bin_size * (bins + 1) = %lld",
+                             (unsigned long long)spectrum[M], max_count, (long long)bin_size * (bins + 1));
+    const uint32_t S32 = bin_size > 0xFFFFFFFFl ? 0xFFFFFFFFu : (uint32_t)bin_size;
+    const uint64_t magic = lrb::coverage_magic(S32);
+    std::fill(mass, mass + bins, 0ull);
+    for (uint64_t c = 0; c < M; ++c)
+        if (spectrum[c]) mass[lrb::coverage_bin((uint32_t)c, S32, magic, (uint32_t)bins)] += c * spectrum[c];
+    mass[bins - 1] += spectrum[M + 1];
+    return LRB_OK;
+}
+
+extern "C" int lrb_write_spectrum_txt(const char* path, const uint64_t* spectrum, uint32_t max_count) {
+    if (!path || !spectrum) return lrb_set_error(LRB_EINVAL, "lrb_write_spectrum_txt: null argument");
+    FILE* f = fopen(path, "w");
+    if (!f) return lrb_set_error(LRB_EIO, "cannot open %s for writing", path);
+    bool ok = true;
+    for (uint32_t c = 1; c < max_count && ok; ++c)
+        if (spectrum[c]) ok = fprintf(f, "%u %llu\n", c, (unsigned long long)spectrum[c]) > 0;
+    if (ok && spectrum[max_count]) ok = fprintf(f, "%u %llu\n", max_count, (unsigned long long)spectrum[max_count]) > 0;
+    if (fclose(f) != 0) ok = false;
+    if (!ok) return lrb_set_error(LRB_EIO, "short write to %s", path);
     return LRB_OK;
 }

@@ -8,6 +8,7 @@
 //   * count  : one THREAD per block, grid-stride; read-oblivious because padding slots are invalid;
 //     one RED.ADD.U32 per valid window on the bit-15-clear key of {val, rc(val)}.
 //   * mirror : 64x64 tiled "transpose" T[x] = T[rc(x)] for bit-15-set x (coalesced both ways).
+//   * spectrum: grid-stride 16-byte reads of the bit-15-clear half; small counts into per-lane shared counters.
 // No tensor cores anywhere: nothing here is a dense contraction (BASELINE.json north_star).
 #include <cuda_runtime.h>
 #include <algorithm>
@@ -147,6 +148,113 @@ __global__ void __launch_bounds__(256) k_mirror_v4(uint32_t* __restrict__ table)
         const uint4 o = make_uint4(tile[s0][col], tile[s1][col], tile[s2][col], tile[s3][col]);
         __stcs(reinterpret_cast<uint4*>(table + mirror_dst_index(t, a, c4)), o);
     }
+}
+
+// ------------------------------------------------------------------------------------------------
+// abundance spectrum of the canonical half (no reference counterpart): spectrum[c] += #keys with T == c (c < M),
+// [M] += #keys with T >= M, [M+1] += their sum, [M+2] = max.  Canonical index ci in [0, 2^29) = (row:14 | col:15) maps to
+// the table word (row << 16) | col; the kernel walks 16-byte units of 4 canonical entries, which never straddle a row.
+// The values are heavily concentrated (zeros of a sparse table, the error floor at small counts), so one shared-memory
+// atomic per entry into one histogram would serialise on a few addresses.  Counts below kSpecLaneBins go to counters
+// private to the lane instead — s_lane[warp][c][lane], so lane l only ever touches bank l and a warp's update is one
+// conflict-free RED whatever the values — and are summed over the lanes once per CTA.  Larger counts are spread out
+// (genomic peaks) and take the CTA's shared histogram; counts past that take global u64 atomics.  A thread whose 4
+// values are equal adds them as one update of 4.
+// ------------------------------------------------------------------------------------------------
+constexpr int kSpecThreads = 256;
+constexpr int kSpecWarps = kSpecThreads / 32;
+constexpr int kSpecUnroll = 4;              // 16-byte loads in flight per thread
+constexpr uint32_t kSpecLaneBins = 32;      // counts below this: per-lane counters
+constexpr uint32_t kSpecSmemBins = 8192;    // counts below this: the CTA's shared histogram; above: global u64 atomics
+constexpr size_t kSpecSmem = sizeof(uint32_t) * (kSpecSmemBins + (size_t)kSpecWarps * kSpecLaneBins * 32);  // 64 KiB
+
+__device__ __forceinline__ uint64_t canon_word(uint64_t ci) { return ((ci >> 15) << 16) | (ci & 0x7FFFu); }
+
+__device__ __forceinline__ void smem_add(uint32_t* p, uint32_t n) {  // fire-and-forget shared-memory add (RED)
+    asm volatile("red.shared.add.u32 [%0], %1;" ::"r"((uint32_t)__cvta_generic_to_shared(p)), "r"(n) : "memory");
+}
+
+struct SpecAcc {
+    uint32_t n_over = 0, vmax = 0;
+    uint64_t sum_over = 0;
+};
+
+// table value v counted w times
+__device__ __forceinline__ void spec_add(uint32_t* s_hist, uint32_t* my_lane, unsigned long long* spec, uint32_t M, uint32_t v,
+                                         uint32_t w, SpecAcc& a) {
+    if (v < M) {
+        if (v < kSpecLaneBins) smem_add(my_lane + v * 32u, w);
+        else if (v < kSpecSmemBins) smem_add(s_hist + v, w);
+        else atomicAdd(spec + v, (unsigned long long)w);
+    } else {
+        a.n_over += w;
+        a.sum_over += (uint64_t)v * w;
+    }
+    a.vmax = max(a.vmax, v);
+}
+
+__global__ void __launch_bounds__(kSpecThreads)
+k_table_spectrum(const uint32_t* __restrict__ table, uint64_t u_beg, uint64_t u_end, uint64_t e0_lo, uint64_t e0_hi,
+                 uint64_t e1_lo, uint64_t e1_hi, uint32_t M, unsigned long long* __restrict__ spec) {
+    extern __shared__ uint32_t s_spec[];
+    uint32_t* s_hist = s_spec;                                   // [kSpecSmemBins]
+    uint32_t* s_lane = s_spec + kSpecSmemBins;                   // [kSpecWarps][kSpecLaneBins][32]
+    for (uint32_t i = threadIdx.x; i < kSpecSmemBins + kSpecWarps * kSpecLaneBins * 32; i += kSpecThreads) s_spec[i] = 0;
+    __syncthreads();
+
+    SpecAcc a;
+    const uint32_t lane = threadIdx.x & 31u, warp_in_cta = threadIdx.x >> 5;
+    uint32_t* my_lane = s_lane + warp_in_cta * (kSpecLaneBins * 32) + lane;
+    const uint64_t n_units = u_end - u_beg;
+    const uint64_t stride = (uint64_t)gridDim.x * kSpecThreads * kSpecUnroll;
+    for (uint64_t base = ((uint64_t)blockIdx.x * kSpecWarps + warp_in_cta) * (32 * kSpecUnroll); base < n_units; base += stride) {
+        uint4 q[kSpecUnroll];
+#pragma unroll
+        for (int k = 0; k < kSpecUnroll; ++k) {   // a warp reads 4 x 512 contiguous bytes
+            const uint64_t u = base + (uint64_t)k * 32 + lane;
+            if (u < n_units) q[k] = __ldcs(reinterpret_cast<const uint4*>(table + canon_word((u_beg + u) * 4)));
+        }
+#pragma unroll
+        for (int k = 0; k < kSpecUnroll; ++k) {
+            if (base + (uint64_t)k * 32 + lane >= n_units) continue;
+            if (q[k].x == q[k].y && q[k].x == q[k].z && q[k].x == q[k].w) {
+                spec_add(s_hist, my_lane, spec, M, q[k].x, 4u, a);
+            } else {
+                spec_add(s_hist, my_lane, spec, M, q[k].x, 1u, a);
+                spec_add(s_hist, my_lane, spec, M, q[k].y, 1u, a);
+                spec_add(s_hist, my_lane, spec, M, q[k].z, 1u, a);
+                spec_add(s_hist, my_lane, spec, M, q[k].w, 1u, a);
+            }
+        }
+    }
+    // the < 8 entries before the first / after the last whole unit (key ranges not aligned to 4)
+    if (blockIdx.x == 0 && threadIdx.x < 16) {
+        const uint64_t ci = threadIdx.x < 8 ? e0_lo + threadIdx.x : e1_lo + (threadIdx.x - 8);
+        if (ci < (threadIdx.x < 8 ? e0_hi : e1_hi)) spec_add(s_hist, my_lane, spec, M, __ldg(table + canon_word(ci)), 1u, a);
+    }
+
+    a.n_over = __reduce_add_sync(0xFFFFFFFFu, a.n_over);
+    a.vmax = __reduce_max_sync(0xFFFFFFFFu, a.vmax);
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) a.sum_over += __shfl_xor_sync(0xFFFFFFFFu, a.sum_over, o);
+    if (lane == 0) {
+        if (a.n_over) {
+            atomicAdd(spec + M, (unsigned long long)a.n_over);
+            atomicAdd(spec + M + 1, (unsigned long long)a.sum_over);
+        }
+        atomicMax(spec + M + 2, (unsigned long long)a.vmax);
+    }
+    __syncwarp();
+    // lane c sums count c over the warp's 32 lane counters (rotated start: the 32 lanes read 32 different banks)
+    if (lane < kSpecLaneBins) {
+        const uint32_t* row = s_lane + warp_in_cta * (kSpecLaneBins * 32) + lane * 32u;
+        uint32_t n = 0;
+        for (uint32_t j = 0; j < 32; ++j) n += row[(lane + j) & 31u];
+        if (n) smem_add(s_hist + lane, n);
+    }
+    __syncthreads();
+    for (uint32_t i = threadIdx.x; i < min(M, kSpecSmemBins); i += kSpecThreads)
+        if (s_hist[i]) atomicAdd(spec + i, (unsigned long long)s_hist[i]);
 }
 
 // validity bitmap from the read lengths (one warp per read), then the sparse exceptions on top
@@ -380,6 +488,34 @@ extern "C" int lrb_dev_mirror(uint32_t* table, void* stream) {
     static const bool scalar = getenv("LRB_MIRROR_SCALAR") && atoi(getenv("LRB_MIRROR_SCALAR")) > 0;   // round-1 kernel, for A/B timing
     if (scalar) LRB_LAUNCH("k_mirror", (cudaStream_t)stream, k_mirror<<<1u << 17, 256, 0, (cudaStream_t)stream>>>(table));
     else LRB_LAUNCH("k_mirror", (cudaStream_t)stream, k_mirror_v4<<<1u << 17, 256, 0, (cudaStream_t)stream>>>(table));
+    LRB_CUDA(cudaGetLastError());
+    return LRB_OK;
+}
+
+// canonical (bit-15-clear) keys below `key` (key <= 2^30): 2^15 per complete 2^16-entry row, then the clear half of its row
+static uint64_t canon_rank(uint64_t key) { return ((key >> 16) << 15) + std::min<uint64_t>(key & 0xFFFFu, 0x8000u); }
+
+extern "C" int lrb_dev_table_spectrum(const uint32_t* table, uint32_t key_lo, uint32_t key_hi, uint32_t max_count,
+                                      uint64_t* spectrum, void* stream) {
+    if (!table || !spectrum) return lrb_set_error(LRB_EINVAL, "lrb_dev_table_spectrum: null argument");
+    if ((uintptr_t)table & 15u) return lrb_set_error(LRB_EINVAL, "lrb_dev_table_spectrum: the table must be 16-byte aligned");
+    if (max_count < 2 || max_count > LRB_SPECTRUM_MAX_COUNT)
+        return lrb_set_error(LRB_EINVAL, "lrb_dev_table_spectrum: max_count must be in [2, %u] (got %u)", LRB_SPECTRUM_MAX_COUNT, max_count);
+    const uint64_t hi = std::min<uint64_t>(key_hi, kTableEntries);
+    if (key_lo >= hi) return LRB_OK;
+    const uint64_t ci_lo = canon_rank(key_lo), ci_hi = canon_rank(hi);
+    if (ci_lo >= ci_hi) return LRB_OK;
+    // whole 4-entry units [u_beg, u_end); the entries outside them are the edges e0 (head) and e1 (tail), < 8 in all
+    uint64_t u_beg = (ci_lo + 3) / 4, u_end = ci_hi / 4;
+    uint64_t e0_lo = ci_lo, e0_hi = u_beg * 4, e1_lo = u_end * 4, e1_hi = ci_hi;
+    if (u_beg >= u_end) { u_end = u_beg; e0_hi = ci_hi; e1_lo = e1_hi = 0; }
+    const uint64_t per_cta = (uint64_t)kSpecThreads * kSpecUnroll;
+    const uint64_t want = std::max<uint64_t>(1, (u_end - u_beg + per_cta - 1) / per_cta);
+    const unsigned grid = (unsigned)std::min<uint64_t>(want, (uint64_t)sm_count() * 3);  // 3 x 64 KiB per SM
+    cudaStream_t st = (cudaStream_t)stream;
+    LRB_CUDA(cudaFuncSetAttribute(k_table_spectrum, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSpecSmem));
+    LRB_LAUNCH("k_table_spectrum", st, k_table_spectrum<<<grid, kSpecThreads, kSpecSmem, st>>>(table, u_beg, u_end, e0_lo, e0_hi, e1_lo, e1_hi,
+                                                                                  max_count, reinterpret_cast<unsigned long long*>(spectrum)));
     LRB_CUDA(cudaGetLastError());
     return LRB_OK;
 }

@@ -184,6 +184,13 @@ class Context:
     def table_save(self, path):
         check(lib.lrb_ctx_table_save(self._h, str(path).encode()))
 
+    def table_spectrum(self, max_count=65536):
+        """Abundance spectrum of the context's table: u64[max_count + 3] = n_c for c < max_count (canonical 15-mers
+        counted c times), then keys counted >= max_count, their sum, and the largest count (lrb_dev_table_spectrum)."""
+        spec = np.zeros(_spectrum_len(max_count), dtype=np.uint64)
+        check(lib.lrb_ctx_table_spectrum(self._h, int(max_count), _ptr(spec)))
+        return spec
+
     def close(self):
         if self._h:
             lib.lrb_ctx_destroy(self._h)
@@ -284,6 +291,37 @@ def dev_fill_valid(dr, exc_blk=None, exc_word=None):
 
 def dev_mirror(table):
     check(lib.lrb_dev_mirror(C.c_void_p(table.data_ptr()), _stream()))
+
+
+def _spectrum_len(max_count):
+    if not 0 <= int(max_count) < 2 ** 32:   # the C ABI takes a u32; range [2, SPECTRUM_MAX_COUNT] is checked there
+        raise _lib.LrbError(_lib.LRB_EINVAL, f"max_count {max_count} out of range")
+    return int(max_count) + 3
+
+
+def dev_table_spectrum(table, max_count, key_lo=0, key_hi=_lib.TABLE_ENTRIES, out=None):
+    """Accumulate the spectrum of the bit-15-clear keys of table[key_lo, key_hi) into `out` (int64 tensor of
+    max_count + 3 words read as u64, zeroed here when not given) and return it."""
+    import torch
+    n = _spectrum_len(max_count)
+    if out is None:
+        out = torch.zeros(n, dtype=torch.int64, device=table.device)
+    elif out.numel() < n or out.element_size() != 8 or not out.is_contiguous():
+        raise _lib.LrbError(_lib.LRB_EINVAL, f"spectrum buffer must be {n} contiguous 8-byte words")
+    check(lib.lrb_dev_table_spectrum(C.c_void_p(table.data_ptr()), int(key_lo), min(int(key_hi), _lib.TABLE_ENTRIES), int(max_count),
+                                     C.c_void_p(out.data_ptr()), _stream()))
+    return out
+
+
+def spectrum_bin_mass(spectrum, bin_size, bins):
+    """Windows per coverage bin implied by a spectrum (lrb_spectrum_bin_mass): equals hist.sum(0) of a search of the
+    reads the table was counted from, with the same bin_size / bins."""
+    spec = np.ascontiguousarray(spectrum, dtype=np.uint64)
+    if spec.size < 3:
+        raise _lib.LrbError(_lib.LRB_EINVAL, "a spectrum has max_count + 3 words")
+    mass = np.zeros(max(int(bins), 1), dtype=np.uint64)
+    check(lib.lrb_spectrum_bin_mass(_ptr(spec), spec.size - 3, int(bin_size), int(bins), _ptr(mass)))
+    return mass
 
 
 def dev_search(dr, table, bin_size, bins, hist, sums, tile_lo=0, tile_hi=None, key_lo=0, key_hi=_lib.TABLE_ENTRIES):

@@ -50,6 +50,16 @@ def run_15mer_vecs(reads_path, output, bin_size, bin_count, threads):
     check_proc(o, "Counting 15-mer profiles")
 
 
+def run_15mer_histo(output, threads, max_count=65536):
+    """Abundance spectrum of {output}/profiles/15mers-counts as {output}/profiles/15mers-histo (jellyfish `histo`
+    layout: "count n_kmers" lines of canonical 15-mers), to choose -bs / -bc from (INTEGRATION.md).  No reference
+    counterpart; `threads` is accepted for symmetry with the other runners."""
+    logger.debug(f"LIB::lrb_table_spectrum \"{output}/profiles/15mers-counts\" \"{output}/profiles/15mers-histo\" {max_count}")
+    o = _lib.lib.lrb_table_spectrum(os.fsencode(f"{output}/profiles/15mers-counts"), os.fsencode(f"{output}/profiles/15mers-histo"),
+                                    int(max_count))
+    check_proc(o, "15-mer abundance spectrum")
+
+
 def run_profile(reads_path, output, k_size, bin_size, bin_count, threads, write_table=True, write_npy=False, n_gpus=0):
     """Fused stages 1_1 + 1_2 + 2_1: leaves com_profs, cov_profs (and 15mers-counts unless write_table=False,
     needed by --resume with changed -bs/-bc) in {output}/profiles, byte-identical to the three separate calls.
