@@ -89,6 +89,25 @@ int lrb_reads_exceptions(const lrb_reads* r, const uint32_t** blk, const uint32_
 int lrb_reads_slice(const lrb_reads* r, uint64_t read_lo, uint64_t read_hi, lrb_reads** out);
 void lrb_reads_free(lrb_reads* r);
 
+/* Segment reader: the records of a FASTA/FASTQ file (plain or gzip, same semantics as lrb_reads_from_file) as a sequence of
+ * read sets of bounded size, so that host memory does not grow with the file and no read set reaches the 2^32-block limit
+ * of one lrb_reads.  A SEGMENT is a contiguous run of whole records of at most `segment_bases` bases (a longer record forms
+ * a segment on its own) and always below 2^32 blocks; the concatenated segments are exactly lrb_reads_from_file's read
+ * set.  The file is read in chunks (plain files with pread, never mapped whole), so one segment needs its packed stream
+ * (0.375 B/base) + two chunks + one record.
+ * segment_bases = 0: automatic — the bases whose stream plus the rows of a fused k = 5 / 32-bin profile (2180 B per read,
+ * counted as 2.18 B/base at 1 kb per read) fit half of MemAvailable at open time, capped 2^28 blocks below the block
+ * limit; LRB_SEGMENT_BASES=n overrides it.  A missing or unreadable file is an empty stream.
+ * lrb_reader_next: the next segment as an ordinary read set (exception list built; free with lrb_reads_free), or *out =
+ * NULL at the end.  lrb_reader_rewind: start again from the first record.  lrb_reader_tell: reads, bases and segments
+ * delivered since open / rewind; *at_end = 1 once no record is left (any argument may be NULL). */
+typedef struct lrb_reader lrb_reader;
+int lrb_reader_open(const char* path, int threads, uint64_t segment_bases, lrb_reader** out);
+int lrb_reader_next(lrb_reader* reader, lrb_reads** out);
+int lrb_reader_rewind(lrb_reader* reader);
+int lrb_reader_tell(const lrb_reader* reader, uint64_t* reads, uint64_t* bases, uint64_t* segments, int* at_end);
+void lrb_reader_close(lrb_reader* reader);
+
 /* ------------------------------------------------------------------------------------------------
  * Device-pointer level (the kernels).  All pointers are DEVICE pointers; `stream` is a cudaStream_t
  * passed as void* (NULL = default stream).  Calls are asynchronous on that stream.
@@ -269,13 +288,18 @@ void lrb_ctx_destroy(lrb_ctx* ctx);
  * comp_counts[N*P] (P from k), cov_hist[N*bins], cov_sums[N] are HOST buffers (may be NULL to skip the
  * corresponding phase).  If table_host != NULL the 4 GiB table is copied back as well.
  * flags: LRB_PROFILE_USE_LOADED_TABLE — skip the count phase and search the table already in the context;
- *        LRB_PROFILE_KEEP_TABLE — count even when neither the search nor table_host asks for it (lrb_ctx_table_save follows).
+ *        LRB_PROFILE_KEEP_TABLE — count even when neither the search nor table_host asks for it (lrb_ctx_table_save follows);
+ *        LRB_PROFILE_ADD_TO_TABLE — count, ADDING this read set's windows to the complete table already in the context
+ *        (after a count or lrb_ctx_table_load) instead of starting from zero: tables of read sets profiled one after another
+ *        this way equal the table of their union (segments of one file, lrb_reader_*).  Needs a table; on any error the
+ *        context holds no table afterwards (it may be partly added to).
  * Bounded device memory: a read set whose working set (8.6 B per base of lists beside the 4 GiB table) does not fit is
  * processed in BATCHES — the table accumulates over the batches, then every batch is shipped and partitioned again for
  * the search — with a one-line notice on stderr; results are identical (tests force this with LRB_BATCH_BASES).  This
  * is the reference's constant-memory behaviour (count-15mers.cpp:75-99: reads stream through a bounded queue). */
 #define LRB_PROFILE_USE_LOADED_TABLE 1
 #define LRB_PROFILE_KEEP_TABLE 2
+#define LRB_PROFILE_ADD_TO_TABLE 4
 int lrb_profile_host(lrb_ctx* ctx, const lrb_reads* reads, int k, long bin_size, int bins, uint32_t* comp_counts,
                      uint32_t* cov_hist, uint32_t* cov_sums, uint32_t* table_host, int flags);
 /* How the last lrb_profile_host call ran. */
@@ -331,6 +355,18 @@ int lrb_write_composition_npy(const char* path, const uint32_t* counts, const ui
                               int k, int threads);
 int lrb_write_coverage_npy(const char* path, const uint32_t* hist, const uint32_t* sums, uint64_t n_reads, int bins,
                            int threads);
+/* The same four writers for a file written in parts (one segment of rows at a time): the rows go after the `row0` rows
+ * already in the file; row0 = 0 creates / truncates it.  The .npy forms rewrite the header with row0 + n_reads rows each
+ * time (its size, 128 bytes, does not depend on the shape), so after the last part the file is the one-shot writer's,
+ * byte for byte, and so are the text files. */
+int lrb_append_composition_txt(const char* path, const uint32_t* counts, const uint32_t* read_len, uint64_t n_reads, int k,
+                               int threads, uint64_t row0);
+int lrb_append_coverage_txt(const char* path, const uint32_t* hist, const uint32_t* sums, uint64_t n_reads, int bins,
+                            int threads, uint64_t row0);
+int lrb_append_composition_npy(const char* path, const uint32_t* counts, const uint32_t* read_len, uint64_t n_reads, int k,
+                               int threads, uint64_t row0);
+int lrb_append_coverage_npy(const char* path, const uint32_t* hist, const uint32_t* sums, uint64_t n_reads, int bins,
+                            int threads, uint64_t row0);
 int lrb_table_write_file(const char* path, const uint32_t* table);  /* u64 2^30, then 2^30 u32 */
 int lrb_table_read_file(const char* path, uint32_t* table);
 /* What a spectrum (lrb_dev_table_spectrum layout) implies for the coverage profile with -bs bin_size -bc bins:
@@ -359,7 +395,12 @@ int lrb_search_15mers(const char* table_path, const char* reads_path, const char
  * malformed table file: LRB_EIO / LRB_EFORMAT; no device: LRB_ECUDA.  No reference counterpart. */
 int lrb_table_spectrum(const char* table_path, const char* out_txt, uint32_t max_count);
 /* Fused stage: parse once, keep reads + table in HBM, write com_profs, cov_profs (and 15mers-counts if
- * write_table) into out_dir/profiles/; write_npy additionally emits com_profs.npy / cov_profs.npy. */
+ * write_table) into out_dir/profiles/; write_npy additionally emits com_profs.npy / cov_profs.npy.
+ * Input larger than one segment (lrb_reader_open with the budget of the call's rows; a plain file no larger in bytes than
+ * the budget is read whole as before): the file-level calls above and below go segment by segment and append the rows —
+ * count: one pass adding each segment to the table; search: one pass against the loaded table; fused: pass 1 writes the
+ * composition rows and counts, pass 2 reads the file again and writes the coverage rows.  The files are those of a
+ * one-segment run, byte for byte; one line on stderr gives the number of segments and passes. */
 int lrb_profile(const char* reads_path, const char* out_dir, int k, long bin_size, int bins, int threads,
                 int write_table, int write_npy);
 /* The same on n_gpus GPUs of this node (devices LRB_DEVICE.. ; n_gpus <= 0: LRB_GPUS from the environment, default 1),

@@ -50,7 +50,7 @@ class RunInfo(C.Structure):
                 ("host_plan_ms", C.c_float), ("host_enqueue_ms", C.c_float)]
 
 
-PROFILE_USE_LOADED_TABLE, PROFILE_KEEP_TABLE = 1, 2
+PROFILE_USE_LOADED_TABLE, PROFILE_KEEP_TABLE, PROFILE_ADD_TO_TABLE = 1, 2, 4
 
 
 class SynthParams(C.Structure):
@@ -78,6 +78,11 @@ _SIG = {
     "lrb_reads_free": (None, [_P]),
     "lrb_reads_index_valid": (C.c_int, [_P, C.c_int, _P]),
     "lrb_reads_exceptions": (C.c_int, [_P, C.POINTER(_P), C.POINTER(_P), C.POINTER(C.c_uint64)]),
+    "lrb_reader_open": (C.c_int, [C.c_char_p, C.c_int, C.c_uint64, C.POINTER(_P)]),
+    "lrb_reader_next": (C.c_int, [_P, C.POINTER(_P)]),
+    "lrb_reader_rewind": (C.c_int, [_P]),
+    "lrb_reader_tell": (C.c_int, [_P, _P, _P, _P, _P]),
+    "lrb_reader_close": (None, [_P]),
     "lrb_dev_fill_valid": (C.c_int, [C.POINTER(ReadsView), _P, _P, C.c_uint64, _P]),
     "lrb_dev_composition": (C.c_int, [C.POINTER(ReadsView), C.c_int, _P, C.c_uint64, C.c_uint64, _P]),
     "lrb_dev_count": (C.c_int, [C.POINTER(ReadsView), _P, C.c_uint64, C.c_uint64, C.c_uint32, C.c_uint32, _P]),
@@ -122,6 +127,10 @@ _SIG = {
     "lrb_write_coverage_txt": (C.c_int, [C.c_char_p, _P, _P, C.c_uint64, C.c_int, C.c_int]),
     "lrb_write_composition_npy": (C.c_int, [C.c_char_p, _P, _P, C.c_uint64, C.c_int, C.c_int]),
     "lrb_write_coverage_npy": (C.c_int, [C.c_char_p, _P, _P, C.c_uint64, C.c_int, C.c_int]),
+    "lrb_append_composition_txt": (C.c_int, [C.c_char_p, _P, _P, C.c_uint64, C.c_int, C.c_int, C.c_uint64]),
+    "lrb_append_coverage_txt": (C.c_int, [C.c_char_p, _P, _P, C.c_uint64, C.c_int, C.c_int, C.c_uint64]),
+    "lrb_append_composition_npy": (C.c_int, [C.c_char_p, _P, _P, C.c_uint64, C.c_int, C.c_int, C.c_uint64]),
+    "lrb_append_coverage_npy": (C.c_int, [C.c_char_p, _P, _P, C.c_uint64, C.c_int, C.c_int, C.c_uint64]),
     "lrb_table_write_file": (C.c_int, [C.c_char_p, _P]),
     "lrb_table_read_file": (C.c_int, [C.c_char_p, _P]),
     "lrb_spectrum_bin_mass": (C.c_int, [_P, C.c_uint32, C.c_long, C.c_int, _P]),

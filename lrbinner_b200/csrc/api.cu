@@ -242,7 +242,7 @@ struct Job {
     int k = 0, P = 0, bins = 1;
     long bin_size = 1;
     uint32_t *comp = nullptr, *hist = nullptr, *sums = nullptr, *table_host = nullptr;
-    bool do_comp = false, do_search = false, do_count = false, use_loaded = false;
+    bool do_comp = false, do_search = false, do_count = false, use_loaded = false, add_to_table = false;
     bool use_part = true, want_smem_env = false, force_l2 = false, comp_pinned = false;
     int bucket_shift = 24, h2d_chunks = 16;
     bool force_ship_valid = false;
@@ -394,9 +394,11 @@ int enqueue_upload(lrb_ctx* c, const lrb_reads* r, const Job& J, const ChunkPlan
 }
 
 // Pass 1 of one batch.  row0 = index of the batch's first read in the caller's output arrays.  with_rids: the lists will
-// also serve the search (single-batch mode).  timed: record the phase events of lrb_ctx_last_timings.
+// also serve the search (single-batch mode).  timed: record the phase events of lrb_ctx_last_timings.  add_into_table: the
+// device's table is complete already (LRB_PROFILE_ADD_TO_TABLE on the primary device): the count adds to it, never zeroes
+// or writes it.
 int stage_front(lrb_ctx* c, const lrb_reads* r, const Job& J, uint64_t row0, bool with_rids, bool defer_comp, bool timed,
-                bool first_batch = false, bool only_batch = false) {
+                bool first_batch = false, bool only_batch = false, bool add_into_table = false) {
     CTX_CUDA(cudaSetDevice(c->device));
     cudaStream_t st = c->stream, sin = c->copy_in, sout = c->copy_out;
     const uint64_t n = r->n_reads, nb = r->n_blocks;
@@ -422,11 +424,11 @@ int stage_front(lrb_ctx* c, const lrb_reads* r, const Job& J, uint64_t row0, boo
     lrb_reads_view& v = c->dview;
     // compute stream: zero the outputs while the first chunk is in flight.  The table is zeroed only when counts will be
     // ADDED to it (several batches, or no lists): a device's only batch WRITES its table slices (apply mode bit 3).
-    const bool count_writes = J.do_count && lists && only_batch;
+    const bool count_writes = J.do_count && lists && only_batch && !add_into_table;
     // experiment (LRB_COMP_BESIDE=1): the composition does not ride along with the chunks but runs on the copy_out stream
     // beside the search, once the count is enqueued (it needs nothing but the packed stream)
     const bool comp_beside = J.do_comp && n && only_batch && lists && J.do_count && J.do_search && env_int("LRB_COMP_BESIDE", 0) > 0;
-    if (J.do_count && first_batch && !count_writes)
+    if (J.do_count && first_batch && !count_writes && !add_into_table)
         CTX_CUDA(cudaMemsetAsync(c->table.p, 0, sizeof(uint32_t) * (size_t)kTableEntries, st));
     if (J.do_comp && n && !comp_beside) CTX_CUDA(cudaMemsetAsync(c->comp.p, 0, sizeof(uint32_t) * n * J.P, st));
     CTX_CUDA(cudaStreamWaitEvent(st, c->sync_ev[0], 0));  // index arrays (and validity exceptions) are on the device
@@ -636,9 +638,8 @@ int enqueue_exchange(std::vector<DevPlan>& plans, int n_buckets, int shift, bool
 
 // Seam-to-seam pipeline (see the block comment above).  Phase timings of device 0's first batch
 // (lrb_ctx_last_timings) overlap; [6] is the whole call on device 0's stream; lrb_ctx_last_info has the wall clock.
-extern "C" int lrb_profile_host(lrb_ctx* c, const lrb_reads* r, int k, long bin_size, int bins, uint32_t* comp_counts,
-                                uint32_t* cov_hist, uint32_t* cov_sums, uint32_t* table_host, int flags) {
-    if (!c || !r) return lrb_set_error(LRB_EINVAL, "lrb_profile_host: null argument");
+static int profile_host(lrb_ctx* c, const lrb_reads* r, int k, long bin_size, int bins, uint32_t* comp_counts,
+                        uint32_t* cov_hist, uint32_t* cov_sums, uint32_t* table_host, int flags) {
     Job J;
     J.reads = r; J.k = k; J.P = comp_width(k); J.bins = bins; J.bin_size = bin_size;
     J.comp = comp_counts; J.hist = cov_hist; J.sums = cov_sums; J.table_host = table_host;
@@ -649,8 +650,10 @@ extern "C" int lrb_profile_host(lrb_ctx* c, const lrb_reads* r, int k, long bin_
     if (J.do_search && bin_size <= 0) return lrb_set_error(LRB_EINVAL, "bin_size must be >= 1 (the reference divides by it)");
     if (J.do_search && (bins <= 0 || bins > LRB_MAX_BINS)) return lrb_set_error(LRB_EINVAL, "bins must be in [1, %d]", LRB_MAX_BINS);
     J.use_loaded = (flags & LRB_PROFILE_USE_LOADED_TABLE) != 0;
-    if (J.use_loaded && !c->table_ready) return lrb_set_error(LRB_EINVAL, "no table loaded in this context");
-    J.do_count = !J.use_loaded && (J.do_search || table_host || (flags & LRB_PROFILE_KEEP_TABLE));
+    J.add_to_table = (flags & LRB_PROFILE_ADD_TO_TABLE) != 0;
+    if (J.use_loaded && J.add_to_table) return lrb_set_error(LRB_EINVAL, "LRB_PROFILE_USE_LOADED_TABLE and LRB_PROFILE_ADD_TO_TABLE exclude each other");
+    if ((J.use_loaded || J.add_to_table) && !c->table_ready) return lrb_set_error(LRB_EINVAL, "no table loaded in this context");
+    J.do_count = !J.use_loaded && (J.do_search || table_host || (flags & (LRB_PROFILE_KEEP_TABLE | LRB_PROFILE_ADD_TO_TABLE)));
     {
         const char* e = getenv("LRB_TABLE_PATH");
         if (e && !strcmp(e, "direct")) J.use_part = false;   // one random HBM access per window (kernels.cu): experiments only
@@ -760,6 +763,9 @@ extern "C" int lrb_profile_host(lrb_ctx* c, const lrb_reads* r, int k, long bin_
     info.host_plan_ms = since0();
 
     // ---- pass 1 -----------------------------------------------------------------------------------------------------
+    // Adding to the table: device 0 counts into its complete table, every other device into a private table from zero, so
+    // that after the exchange  sum over devices of the canonical halves = previous table + this read set;  the mirror then
+    // rebuilds the other half on device 0 as for any count.
     c->table_ready = J.use_loaded ? c->table_ready : false;
     if (J.use_loaded && multi) {   // the loaded table lives on device 0: hand it to the others
         CTX_CUDA(cudaSetDevice(c->device));
@@ -783,7 +789,7 @@ extern "C" int lrb_profile_host(lrb_ctx* c, const lrb_reads* r, int k, long bin_
             if (b.r0 == 0 && b.r1 == n) s = const_cast<lrb_reads*>(r);
             else { if ((rc2 = lrb_reads_slice(r, b.r0, b.r1, &s))) break; owned = true; }
             rc2 = stage_front(x, s, J, b.r0, /*with_rids=*/single && J.do_search, /*defer_comp=*/single && !J.comp_pinned, /*timed=*/x == c && i == 0,
-                              /*first_batch=*/i == 0, /*only_batch=*/single);
+                              /*first_batch=*/i == 0, /*only_batch=*/single, /*add_into_table=*/J.add_to_table && x == c);
             if (single && !rc2) { p.kept = s; p.kept_owned = owned; break; }
             if (!rc2) rc2 = sync_ctx(x);   // the buffers are re-used by the next batch
             if (owned) lrb_reads_free(s);
@@ -913,6 +919,14 @@ extern "C" int lrb_profile_host(lrb_ctx* c, const lrb_reads* r, int k, long bin_
     info.lists_reused = !streamed && J.use_part && J.do_count && J.do_search;
     info.wall_ms = (float)std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - wall0).count();
     return LRB_OK;
+}
+
+extern "C" int lrb_profile_host(lrb_ctx* c, const lrb_reads* r, int k, long bin_size, int bins, uint32_t* comp_counts,
+                                uint32_t* cov_hist, uint32_t* cov_sums, uint32_t* table_host, int flags) {
+    if (!c || !r) return lrb_set_error(LRB_EINVAL, "lrb_profile_host: null argument");
+    const int rc = profile_host(c, r, k, bin_size, bins, comp_counts, cov_hist, cov_sums, table_host, flags);
+    if (rc && (flags & LRB_PROFILE_ADD_TO_TABLE)) c->table_ready = false;   // the table may hold part of this read set
+    return rc;
 }
 
 extern "C" int lrb_ctx_last_timings(const lrb_ctx* c, float* ms7) {
@@ -1127,10 +1141,6 @@ struct CtxGuard {
     lrb_ctx* c = nullptr;
     ~CtxGuard() { lrb_ctx_destroy(c); }
 };
-struct ReadsGuard {
-    lrb_reads* r = nullptr;
-    ~ReadsGuard() { lrb_reads_free(r); }
-};
 
 int default_device() {
     const char* e = getenv("LRB_DEVICE");
@@ -1161,6 +1171,65 @@ int make_dir(const char* path) {
     return lrb_set_error(LRB_EIO, "cannot create directory %s: %s", path, strerror(errno));
 }
 
+// The reads of a file-level call: one read set (lrb_reads_from_file) when the input fits one segment, else the segment
+// reader positioned after its first segment.  Host memory then holds one segment's packed stream and result rows, whatever
+// the size of the file, and no read set reaches the 2^32-block limit.
+struct Input {
+    lrb_reads* whole = nullptr;   // the input as one read set, or
+    lrb_reader* rd = nullptr;     // its reader, with the current segment in `seg`
+    lrb_reads* seg = nullptr;
+    ~Input() { lrb_reads_free(whole); lrb_reads_free(seg); lrb_reader_close(rd); }
+};
+
+bool is_gzip(const char* path) {
+    unsigned char magic[2] = {0, 0};
+    const int fd = open(path, O_RDONLY);
+    const bool gz = fd >= 0 && pread(fd, magic, 2, 0) == 2 && magic[0] == 0x1f && magic[1] == 0x8b;
+    if (fd >= 0) close(fd);
+    return gz;
+}
+
+// row_bytes: host bytes of result rows per read.  A missing file, or a plain file no larger in bytes than the segment budget,
+// is read whole as before; otherwise the reader decides, and a first segment that is the whole stream is used as one read set.
+int open_input(const char* path, int threads, uint64_t row_bytes, Input& in) {
+    const uint64_t budget = lrb_segment_budget(row_bytes + 16);   // + read_len, read_blk and >= 1 tile per read
+    struct stat st;
+    if (stat(path, &st) != 0 || (S_ISREG(st.st_mode) && (uint64_t)st.st_size <= budget && !is_gzip(path)))
+        return lrb_reads_from_file(path, threads, &in.whole);
+    int rc, at_end = 0;
+    if ((rc = lrb_reader_open(path, threads, budget, &in.rd)) || (rc = lrb_reader_next(in.rd, &in.seg))) return rc;
+    lrb_reader_tell(in.rd, nullptr, nullptr, nullptr, &at_end);
+    if (!at_end) return LRB_OK;
+    std::swap(in.whole, in.seg);
+    return in.whole ? LRB_OK : lrb_reads_from_lengths(nullptr, 0, &in.whole);   // no record at all: an empty read set
+}
+
+// f(segment, index of its first read) for every segment from the current one on; rewind: from the first record again
+template <class F>
+int each_segment(Input& in, bool rewind, F f) {
+    int rc;
+    if (rewind) {
+        lrb_reads_free(in.seg);
+        in.seg = nullptr;
+        if ((rc = lrb_reader_rewind(in.rd)) || (rc = lrb_reader_next(in.rd, &in.seg))) return rc;
+    }
+    for (uint64_t row0 = 0; in.seg;) {
+        if ((rc = f(in.seg, row0))) return rc;
+        row0 += in.seg->n_reads;
+        lrb_reads_free(in.seg);
+        in.seg = nullptr;
+        if ((rc = lrb_reader_next(in.rd, &in.seg))) return rc;
+    }
+    return LRB_OK;
+}
+
+void segments_notice(const Input& in, int passes) {
+    uint64_t reads = 0, bases = 0, segs = 0;
+    lrb_reader_tell(in.rd, &reads, &bases, &segs, nullptr);
+    fprintf(stderr, "[lrb] input: %llu reads / %llu bases in %llu segments (larger than one segment of host memory); %d pass%s over the file\n",
+            (unsigned long long)reads, (unsigned long long)bases, (unsigned long long)segs, passes, passes == 1 ? "" : "es");
+}
+
 }  // namespace
 
 extern "C" int lrb_count_kmers(const char* reads_path, const char* out_txt, int k, int threads) {
@@ -1171,11 +1240,20 @@ extern "C" int lrb_count_kmers(const char* reads_path, const char* out_txt, int 
     if ((rc = truncate_file(out_txt))) return rc;
     CtxGuard cg;
     if ((rc = create_ctx(0, &cg.c))) return rc;
-    ReadsGuard rg;
-    if ((rc = lrb_reads_from_file(reads_path, threads, &rg.r))) return rc;
-    std::vector<uint32_t> counts((size_t)rg.r->n_reads * P + 1);
-    if ((rc = lrb_profile_host(cg.c, rg.r, k, 1, 1, counts.data(), nullptr, nullptr, nullptr, 0))) return rc;
-    return lrb_write_composition_txt(out_txt, counts.data(), rg.r->read_len, rg.r->n_reads, k, threads);
+    Input in;
+    if ((rc = open_input(reads_path, threads, 4ull * P, in))) return rc;
+    if (in.whole) {
+        std::vector<uint32_t> counts((size_t)in.whole->n_reads * P + 1);
+        if ((rc = lrb_profile_host(cg.c, in.whole, k, 1, 1, counts.data(), nullptr, nullptr, nullptr, 0))) return rc;
+        return lrb_write_composition_txt(out_txt, counts.data(), in.whole->read_len, in.whole->n_reads, k, threads);
+    }
+    rc = each_segment(in, false, [&](const lrb_reads* s, uint64_t row0) -> int {
+        std::vector<uint32_t> counts((size_t)s->n_reads * P + 1);
+        const int rc2 = lrb_profile_host(cg.c, s, k, 1, 1, counts.data(), nullptr, nullptr, nullptr, 0);
+        return rc2 ? rc2 : lrb_append_composition_txt(out_txt, counts.data(), s->read_len, s->n_reads, k, threads, row0);
+    });
+    if (!rc) segments_notice(in, 1);
+    return rc;
 }
 
 extern "C" int lrb_count_15mers(const char* reads_path, const char* out_table, int threads) {
@@ -1183,10 +1261,15 @@ extern "C" int lrb_count_15mers(const char* reads_path, const char* out_table, i
     int rc;
     CtxGuard cg;
     if ((rc = create_ctx(0, &cg.c))) return rc;
-    ReadsGuard rg;
-    if ((rc = lrb_reads_from_file(reads_path, threads, &rg.r))) return rc;
+    Input in;
+    if ((rc = open_input(reads_path, threads, 0, in))) return rc;
     // the same key-partitioned count as the fused stage; the table stays in the context and is streamed to the file
-    if ((rc = lrb_profile_host(cg.c, rg.r, 0, 1, 1, nullptr, nullptr, nullptr, nullptr, LRB_PROFILE_KEEP_TABLE))) return rc;
+    if (in.whole) rc = lrb_profile_host(cg.c, in.whole, 0, 1, 1, nullptr, nullptr, nullptr, nullptr, LRB_PROFILE_KEEP_TABLE);
+    else rc = each_segment(in, false, [&](const lrb_reads* s, uint64_t row0) -> int {
+        return lrb_profile_host(cg.c, s, 0, 1, 1, nullptr, nullptr, nullptr, nullptr, row0 ? LRB_PROFILE_ADD_TO_TABLE : LRB_PROFILE_KEEP_TABLE);
+    });
+    if (rc) return rc;
+    if (!in.whole) segments_notice(in, 1);
     return lrb_ctx_table_save(cg.c, out_table);
 }
 
@@ -1200,12 +1283,18 @@ extern "C" int lrb_search_15mers(const char* table_path, const char* reads_path,
     if ((rc = create_ctx(0, &cg.c))) return rc;
     if ((rc = lrb_ctx_table_load(cg.c, table_path))) return rc;
     if ((rc = truncate_file(out_txt))) return rc;
-    ReadsGuard rg;
-    if ((rc = lrb_reads_from_file(reads_path, threads, &rg.r))) return rc;
-    const uint64_t n = rg.r->n_reads;
-    std::vector<uint32_t> hist((size_t)n * bins + 1), sums(n + 1);
-    if ((rc = lrb_profile_host(cg.c, rg.r, 0, bin_size, bins, nullptr, hist.data(), sums.data(), nullptr, LRB_PROFILE_USE_LOADED_TABLE))) return rc;
-    return lrb_write_coverage_txt(out_txt, hist.data(), sums.data(), n, bins, threads);
+    Input in;
+    if ((rc = open_input(reads_path, threads, 4ull * ((uint64_t)bins + 1), in))) return rc;
+    auto search = [&](const lrb_reads* s, uint64_t row0) -> int {
+        const uint64_t n = s->n_reads;
+        std::vector<uint32_t> hist((size_t)n * bins + 1), sums(n + 1);
+        const int rc2 = lrb_profile_host(cg.c, s, 0, bin_size, bins, nullptr, hist.data(), sums.data(), nullptr, LRB_PROFILE_USE_LOADED_TABLE);
+        return rc2 ? rc2 : lrb_append_coverage_txt(out_txt, hist.data(), sums.data(), n, bins, threads, row0);
+    };
+    if (in.whole) return search(in.whole, 0);
+    if ((rc = each_segment(in, false, search))) return rc;
+    segments_notice(in, 1);
+    return LRB_OK;
 }
 
 extern "C" int lrb_table_spectrum(const char* table_path, const char* out_txt, uint32_t max_count) {
@@ -1233,16 +1322,43 @@ extern "C" int lrb_profile_multi(const char* reads_path, const char* out_dir, in
     if ((rc = make_dir(out_dir)) || (rc = make_dir(prof.c_str()))) return rc;
     CtxGuard cg;
     if ((rc = create_ctx(n_gpus, &cg.c))) return rc;
-    ReadsGuard rg;
-    if ((rc = lrb_reads_from_file(reads_path, threads, &rg.r))) return rc;
-    const uint64_t n = rg.r->n_reads;
-    std::vector<uint32_t> counts((size_t)n * P + 1), hist((size_t)n * bins + 1), sums(n + 1);
-    if ((rc = lrb_profile_host(cg.c, rg.r, k, bin_size, bins, counts.data(), hist.data(), sums.data(), nullptr, 0))) return rc;
-    if ((rc = lrb_write_composition_txt((prof + "/com_profs").c_str(), counts.data(), rg.r->read_len, n, k, threads))) return rc;
-    if ((rc = lrb_write_coverage_txt((prof + "/cov_profs").c_str(), hist.data(), sums.data(), n, bins, threads))) return rc;
-    if (write_npy) {
-        if ((rc = lrb_write_composition_npy((prof + "/com_profs.npy").c_str(), counts.data(), rg.r->read_len, n, k, threads))) return rc;
-        if ((rc = lrb_write_coverage_npy((prof + "/cov_profs.npy").c_str(), hist.data(), sums.data(), n, bins, threads))) return rc;
+    Input in;
+    if ((rc = open_input(reads_path, threads, 4ull * ((uint64_t)P + bins + 1), in))) return rc;
+    const std::string com = prof + "/com_profs", cov = prof + "/cov_profs", com_npy = com + ".npy", cov_npy = cov + ".npy";
+    if (in.whole) {
+        const lrb_reads* r = in.whole;
+        const uint64_t n = r->n_reads;
+        std::vector<uint32_t> counts((size_t)n * P + 1), hist((size_t)n * bins + 1), sums(n + 1);
+        if ((rc = lrb_profile_host(cg.c, r, k, bin_size, bins, counts.data(), hist.data(), sums.data(), nullptr, 0))) return rc;
+        if ((rc = lrb_write_composition_txt(com.c_str(), counts.data(), r->read_len, n, k, threads))) return rc;
+        if ((rc = lrb_write_coverage_txt(cov.c_str(), hist.data(), sums.data(), n, bins, threads))) return rc;
+        if (write_npy) {
+            if ((rc = lrb_write_composition_npy(com_npy.c_str(), counts.data(), r->read_len, n, k, threads))) return rc;
+            if ((rc = lrb_write_coverage_npy(cov_npy.c_str(), hist.data(), sums.data(), n, bins, threads))) return rc;
+        }
+    } else {
+        // pass 1: composition rows, and every segment counted into the one table
+        rc = each_segment(in, false, [&](const lrb_reads* s, uint64_t row0) -> int {
+            const uint64_t n = s->n_reads;
+            std::vector<uint32_t> counts((size_t)n * P + 1);
+            int rc2 = lrb_profile_host(cg.c, s, k, bin_size, bins, counts.data(), nullptr, nullptr, nullptr,
+                                       row0 ? LRB_PROFILE_ADD_TO_TABLE : LRB_PROFILE_KEEP_TABLE);
+            if (!rc2) rc2 = lrb_append_composition_txt(com.c_str(), counts.data(), s->read_len, n, k, threads, row0);
+            if (!rc2 && write_npy) rc2 = lrb_append_composition_npy(com_npy.c_str(), counts.data(), s->read_len, n, k, threads, row0);
+            return rc2;
+        });
+        if (rc) return rc;
+        // pass 2: the file again, every segment searched against the finished table
+        rc = each_segment(in, true, [&](const lrb_reads* s, uint64_t row0) -> int {
+            const uint64_t n = s->n_reads;
+            std::vector<uint32_t> hist((size_t)n * bins + 1), sums(n + 1);
+            int rc2 = lrb_profile_host(cg.c, s, k, bin_size, bins, nullptr, hist.data(), sums.data(), nullptr, LRB_PROFILE_USE_LOADED_TABLE);
+            if (!rc2) rc2 = lrb_append_coverage_txt(cov.c_str(), hist.data(), sums.data(), n, bins, threads, row0);
+            if (!rc2 && write_npy) rc2 = lrb_append_coverage_npy(cov_npy.c_str(), hist.data(), sums.data(), n, bins, threads, row0);
+            return rc2;
+        });
+        if (rc) return rc;
+        segments_notice(in, 2);
     }
     if (write_table && (rc = lrb_ctx_table_save(cg.c, (prof + "/15mers-counts").c_str()))) return rc;
     return LRB_OK;

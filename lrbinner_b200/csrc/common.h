@@ -58,3 +58,6 @@ struct lrb_reads {
 // page-locked when asked for and a CUDA device is usable, plain aligned memory otherwise (host-only unit tests)
 void* lrb_host_alloc(size_t bytes, bool* pinned, bool want_pinned = true);
 void lrb_host_free(void* p, bool pinned);
+
+// bases per segment of the segment reader for result rows of `row_bytes_per_read` (lrb_reader_open: segment_bases = 0)
+uint64_t lrb_segment_budget(uint64_t row_bytes_per_read);

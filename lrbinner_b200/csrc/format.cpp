@@ -88,10 +88,12 @@ bool pwrite_all(int fd, const char* p, size_t n, uint64_t off) {
 
 // Fixed-width rows: every thread formats blocks of its share of the rows into a private buffer and writes them at their
 // final offset (pwrite), so neither the text nor the file copy is ever serial and nothing of file size sits in memory.
-// row(i, dst) fills row i (row_bytes bytes).
+// row(i, dst) fills row i (row_bytes bytes).  The rows go after `row0` rows already in the file (row0 = 0: a new file); the
+// head, if any, is (re)written at offset 0.
 template <class RowFn>
-int write_fixed_rows(const char* path, const void* head, size_t head_bytes, uint64_t n_rows, size_t row_bytes, int threads, RowFn row) {
-    const int fd = open(path, O_WRONLY | O_CREAT | O_TRUNC, 0644);
+int write_fixed_rows(const char* path, const void* head, size_t head_bytes, uint64_t n_rows, size_t row_bytes, int threads, RowFn row,
+                     uint64_t row0) {
+    const int fd = open(path, O_WRONLY | O_CREAT | (row0 ? 0 : O_TRUNC), 0644);
     if (fd < 0) return lrb_set_error(LRB_EIO, "cannot open %s for writing", path);
     bool ok = !head_bytes || pwrite_all(fd, (const char*)head, head_bytes, 0);
     if (threads < 1) threads = 1;
@@ -105,7 +107,7 @@ int write_fixed_rows(const char* path, const void* head, size_t head_bytes, uint
         for (uint64_t lo = a; lo < b; lo += block_rows) {
             const uint64_t hi = std::min(b, lo + block_rows);
             for (uint64_t i = lo; i < hi; ++i) row(i, buf.data() + (size_t)(i - lo) * row_bytes);
-            if (!pwrite_all(fd, buf.data(), (size_t)(hi - lo) * row_bytes, head_bytes + lo * row_bytes)) { failed[(size_t)t] = 1; return; }
+            if (!pwrite_all(fd, buf.data(), (size_t)(hi - lo) * row_bytes, head_bytes + (row0 + lo) * row_bytes)) { failed[(size_t)t] = 1; return; }
         }
     };
     if (ok && n_rows) {
@@ -123,10 +125,13 @@ int write_fixed_rows(const char* path, const void* head, size_t head_bytes, uint
 }
 
 template <class RowFn>
-int write_rows(const char* path, uint64_t n_rows, size_t row_bytes, int threads, RowFn row) {
-    return write_fixed_rows(path, nullptr, 0, n_rows, row_bytes, threads, row);
+int write_rows(const char* path, uint64_t n_rows, size_t row_bytes, int threads, RowFn row, uint64_t row0) {
+    return write_fixed_rows(path, nullptr, 0, n_rows, row_bytes, threads, row, row0);
 }
 
+// 10 + len("{'descr': '<f8', 'fortran_order': False, 'shape': (R, C), }\n") = 69 + digits(R) + digits(C) <= 128 for any
+// u64 R and C < 10^39, so the header is 128 bytes for every shape: a file written in parts can take the final row count
+// in place.
 std::string npy_header(uint64_t rows, uint64_t cols) {
     char dict[160];
     snprintf(dict, sizeof dict, "{'descr': '<f8', 'fortran_order': False, 'shape': (%llu, %llu), }",
@@ -145,20 +150,21 @@ std::string npy_header(uint64_t rows, uint64_t cols) {
 }
 
 template <class RowFn>
-int write_npy(const char* path, uint64_t n_rows, uint64_t cols, int threads, RowFn row) {
-    const std::string h = npy_header(n_rows, cols);
+int write_npy(const char* path, uint64_t n_rows, uint64_t cols, int threads, RowFn row, uint64_t row0) {
+    const std::string h = npy_header(row0 + n_rows, cols);
+    if (h.size() != 128) return lrb_set_error(LRB_EINVAL, "npy header of %zu bytes", h.size());
     return write_fixed_rows(path, h.data(), h.size(), n_rows, (size_t)cols * 8, threads,
-                            [&](uint64_t i, char* dst) { row(i, reinterpret_cast<double*>(dst)); });
+                            [&](uint64_t i, char* dst) { row(i, reinterpret_cast<double*>(dst)); }, row0);
 }
 
 inline uint32_t comp_total(uint32_t len, int k) { return len >= (uint32_t)k ? len - (uint32_t)k + 1u : 0u; }
 
 }  // namespace
 
-extern "C" int lrb_write_composition_txt(const char* path, const uint32_t* counts, const uint32_t* read_len,
-                                         uint64_t n_reads, int k, int threads) {
+extern "C" int lrb_append_composition_txt(const char* path, const uint32_t* counts, const uint32_t* read_len,
+                                         uint64_t n_reads, int k, int threads, uint64_t row0) {
     const int P = comp_width(k);
-    if (!path || !P || (n_reads && (!counts || !read_len))) return lrb_set_error(LRB_EINVAL, "lrb_write_composition_txt: bad argument");
+    if (!path || !P || (n_reads && (!counts || !read_len))) return lrb_set_error(LRB_EINVAL, "lrb_append_composition_txt: bad argument");
     const size_t row_bytes = (size_t)P * 9 + 1;  // "d.dddddd " x P, then '\n'  (count-kmers.cpp:110-118)
     return write_rows(path, n_reads, row_bytes, threads, [=](uint64_t i, char* dst) {
         const uint32_t total = comp_total(read_len[i], k);
@@ -168,12 +174,17 @@ extern "C" int lrb_write_composition_txt(const char* path, const uint32_t* count
             dst[(size_t)j * 9 + 8] = ' ';
         }
         dst[row_bytes - 1] = '\n';
-    });
+    }, row0);
 }
 
-extern "C" int lrb_write_coverage_txt(const char* path, const uint32_t* hist, const uint32_t* sums, uint64_t n_reads,
-                                      int bins, int threads) {
-    if (!path || bins <= 0 || (n_reads && (!hist || !sums))) return lrb_set_error(LRB_EINVAL, "lrb_write_coverage_txt: bad argument");
+extern "C" int lrb_write_composition_txt(const char* path, const uint32_t* counts, const uint32_t* read_len,
+                                         uint64_t n_reads, int k, int threads) {
+    return lrb_append_composition_txt(path, counts, read_len, n_reads, k, threads, 0);
+}
+
+extern "C" int lrb_append_coverage_txt(const char* path, const uint32_t* hist, const uint32_t* sums, uint64_t n_reads,
+                                      int bins, int threads, uint64_t row0) {
+    if (!path || bins <= 0 || (n_reads && (!hist || !sums))) return lrb_set_error(LRB_EINVAL, "lrb_append_coverage_txt: bad argument");
     const size_t row_bytes = (size_t)bins * 9;  // values separated by ' ', '\n' after the last (search-15mers.cpp:35-48)
     return write_rows(path, n_reads, row_bytes, threads, [=](uint64_t i, char* dst) {
         const uint32_t* c = hist + (size_t)i * bins;
@@ -181,27 +192,42 @@ extern "C" int lrb_write_coverage_txt(const char* path, const uint32_t* hist, co
             put_fixed6(dst + (size_t)j * 9, lrb::fixed6(c[j], sums[i], true));
             dst[(size_t)j * 9 + 8] = (j == bins - 1) ? '\n' : ' ';
         }
-    });
+    }, row0);
 }
 
-extern "C" int lrb_write_composition_npy(const char* path, const uint32_t* counts, const uint32_t* read_len,
-                                         uint64_t n_reads, int k, int threads) {
+extern "C" int lrb_write_coverage_txt(const char* path, const uint32_t* hist, const uint32_t* sums, uint64_t n_reads,
+                                      int bins, int threads) {
+    return lrb_append_coverage_txt(path, hist, sums, n_reads, bins, threads, 0);
+}
+
+extern "C" int lrb_append_composition_npy(const char* path, const uint32_t* counts, const uint32_t* read_len,
+                                         uint64_t n_reads, int k, int threads, uint64_t row0) {
     const int P = comp_width(k);
-    if (!path || !P || (n_reads && (!counts || !read_len))) return lrb_set_error(LRB_EINVAL, "lrb_write_composition_npy: bad argument");
+    if (!path || !P || (n_reads && (!counts || !read_len))) return lrb_set_error(LRB_EINVAL, "lrb_append_composition_npy: bad argument");
     return write_npy(path, n_reads, (uint64_t)P, threads, [=](uint64_t i, double* dst) {
         const uint32_t total = comp_total(read_len[i], k);
         const uint32_t* c = counts + (size_t)i * P;
         for (int j = 0; j < P; ++j) dst[j] = (double)lrb::fixed6(c[j], total, false) / 1e6;  // == float("%f" text)
-    });
+    }, row0);
+}
+
+extern "C" int lrb_write_composition_npy(const char* path, const uint32_t* counts, const uint32_t* read_len,
+                                         uint64_t n_reads, int k, int threads) {
+    return lrb_append_composition_npy(path, counts, read_len, n_reads, k, threads, 0);
+}
+
+extern "C" int lrb_append_coverage_npy(const char* path, const uint32_t* hist, const uint32_t* sums, uint64_t n_reads,
+                                      int bins, int threads, uint64_t row0) {
+    if (!path || bins <= 0 || (n_reads && (!hist || !sums))) return lrb_set_error(LRB_EINVAL, "lrb_append_coverage_npy: bad argument");
+    return write_npy(path, n_reads, (uint64_t)bins, threads, [=](uint64_t i, double* dst) {
+        const uint32_t* c = hist + (size_t)i * bins;
+        for (int j = 0; j < bins; ++j) dst[j] = (double)lrb::fixed6(c[j], sums[i], true) / 1e6;
+    }, row0);
 }
 
 extern "C" int lrb_write_coverage_npy(const char* path, const uint32_t* hist, const uint32_t* sums, uint64_t n_reads,
                                       int bins, int threads) {
-    if (!path || bins <= 0 || (n_reads && (!hist || !sums))) return lrb_set_error(LRB_EINVAL, "lrb_write_coverage_npy: bad argument");
-    return write_npy(path, n_reads, (uint64_t)bins, threads, [=](uint64_t i, double* dst) {
-        const uint32_t* c = hist + (size_t)i * bins;
-        for (int j = 0; j < bins; ++j) dst[j] = (double)lrb::fixed6(c[j], sums[i], true) / 1e6;
-    });
+    return lrb_append_coverage_npy(path, hist, sums, n_reads, bins, threads, 0);
 }
 
 // ---- 15mers-counts file (kmer_utils.h:89-112): u64 size (= 2^30), then size little-endian u32 -----

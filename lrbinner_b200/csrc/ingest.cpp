@@ -548,14 +548,25 @@ static int index_valid(lrb_reads* r, int threads) {
 
 }  // namespace
 
-// ---- gzip input, streamed ------------------------------------------------------------------------------------------
-// A gzip stream cannot be split, but it need not be inflated as a whole either (round 1 did: a 100 Gbase .gz needed 100 GB
-// of RAM).  The file is inflated in chunks by a producer thread while the previous chunk is parsed (all `threads`
-// ranges) and packed; a record whose parse ran into the end of the data available so far is kept back, with everything
-// after it, for the next round.  Host memory: the packed stream (0.375 B/base) + two chunks + one record.
-// Record semantics are parse_range's, so the result equals the whole-image parse (tests: every fixture and the fuzz
-// files, gzip-compressed, with chunks of 1 .. 4096 bytes, against the oracle reader).
+// ---- segment reader: the read stream in chunks, delivered as read sets of bounded size -----------------------------------
+// The file is read in chunks (gzip: inflated by zlib; plain: pread windows, never mapped whole) by a producer thread while
+// the previous chunk is parsed (all `threads` ranges) and packed; a record whose parse ran into the end of the data read so
+// far is kept back, with everything after it, for the next round.  Records go into the current SEGMENT until the next one
+// would take it past its budget of bases or past kSegmentMaxBlocks; that record then starts the next segment (parsed again
+// from its header), and a record longer than the budget forms a segment on its own.  Host memory: one segment's packed
+// stream (0.375 B/base) + two chunks + one record, whatever the file's size.  Record semantics are parse_range's, so the
+// concatenated segments equal the whole-image parse (tests: every fixture and the fuzz files, plain and gzip, with chunks
+// and budgets down to 1 byte / 1 base, against the oracle reader).
 namespace {
+
+// A read set indexes its blocks with u32 (2^32 - 16 at most, build_layout); segments stay 2^28 blocks (8.6 Gbases) below.
+constexpr uint64_t kSegmentMaxBlocks = 0xF0000000ull;
+constexpr uint64_t kSegmentMaxBases = kSegmentMaxBlocks * 32;
+// lrb_reader_open(.., 0, ..) sizes segments for the largest rows of a fused call: k = 5 composition + 32 coverage bins + sum
+constexpr uint64_t kDefaultRowBytes = 4 * (512 + 32 + 1);
+// the per-read estimate that turns result rows into bytes per base: long reads (ONT / HiFi) are several kb, so 1 kb is
+// conservative for them; a read set of much shorter reads holds proportionally more rows per segment
+constexpr uint64_t kReadLenEstimate = 1000;
 
 struct GrowWords {
     uint32_t* p = nullptr;
@@ -571,51 +582,137 @@ struct GrowWords {
     }
 };
 
-int reads_from_gz_stream(const char* path, int threads, lrb_reads** out) {
-    gzFile f = gzopen(path, "rb");
-    if (!f) { *out = new lrb_reads(); return build_layout(*out, true, false); }   // unreadable == empty stream, like the tools
-    gzbuffer(f, 1 << 20);
+uint64_t mem_available_bytes() {
+    if (FILE* f = fopen("/proc/meminfo", "r")) {
+        char line[256];
+        unsigned long long kb = 0;
+        bool found = false;
+        while (!found && fgets(line, sizeof line, f)) found = sscanf(line, "MemAvailable: %llu kB", &kb) == 1;
+        fclose(f);
+        if (found) return (uint64_t)kb << 10;
+    }
+    return (uint64_t)sysconf(_SC_AVPHYS_PAGES) * (uint64_t)sysconf(_SC_PAGESIZE);
+}
+
+}  // namespace
+
+uint64_t lrb_segment_budget(uint64_t row_bytes_per_read) {
+    const char* e = getenv("LRB_SEGMENT_BASES");   // tests: segments of a few bases
+    if (e && atoll(e) > 0) return std::min<uint64_t>((uint64_t)atoll(e), kSegmentMaxBases);
+    // half of MemAvailable for the stream (0.375 B/base) + the rows (row_bytes per kReadLenEstimate bases)
+    const double per_base = 0.375 + (double)row_bytes_per_read / (double)kReadLenEstimate;
+    const double bases = (double)(mem_available_bytes() / 2) / per_base;
+    return (uint64_t)std::max(1.0, std::min(bases, (double)kSegmentMaxBases));
+}
+
+struct lrb_reader {
+    std::string path;
+    int threads = 1;
+    uint64_t budget = kSegmentMaxBases;     // bases per segment
+    uint64_t max_blocks = kSegmentMaxBlocks;
+    bool whole = false;                      // one read set of the whole stream: passing max_blocks is an error, not a cut
     size_t chunk = 64u << 20;   // measured (200 MB FASTA, 8 threads): 64 MiB chunks 1.16 s, one 256 MiB chunk 1.52 s, whole image 1.19 s
-    {
-        const char* e = getenv("LRB_GZ_CHUNK");   // tests: chunks of a few bytes
-        if (e && atoll(e) > 0) chunk = (size_t)atoll(e);
-    }
     size_t min_chunk = 8u << 20;
-    {
-        const char* e = getenv("LRB_PARSE_CHUNK");
-        if (e && atoll(e) > 0) min_chunk = (size_t)atoll(e);
-    }
-    threads = std::max(1, std::min(threads, 64));
-    std::vector<unsigned char> work, next(chunk);
+    bool gz = false;
+    gzFile f = nullptr;
+    int fd = -1;
+    uint64_t file_off = 0;
+    std::vector<unsigned char> work, next;
     size_t next_n = 0;
     bool next_eof = false;
-    auto inflate = [&]() {   // fills `next`; short read == end of the stream (or a damaged one: the tools stop quietly there too)
+    bool pending = false;   // `work` holds complete records not delivered yet: the last segment was cut inside it
+    bool done = false;
+    uint64_t reads_out = 0, bases_out = 0, segments_out = 0;
+
+    ~lrb_reader() {
+        if (f) gzclose(f);
+        if (fd >= 0) close(fd);
+    }
+    // fills `next`; a short read is the end of the stream (or of a damaged one: the tools stop quietly there too)
+    void fill_next() {
         next_n = 0;
         next_eof = false;
         while (next_n < chunk) {
-            const int got = gzread(f, next.data() + next_n, (unsigned)std::min<size_t>(chunk - next_n, 1u << 30));
+            const size_t want = std::min<size_t>(chunk - next_n, 1u << 30);
+            const long got = gz ? (long)gzread(f, next.data() + next_n, (unsigned)want) : (long)pread(fd, next.data() + next_n, want, (off_t)file_off);
             if (got <= 0) { next_eof = true; break; }
+            if (!gz) file_off += (uint64_t)got;
             next_n += (size_t)got;
         }
-    };
+    }
+    void start() {
+        work.clear();
+        pending = false;
+        done = !f && fd < 0;   // unreadable file == empty stream, like the tools
+        reads_out = bases_out = segments_out = 0;
+        next_n = 0;
+        next_eof = true;
+        if (!done) fill_next();
+    }
+};
+
+namespace {
+
+int reader_open(const char* path, int threads, uint64_t segment_bases, bool whole, lrb_reader** out) {
+    lrb_reader* rd = new lrb_reader();
+    rd->path = path;
+    rd->threads = std::max(1, std::min(threads, 64));
+    rd->whole = whole;
+    if (whole) { rd->budget = UINT64_MAX; rd->max_blocks = 0xFFFFFFF0ull; }
+    else rd->budget = std::min<uint64_t>(segment_bases ? segment_bases : lrb_segment_budget(kDefaultRowBytes), kSegmentMaxBases);
+    {
+        const char* e = getenv("LRB_GZ_CHUNK");   // tests: chunks of a few bytes (plain files too)
+        if (e && atoll(e) > 0) rd->chunk = (size_t)atoll(e);
+        e = getenv("LRB_PARSE_CHUNK");
+        if (e && atoll(e) > 0) rd->min_chunk = (size_t)atoll(e);
+    }
+    // a regular plain file is read with pread; gzip (and anything that is not a regular file) goes through zlib, which passes
+    // plain data through unchanged (io_utils.h:143)
+    const int fd = open(path, O_RDONLY);
+    struct stat st;
+    unsigned char magic[2] = {0, 0};
+    const bool regular = fd >= 0 && fstat(fd, &st) == 0 && S_ISREG(st.st_mode);
+    rd->gz = !regular || (pread(fd, magic, 2, 0) == 2 && magic[0] == 0x1f && magic[1] == 0x8b);
+    if (rd->gz) {
+        if (fd >= 0) close(fd);
+        if (fd >= 0 && (rd->f = gzopen(path, "rb"))) gzbuffer(rd->f, 1 << 20);
+    } else {
+        rd->fd = fd;
+    }
+    rd->next.resize(rd->chunk);
+    rd->start();
+    *out = rd;
+    return LRB_OK;
+}
+
+// The next segment (NULL once the stream is exhausted).
+int reader_next(lrb_reader* rd, lrb_reads** out) {
+    *out = nullptr;
     std::vector<uint32_t> lens;
     GrowWords codes, valid;
-    uint64_t blk = 0;
+    uint64_t blk = 0, bases = 0;
     int rc = LRB_OK;
-    inflate();
-    bool eof = false;
+    bool full = false;
     struct Item { const unsigned char* s; uint32_t len; uint64_t blk; };
     std::vector<Item> items;
     std::vector<Parsed> parts;
-    while (!eof && rc == LRB_OK) {
-        work.insert(work.end(), next.begin(), next.begin() + (ptrdiff_t)next_n);
-        eof = next_eof;
+    std::vector<unsigned char>& work = rd->work;
+    const int threads = rd->threads;
+    while (!full && !rd->done && rc == LRB_OK) {
+        bool eof;   // nothing follows `work` in the stream
         std::thread producer;
-        if (!eof) producer = std::thread(inflate);   // the next chunk inflates while this one is parsed and packed
+        if (!rd->pending) {
+            work.insert(work.end(), rd->next.begin(), rd->next.begin() + (ptrdiff_t)rd->next_n);
+            rd->next_n = 0;
+            eof = rd->next_eof;
+            if (!eof) producer = std::thread([rd]() { rd->fill_next(); });   // the next chunk is read while this one is parsed and packed
+        } else {
+            eof = rd->next_eof && rd->next_n == 0;
+        }
         bool ended = false;
-        parse_all(work.data(), work.size(), threads, min_chunk, parts, true, &ended);
+        parse_all(work.data(), work.size(), threads, rd->min_chunk, parts, true, &ended);
         size_t carry_from = work.size();
-        bool stop = false;
+        bool stop = eof;   // the stream ends for good behind this round's records
         if (!eof) {
             Parsed& last = parts.back();
             if (ended && !last.end_touched) stop = true;            // a malformed record ends the stream for good (kseq.h:209-214)
@@ -626,14 +723,25 @@ int reads_from_gz_stream(const char* path, int threads, lrb_reads** out) {
             } else carry_from = last.open_hdr;
         }
         items.clear();
-        for (auto& p : parts)
-            for (const Record& rec : p.recs) {
+        for (size_t pi = 0; pi < parts.size() && !full && rc == LRB_OK; ++pi) {
+            Parsed& p = parts[pi];
+            for (size_t j = 0; j < p.recs.size(); ++j) {
+                const Record& rec = p.recs[j];
+                const uint64_t nb = (uint64_t)rec.len / 32 + 1;
+                if (blk + nb > rd->max_blocks && rd->whole) { rc = lrb_set_error(LRB_EINVAL, "read set too large: more than 2^32 blocks (137 Gbases)"); break; }
+                if (!lens.empty() && (bases + rec.len > rd->budget || blk + nb > rd->max_blocks)) {   // starts the next segment
+                    carry_from = (size_t)p.hdr[j];
+                    full = true;
+                    break;
+                }
                 items.push_back({rec.in_pool ? (const unsigned char*)p.pool.data() + rec.off : work.data() + rec.off, rec.len, blk});
-                blk += (uint64_t)rec.len / 32 + 1;
+                blk += nb;
+                bases += rec.len;
                 lens.push_back(rec.len);
             }
-        if (blk > 0xFFFFFFF0ull) rc = lrb_set_error(LRB_EINVAL, "read set too large: more than 2^32 blocks (137 Gbases)");
-        else if (!codes.need(2 * blk + 2) || !valid.need(blk + 1)) rc = lrb_set_error(LRB_ENOMEM, "out of memory (packed stream, %llu blocks)", (unsigned long long)blk);
+        }
+        if (rc == LRB_OK && (!codes.need(2 * blk + 2) || !valid.need(blk + 1)))
+            rc = lrb_set_error(LRB_ENOMEM, "out of memory (packed stream, %llu blocks)", (unsigned long long)blk);
         if (rc == LRB_OK && !items.empty()) {
             const int T = items.size() < 64 ? 1 : threads;
             auto work_fn = [&](size_t lo, size_t hi) {
@@ -657,11 +765,12 @@ int reads_from_gz_stream(const char* path, int threads, lrb_reads** out) {
             }
         }
         if (producer.joinable()) producer.join();
-        if (stop) break;
-        if (!eof) work.erase(work.begin(), work.begin() + (ptrdiff_t)carry_from);
+        rd->pending = full;
+        if (full || !stop) work.erase(work.begin(), work.begin() + (ptrdiff_t)carry_from);
+        else { rd->done = true; work.clear(); }
     }
-    gzclose(f);
-    if (rc) { free(codes.p); free(valid.p); return rc; }
+    if (rc) { free(codes.p); free(valid.p); rd->done = true; return rc; }
+    if (lens.empty() && !rd->whole) { free(codes.p); free(valid.p); return LRB_OK; }
     lrb_reads* r = new lrb_reads();
     r->n_reads = lens.size();
     r->read_len = (uint32_t*)malloc(sizeof(uint32_t) * (lens.size() + 1));
@@ -671,11 +780,53 @@ int reads_from_gz_stream(const char* path, int threads, lrb_reads** out) {
     r->valid = valid.p;
     r->pinned = false;
     if ((rc = build_layout(r, false, false, /*alloc_stream=*/false)) || (rc = index_valid(r, threads))) { free_reads(r); return rc; }
+    rd->reads_out += r->n_reads;
+    rd->bases_out += r->total_bases;
+    rd->segments_out += 1;
     *out = r;
     return LRB_OK;
 }
 
+// gzip input of lrb_reads_from_file: the whole stream as one read set, read in chunks (round 1 inflated the whole file:
+// a 100 Gbase .gz needed 100 GB of RAM; this needs the packed stream + two chunks + one record)
+int reads_from_gz_stream(const char* path, int threads, lrb_reads** out) {
+    lrb_reader* rd = nullptr;
+    reader_open(path, threads, 0, /*whole=*/true, &rd);
+    const int rc = reader_next(rd, out);
+    delete rd;
+    return rc;
+}
+
 }  // namespace
+
+extern "C" int lrb_reader_open(const char* path, int threads, uint64_t segment_bases, lrb_reader** out) {
+    if (!path || !out) return lrb_set_error(LRB_EINVAL, "lrb_reader_open: null argument");
+    return reader_open(path, threads, segment_bases, /*whole=*/false, out);
+}
+
+extern "C" int lrb_reader_next(lrb_reader* rd, lrb_reads** out) {
+    if (!rd || !out) return lrb_set_error(LRB_EINVAL, "lrb_reader_next: null argument");
+    return reader_next(rd, out);
+}
+
+extern "C" int lrb_reader_rewind(lrb_reader* rd) {
+    if (!rd) return lrb_set_error(LRB_EINVAL, "lrb_reader_rewind: null argument");
+    if (rd->f && gzrewind(rd->f) != 0) return lrb_set_error(LRB_EIO, "cannot rewind %s", rd->path.c_str());
+    rd->file_off = 0;
+    rd->start();
+    return LRB_OK;
+}
+
+extern "C" int lrb_reader_tell(const lrb_reader* rd, uint64_t* reads, uint64_t* bases, uint64_t* segments, int* at_end) {
+    if (!rd) return lrb_set_error(LRB_EINVAL, "lrb_reader_tell: null argument");
+    if (reads) *reads = rd->reads_out;
+    if (bases) *bases = rd->bases_out;
+    if (segments) *segments = rd->segments_out;
+    if (at_end) *at_end = rd->done ? 1 : 0;
+    return LRB_OK;
+}
+
+extern "C" void lrb_reader_close(lrb_reader* rd) { delete rd; }
 
 extern "C" int lrb_reads_index_valid(lrb_reads* r, int threads, uint64_t* n_exceptions) {
     if (!r) return lrb_set_error(LRB_EINVAL, "lrb_reads_index_valid: null argument");

@@ -2,6 +2,7 @@
 
   PackedReads  — a read set in the packed host layout (lrb_reads*), from a FASTA/FASTQ file, from
                  ASCII bases, or layout-only from lengths.
+  SegmentReader / read_segments — a FASTA/FASTQ file as consecutive read sets of bounded size (lrb_reader_*).
   Context      — one GPU: seam-to-seam `profile()` over host buffers (lrb_profile_host).
   DeviceReads / dev_* — torch-tensor plumbing for the device-pointer level (lrb_dev_*): used by the
                  device-resident benchmark and the multi-GPU driver (lrbinner_b200/dist.py), where
@@ -122,6 +123,60 @@ class PackedReads:
             pass
 
 
+class SegmentReader:
+    """Owns an lrb_reader*: the records of a FASTA/FASTQ file (plain or gzip) as consecutive PackedReads of at most
+    `segment_bases` bases each (a longer read forms a segment on its own; 0 = sized from the host's available memory).
+    Concatenated, the segments are PackedReads.from_file(path)."""
+
+    def __init__(self, path, segment_bases=0, threads=8):
+        self._h = C.c_void_p()
+        check(lib.lrb_reader_open(str(path).encode(), int(threads), int(segment_bases), C.byref(self._h)))
+
+    def next(self):
+        """The next segment, or None at the end of the file."""
+        h = C.c_void_p()
+        check(lib.lrb_reader_next(self._h, C.byref(h)))
+        return PackedReads(h) if h.value else None
+
+    def __iter__(self):
+        while True:
+            seg = self.next()
+            if seg is None:
+                return
+            yield seg
+
+    def rewind(self):
+        check(lib.lrb_reader_rewind(self._h))
+
+    def tell(self):
+        """dict(reads, bases, segments) delivered since open / rewind, and at_end (no record left)."""
+        v = [C.c_uint64(0), C.c_uint64(0), C.c_uint64(0)]
+        at_end = C.c_int(0)
+        check(lib.lrb_reader_tell(self._h, C.byref(v[0]), C.byref(v[1]), C.byref(v[2]), C.byref(at_end)))
+        return {"reads": v[0].value, "bases": v[1].value, "segments": v[2].value, "at_end": bool(at_end.value)}
+
+    def close(self):
+        if self._h:
+            lib.lrb_reader_close(self._h)
+            self._h = None
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+
+def read_segments(path, segment_bases=0, threads=8):
+    """Generator of the segments of a FASTA/FASTQ file as PackedReads (see SegmentReader); the reader lives as long as
+    the generator."""
+    reader = SegmentReader(path, segment_bases, threads)
+    try:
+        yield from reader
+    finally:
+        reader.close()
+
+
 class Context:
     """One GPU, or several driven from this process (device = an ordinal or a list of ordinals; the first is the
     primary and ends up with the complete table).  profile() is the seam-to-seam call: host buffers in, host buffers out."""
@@ -136,9 +191,11 @@ class Context:
         self.device = device
 
     def profile(self, reads, k=None, bin_size=None, bins=None, want_table=False, use_loaded_table=False, out=None,
-                keep_table=False):
+                keep_table=False, add_to_table=False):
         """Returns dict(comp=[N,P] u32, hist=[N,bins] u32, sums=[N] u32, table=[2^30] u32) for the requested parts.
-        `out` may carry preallocated (ideally page-locked) arrays under the same keys."""
+        `out` may carry preallocated (ideally page-locked) arrays under the same keys.  add_to_table: count these reads
+        INTO the context's complete table (from an earlier count or table_load) instead of from zero; on failure the
+        context holds no table."""
         n = reads.n_reads
         out = dict(out or {})
         comp = hist = sums = table = None
@@ -162,7 +219,8 @@ class Context:
                                    _ptr(comp) if comp is not None else None, _ptr(hist) if hist is not None else None,
                                    _ptr(sums) if sums is not None else None, _ptr(table) if table is not None else None,
                                    (_lib.PROFILE_USE_LOADED_TABLE if use_loaded_table else 0) |
-                                   (_lib.PROFILE_KEEP_TABLE if keep_table else 0)))
+                                   (_lib.PROFILE_KEEP_TABLE if keep_table else 0) |
+                                   (_lib.PROFILE_ADD_TO_TABLE if add_to_table else 0)))
         return {"comp": comp, "hist": hist, "sums": sums, "table": table}
 
     def info(self):
