@@ -40,6 +40,7 @@ extern "C" {
 #define LRB_TABLE_ENTRIES (1ull << 30) /* 4^15, count-15mers.cpp:99 */
 #define LRB_TILE_BLOCKS 256            /* 32-slot blocks of one read per warp tile */
 #define LRB_MAX_BINS 4096              /* coverage histogram width accepted by lrb_dev_search */
+#define LRB_MAX_COV_SETTINGS 8         /* (bin size, bin count) settings binned in one search (*_settings calls) */
 
 int lrb_version(void);
 const char* lrb_last_error(void);
@@ -234,6 +235,14 @@ int lrb_dev_partition_apply(const lrb_partition* part, int mode, uint32_t* table
  * that includes the last bucket. */
 int lrb_dev_partition_apply_range(const lrb_partition* part, int mode, int bucket_lo, int bucket_hi, uint32_t* table,
                                   long bin_size, int bins, uint32_t* hist, uint32_t* sums, void* stream);
+/* Search for n coverage settings at once (no reference counterpart: the reference runs search-15mers once per -bs/-bc).
+ * Every window's count is gathered once and binned by each setting (bin_sizes[m], bins[m]) into rows of W = sum of bins[m]
+ * words: setting 0's bins, then setting 1's, ...  Row r of setting m is hist[r*W + sum_{j<m} bins[j] + b]; sums[r] (the
+ * read's valid windows, the same for every setting) is rewritten by the call that includes the last bucket, as in mode 2.
+ * LRB_EINVAL unless 1 <= n <= LRB_MAX_COV_SETTINGS, every bin_size >= 1, every bins in [1, LRB_MAX_BINS], W <= LRB_MAX_BINS
+ * and no (bin_size, bins) pair repeats.  n = 1 is mode 2 of lrb_dev_partition_apply_range, row for row. */
+int lrb_dev_partition_search_settings(const lrb_partition* part, int bucket_lo, int bucket_hi, const uint32_t* table, int n,
+                                      const long* bin_sizes, const int* bins, uint32_t* hist, uint32_t* sums, void* stream);
 
 /* Pack ASCII on the device: bases[] (device, concatenated) -> codes/valid of `dev` (layout prebuilt). */
 int lrb_dev_pack_ascii(const lrb_reads_view* dev, const char* bases, const uint64_t* offsets, void* stream);
@@ -302,6 +311,14 @@ void lrb_ctx_destroy(lrb_ctx* ctx);
 #define LRB_PROFILE_ADD_TO_TABLE 4
 int lrb_profile_host(lrb_ctx* ctx, const lrb_reads* reads, int k, long bin_size, int bins, uint32_t* comp_counts,
                      uint32_t* cov_hist, uint32_t* cov_sums, uint32_t* table_host, int flags);
+/* The same with n coverage settings searched in one pass over the table (lrb_dev_partition_search_settings): cov_hist[N*W],
+ * W = sum of bins[m], holds for every read setting 0's bins, then setting 1's, ...; cov_sums[N] is shared by all settings.
+ * Every flag and part of lrb_profile_host works alongside (composition, count, KEEP / ADD_TO / USE_LOADED_TABLE, batches,
+ * several devices); lrb_profile_host is its n = 1 case.  The settings are checked as in lrb_dev_partition_search_settings
+ * when coverage is asked for, before any device work; n > 1 under LRB_TABLE_PATH=direct is refused (LRB_EINVAL).  The
+ * experiment switches LRB_SEARCH_LUT and LRB_SEARCH_HINT act on single-setting calls only. */
+int lrb_profile_host_settings(lrb_ctx* ctx, const lrb_reads* reads, int k, int n, const long* bin_sizes, const int* bins,
+                              uint32_t* comp_counts, uint32_t* cov_hist, uint32_t* cov_sums, uint32_t* table_host, int flags);
 /* How the last lrb_profile_host call ran. */
 typedef struct {
     int n_devices;            /* GPUs that took part */
@@ -391,6 +408,13 @@ int lrb_count_kmers(const char* reads_path, const char* out_txt, int k, int thre
 int lrb_count_15mers(const char* reads_path, const char* out_table, int threads);
 int lrb_search_15mers(const char* table_path, const char* reads_path, const char* out_txt, long bin_size, int bins,
                       int threads);
+/* lrb_search_15mers for n settings with one table load and one parse: out_txts[m] receives the coverage text of
+ * (bin_sizes[m], bins[m]), byte for byte the file lrb_search_15mers writes for that setting; out_npys (may be NULL, or
+ * hold NULLs) the matching .npy.  Input larger than one segment is read segment by segment (rows of 4 (W + 1) bytes per
+ * read) and every file gets its rows appended in file order.  The arguments are checked before any file or device is
+ * touched (LRB_EINVAL as for lrb_profile_host_settings; a NULL path too).  No reference counterpart. */
+int lrb_search_15mers_settings(const char* table_path, const char* reads_path, int n, const long* bin_sizes, const int* bins,
+                               const char* const* out_txts, const char* const* out_npys, int threads);
 /* Abundance spectrum of a 15mers-counts file as lrb_write_spectrum_txt text (loaded on device LRB_DEVICE).  Missing or
  * malformed table file: LRB_EIO / LRB_EFORMAT; no device: LRB_ECUDA.  No reference counterpart. */
 int lrb_table_spectrum(const char* table_path, const char* out_txt, uint32_t max_count);

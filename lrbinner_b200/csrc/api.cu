@@ -239,8 +239,11 @@ namespace {
 
 struct Job {
     const lrb_reads* reads = nullptr;
-    int k = 0, P = 0, bins = 1;
-    long bin_size = 1;
+    int k = 0, P = 0, bins = 1;       // bins: width of a coverage row, the sum of the settings' bin counts
+    long bin_size = 1;                // setting 0's (the only one the direct search takes)
+    int n_set = 1;                    // coverage settings binned in one search (lrb_profile_host_settings)
+    long set_bs[LRB_MAX_COV_SETTINGS] = {1};
+    int set_bins[LRB_MAX_COV_SETTINGS] = {1};
     uint32_t *comp = nullptr, *hist = nullptr, *sums = nullptr, *table_host = nullptr;
     bool do_comp = false, do_search = false, do_count = false, use_loaded = false, add_to_table = false;
     bool use_part = true, want_smem_env = false, force_l2 = false, comp_pinned = false;
@@ -483,6 +486,9 @@ int stage_front(lrb_ctx* c, const lrb_reads* r, const Job& J, uint64_t row0, boo
 // Pass 2: coverage rows of the batch's reads against the device's (finished) table, buckets [b_lo, b_hi) of the lists.
 int search_lists(lrb_ctx* c, const Job& J, uint64_t n, int b_lo, int b_hi) {
     if (!n) return LRB_OK;
+    if (J.n_set > 1)
+        return lrb_dev_partition_search_settings(&c->part, b_lo, b_hi, (const uint32_t*)c->table.p, J.n_set, J.set_bs, J.set_bins,
+                                                 (uint32_t*)c->hist.p, (uint32_t*)c->sums.p, c->stream);
     return lrb_dev_partition_apply_range(&c->part, 2, b_lo, b_hi, (uint32_t*)c->table.p, J.bin_size, J.bins, (uint32_t*)c->hist.p,
                                          (uint32_t*)c->sums.p, c->stream);
 }
@@ -638,26 +644,40 @@ int enqueue_exchange(std::vector<DevPlan>& plans, int n_buckets, int shift, bool
 
 // Seam-to-seam pipeline (see the block comment above).  Phase timings of device 0's first batch
 // (lrb_ctx_last_timings) overlap; [6] is the whole call on device 0's stream; lrb_ctx_last_info has the wall clock.
-static int profile_host(lrb_ctx* c, const lrb_reads* r, int k, long bin_size, int bins, uint32_t* comp_counts,
-                        uint32_t* cov_hist, uint32_t* cov_sums, uint32_t* table_host, int flags) {
+static bool direct_table_path() {   // one random HBM access per window (kernels.cu): experiments only
+    const char* e = getenv("LRB_TABLE_PATH");
+    return e && !strcmp(e, "direct");
+}
+
+static int profile_host(lrb_ctx* c, const lrb_reads* r, int k, int n_set, const long* bin_sizes, const int* bins,
+                        uint32_t* comp_counts, uint32_t* cov_hist, uint32_t* cov_sums, uint32_t* table_host, int flags) {
     Job J;
-    J.reads = r; J.k = k; J.P = comp_width(k); J.bins = bins; J.bin_size = bin_size;
+    J.reads = r; J.k = k; J.P = comp_width(k);
     J.comp = comp_counts; J.hist = cov_hist; J.sums = cov_sums; J.table_host = table_host;
     J.do_comp = comp_counts != nullptr;
     if (J.do_comp && !J.P) return lrb_set_error(LRB_EINVAL, "k must be 3, 4 or 5 (got %d)", k);
     J.do_search = cov_hist || cov_sums;
     if (J.do_search && (!cov_hist || !cov_sums)) return lrb_set_error(LRB_EINVAL, "cov_hist and cov_sums go together");
-    if (J.do_search && bin_size <= 0) return lrb_set_error(LRB_EINVAL, "bin_size must be >= 1 (the reference divides by it)");
-    if (J.do_search && (bins <= 0 || bins > LRB_MAX_BINS)) return lrb_set_error(LRB_EINVAL, "bins must be in [1, %d]", LRB_MAX_BINS);
+    if (J.do_search) {
+        uint32_t W = 0;
+        const int rc = lrb_check_cov_settings("lrb_profile_host", n_set, bin_sizes, bins, &W);
+        if (rc) return rc;
+        if (n_set > 1 && direct_table_path())
+            return lrb_set_error(LRB_EINVAL, "LRB_TABLE_PATH=direct searches one coverage setting per call (%d settings asked for)", n_set);
+        J.n_set = n_set;
+        std::copy(bin_sizes, bin_sizes + n_set, J.set_bs);
+        std::copy(bins, bins + n_set, J.set_bins);
+        J.bin_size = bin_sizes[0];
+        J.bins = (int)W;
+    }
     J.use_loaded = (flags & LRB_PROFILE_USE_LOADED_TABLE) != 0;
     J.add_to_table = (flags & LRB_PROFILE_ADD_TO_TABLE) != 0;
     if (J.use_loaded && J.add_to_table) return lrb_set_error(LRB_EINVAL, "LRB_PROFILE_USE_LOADED_TABLE and LRB_PROFILE_ADD_TO_TABLE exclude each other");
     if ((J.use_loaded || J.add_to_table) && !c->table_ready) return lrb_set_error(LRB_EINVAL, "no table loaded in this context");
     J.do_count = !J.use_loaded && (J.do_search || table_host || (flags & (LRB_PROFILE_KEEP_TABLE | LRB_PROFILE_ADD_TO_TABLE)));
     {
-        const char* e = getenv("LRB_TABLE_PATH");
-        if (e && !strcmp(e, "direct")) J.use_part = false;   // one random HBM access per window (kernels.cu): experiments only
-        e = getenv("LRB_COUNT_PATH");
+        if (direct_table_path()) J.use_part = false;
+        const char* e = getenv("LRB_COUNT_PATH");
         J.want_smem_env = e && !strcmp(e, "smem");
         J.force_l2 = e && !strcmp(e, "l2");
         const int bl = env_int("LRB_BUCKET_LOG2", 24);
@@ -921,12 +941,17 @@ static int profile_host(lrb_ctx* c, const lrb_reads* r, int k, long bin_size, in
     return LRB_OK;
 }
 
-extern "C" int lrb_profile_host(lrb_ctx* c, const lrb_reads* r, int k, long bin_size, int bins, uint32_t* comp_counts,
-                                uint32_t* cov_hist, uint32_t* cov_sums, uint32_t* table_host, int flags) {
+extern "C" int lrb_profile_host_settings(lrb_ctx* c, const lrb_reads* r, int k, int n, const long* bin_sizes, const int* bins,
+                                         uint32_t* comp_counts, uint32_t* cov_hist, uint32_t* cov_sums, uint32_t* table_host, int flags) {
     if (!c || !r) return lrb_set_error(LRB_EINVAL, "lrb_profile_host: null argument");
-    const int rc = profile_host(c, r, k, bin_size, bins, comp_counts, cov_hist, cov_sums, table_host, flags);
+    const int rc = profile_host(c, r, k, n, bin_sizes, bins, comp_counts, cov_hist, cov_sums, table_host, flags);
     if (rc && (flags & LRB_PROFILE_ADD_TO_TABLE)) c->table_ready = false;   // the table may hold part of this read set
     return rc;
+}
+
+extern "C" int lrb_profile_host(lrb_ctx* c, const lrb_reads* r, int k, long bin_size, int bins, uint32_t* comp_counts,
+                                uint32_t* cov_hist, uint32_t* cov_sums, uint32_t* table_host, int flags) {
+    return lrb_profile_host_settings(c, r, k, 1, &bin_size, &bins, comp_counts, cov_hist, cov_sums, table_host, flags);
 }
 
 extern "C" int lrb_ctx_last_timings(const lrb_ctx* c, float* ms7) {
@@ -1290,6 +1315,43 @@ extern "C" int lrb_search_15mers(const char* table_path, const char* reads_path,
         std::vector<uint32_t> hist((size_t)n * bins + 1), sums(n + 1);
         const int rc2 = lrb_profile_host(cg.c, s, 0, bin_size, bins, nullptr, hist.data(), sums.data(), nullptr, LRB_PROFILE_USE_LOADED_TABLE);
         return rc2 ? rc2 : lrb_append_coverage_txt(out_txt, hist.data(), sums.data(), n, bins, threads, row0);
+    };
+    if (in.whole) return search(in.whole, 0);
+    if ((rc = each_segment(in, false, search))) return rc;
+    segments_notice(in, 1);
+    return LRB_OK;
+}
+
+extern "C" int lrb_search_15mers_settings(const char* table_path, const char* reads_path, int n, const long* bin_sizes, const int* bins,
+                                          const char* const* out_txts, const char* const* out_npys, int threads) {
+    if (!table_path || !reads_path || !out_txts) return lrb_set_error(LRB_EINVAL, "lrb_search_15mers_settings: null path");
+    uint32_t W = 0;
+    int rc = lrb_check_cov_settings("lrb_search_15mers_settings", n, bin_sizes, bins, &W);
+    if (rc) return rc;
+    for (int m = 0; m < n; ++m)
+        if (!out_txts[m]) return lrb_set_error(LRB_EINVAL, "lrb_search_15mers_settings: null output path (setting %d)", m);
+    if (n > 1 && direct_table_path())
+        return lrb_set_error(LRB_EINVAL, "LRB_TABLE_PATH=direct searches one coverage setting per call (%d settings asked for)", n);
+    CtxGuard cg;
+    if ((rc = create_ctx(0, &cg.c))) return rc;
+    if ((rc = lrb_ctx_table_load(cg.c, table_path))) return rc;
+    for (int m = 0; m < n; ++m)
+        if ((rc = truncate_file(out_txts[m]))) return rc;
+    Input in;
+    if ((rc = open_input(reads_path, threads, 4ull * ((uint64_t)W + 1), in))) return rc;
+    // rows of W words come back; each file gets its setting's columns, so the writers are those of lrb_search_15mers
+    auto search = [&](const lrb_reads* s, uint64_t row0) -> int {
+        const uint64_t nr = s->n_reads;
+        std::vector<uint32_t> hist((size_t)nr * W + 1), sums(nr + 1), one;
+        int rc2 = lrb_profile_host_settings(cg.c, s, 0, n, bin_sizes, bins, nullptr, hist.data(), sums.data(), nullptr, LRB_PROFILE_USE_LOADED_TABLE);
+        for (int m = 0, off = 0; m < n && !rc2; off += bins[m], ++m) {
+            const size_t B = (size_t)bins[m];
+            one.resize(nr * B + 1);
+            for (uint64_t r = 0; r < nr; ++r) std::copy_n(hist.data() + r * W + off, B, one.data() + r * B);
+            rc2 = lrb_append_coverage_txt(out_txts[m], one.data(), sums.data(), nr, bins[m], threads, row0);
+            if (!rc2 && out_npys && out_npys[m]) rc2 = lrb_append_coverage_npy(out_npys[m], one.data(), sums.data(), nr, bins[m], threads, row0);
+        }
+        return rc2;
     };
     if (in.whole) return search(in.whole, 0);
     if ((rc = each_segment(in, false, search))) return rc;

@@ -61,3 +61,7 @@ void lrb_host_free(void* p, bool pinned);
 
 // bases per segment of the segment reader for result rows of `row_bytes_per_read` (lrb_reader_open: segment_bases = 0)
 uint64_t lrb_segment_budget(uint64_t row_bytes_per_read);
+
+// n coverage settings (bin_sizes[m], bins[m]) of one search: 1 <= n <= LRB_MAX_COV_SETTINGS, bin_size >= 1, bins in
+// [1, LRB_MAX_BINS], no pair twice, row width W = sum of bins <= LRB_MAX_BINS (into *width).  LRB_EINVAL naming `who`.
+int lrb_check_cov_settings(const char* who, int n, const long* bin_sizes, const int* bins, uint32_t* width);

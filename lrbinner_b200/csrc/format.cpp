@@ -270,6 +270,23 @@ extern "C" int lrb_table_read_file(const char* path, uint32_t* table) {
     return LRB_OK;
 }
 
+int lrb_check_cov_settings(const char* who, int n, const long* bin_sizes, const int* bins, uint32_t* width) {
+    if (n < 1 || n > LRB_MAX_COV_SETTINGS) return lrb_set_error(LRB_EINVAL, "%s: the number of settings must be in [1, %d] (got %d)", who, LRB_MAX_COV_SETTINGS, n);
+    if (!bin_sizes || !bins) return lrb_set_error(LRB_EINVAL, "%s: null bin_sizes / bins", who);
+    uint64_t W = 0;
+    for (int m = 0; m < n; ++m) {
+        if (bin_sizes[m] < 1) return lrb_set_error(LRB_EINVAL, "%s: bin_size must be >= 1 (setting %d: got %ld)", who, m, bin_sizes[m]);
+        if (bins[m] < 1 || bins[m] > LRB_MAX_BINS) return lrb_set_error(LRB_EINVAL, "%s: bins must be in [1, %d] (setting %d: got %d)", who, LRB_MAX_BINS, m, bins[m]);
+        for (int j = 0; j < m; ++j)
+            if (bin_sizes[j] == bin_sizes[m] && bins[j] == bins[m])
+                return lrb_set_error(LRB_EINVAL, "%s: setting %d repeats setting %d (bin_size %ld, bins %d)", who, m, j, bin_sizes[m], bins[m]);
+        W += (uint64_t)bins[m];
+    }
+    if (W > LRB_MAX_BINS) return lrb_set_error(LRB_EINVAL, "%s: the settings' bins add up to %llu, more than %d", who, (unsigned long long)W, LRB_MAX_BINS);
+    if (width) *width = (uint32_t)W;
+    return LRB_OK;
+}
+
 // ---- abundance spectrum of the table (lrb_dev_table_spectrum layout: n_c for c < M, then n_over, sum_over, max) ----
 extern "C" int lrb_spectrum_bin_mass(const uint64_t* spectrum, uint32_t max_count, long bin_size, int bins, uint64_t* mass) {
     if (!spectrum || !mass) return lrb_set_error(LRB_EINVAL, "lrb_spectrum_bin_mass: null argument");

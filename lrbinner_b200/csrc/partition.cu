@@ -25,7 +25,9 @@
 //   k_count_keys    per bucket: RED.ADD.U32 table[key]                              (L2-resident atomics)
 //   k_search_keys   per bucket, warp per run: count = table[key] (an L2 hit), bucket rule, aggregation of equal
 //                   (read, bin) entries of the warp, RED into hist[read][bin]
-//   k_row_sums      sums[read] = sum of hist[read][*]  (every window lands in exactly one bin)
+//   k_search_settings  the same walk, the gathered count binned by up to 8 (bin size, bin count) settings into one
+//                   row of their concatenated bins (lrb_dev_partition_search_settings)
+//   k_row_sums      sums[read] = sum of hist[read][*]  (every window lands in exactly one bin of each setting)
 //
 // The stream can be added in several chunks (lrb_dev_partition_add), each with its own regions, so the
 // partition of chunk i overlaps the host-to-device copy of chunk i+1; everything is asynchronous on the
@@ -982,25 +984,18 @@ __device__ __forceinline__ uint32_t ldg_hint(const uint32_t* a, uint64_t pol) {
     return v;
 }
 
-template <bool USE_LUT, int U, int HINT = 0>
-__global__ void __launch_bounds__(256)
-k_search_keys(const uint32_t* __restrict__ ents, const PartMeta* __restrict__ meta, int bucket0, int n_chunks, ChunkList L,
-              StepTables T, uint32_t bucket_base0, uint32_t hi_mask2, int shift, const uint32_t* __restrict__ table, uint32_t S32,
-              uint64_t magic, uint32_t B, uint32_t* __restrict__ hist) {
-    // one launch may cover several buckets (gridDim.y): CTAs are dispatched x-fastest, so the buckets are still worked on
-    // one after the other (their slices take turns in L2) but the tail of one overlaps the head of the next
-    const int bucket = bucket0 + (int)blockIdx.y;
-    const uint32_t bucket_base = bucket_base0 + ((uint32_t)blockIdx.y << shift);
-    __shared__ uint32_t s_bnd[8][kTaskRuns + 1];  // per warp: start of each run of the span, [kTaskRuns] = end of the span
-    __shared__ uint32_t s_r0[8][kTaskRuns];       // per warp: read index of each run's step relative to the span's first
-    __shared__ uint16_t s_lut[USE_LUT ? kBinLut : 2];
-    if (meta->overflow) return;
-    // every count >= (B+1)*S lands in the last bin (pos >= B), so the table covers the whole rule
-    const uint32_t lut_top = USE_LUT ? (B + 1u) * S32 : 0u;
-    if (USE_LUT) {
-        for (uint32_t i = threadIdx.x; i <= lut_top; i += blockDim.x) s_lut[i] = (uint16_t)coverage_bin(i, S32, magic, B);
-        __syncthreads();
-    }
+// The walk over the entries of one bucket, shared by the single-setting search and the multi-setting one: put(hbase, cnt,
+// act, lane, seek, row) bins the gathered count `cnt` of an entry and adds it to the histogram row row() (relative to
+// hbase, whose rows are `pitch` words apart) after seek(); both only where act (the lane has an entry).  put is called by
+// every lane of the warp together, so it may use warp-wide primitives.  One launch may cover several buckets (gridDim.y):
+// CTAs are dispatched x-fastest, so the buckets are still worked on one after the other (their slices take turns in L2)
+// but the tail of one overlaps the head of the next.
+template <int U, int HINT, class Put>
+__device__ __forceinline__ void search_keys_body(const uint32_t* __restrict__ ents, const PartMeta* __restrict__ meta, int bucket,
+                                                 int n_chunks, const ChunkList& L, const StepTables& T, uint32_t bucket_base,
+                                                 uint32_t hi_mask2, int shift, const uint32_t* __restrict__ table,
+                                                 uint32_t* __restrict__ hist, uint32_t pitch, uint32_t (*s_bnd)[kTaskRuns + 1],
+                                                 uint32_t (*s_r0)[kTaskRuns], Put put) {
     const uint32_t lane = threadIdx.x & 31u, wl = threadIdx.x >> 5;
     const uint32_t warp = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, n_warps = (gridDim.x * blockDim.x) >> 5;
     const uint64_t pol = HINT ? l2_policy_evict_last() : 0ull;
@@ -1023,17 +1018,13 @@ k_search_keys(const uint32_t* __restrict__ ents, const PartMeta* __restrict__ me
         if (lane < kTaskRuns) r0[lane] = my_r0 - rbase;
         __syncwarp();
         const uint32_t span_beg = bnd[0], span_end = bnd[kTaskRuns];
-        uint32_t* __restrict__ hbase = hist + (size_t)rbase * B;
+        uint32_t* __restrict__ hbase = hist + (size_t)rbase * pitch;
         uint32_t cur = 0, nxt = bnd[1], rr = 0;  // run of this lane's current entry, its end, its relative read base
         auto emit = [&](uint32_t e, uint32_t cnt, uint32_t i, bool act) {
-            uint32_t cell = 0xFFFFFFFFu;
-            if (act) {
-                while (i >= nxt) { ++cur; nxt = bnd[cur + 1]; rr = r0[cur]; }  // runs may be empty; i < bnd[kTaskRuns] bounds cur
-                const uint32_t bin = USE_LUT ? s_lut[min(cnt, lut_top)] : coverage_bin(cnt, S32, magic, B);
-                cell = (rr + (e >> rsh)) * B + bin;
-            }
-            const uint32_t peers = __match_any_sync(0xFFFFFFFFu, cell);
-            if (act && (uint32_t)__ffs(peers) - 1u == lane) atomicAdd(hbase + cell, (uint32_t)__popc(peers));
+            // seek(): move to the run of entry i (active lanes only); row(): then the entry's read, relative to hbase
+            auto seek = [&]() { while (i >= nxt) { ++cur; nxt = bnd[cur + 1]; rr = r0[cur]; } };  // runs may be empty; i < bnd[kTaskRuns] bounds cur
+            auto row = [&]() { return rr + (e >> rsh); };
+            put(hbase, cnt, act, lane, seek, row);
         };
         uint32_t i0 = span_beg;
         constexpr uint32_t kStep = 32u * U;
@@ -1089,14 +1080,94 @@ k_search_keys(const uint32_t* __restrict__ ents, const PartMeta* __restrict__ me
     }
 }
 
-// sums[r] = number of windows of read r that were bucketed so far = sum of its histogram row
-__global__ void __launch_bounds__(256) k_row_sums(const uint32_t* __restrict__ hist, uint32_t* __restrict__ sums, uint64_t n_reads, uint32_t B) {
+// hist[read][bin(table[key])] += 1 for one (bin size, bin count): rows of B bins
+template <bool USE_LUT, int U, int HINT = 0>
+__global__ void __launch_bounds__(256)
+k_search_keys(const uint32_t* __restrict__ ents, const PartMeta* __restrict__ meta, int bucket0, int n_chunks, ChunkList L,
+              StepTables T, uint32_t bucket_base0, uint32_t hi_mask2, int shift, const uint32_t* __restrict__ table, uint32_t S32,
+              uint64_t magic, uint32_t B, uint32_t* __restrict__ hist) {
+    const int bucket = bucket0 + (int)blockIdx.y;
+    const uint32_t bucket_base = bucket_base0 + ((uint32_t)blockIdx.y << shift);
+    __shared__ uint32_t s_bnd[8][kTaskRuns + 1];  // per warp: start of each run of the span, [kTaskRuns] = end of the span
+    __shared__ uint32_t s_r0[8][kTaskRuns];       // per warp: read index of each run's step relative to the span's first
+    __shared__ uint16_t s_lut[USE_LUT ? kBinLut : 2];
+    if (meta->overflow) return;
+    // every count >= (B+1)*S lands in the last bin (pos >= B), so the table covers the whole rule
+    const uint32_t lut_top = USE_LUT ? (B + 1u) * S32 : 0u;
+    if (USE_LUT) {
+        for (uint32_t i = threadIdx.x; i <= lut_top; i += blockDim.x) s_lut[i] = (uint16_t)coverage_bin(i, S32, magic, B);
+        __syncthreads();
+    }
+    search_keys_body<U, HINT>(ents, meta, bucket, n_chunks, L, T, bucket_base, hi_mask2, shift, table, hist, B, s_bnd, s_r0,
+                              [&](uint32_t* hbase, uint32_t cnt, bool act, uint32_t lane, auto seek, auto row) {
+                                  uint32_t cell = 0xFFFFFFFFu;
+                                  if (act) {
+                                      seek();
+                                      const uint32_t bin = USE_LUT ? s_lut[min(cnt, lut_top)] : coverage_bin(cnt, S32, magic, B);
+                                      cell = row() * B + bin;
+                                  }
+                                  const uint32_t peers = __match_any_sync(0xFFFFFFFFu, cell);
+                                  if (act && (uint32_t)__ffs(peers) - 1u == lane) atomicAdd(hbase + cell, (uint32_t)__popc(peers));
+                              });
+}
+
+// Several (bin size, bin count) settings in one pass: the count gathered for a window is binned once per setting, into
+// rows of W = sum of B_m words that hold setting 0's bins, then setting 1's, ...  The gather (the cost of the search)
+// happens once; each further setting adds one bin computation, one __match_any_sync and the REDs of its cells.
+struct CovSettings {
+    uint64_t magic[LRB_MAX_COV_SETTINGS];
+    uint32_t S32[LRB_MAX_COV_SETTINGS], B[LRB_MAX_COV_SETTINGS], off[LRB_MAX_COV_SETTINGS];
+    uint32_t n, W;
+};
+
+template <int U>
+__global__ void __launch_bounds__(256)
+k_search_settings(const uint32_t* __restrict__ ents, const PartMeta* __restrict__ meta, int bucket0, int n_chunks, ChunkList L,
+                  StepTables T, uint32_t bucket_base0, uint32_t hi_mask2, int shift, const uint32_t* __restrict__ table,
+                  const __grid_constant__ CovSettings C, uint32_t* __restrict__ hist) {
+    const int bucket = bucket0 + (int)blockIdx.y;
+    const uint32_t bucket_base = bucket_base0 + ((uint32_t)blockIdx.y << shift);
+    __shared__ uint32_t s_bnd[8][kTaskRuns + 1];
+    __shared__ uint32_t s_r0[8][kTaskRuns];
+    if (meta->overflow) return;
+    search_keys_body<U, 0>(ents, meta, bucket, n_chunks, L, T, bucket_base, hi_mask2, shift, table, hist, C.W, s_bnd, s_r0,
+                           [&](uint32_t* hbase, uint32_t cnt, bool act, uint32_t lane, auto seek, auto row) {
+                               uint32_t base = 0;
+                               if (act) {
+                                   seek();
+                                   base = row() * C.W;
+                               }
+                               for (uint32_t m = 0; m < C.n; ++m) {
+                                   uint32_t cell = 0xFFFFFFFFu;
+                                   if (act) cell = base + C.off[m] + coverage_bin(cnt, C.S32[m], C.magic[m], C.B[m]);
+                                   const uint32_t peers = __match_any_sync(0xFFFFFFFFu, cell);
+                                   if (act && (uint32_t)__ffs(peers) - 1u == lane) atomicAdd(hbase + cell, (uint32_t)__popc(peers));
+                               }
+                           });
+}
+
+// sums[r] = number of windows of read r that were bucketed so far = sum of the B bins that start its histogram row (every
+// setting of a row counts each window once, so the first one does)
+__global__ void __launch_bounds__(256) k_row_sums(const uint32_t* __restrict__ hist, uint32_t* __restrict__ sums, uint64_t n_reads, uint32_t B,
+                                                  uint32_t pitch) {
     const uint64_t r = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (r >= n_reads) return;
-    const uint32_t* row = hist + r * B;
+    const uint32_t* row = hist + r * pitch;
     uint32_t s = 0;
     for (uint32_t i = 0; i < B; ++i) s += row[i];
     sums[r] = s;
+}
+
+// search tasks of every chunk of the partition (L.task0 = prefix of tasks per chunk)
+ChunkList chunk_list(const lrb_partition* part) {
+    ChunkList L;
+    L.task0[0] = 0;
+    for (int c = 0; c < kMaxChunks; ++c) {
+        L.step0[c] = c < part->n_chunks ? part->chunk_step0[c] : 0u;
+        L.nsteps[c] = c < part->n_chunks ? part->chunk_nsteps[c] : 0u;
+        L.task0[c + 1] = L.task0[c] + (L.nsteps[c] + kTaskRuns - 1) / kTaskRuns;
+    }
+    return L;
 }
 
 uint32_t l2_strided() {  // which rows a k2_partition warp sweeps: "strided" (warp + 16 j, default: 2 ms faster) or "block" (16 warp + j)
@@ -1108,6 +1179,10 @@ int sms() {
     int dev = 0, n = 148;
     if (cudaGetDevice(&dev) == cudaSuccess) cudaDeviceGetAttribute(&n, cudaDevAttrMultiProcessorCount, dev);
     return n > 0 ? n : 148;
+}
+
+unsigned search_grid(const ChunkList& L, int n_chunks) {  // CTAs per bucket of the search: 8 warps (tasks) per CTA
+    return (unsigned)std::min<uint64_t>((uint64_t)sms() * 8, (L.task0[n_chunks] + 7) / 8 + 1);
 }
 
 }  // namespace
@@ -1338,18 +1413,11 @@ extern "C" int lrb_dev_partition_apply_range(const lrb_partition* part, int mode
     const uint64_t magic = coverage_magic(S32);
     const PartMeta* meta = reinterpret_cast<const PartMeta*>(part->small);
     const StepTables T = step_tables(part->steps, part->step_capacity);
-    ChunkList L;
-    L.task0[0] = 0;
-    for (int c = 0; c < kMaxChunks; ++c) {
-        L.step0[c] = c < part->n_chunks ? part->chunk_step0[c] : 0u;
-        L.nsteps[c] = c < part->n_chunks ? part->chunk_nsteps[c] : 0u;
-        L.task0[c + 1] = L.task0[c] + (L.nsteps[c] + kTaskRuns - 1) / kTaskRuns;
-    }
-    const uint32_t n_tasks = L.task0[part->n_chunks];
+    const ChunkList L = chunk_list(part);
     const int shift = part->shift;
     const uint32_t hi_mask2 = ((1u << shift) - 1u) & ~0xFFFFu;
     const unsigned grid = (unsigned)sms() * 8;
-    const unsigned sgrid = (unsigned)std::min<uint64_t>(grid, (n_tasks + 7) / 8 + 1);  // 8 warps (tasks) per CTA
+    const unsigned sgrid = search_grid(L, part->n_chunks);
     // bin rule through a shared-memory table instead of arithmetic: measured slower on B200 (the extra LDS competes with
     // the gathers for the memory pipe), kept behind LRB_SEARCH_LUT=1 for experiments
     const char* lut_env = getenv("LRB_SEARCH_LUT");
@@ -1405,7 +1473,49 @@ extern "C" int lrb_dev_partition_apply_range(const lrb_partition* part, int mode
         }
     }
     if (do_search && part->n_reads && bucket_hi == part->n_buckets)
-        LRB_LAUNCH("k_row_sums", st, k_row_sums<<<(unsigned)((part->n_reads + 255) / 256), 256, 0, st>>>(hist, sums, part->n_reads, (uint32_t)bins));
+        LRB_LAUNCH("k_row_sums", st, k_row_sums<<<(unsigned)((part->n_reads + 255) / 256), 256, 0, st>>>(hist, sums, part->n_reads, (uint32_t)bins, (uint32_t)bins));
+    LRB_CUDA(cudaGetLastError());
+    return LRB_OK;
+}
+
+// Several coverage settings in one search (k_search_settings): hist rows of W = sum of bins[m] words, setting m's bins at
+// column sum_{j<m} bins[j]; sums are rewritten by the call that includes the last bucket.  n = 1 is mode 2 of
+// lrb_dev_partition_apply_range (where the experiment switches LRB_SEARCH_LUT / _HINT / _UNROLL apply).
+extern "C" int lrb_dev_partition_search_settings(const lrb_partition* part, int bucket_lo, int bucket_hi, const uint32_t* table, int n,
+                                                 const long* bin_sizes, const int* bins, uint32_t* hist, uint32_t* sums, void* stream) {
+    if (!part || !table || !hist || !sums) return lrb_set_error(LRB_EINVAL, "lrb_dev_partition_search_settings: null argument");
+    uint32_t W = 0;
+    const int rc = lrb_check_cov_settings("lrb_dev_partition_search_settings", n, bin_sizes, bins, &W);
+    if (rc) return rc;
+    if (n == 1)
+        return lrb_dev_partition_apply_range(part, 2, bucket_lo, bucket_hi, const_cast<uint32_t*>(table), bin_sizes[0], bins[0], hist, sums, stream);
+    if (!part->has_rids) return lrb_set_error(LRB_EINVAL, "lrb_dev_partition_search_settings: partition was built without read ids");
+    if (bucket_lo < 0) bucket_lo = 0;
+    if (bucket_hi > part->n_buckets) bucket_hi = part->n_buckets;
+    if (part->n_chunks == 0) return LRB_OK;
+    cudaStream_t st = (cudaStream_t)stream;
+    CovSettings C = {};
+    C.n = (uint32_t)n;
+    C.W = W;
+    for (int m = 0, off = 0; m < n; off += bins[m], ++m) {
+        C.S32[m] = bin_sizes[m] > 0xFFFFFFFFl ? 0xFFFFFFFFu : (uint32_t)bin_sizes[m];
+        C.magic[m] = coverage_magic(C.S32[m]);
+        C.B[m] = (uint32_t)bins[m];
+        C.off[m] = (uint32_t)off;
+    }
+    const PartMeta* meta = reinterpret_cast<const PartMeta*>(part->small);
+    const ChunkList L = chunk_list(part);
+    const int shift = part->shift;
+    const uint32_t hi_mask2 = ((1u << shift) - 1u) & ~0xFFFFu;
+    if (bucket_hi > bucket_lo) {
+        const dim3 gs(search_grid(L, part->n_chunks), (unsigned)(bucket_hi - bucket_lo));
+        LRB_LAUNCH("k_search_settings", st, k_search_settings<8><<<gs, 256, 0, st>>>(part->keys, meta, bucket_lo, part->n_chunks, L,
+                                                                                     step_tables(part->steps, part->step_capacity),
+                                                                                     part->key_lo + ((uint32_t)bucket_lo << shift),
+                                                                                     hi_mask2, shift, table, C, hist));
+    }
+    if (part->n_reads && bucket_hi == part->n_buckets)
+        LRB_LAUNCH("k_row_sums", st, k_row_sums<<<(unsigned)((part->n_reads + 255) / 256), 256, 0, st>>>(hist, sums, part->n_reads, (uint32_t)bins[0], W));
     LRB_CUDA(cudaGetLastError());
     return LRB_OK;
 }

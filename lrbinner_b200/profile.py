@@ -191,22 +191,30 @@ class Context:
         self.device = device
 
     def profile(self, reads, k=None, bin_size=None, bins=None, want_table=False, use_loaded_table=False, out=None,
-                keep_table=False, add_to_table=False):
+                keep_table=False, add_to_table=False, coverage=None):
         """Returns dict(comp=[N,P] u32, hist=[N,bins] u32, sums=[N] u32, table=[2^30] u32) for the requested parts.
         `out` may carry preallocated (ideally page-locked) arrays under the same keys.  add_to_table: count these reads
         INTO the context's complete table (from an earlier count or table_load) instead of from zero; on failure the
-        context holds no table."""
+        context holds no table.
+        coverage=[(bin_size, bins), ...] (instead of bin_size / bins): up to 8 settings searched in one pass over the table
+        (lrb_profile_host_settings).  hist is then [N, W], W = the sum of the bins, with each setting's columns after those of
+        the settings before it; hists[m] is the [N, bins_m] view of setting m, and sums are the same for every setting."""
+        if coverage is not None and (bin_size is not None or bins is not None):
+            raise _lib.LrbError(_lib.LRB_EINVAL, "coverage=[(bin_size, bins), ...] replaces bin_size / bins: give one or the other")
         n = reads.n_reads
         out = dict(out or {})
-        comp = hist = sums = table = None
+        comp = hist = sums = table = hists = None
+        set_bs, set_bins = _settings_arrays(coverage if coverage is not None else
+                                            [(bin_size if bin_size is not None else 1, bins if bins is not None else 1)])
         if k is not None:
             comp = out.get("comp")
             if comp is None:
                 comp = np.zeros((n, COMP_WIDTH[k]), dtype=np.uint32)
-        if bins is not None:
+        if bins is not None or coverage is not None:
+            width = max(int(np.clip(set_bins, 1, None).sum()), 1)
             hist = out.get("hist")
-            if hist is None:
-                hist = np.zeros((n, max(int(bins), 1)), dtype=np.uint32)
+            if hist is None:   # a width the library refuses (it checks the settings before any work) gets no real buffer
+                hist = np.zeros((n, width if coverage is None or width <= _lib.MAX_BINS else 1), dtype=np.uint32)
             sums = out.get("sums")
             if sums is None:
                 sums = np.zeros(n, dtype=np.uint32)
@@ -214,14 +222,17 @@ class Context:
             table = out.get("table")
             if table is None:
                 table = np.empty(_lib.TABLE_ENTRIES, dtype=np.uint32)
-        check(lib.lrb_profile_host(self._h, reads._h, int(k) if k is not None else 0,
-                                   int(bin_size) if bin_size is not None else 1, int(bins) if bins is not None else 1,
-                                   _ptr(comp) if comp is not None else None, _ptr(hist) if hist is not None else None,
-                                   _ptr(sums) if sums is not None else None, _ptr(table) if table is not None else None,
-                                   (_lib.PROFILE_USE_LOADED_TABLE if use_loaded_table else 0) |
-                                   (_lib.PROFILE_KEEP_TABLE if keep_table else 0) |
-                                   (_lib.PROFILE_ADD_TO_TABLE if add_to_table else 0)))
-        return {"comp": comp, "hist": hist, "sums": sums, "table": table}
+        check(lib.lrb_profile_host_settings(self._h, reads._h, int(k) if k is not None else 0, len(set_bs), _ptr(set_bs),
+                                            _ptr(set_bins), _ptr(comp) if comp is not None else None,
+                                            _ptr(hist) if hist is not None else None, _ptr(sums) if sums is not None else None,
+                                            _ptr(table) if table is not None else None,
+                                            (_lib.PROFILE_USE_LOADED_TABLE if use_loaded_table else 0) |
+                                            (_lib.PROFILE_KEEP_TABLE if keep_table else 0) |
+                                            (_lib.PROFILE_ADD_TO_TABLE if add_to_table else 0)))
+        if coverage is not None:
+            offs = np.concatenate([[0], np.cumsum(set_bins)])
+            hists = [hist[:, offs[m]:offs[m + 1]] for m in range(len(set_bins))]
+        return {"comp": comp, "hist": hist, "hists": hists, "sums": sums, "table": table}
 
     def info(self):
         """How the last profile() ran: devices, batches, table path, wall / exchange milliseconds."""
@@ -462,6 +473,22 @@ class PartitionWorkspace:
                                                 C.c_void_p(table.data_ptr()), bin_size, bins,
                                                 C.c_void_p(hist.data_ptr()) if hist is not None else None,
                                                 C.c_void_p(sums.data_ptr()) if sums is not None else None, _stream()))
+
+    def search_settings(self, table, settings, hist, sums, bucket_lo=0, bucket_hi=None):
+        """Search for several (bin_size, bins) settings at once (lrb_dev_partition_search_settings): hist is [N, W] with
+        W = the sum of the bins, each setting's columns after those of the settings before it; hist and sums zeroed by the
+        caller as for apply(search=True)."""
+        bs, bc = _settings_arrays(settings)
+        check(lib.lrb_dev_partition_search_settings(C.byref(self.part), bucket_lo, 64 if bucket_hi is None else bucket_hi,
+                                                    C.c_void_p(table.data_ptr()), len(bs), _ptr(bs), _ptr(bc),
+                                                    C.c_void_p(hist.data_ptr()), C.c_void_p(sums.data_ptr()), _stream()))
+
+
+def _settings_arrays(settings):
+    """(bin_sizes as C long, bins as C int) arrays of a list of (bin_size, bins) settings"""
+    settings = [(int(s), int(b)) for s, b in settings]
+    return (np.array([s for s, _ in settings], dtype=np.dtype(f"i{C.sizeof(C.c_long)}")),
+            np.array([b for _, b in settings], dtype=np.int32))
 
 
 def dev_table15_partitioned(dr, ws, table, do_count=True, bin_size=1, bins=1, hist=None, sums=None, blk_lo=0, blk_hi=None,

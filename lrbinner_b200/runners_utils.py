@@ -13,6 +13,7 @@ liblrb200.so (CUDA, sm_100a) through ctypes:
 A maintainer switches LRBinner over with one import line in mbcclr_utils/pipelines.py (INTEGRATION.md).
 run_profile() is the fused fast path for stages 1_1 + 1_2 + 2_1 (parse once, table stays in HBM).
 """
+import ctypes as C
 import logging
 import os
 import sys
@@ -48,6 +49,27 @@ def run_15mer_vecs(reads_path, output, bin_size, bin_count, threads):
     o = _lib.lib.lrb_search_15mers(os.fsencode(f"{output}/profiles/15mers-counts"), os.fsencode(reads_path),
                                    os.fsencode(f"{output}/profiles/cov_profs"), int(bin_size), int(bin_count), int(threads))
     check_proc(o, "Counting 15-mer profiles")
+
+
+def run_15mer_vecs_settings(reads_path, output, settings, threads, write_npy=False):
+    """Coverage profiles for several -bs / -bc settings at once: one load of {output}/profiles/15mers-counts and one parse
+    of the reads (lrb_search_15mers_settings), writing {output}/profiles/cov_profs_bs{S}_bc{B} (and .npy with write_npy)
+    for every (S, B) in `settings` (at most 8, no pair twice), each byte for byte the cov_profs that run_15mer_vecs
+    writes for that setting.  cov_profs itself is never touched, so a checkpointed run stays consistent: copy the chosen
+    file to cov_profs and resume from stage 3_1 (INTEGRATION.md).  No reference counterpart."""
+    settings = [(int(s), int(b)) for s, b in settings]
+    if not os.path.isdir(f"{output}/profiles"):
+        os.makedirs(f"{output}/profiles")
+    n = len(settings)
+    outs = [os.fsencode(f"{output}/profiles/cov_profs_bs{s}_bc{b}") for s, b in settings]
+    txts = (C.c_char_p * max(n, 1))(*outs)
+    npys = (C.c_char_p * max(n, 1))(*[o + b".npy" for o in outs]) if write_npy else None
+    bs = (C.c_long * max(n, 1))(*[s for s, _ in settings])
+    bc = (C.c_int * max(n, 1))(*[b for _, b in settings])
+    logger.debug(f"LIB::lrb_search_15mers_settings \"{output}/profiles/15mers-counts\" \"{reads_path}\" {settings} {threads}")
+    o = _lib.lib.lrb_search_15mers_settings(os.fsencode(f"{output}/profiles/15mers-counts"), os.fsencode(reads_path), n, bs, bc,
+                                            txts, npys, int(threads))
+    check_proc(o, "Counting 15-mer profiles for several settings")
 
 
 def run_15mer_histo(output, threads, max_count=65536):
