@@ -41,6 +41,7 @@ extern "C" {
 #define LRB_TILE_BLOCKS 256            /* 32-slot blocks of one read per warp tile */
 #define LRB_MAX_BINS 4096              /* coverage histogram width accepted by lrb_dev_search */
 #define LRB_MAX_COV_SETTINGS 8         /* (bin size, bin count) settings binned in one search (*_settings calls) */
+#define LRB_MAX_SAMPLE_TABLES 8        /* sample tables searched in one call (*_samples calls) and sample slots of a context */
 
 int lrb_version(void);
 const char* lrb_last_error(void);
@@ -140,6 +141,11 @@ int lrb_dev_mirror(uint32_t* table, void* stream);
 #define LRB_SPECTRUM_MAX_COUNT (1u << 24)
 int lrb_dev_table_spectrum(const uint32_t* table, uint32_t key_lo, uint32_t key_hi, uint32_t max_count, uint64_t* spectrum,
                            void* stream);
+/* Compact form of a sample table: only its canonical (bit-15-clear) half, 2^29 u32 = 2 GiB, entry i holding
+ * table[((i >> 15) << 16) | (i & 0x7FFF)].  The multi-table search reads sample tables only at bit-15-clear keys, so it
+ * takes them in this form.  `table` is a full-layout 2^30-entry table (the other half need not be mirrored). */
+#define LRB_COMPACT_ENTRIES (1ull << 29)
+int lrb_dev_table_compact(const uint32_t* table, uint32_t* compact, void* stream);
 
 /* Multi-GPU table exchange helpers (the reference has no counterpart: it is single-process; SURVEY.md 8e).
  * lrb_dev_copy2d: pitched device-to-device copy on the copy engines; src may be a peer GPU's table mapped into this
@@ -243,6 +249,23 @@ int lrb_dev_partition_apply_range(const lrb_partition* part, int mode, int bucke
  * and no (bin_size, bins) pair repeats.  n = 1 is mode 2 of lrb_dev_partition_apply_range, row for row. */
 int lrb_dev_partition_search_settings(const lrb_partition* part, int bucket_lo, int bucket_hi, const uint32_t* table, int n,
                                       const long* bin_sizes, const int* bins, uint32_t* hist, uint32_t* sums, void* stream);
+/* Search the partition's reads against n compact sample tables at once (differential coverage; no reference counterpart:
+ * the reference runs search-15mers once per table).  compact_tables is a HOST array of n device pointers to
+ * lrb_dev_table_compact tables; table t is binned with (bin_sizes[t], bins[t]) into rows of W = sum of bins[t] words:
+ * table 0's bins, then table 1's, ...  Row r of table t is hist[r*W + sum_{j<t} bins[j] + b] and equals row r of a
+ * single-table search with that table's full layout, for every table that is symmetric (T[x] == T[revcomp x], as every
+ * counted table is): like every partitioned search, only the bit-15-clear member of each {x, revcomp x} pair is read.
+ * sums[r] (the read's valid windows, the same for every table) is rewritten by the call that includes the last bucket.
+ * One walk over the lists per group of tables (the group size is measured, DESIGN.md section 4).  LRB_EINVAL unless
+ * 1 <= n <= LRB_MAX_SAMPLE_TABLES, every bin_size >= 1, every bins in [1, LRB_MAX_BINS], W <= LRB_MAX_BINS, no
+ * (table pointer, bin_size, bins) repeats, the partition has read ids and starts at a bucket boundary. */
+int lrb_dev_partition_search_samples(const lrb_partition* part, int bucket_lo, int bucket_hi, const uint32_t* const* compact_tables,
+                                     int n, const long* bin_sizes, const int* bins, uint32_t* hist, uint32_t* sums, void* stream);
+/* The same with the group size given: 1 (one walk per table) or 2 (two tables per walk); 0 is the default of
+ * lrb_dev_partition_search_samples.  For measuring the two against each other. */
+int lrb_dev_partition_search_samples_grouped(const lrb_partition* part, int bucket_lo, int bucket_hi,
+                                             const uint32_t* const* compact_tables, int n, const long* bin_sizes, const int* bins,
+                                             uint32_t* hist, uint32_t* sums, int group, void* stream);
 
 /* Pack ASCII on the device: bases[] (device, concatenated) -> codes/valid of `dev` (layout prebuilt). */
 int lrb_dev_pack_ascii(const lrb_reads_view* dev, const char* bases, const uint64_t* offsets, void* stream);
@@ -319,6 +342,28 @@ int lrb_profile_host(lrb_ctx* ctx, const lrb_reads* reads, int k, long bin_size,
  * experiment switches LRB_SEARCH_LUT and LRB_SEARCH_HINT act on single-setting calls only. */
 int lrb_profile_host_settings(lrb_ctx* ctx, const lrb_reads* reads, int k, int n, const long* bin_sizes, const int* bins,
                               uint32_t* comp_counts, uint32_t* cov_hist, uint32_t* cov_sums, uint32_t* table_host, int flags);
+/* Sample slots: a context holds up to LRB_MAX_SAMPLE_TABLES sample tables beside its own table, each in compact form
+ * (lrb_dev_table_compact, 2 GiB) on EVERY device of the context (the multi-device search shards reads, so every device
+ * needs every table).  Loading or keeping into a slot replaces what it held; neither touches the context's own table.
+ * lrb_ctx_sample_table_load reads only the canonical rows of a 15mers-counts file (2^14 rows of 128 KiB at a 256 KiB
+ * stride: 2 GiB of the 4 GiB); the header and the file size are checked first: missing file LRB_EIO, bad header or size
+ * LRB_EFORMAT.  lrb_ctx_sample_table_keep compacts the context's own complete table into the slot (LRB_EINVAL when the
+ * context holds none).  lrb_ctx_sample_table_free releases the slot's memory. */
+int lrb_ctx_sample_table_load(lrb_ctx* ctx, int slot, const char* path);
+int lrb_ctx_sample_table_keep(lrb_ctx* ctx, int slot);
+int lrb_ctx_sample_table_free(lrb_ctx* ctx, int slot);
+/* Host side of lrb_ctx_sample_table_load: canonical rows [row_lo, row_hi) (row j = entries j 2^16 .. j 2^16 + 2^15 - 1)
+ * of a 15mers-counts file into compact[(row_hi - row_lo) 2^15], after the same header and size checks. */
+int lrb_table_read_canonical(const char* path, uint32_t row_lo, uint32_t row_hi, uint32_t* compact);
+/* lrb_profile_host_settings with coverage against n sample slots instead of the context's table: slot slots[t] binned with
+ * (bin_sizes[t], bins[t]) into cov_hist[N*W], W = sum of bins[t], table 0's bins first (lrb_dev_partition_search_samples).
+ * The context's own table is not searched (keep it into a slot to search it).  Composition, the count flags
+ * (KEEP_TABLE, ADD_TO_TABLE, table_host), batches and several devices work alongside; coverage itself needs no count.
+ * LRB_EINVAL before any device work for an empty or out-of-range slot, bad settings, the same (slot, bin_size, bins)
+ * twice, and LRB_TABLE_PATH=direct (the direct kernels read only the full-layout table). */
+int lrb_profile_host_samples(lrb_ctx* ctx, const lrb_reads* reads, int k, int n, const int* slots, const long* bin_sizes,
+                             const int* bins, uint32_t* comp_counts, uint32_t* cov_hist, uint32_t* cov_sums, uint32_t* table_host,
+                             int flags);
 /* How the last lrb_profile_host call ran. */
 typedef struct {
     int n_devices;            /* GPUs that took part */
@@ -415,6 +460,15 @@ int lrb_search_15mers(const char* table_path, const char* reads_path, const char
  * touched (LRB_EINVAL as for lrb_profile_host_settings; a NULL path too).  No reference counterpart. */
 int lrb_search_15mers_settings(const char* table_path, const char* reads_path, int n, const long* bin_sizes, const int* bins,
                                const char* const* out_txts, const char* const* out_npys, int threads);
+/* Differential coverage: the reads against n 15mers-counts files at once, each loaded once into a sample slot (canonical
+ * rows only) and the reads parsed once.  Line r of out_txt holds table 0's bins, then table 1's, ... (W = sum of bins[t]
+ * values): block t is, byte for byte, line r of lrb_search_15mers(table_paths[t], reads, bin_sizes[t], bins[t]) for every
+ * symmetric (counted) table, and the blocks are joined by one space.  out_npy (may be NULL) gets the [N, W] float rows.
+ * Input larger than one segment is read segment by segment (rows of 4 (W + 1) bytes per read).  LRB_GPUS is honoured.
+ * Arguments are checked before any file or device work (LRB_EINVAL: a NULL path, n, the settings, the same (path, bin_size,
+ * bins) twice).  No reference counterpart. */
+int lrb_search_15mers_samples(const char* const* table_paths, int n, const long* bin_sizes, const int* bins, const char* reads_path,
+                              const char* out_txt, const char* out_npy, int threads);
 /* Abundance spectrum of a 15mers-counts file as lrb_write_spectrum_txt text (loaded on device LRB_DEVICE).  Missing or
  * malformed table file: LRB_EIO / LRB_EFORMAT; no device: LRB_ECUDA.  No reference counterpart. */
 int lrb_table_spectrum(const char* table_path, const char* out_txt, uint32_t max_count);

@@ -14,6 +14,8 @@ TABLE_ENTRIES = 1 << 30
 TILE_BLOCKS = 256
 MAX_BINS = 4096
 MAX_COV_SETTINGS = 8
+MAX_SAMPLE_TABLES = 8
+COMPACT_ENTRIES = 1 << 29
 SPECTRUM_MAX_COUNT = 1 << 24
 
 
@@ -103,6 +105,9 @@ _SIG = {
     "lrb_dev_partition_apply": (C.c_int, [_P, C.c_int, _P, C.c_long, C.c_int, _P, _P, _P]),
     "lrb_dev_partition_apply_range": (C.c_int, [_P, C.c_int, C.c_int, C.c_int, _P, C.c_long, C.c_int, _P, _P, _P]),
     "lrb_dev_partition_search_settings": (C.c_int, [_P, C.c_int, C.c_int, _P, C.c_int, _P, _P, _P, _P, _P]),
+    "lrb_dev_partition_search_samples": (C.c_int, [_P, C.c_int, C.c_int, _P, C.c_int, _P, _P, _P, _P, _P]),
+    "lrb_dev_partition_search_samples_grouped": (C.c_int, [_P, C.c_int, C.c_int, _P, C.c_int, _P, _P, _P, _P, C.c_int, _P]),
+    "lrb_dev_table_compact": (C.c_int, [_P, _P, _P]),
     "lrb_dev_pack_ascii": (C.c_int, [C.POINTER(ReadsView), _P, _P, _P]),
     "lrb_dev_format_composition": (C.c_int, [_P, _P, C.c_uint64, C.c_int, _P, _P]),
     "lrb_dev_format_coverage": (C.c_int, [_P, _P, C.c_uint64, C.c_int, _P, _P]),
@@ -116,6 +121,11 @@ _SIG = {
     "lrb_ctx_last_info": (C.c_int, [_P, _P]),
     "lrb_profile_host": (C.c_int, [_P, _P, C.c_int, C.c_long, C.c_int, _P, _P, _P, _P, C.c_int]),
     "lrb_profile_host_settings": (C.c_int, [_P, _P, C.c_int, C.c_int, _P, _P, _P, _P, _P, _P, C.c_int]),
+    "lrb_profile_host_samples": (C.c_int, [_P, _P, C.c_int, C.c_int, _P, _P, _P, _P, _P, _P, _P, C.c_int]),
+    "lrb_ctx_sample_table_load": (C.c_int, [_P, C.c_int, C.c_char_p]),
+    "lrb_ctx_sample_table_keep": (C.c_int, [_P, C.c_int]),
+    "lrb_ctx_sample_table_free": (C.c_int, [_P, C.c_int]),
+    "lrb_table_read_canonical": (C.c_int, [C.c_char_p, C.c_uint32, C.c_uint32, _P]),
     "lrb_ctx_last_timings": (C.c_int, [_P, _P]),
     "lrb_pinned_alloc": (_P, [C.c_size_t]),
     "lrb_pinned_free": (None, [_P]),
@@ -143,6 +153,7 @@ _SIG = {
     "lrb_count_15mers": (C.c_int, [C.c_char_p, C.c_char_p, C.c_int]),
     "lrb_search_15mers": (C.c_int, [C.c_char_p, C.c_char_p, C.c_char_p, C.c_long, C.c_int, C.c_int]),
     "lrb_search_15mers_settings": (C.c_int, [C.c_char_p, C.c_char_p, C.c_int, _P, _P, _P, _P, C.c_int]),
+    "lrb_search_15mers_samples": (C.c_int, [_P, C.c_int, _P, _P, C.c_char_p, C.c_char_p, C.c_char_p, C.c_int]),
     "lrb_table_spectrum": (C.c_int, [C.c_char_p, C.c_char_p, C.c_uint32]),
     "lrb_profile": (C.c_int, [C.c_char_p, C.c_char_p, C.c_int, C.c_long, C.c_int, C.c_int, C.c_int, C.c_int]),
     "lrb_profile_multi": (C.c_int, [C.c_char_p, C.c_char_p, C.c_int, C.c_long, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int]),

@@ -98,6 +98,8 @@ struct lrb_ctx {
     DevBuf stage;                                         // multi-GPU exchange: rows pulled from the peers
     lrb_partition part = {};
     bool table_ready = false;  // holds a complete (mirrored) table
+    DevBuf sample[LRB_MAX_SAMPLE_TABLES];               // sample slots: compact tables (lrb_dev_table_compact), 2 GiB each
+    bool sample_ready[LRB_MAX_SAMPLE_TABLES] = {};
     lrb_reads_view dview = {};
     float ms[7] = {0, 0, 0, 0, 0, 0, 0};
     std::vector<lrb_ctx*> peers;   // devices 1.. of a multi-GPU context (owned by the context of devices[0])
@@ -205,6 +207,7 @@ extern "C" void lrb_ctx_destroy(lrb_ctx* c) {
     for (DevBuf* b : {&c->codes, &c->valid, &c->read_len, &c->read_blk, &c->tile_read, &c->tile_blk, &c->table, &c->comp,
                       &c->hist, &c->sums, &c->text, &c->part_keys, &c->part_small, &c->part_steps, &c->part_sub, &c->blk_read, &c->exc_blk, &c->exc_valid, &c->stage})
         b->release();
+    for (DevBuf& b : c->sample) b.release();
     for (auto& ev : c->ev) if (ev) cudaEventDestroy(ev);
     for (auto& ev : c->xev) if (ev) cudaEventDestroy(ev);
     for (auto& ev : c->sync_ev) if (ev) cudaEventDestroy(ev);
@@ -244,6 +247,8 @@ struct Job {
     int n_set = 1;                    // coverage settings binned in one search (lrb_profile_host_settings)
     long set_bs[LRB_MAX_COV_SETTINGS] = {1};
     int set_bins[LRB_MAX_COV_SETTINGS] = {1};
+    int n_samp = 0;                   // > 0: coverage against these sample slots (lrb_profile_host_samples), setting t each
+    int samp_slot[LRB_MAX_SAMPLE_TABLES] = {};
     uint32_t *comp = nullptr, *hist = nullptr, *sums = nullptr, *table_host = nullptr;
     bool do_comp = false, do_search = false, do_count = false, use_loaded = false, add_to_table = false;
     bool use_part = true, want_smem_env = false, force_l2 = false, comp_pinned = false;
@@ -275,7 +280,8 @@ bool host_ptr_is_pinned(const void* p) {
     return a.type == cudaMemoryTypeHost;
 }
 
-// bytes of device memory a batch of `blocks` blocks / `reads` reads needs beside the table
+// bytes of device memory a batch of `blocks` blocks / `reads` reads needs beside the table and the sample slots (both are
+// allocated before the batches are planned, so the free memory the plan starts from already leaves them out)
 uint64_t batch_bytes(const Job& J, uint64_t blocks, uint64_t reads, uint64_t tiles) {
     uint64_t b = blocks * 12 + 64;                                        // codes + valid
     b += reads * 8 + tiles * 8 + 64;                                      // read_len, read_blk, tiles
@@ -486,6 +492,12 @@ int stage_front(lrb_ctx* c, const lrb_reads* r, const Job& J, uint64_t row0, boo
 // Pass 2: coverage rows of the batch's reads against the device's (finished) table, buckets [b_lo, b_hi) of the lists.
 int search_lists(lrb_ctx* c, const Job& J, uint64_t n, int b_lo, int b_hi) {
     if (!n) return LRB_OK;
+    if (J.n_samp) {
+        const uint32_t* tabs[LRB_MAX_SAMPLE_TABLES];
+        for (int t = 0; t < J.n_samp; ++t) tabs[t] = (const uint32_t*)c->sample[J.samp_slot[t]].p;
+        return lrb_dev_partition_search_samples(&c->part, b_lo, b_hi, tabs, J.n_samp, J.set_bs, J.set_bins, (uint32_t*)c->hist.p,
+                                                (uint32_t*)c->sums.p, c->stream);
+    }
     if (J.n_set > 1)
         return lrb_dev_partition_search_settings(&c->part, b_lo, b_hi, (const uint32_t*)c->table.p, J.n_set, J.set_bs, J.set_bins,
                                                  (uint32_t*)c->hist.p, (uint32_t*)c->sums.p, c->stream);
@@ -649,7 +661,19 @@ static bool direct_table_path() {   // one random HBM access per window (kernels
     return e && !strcmp(e, "direct");
 }
 
-static int profile_host(lrb_ctx* c, const lrb_reads* r, int k, int n_set, const long* bin_sizes, const int* bins,
+// slot numbers in range, then the settings of the tables, the same slot with the same setting twice refused
+static int check_sample_slots(int n, const int* slots, const long* bin_sizes, const int* bins, uint32_t* W) {
+    uint64_t ids[LRB_MAX_SAMPLE_TABLES] = {};
+    for (int t = 0; t < n && t < LRB_MAX_SAMPLE_TABLES; ++t) {
+        if (slots[t] < 0 || slots[t] >= LRB_MAX_SAMPLE_TABLES)
+            return lrb_set_error(LRB_EINVAL, "lrb_profile_host_samples: slot must be in [0, %d) (table %d: got %d)", LRB_MAX_SAMPLE_TABLES, t, slots[t]);
+        ids[t] = (uint64_t)slots[t];
+    }
+    return lrb_check_table_settings("lrb_profile_host_samples", n, ids, bin_sizes, bins, W);
+}
+
+// slots: NULL, or the sample slot of each of the n_set settings (coverage against those instead of the context's table)
+static int profile_host(lrb_ctx* c, const lrb_reads* r, int k, int n_set, const long* bin_sizes, const int* bins, const int* slots,
                         uint32_t* comp_counts, uint32_t* cov_hist, uint32_t* cov_sums, uint32_t* table_host, int flags) {
     Job J;
     J.reads = r; J.k = k; J.P = comp_width(k);
@@ -658,10 +682,21 @@ static int profile_host(lrb_ctx* c, const lrb_reads* r, int k, int n_set, const 
     if (J.do_comp && !J.P) return lrb_set_error(LRB_EINVAL, "k must be 3, 4 or 5 (got %d)", k);
     J.do_search = cov_hist || cov_sums;
     if (J.do_search && (!cov_hist || !cov_sums)) return lrb_set_error(LRB_EINVAL, "cov_hist and cov_sums go together");
+    if (slots && !J.do_search) return lrb_set_error(LRB_EINVAL, "lrb_profile_host_samples: sample tables need cov_hist and cov_sums");
     if (J.do_search) {
         uint32_t W = 0;
-        const int rc = lrb_check_cov_settings("lrb_profile_host", n_set, bin_sizes, bins, &W);
-        if (rc) return rc;
+        int rc;
+        if (slots) {
+            if ((rc = check_sample_slots(n_set, slots, bin_sizes, bins, &W))) return rc;
+            for (int t = 0; t < n_set; ++t)
+                if (!c->sample_ready[slots[t]]) return lrb_set_error(LRB_EINVAL, "lrb_profile_host_samples: sample slot %d is empty (table %d)", slots[t], t);
+            if (direct_table_path())
+                return lrb_set_error(LRB_EINVAL, "lrb_profile_host_samples: LRB_TABLE_PATH=direct reads only the full-layout table, not sample slots");
+            J.n_samp = n_set;
+            std::copy(slots, slots + n_set, J.samp_slot);
+        } else if ((rc = lrb_check_cov_settings("lrb_profile_host", n_set, bin_sizes, bins, &W))) {
+            return rc;
+        }
         if (n_set > 1 && direct_table_path())
             return lrb_set_error(LRB_EINVAL, "LRB_TABLE_PATH=direct searches one coverage setting per call (%d settings asked for)", n_set);
         J.n_set = n_set;
@@ -674,7 +709,7 @@ static int profile_host(lrb_ctx* c, const lrb_reads* r, int k, int n_set, const 
     J.add_to_table = (flags & LRB_PROFILE_ADD_TO_TABLE) != 0;
     if (J.use_loaded && J.add_to_table) return lrb_set_error(LRB_EINVAL, "LRB_PROFILE_USE_LOADED_TABLE and LRB_PROFILE_ADD_TO_TABLE exclude each other");
     if ((J.use_loaded || J.add_to_table) && !c->table_ready) return lrb_set_error(LRB_EINVAL, "no table loaded in this context");
-    J.do_count = !J.use_loaded && (J.do_search || table_host || (flags & (LRB_PROFILE_KEEP_TABLE | LRB_PROFILE_ADD_TO_TABLE)));
+    J.do_count = !J.use_loaded && ((J.do_search && !J.n_samp) || table_host || (flags & (LRB_PROFILE_KEEP_TABLE | LRB_PROFILE_ADD_TO_TABLE)));
     {
         if (direct_table_path()) J.use_part = false;
         const char* e = getenv("LRB_COUNT_PATH");
@@ -689,7 +724,7 @@ static int profile_host(lrb_ctx* c, const lrb_reads* r, int k, int n_set, const 
     J.comp_pinned = host_ptr_is_pinned(comp_counts);
     const auto wall0 = std::chrono::steady_clock::now();
     const uint64_t n = r->n_reads, nb = r->n_blocks;
-    const bool need_table = J.do_count || J.do_search;
+    const bool need_table = J.do_count || (J.do_search && !J.n_samp);   // sample slots are allocated already
 
     // ---- devices and their read ranges (contiguous, balanced by blocks) ------------------------------------------
     std::vector<DevPlan> plans;
@@ -786,7 +821,7 @@ static int profile_host(lrb_ctx* c, const lrb_reads* r, int k, int n_set, const 
     // Adding to the table: device 0 counts into its complete table, every other device into a private table from zero, so
     // that after the exchange  sum over devices of the canonical halves = previous table + this read set;  the mirror then
     // rebuilds the other half on device 0 as for any count.
-    c->table_ready = J.use_loaded ? c->table_ready : false;
+    c->table_ready = (J.use_loaded || (J.n_samp && !J.do_count)) ? c->table_ready : false;   // a search of sample slots leaves it
     if (J.use_loaded && multi) {   // the loaded table lives on device 0: hand it to the others
         CTX_CUDA(cudaSetDevice(c->device));
         CTX_CUDA(cudaEventRecord(c->counted, c->stream));
@@ -944,8 +979,20 @@ static int profile_host(lrb_ctx* c, const lrb_reads* r, int k, int n_set, const 
 extern "C" int lrb_profile_host_settings(lrb_ctx* c, const lrb_reads* r, int k, int n, const long* bin_sizes, const int* bins,
                                          uint32_t* comp_counts, uint32_t* cov_hist, uint32_t* cov_sums, uint32_t* table_host, int flags) {
     if (!c || !r) return lrb_set_error(LRB_EINVAL, "lrb_profile_host: null argument");
-    const int rc = profile_host(c, r, k, n, bin_sizes, bins, comp_counts, cov_hist, cov_sums, table_host, flags);
+    const int rc = profile_host(c, r, k, n, bin_sizes, bins, nullptr, comp_counts, cov_hist, cov_sums, table_host, flags);
     if (rc && (flags & LRB_PROFILE_ADD_TO_TABLE)) c->table_ready = false;   // the table may hold part of this read set
+    return rc;
+}
+
+extern "C" int lrb_profile_host_samples(lrb_ctx* c, const lrb_reads* r, int k, int n, const int* slots, const long* bin_sizes,
+                                        const int* bins, uint32_t* comp_counts, uint32_t* cov_hist, uint32_t* cov_sums, uint32_t* table_host,
+                                        int flags) {
+    if (!r || !slots) return lrb_set_error(LRB_EINVAL, "lrb_profile_host_samples: null argument");
+    int rc = check_sample_slots(n, slots, bin_sizes, bins, nullptr);   // before the context: no device needed to refuse
+    if (rc) return rc;
+    if (!c) return lrb_set_error(LRB_EINVAL, "lrb_profile_host_samples: null context");
+    rc = profile_host(c, r, k, n, bin_sizes, bins, slots, comp_counts, cov_hist, cov_sums, table_host, flags);
+    if (rc && (flags & LRB_PROFILE_ADD_TO_TABLE)) c->table_ready = false;
     return rc;
 }
 
@@ -1085,6 +1132,146 @@ extern "C" int lrb_ctx_table_load(lrb_ctx* c, const char* path) {
     close(fd);
     if (!rc) c->table_ready = true;
     return rc;
+}
+
+// ---- sample slots: compact tables (canonical halves) on every device of the context ----------------------------------
+namespace {
+
+constexpr uint64_t kCanonRows = (uint64_t)kTableEntries >> 16;   // 2^14 rows of 2^16 entries; the first 2^15 of each are canonical
+constexpr size_t kCanonRowBytes = 4u << 15;                       // 128 KiB of a row read, at a stride of 256 KiB
+constexpr size_t kCompactBytes = sizeof(uint32_t) * (size_t)LRB_COMPACT_ENTRIES;
+
+// open a 15mers-counts file after checking its header and its size (reading only canonical rows would not notice a file
+// cut short by less than one row)
+int open_table_file(const char* path, int* fd_out) {
+    const int fd = open(path, O_RDONLY);
+    if (fd < 0) return lrb_set_error(LRB_EIO, "cannot open table file %s", path);
+    uint64_t size = 0;
+    struct stat st;
+    if (pread(fd, &size, sizeof size, 0) != (ssize_t)sizeof size || size != kTableEntries || fstat(fd, &st) != 0 ||
+        (uint64_t)st.st_size != sizeof size + 4ull * kTableEntries) {
+        close(fd);
+        return lrb_set_error(LRB_EFORMAT, "%s is not a 4^15-entry 15mers-counts file (header or size)", path);
+    }
+    *fd_out = fd;
+    return LRB_OK;
+}
+
+// canonical rows [row_lo, row_hi) of the open table file side by side into dst (split over threads like the table load)
+bool read_canonical_rows(int fd, uint64_t row_lo, uint64_t row_hi, char* dst) {
+    return split_io(dst, (size_t)(row_hi - row_lo) * kCanonRowBytes, 0, [&](char* p, size_t len, off_t at) {
+        while (len) {   // `at` is the byte offset in dst; its row and the place inside the row give the file offset
+            const uint64_t row = row_lo + (uint64_t)at / kCanonRowBytes, in_row = (uint64_t)at % kCanonRowBytes;
+            size_t want = std::min<size_t>(len, kCanonRowBytes - in_row);
+            const ssize_t r = pread(fd, p, want, (off_t)(sizeof(uint64_t) + row * 2 * kCanonRowBytes + in_row));
+            if (r <= 0) return false;
+            p += r; len -= (size_t)r; at += r;
+        }
+        return true;
+    });
+}
+
+int check_slot(const lrb_ctx* c, int slot, const char* who) {
+    if (!c) return lrb_set_error(LRB_EINVAL, "%s: null context", who);
+    if (slot < 0 || slot >= LRB_MAX_SAMPLE_TABLES) return lrb_set_error(LRB_EINVAL, "%s: slot must be in [0, %d) (got %d)", who, LRB_MAX_SAMPLE_TABLES, slot);
+    return LRB_OK;
+}
+
+std::vector<lrb_ctx*> ctx_devices(lrb_ctx* c) {
+    std::vector<lrb_ctx*> d{c};
+    for (lrb_ctx* p : c->peers) d.push_back(p);
+    return d;
+}
+
+// the slot's buffer on every device, marked empty until it is filled
+int reserve_slot(lrb_ctx* c, int slot) {
+    for (lrb_ctx* x : ctx_devices(c)) {
+        x->sample_ready[slot] = false;
+        CTX_CUDA(cudaSetDevice(x->device));
+        int rc;
+        if ((rc = x->sample[slot].reserve(kCompactBytes))) return rc;
+    }
+    CTX_CUDA(cudaSetDevice(c->device));
+    return LRB_OK;
+}
+
+// device 0's slot to the other devices (after the work already on device 0's stream), then wait; all slots ready
+int broadcast_slot(lrb_ctx* c, int slot) {
+    CTX_CUDA(cudaSetDevice(c->device));
+    for (lrb_ctx* p : c->peers)
+        CTX_CUDA(cudaMemcpyPeerAsync(p->sample[slot].p, p->device, c->sample[slot].p, c->device, kCompactBytes, c->stream));
+    CTX_CUDA(cudaStreamSynchronize(c->stream));
+    for (lrb_ctx* x : ctx_devices(c)) x->sample_ready[slot] = true;
+    return LRB_OK;
+}
+
+}  // namespace
+
+extern "C" int lrb_table_read_canonical(const char* path, uint32_t row_lo, uint32_t row_hi, uint32_t* compact) {
+    if (!path || !compact) return lrb_set_error(LRB_EINVAL, "lrb_table_read_canonical: null argument");
+    if (row_lo > row_hi || row_hi > kCanonRows)
+        return lrb_set_error(LRB_EINVAL, "lrb_table_read_canonical: rows [%u, %u) outside [0, %llu)", row_lo, row_hi, (unsigned long long)kCanonRows);
+    int fd = -1, rc;
+    if ((rc = open_table_file(path, &fd))) return rc;
+    const bool ok = read_canonical_rows(fd, row_lo, row_hi, (char*)compact);
+    close(fd);
+    return ok ? LRB_OK : lrb_set_error(LRB_EFORMAT, "%s is truncated", path);
+}
+
+extern "C" int lrb_ctx_sample_table_load(lrb_ctx* c, int slot, const char* path) {
+    int rc;
+    if ((rc = check_slot(c, slot, "lrb_ctx_sample_table_load"))) return rc;
+    if (!path) return lrb_set_error(LRB_EINVAL, "lrb_ctx_sample_table_load: null path");
+    int fd = -1;
+    if ((rc = open_table_file(path, &fd))) return rc;
+    if ((rc = reserve_slot(c, slot))) { close(fd); return rc; }
+    // the rows of a 64 MiB staging buffer are read while the other one is on its way to device 0
+    bool pin = false, pin2 = false;
+    char* stage[2] = {(char*)lrb_host_alloc(kTableChunk, &pin), (char*)lrb_host_alloc(kTableChunk, &pin2)};
+    if (!stage[0] || !stage[1]) rc = lrb_set_error(LRB_ENOMEM, "out of memory (staging)");
+    const uint64_t rows_per_chunk = kTableChunk / kCanonRowBytes;
+    cudaEvent_t done[2];
+    cudaEventCreate(&done[0]);
+    cudaEventCreate(&done[1]);
+    bool used[2] = {false, false};
+    int cur = 0;
+    for (uint64_t row = 0; !rc && row < kCanonRows; row += rows_per_chunk, cur ^= 1) {
+        const uint64_t row_hi = std::min(kCanonRows, row + rows_per_chunk);
+        if (used[cur]) cudaEventSynchronize(done[cur]);
+        if (!read_canonical_rows(fd, row, row_hi, stage[cur])) { rc = lrb_set_error(LRB_EFORMAT, "%s is truncated", path); break; }
+        if (cudaMemcpyAsync((char*)c->sample[slot].p + row * kCanonRowBytes, stage[cur], (row_hi - row) * kCanonRowBytes, cudaMemcpyHostToDevice,
+                            c->stream) != cudaSuccess) { rc = lrb_set_error(LRB_ECUDA, "H2D failed"); break; }
+        cudaEventRecord(done[cur], c->stream);
+        used[cur] = true;
+    }
+    if (cudaStreamSynchronize(c->stream) != cudaSuccess && !rc) rc = lrb_set_error(LRB_ECUDA, "H2D failed: %s", cudaGetErrorString(cudaGetLastError()));
+    cudaEventDestroy(done[0]);
+    cudaEventDestroy(done[1]);
+    lrb_host_free(stage[0], pin);
+    lrb_host_free(stage[1], pin2);
+    close(fd);
+    return rc ? rc : broadcast_slot(c, slot);
+}
+
+extern "C" int lrb_ctx_sample_table_keep(lrb_ctx* c, int slot) {
+    int rc;
+    if ((rc = check_slot(c, slot, "lrb_ctx_sample_table_keep"))) return rc;
+    if (!c->table_ready) return lrb_set_error(LRB_EINVAL, "lrb_ctx_sample_table_keep: no table in this context");
+    if ((rc = reserve_slot(c, slot))) return rc;
+    if ((rc = lrb_dev_table_compact((const uint32_t*)c->table.p, (uint32_t*)c->sample[slot].p, c->stream))) return rc;
+    return broadcast_slot(c, slot);
+}
+
+extern "C" int lrb_ctx_sample_table_free(lrb_ctx* c, int slot) {
+    int rc;
+    if ((rc = check_slot(c, slot, "lrb_ctx_sample_table_free"))) return rc;
+    for (lrb_ctx* x : ctx_devices(c)) {
+        CTX_CUDA(cudaSetDevice(x->device));
+        x->sample_ready[slot] = false;
+        x->sample[slot].release();
+    }
+    CTX_CUDA(cudaSetDevice(c->device));
+    return LRB_OK;
 }
 
 extern "C" int lrb_ctx_table_spectrum(lrb_ctx* c, uint32_t max_count, uint64_t* spectrum_host) {
@@ -1351,6 +1538,47 @@ extern "C" int lrb_search_15mers_settings(const char* table_path, const char* re
             rc2 = lrb_append_coverage_txt(out_txts[m], one.data(), sums.data(), nr, bins[m], threads, row0);
             if (!rc2 && out_npys && out_npys[m]) rc2 = lrb_append_coverage_npy(out_npys[m], one.data(), sums.data(), nr, bins[m], threads, row0);
         }
+        return rc2;
+    };
+    if (in.whole) return search(in.whole, 0);
+    if ((rc = each_segment(in, false, search))) return rc;
+    segments_notice(in, 1);
+    return LRB_OK;
+}
+
+extern "C" int lrb_search_15mers_samples(const char* const* table_paths, int n, const long* bin_sizes, const int* bins, const char* reads_path,
+                                         const char* out_txt, const char* out_npy, int threads) {
+    static const char* who = "lrb_search_15mers_samples";
+    if (!table_paths || !reads_path || !out_txt) return lrb_set_error(LRB_EINVAL, "%s: null path", who);
+    // slot of each table: the first entry with the same path string (a table listed twice is loaded once)
+    uint64_t ids[LRB_MAX_SAMPLE_TABLES] = {};
+    int slots[LRB_MAX_SAMPLE_TABLES] = {}, n_slots = 0;
+    for (int t = 0; t < n && t < LRB_MAX_SAMPLE_TABLES; ++t) {
+        if (!table_paths[t]) return lrb_set_error(LRB_EINVAL, "%s: null table path (table %d)", who, t);
+        int j = 0;
+        while (j < t && strcmp(table_paths[j], table_paths[t])) ++j;
+        ids[t] = (uint64_t)j;
+        slots[t] = j == t ? n_slots++ : slots[j];
+    }
+    uint32_t W = 0;
+    int rc = lrb_check_table_settings(who, n, ids, bin_sizes, bins, &W);
+    if (rc) return rc;
+    if (direct_table_path()) return lrb_set_error(LRB_EINVAL, "%s: LRB_TABLE_PATH=direct reads only the full-layout table, not sample slots", who);
+    CtxGuard cg;
+    if ((rc = create_ctx(0, &cg.c))) return rc;
+    for (int t = 0; t < n; ++t)
+        if (ids[t] == (uint64_t)t && (rc = lrb_ctx_sample_table_load(cg.c, slots[t], table_paths[t]))) return rc;
+    if ((rc = truncate_file(out_txt))) return rc;
+    Input in;
+    if ((rc = open_input(reads_path, threads, 4ull * ((uint64_t)W + 1), in))) return rc;
+    // every block of a row is normalised by the same sums (the read's valid windows), so the writers of one table apply at
+    // width W and the line is the n single-table lines joined by one space
+    auto search = [&](const lrb_reads* s, uint64_t row0) -> int {
+        const uint64_t nr = s->n_reads;
+        std::vector<uint32_t> hist((size_t)nr * W + 1), sums(nr + 1);
+        int rc2 = lrb_profile_host_samples(cg.c, s, 0, n, slots, bin_sizes, bins, nullptr, hist.data(), sums.data(), nullptr, 0);
+        if (!rc2) rc2 = lrb_append_coverage_txt(out_txt, hist.data(), sums.data(), nr, (int)W, threads, row0);
+        if (!rc2 && out_npy) rc2 = lrb_append_coverage_npy(out_npy, hist.data(), sums.data(), nr, (int)W, threads, row0);
         return rc2;
     };
     if (in.whole) return search(in.whole, 0);

@@ -65,3 +65,7 @@ uint64_t lrb_segment_budget(uint64_t row_bytes_per_read);
 // n coverage settings (bin_sizes[m], bins[m]) of one search: 1 <= n <= LRB_MAX_COV_SETTINGS, bin_size >= 1, bins in
 // [1, LRB_MAX_BINS], no pair twice, row width W = sum of bins <= LRB_MAX_BINS (into *width).  LRB_EINVAL naming `who`.
 int lrb_check_cov_settings(const char* who, int n, const long* bin_sizes, const int* bins, uint32_t* width);
+
+// The same for n sample tables with one setting each (LRB_MAX_SAMPLE_TABLES at most): ids[t] says which table t is, and only
+// the same (table, bin_size, bins) twice is refused.
+int lrb_check_table_settings(const char* who, int n, const uint64_t* ids, const long* bin_sizes, const int* bins, uint32_t* width);

@@ -270,21 +270,34 @@ extern "C" int lrb_table_read_file(const char* path, uint32_t* table) {
     return LRB_OK;
 }
 
-int lrb_check_cov_settings(const char* who, int n, const long* bin_sizes, const int* bins, uint32_t* width) {
-    if (n < 1 || n > LRB_MAX_COV_SETTINGS) return lrb_set_error(LRB_EINVAL, "%s: the number of settings must be in [1, %d] (got %d)", who, LRB_MAX_COV_SETTINGS, n);
+// ids == nullptr: n settings of one table; else n sample tables, ids[t] telling which table t is (equal ids, same table)
+static int check_settings(const char* who, int n, const uint64_t* ids, const long* bin_sizes, const int* bins, uint32_t* width) {
+    const char* what = ids ? "table" : "setting";
+    const int most = ids ? LRB_MAX_SAMPLE_TABLES : LRB_MAX_COV_SETTINGS;
+    if (n < 1 || n > most) return lrb_set_error(LRB_EINVAL, "%s: the number of %ss must be in [1, %d] (got %d)", who, ids ? "sample table" : "setting", most, n);
     if (!bin_sizes || !bins) return lrb_set_error(LRB_EINVAL, "%s: null bin_sizes / bins", who);
     uint64_t W = 0;
     for (int m = 0; m < n; ++m) {
-        if (bin_sizes[m] < 1) return lrb_set_error(LRB_EINVAL, "%s: bin_size must be >= 1 (setting %d: got %ld)", who, m, bin_sizes[m]);
-        if (bins[m] < 1 || bins[m] > LRB_MAX_BINS) return lrb_set_error(LRB_EINVAL, "%s: bins must be in [1, %d] (setting %d: got %d)", who, LRB_MAX_BINS, m, bins[m]);
+        if (bin_sizes[m] < 1) return lrb_set_error(LRB_EINVAL, "%s: bin_size must be >= 1 (%s %d: got %ld)", who, what, m, bin_sizes[m]);
+        if (bins[m] < 1 || bins[m] > LRB_MAX_BINS) return lrb_set_error(LRB_EINVAL, "%s: bins must be in [1, %d] (%s %d: got %d)", who, LRB_MAX_BINS, what, m, bins[m]);
         for (int j = 0; j < m; ++j)
-            if (bin_sizes[j] == bin_sizes[m] && bins[j] == bins[m])
-                return lrb_set_error(LRB_EINVAL, "%s: setting %d repeats setting %d (bin_size %ld, bins %d)", who, m, j, bin_sizes[m], bins[m]);
+            if (bin_sizes[j] == bin_sizes[m] && bins[j] == bins[m] && (!ids || ids[j] == ids[m]))
+                return lrb_set_error(LRB_EINVAL, "%s: %s %d repeats %s %d (%sbin_size %ld, bins %d)", who, what, m, what, j, ids ? "same table, " : "",
+                                     bin_sizes[m], bins[m]);
         W += (uint64_t)bins[m];
     }
-    if (W > LRB_MAX_BINS) return lrb_set_error(LRB_EINVAL, "%s: the settings' bins add up to %llu, more than %d", who, (unsigned long long)W, LRB_MAX_BINS);
+    if (W > LRB_MAX_BINS) return lrb_set_error(LRB_EINVAL, "%s: the %ss' bins add up to %llu, more than %d", who, what, (unsigned long long)W, LRB_MAX_BINS);
     if (width) *width = (uint32_t)W;
     return LRB_OK;
+}
+
+int lrb_check_cov_settings(const char* who, int n, const long* bin_sizes, const int* bins, uint32_t* width) {
+    return check_settings(who, n, nullptr, bin_sizes, bins, width);
+}
+
+int lrb_check_table_settings(const char* who, int n, const uint64_t* ids, const long* bin_sizes, const int* bins, uint32_t* width) {
+    if (!ids) return lrb_set_error(LRB_EINVAL, "%s: null table ids", who);
+    return check_settings(who, n, ids, bin_sizes, bins, width);
 }
 
 // ---- abundance spectrum of the table (lrb_dev_table_spectrum layout: n_c for c < M, then n_over, sum_over, max) ----

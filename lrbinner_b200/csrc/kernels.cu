@@ -492,6 +492,14 @@ extern "C" int lrb_dev_mirror(uint32_t* table, void* stream) {
     return LRB_OK;
 }
 
+// canonical half of every 2^16-entry row (its first 2^15 entries) side by side: one pitched copy on the copy engines
+extern "C" int lrb_dev_table_compact(const uint32_t* table, uint32_t* compact, void* stream) {
+    if (!table || !compact) return lrb_set_error(LRB_EINVAL, "lrb_dev_table_compact: null argument");
+    LRB_CUDA(cudaMemcpy2DAsync(compact, 4u << 15, table, 4u << 16, 4u << 15, (size_t)(LRB_TABLE_ENTRIES >> 16), cudaMemcpyDeviceToDevice,
+                               (cudaStream_t)stream));
+    return LRB_OK;
+}
+
 // canonical (bit-15-clear) keys below `key` (key <= 2^30): 2^15 per complete 2^16-entry row, then the clear half of its row
 static uint64_t canon_rank(uint64_t key) { return ((key >> 16) << 15) + std::min<uint64_t>(key & 0xFFFFu, 0x8000u); }
 

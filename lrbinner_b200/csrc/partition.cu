@@ -27,6 +27,8 @@
 //                   (read, bin) entries of the warp, RED into hist[read][bin]
 //   k_search_settings  the same walk, the gathered count binned by up to 8 (bin size, bin count) settings into one
 //                   row of their concatenated bins (lrb_dev_partition_search_settings)
+//   k_search_samples  the same walk over compact sample tables, one or two per launch: each table's count binned by
+//                   its own setting into its column block of one row (lrb_dev_partition_search_samples)
 //   k_row_sums      sums[read] = sum of hist[read][*]  (every window lands in exactly one bin of each setting)
 //
 // The stream can be added in several chunks (lrb_dev_partition_add), each with its own regions, so the
@@ -984,22 +986,21 @@ __device__ __forceinline__ uint32_t ldg_hint(const uint32_t* a, uint64_t pol) {
     return v;
 }
 
-// The walk over the entries of one bucket, shared by the single-setting search and the multi-setting one: put(hbase, cnt,
-// act, lane, seek, row) bins the gathered count `cnt` of an entry and adds it to the histogram row row() (relative to
+// The walk over the entries of one bucket, shared by the single-setting search, the multi-setting one and the multi-table
+// one: load(e) gathers what entry e needs from the table(s) (a count, or one count per table); put(hbase, cnt,
+// act, lane, seek, row) bins the gathered `cnt` of an entry and adds it to the histogram row row() (relative to
 // hbase, whose rows are `pitch` words apart) after seek(); both only where act (the lane has an entry).  put is called by
 // every lane of the warp together, so it may use warp-wide primitives.  One launch may cover several buckets (gridDim.y):
 // CTAs are dispatched x-fastest, so the buckets are still worked on one after the other (their slices take turns in L2)
 // but the tail of one overlaps the head of the next.
-template <int U, int HINT, class Put>
+template <int U, class Load, class Put>
 __device__ __forceinline__ void search_keys_body(const uint32_t* __restrict__ ents, const PartMeta* __restrict__ meta, int bucket,
-                                                 int n_chunks, const ChunkList& L, const StepTables& T, uint32_t bucket_base,
-                                                 uint32_t hi_mask2, int shift, const uint32_t* __restrict__ table,
+                                                 int n_chunks, const ChunkList& L, const StepTables& T, int shift,
                                                  uint32_t* __restrict__ hist, uint32_t pitch, uint32_t (*s_bnd)[kTaskRuns + 1],
-                                                 uint32_t (*s_r0)[kTaskRuns], Put put) {
+                                                 uint32_t (*s_r0)[kTaskRuns], Load load, Put put) {
+    using Count = decltype(load(0u));
     const uint32_t lane = threadIdx.x & 31u, wl = threadIdx.x >> 5;
     const uint32_t warp = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, n_warps = (gridDim.x * blockDim.x) >> 5;
-    const uint64_t pol = HINT ? l2_policy_evict_last() : 0ull;
-    auto gather = [&](uint32_t key) { return HINT ? ldg_hint(table + key, pol) : table[key]; };
     const uint32_t* __restrict__ off_row = T.off + (size_t)bucket * T.cap;
     uint32_t* bnd = s_bnd[wl];
     uint32_t* r0 = s_r0[wl];
@@ -1020,7 +1021,7 @@ __device__ __forceinline__ void search_keys_body(const uint32_t* __restrict__ en
         const uint32_t span_beg = bnd[0], span_end = bnd[kTaskRuns];
         uint32_t* __restrict__ hbase = hist + (size_t)rbase * pitch;
         uint32_t cur = 0, nxt = bnd[1], rr = 0;  // run of this lane's current entry, its end, its relative read base
-        auto emit = [&](uint32_t e, uint32_t cnt, uint32_t i, bool act) {
+        auto emit = [&](uint32_t e, const Count& cnt, uint32_t i, bool act) {
             // seek(): move to the run of entry i (active lanes only); row(): then the entry's read, relative to hbase
             auto seek = [&]() { while (i >= nxt) { ++cur; nxt = bnd[cur + 1]; rr = r0[cur]; } };  // runs may be empty; i < bnd[kTaskRuns] bounds cur
             auto row = [&]() { return rr + (e >> rsh); };
@@ -1029,13 +1030,14 @@ __device__ __forceinline__ void search_keys_body(const uint32_t* __restrict__ en
         uint32_t i0 = span_beg;
         constexpr uint32_t kStep = 32u * U;
         if (i0 + kStep <= span_end) {  // full steps: no predicates; the entries of step t+1 are fetched while step t gathers
-            uint32_t e[U], nx[U], cn[U];
+            uint32_t e[U], nx[U];
+            Count cn[U];
             const uint32_t* src = region + i0 + lane;
 #pragma unroll
             for (int u = 0; u < U; ++u) e[u] = __ldcs(src + 32 * u);
             for (;;) {
 #pragma unroll
-                for (int u = 0; u < U; ++u) cn[u] = gather(entry_key(e[u], bucket_base, hi_mask2));
+                for (int u = 0; u < U; ++u) cn[u] = load(e[u]);
                 const bool more = i0 + 2u * kStep <= span_end;  // warp-uniform
                 if (more) {
                     const uint32_t* nsrc = region + i0 + kStep + lane;
@@ -1053,15 +1055,15 @@ __device__ __forceinline__ void search_keys_body(const uint32_t* __restrict__ en
         for (; i0 + 128u <= span_end; i0 += 128u) {  // (U > 4) full 128-entry steps that are left
             const uint32_t* src = region + i0 + lane;
             const uint32_t e0 = __ldcs(src), e1 = __ldcs(src + 32), e2 = __ldcs(src + 64), e3 = __ldcs(src + 96);
-            const uint32_t c0 = gather(entry_key(e0, bucket_base, hi_mask2)), c1 = gather(entry_key(e1, bucket_base, hi_mask2)),
-                           c2 = gather(entry_key(e2, bucket_base, hi_mask2)), c3 = gather(entry_key(e3, bucket_base, hi_mask2));
+            const Count c0 = load(e0), c1 = load(e1), c2 = load(e2), c3 = load(e3);
             emit(e0, c0, i0 + lane, true);
             emit(e1, c1, i0 + lane + 32u, true);
             emit(e2, c2, i0 + lane + 64u, true);
             emit(e3, c3, i0 + lane + 96u, true);
         }
         if (i0 < span_end) {  // tail of the span
-            uint32_t e[4], cnt[4];
+            uint32_t e[4];
+            Count cnt[4];
             bool act[4];
 #pragma unroll
             for (int u = 0; u < 4; ++u) {
@@ -1070,7 +1072,7 @@ __device__ __forceinline__ void search_keys_body(const uint32_t* __restrict__ en
                 e[u] = act[u] ? __ldcs(region + i) : 0u;
             }
 #pragma unroll
-            for (int u = 0; u < 4; ++u) cnt[u] = act[u] ? gather(entry_key(e[u], bucket_base, hi_mask2)) : 0u;
+            for (int u = 0; u < 4; ++u) cnt[u] = act[u] ? load(e[u]) : Count{};
 #pragma unroll
             for (int u = 0; u < 4; ++u) {
                 if (i0 + 32u * u >= span_end) break;  // warp-uniform
@@ -1078,6 +1080,16 @@ __device__ __forceinline__ void search_keys_body(const uint32_t* __restrict__ en
             }
         }
     }
+}
+
+// load functor of the walk for the full-layout table: the count of the entry's key (HINT = 1: gathers marked evict_last)
+template <int HINT>
+__device__ __forceinline__ auto table_load(const uint32_t* __restrict__ table, uint32_t bucket_base, uint32_t hi_mask2) {
+    const uint64_t pol = HINT ? l2_policy_evict_last() : 0ull;
+    return [=](uint32_t e) {
+        const uint32_t key = entry_key(e, bucket_base, hi_mask2);
+        return HINT ? ldg_hint(table + key, pol) : table[key];
+    };
 }
 
 // hist[read][bin(table[key])] += 1 for one (bin size, bin count): rows of B bins
@@ -1098,7 +1110,7 @@ k_search_keys(const uint32_t* __restrict__ ents, const PartMeta* __restrict__ me
         for (uint32_t i = threadIdx.x; i <= lut_top; i += blockDim.x) s_lut[i] = (uint16_t)coverage_bin(i, S32, magic, B);
         __syncthreads();
     }
-    search_keys_body<U, HINT>(ents, meta, bucket, n_chunks, L, T, bucket_base, hi_mask2, shift, table, hist, B, s_bnd, s_r0,
+    search_keys_body<U>(ents, meta, bucket, n_chunks, L, T, shift, hist, B, s_bnd, s_r0, table_load<HINT>(table, bucket_base, hi_mask2),
                               [&](uint32_t* hbase, uint32_t cnt, bool act, uint32_t lane, auto seek, auto row) {
                                   uint32_t cell = 0xFFFFFFFFu;
                                   if (act) {
@@ -1130,7 +1142,7 @@ k_search_settings(const uint32_t* __restrict__ ents, const PartMeta* __restrict_
     __shared__ uint32_t s_bnd[8][kTaskRuns + 1];
     __shared__ uint32_t s_r0[8][kTaskRuns];
     if (meta->overflow) return;
-    search_keys_body<U, 0>(ents, meta, bucket, n_chunks, L, T, bucket_base, hi_mask2, shift, table, hist, C.W, s_bnd, s_r0,
+    search_keys_body<U>(ents, meta, bucket, n_chunks, L, T, shift, hist, C.W, s_bnd, s_r0, table_load<0>(table, bucket_base, hi_mask2),
                            [&](uint32_t* hbase, uint32_t cnt, bool act, uint32_t lane, auto seek, auto row) {
                                uint32_t base = 0;
                                if (act) {
@@ -1144,6 +1156,65 @@ k_search_settings(const uint32_t* __restrict__ ents, const PartMeta* __restrict_
                                    if (act && (uint32_t)__ffs(peers) - 1u == lane) atomicAdd(hbase + cell, (uint32_t)__popc(peers));
                                }
                            });
+}
+
+// Several sample tables in one walk over the lists.  A sample table is held compact (lrb_dev_table_compact): only its
+// bit-15-clear keys, entry i = T[((i >> 15) << 16) | (i & 0x7FFF)].  A list entry keeps its key inside the bucket with bit
+// 15 dropped in its low shift - 1 bits, so the entry's compact index is (bucket_base >> 1) | (e & (2^(shift-1) - 1)) and a
+// bucket's slice of a compact table is one contiguous 2^(shift-1)-entry range.  k_search_samples gathers each entry's
+// count from the G tables of a group and bins it with that table's setting into that table's column block, one
+// __match_any_sync and aggregated REDs per block as k_search_settings does per setting.  The host runs one walk per group.
+struct SampleGroup {
+    const uint32_t* table[2];  // compact tables of the group
+    uint64_t magic[2];
+    uint32_t S32[2], B[2], off[2];
+    uint32_t W;                // row pitch: the bins of every table of the call
+};
+
+// Tables per walk: one.  Two compact slices of a 2^24-key bucket (64 MiB) would fit the 126 MB L2 beside the list stream
+// and the histogram lines, and fusing them saves one read of the lists per pair; measured on config #2 it is 1.28-1.30x
+// slower than one walk per table for 2, 4 and 8 tables (profiles/r06_samples_bench.jsonl, DESIGN.md section 4).
+constexpr int kSampleGroup = 1;
+
+template <int G>
+struct SampleCounts {
+    uint32_t c[G];
+};
+
+template <int U, int G>
+__global__ void __launch_bounds__(256)
+k_search_samples(const uint32_t* __restrict__ ents, const PartMeta* __restrict__ meta, int bucket0, int n_chunks, ChunkList L,
+                 StepTables T, uint32_t cbase0, int shift, const __grid_constant__ SampleGroup S, uint32_t* __restrict__ hist) {
+    const int bucket = bucket0 + (int)blockIdx.y;
+    const uint32_t cbase = cbase0 + ((uint32_t)blockIdx.y << (shift - 1));
+    const uint32_t emask = (1u << (shift - 1)) - 1u;
+    __shared__ uint32_t s_bnd[8][kTaskRuns + 1];
+    __shared__ uint32_t s_r0[8][kTaskRuns];
+    if (meta->overflow) return;
+    const uint32_t* slice[G];  // the bucket's slice of each table
+#pragma unroll
+    for (int g = 0; g < G; ++g) slice[g] = S.table[g] + cbase;
+    search_keys_body<U>(ents, meta, bucket, n_chunks, L, T, shift, hist, S.W, s_bnd, s_r0,
+                        [&](uint32_t e) {
+                            SampleCounts<G> r;
+#pragma unroll
+                            for (int g = 0; g < G; ++g) r.c[g] = __ldg(slice[g] + (e & emask));
+                            return r;
+                        },
+                        [&](uint32_t* hbase, const SampleCounts<G>& cnt, bool act, uint32_t lane, auto seek, auto row) {
+                            uint32_t base = 0;
+                            if (act) {
+                                seek();
+                                base = row() * S.W;
+                            }
+#pragma unroll
+                            for (int g = 0; g < G; ++g) {
+                                uint32_t cell = 0xFFFFFFFFu;
+                                if (act) cell = base + S.off[g] + coverage_bin(cnt.c[g], S.S32[g], S.magic[g], S.B[g]);
+                                const uint32_t peers = __match_any_sync(0xFFFFFFFFu, cell);
+                                if (act && (uint32_t)__ffs(peers) - 1u == lane) atomicAdd(hbase + cell, (uint32_t)__popc(peers));
+                            }
+                        });
 }
 
 // sums[r] = number of windows of read r that were bucketed so far = sum of the B bins that start its histogram row (every
@@ -1518,4 +1589,68 @@ extern "C" int lrb_dev_partition_search_settings(const lrb_partition* part, int 
         LRB_LAUNCH("k_row_sums", st, k_row_sums<<<(unsigned)((part->n_reads + 255) / 256), 256, 0, st>>>(hist, sums, part->n_reads, (uint32_t)bins[0], W));
     LRB_CUDA(cudaGetLastError());
     return LRB_OK;
+}
+
+// Several compact sample tables in one search (k_search_samples): hist rows of W = sum of bins[t] words, table t's bins at
+// column sum_{j<t} bins[j]; one walk over the lists per group of `group` tables; sums are rewritten by the call that
+// includes the last bucket.
+extern "C" int lrb_dev_partition_search_samples_grouped(const lrb_partition* part, int bucket_lo, int bucket_hi,
+                                                        const uint32_t* const* compact_tables, int n, const long* bin_sizes,
+                                                        const int* bins, uint32_t* hist, uint32_t* sums, int group, void* stream) {
+    static const char* who = "lrb_dev_partition_search_samples";
+    if (!part || !compact_tables || !hist || !sums) return lrb_set_error(LRB_EINVAL, "%s: null argument", who);
+    if (group < 0 || group > 2) return lrb_set_error(LRB_EINVAL, "%s: group must be 0 (the default), 1 or 2 (got %d)", who, group);
+    if (group == 0) group = kSampleGroup;
+    uint64_t ids[LRB_MAX_SAMPLE_TABLES] = {};
+    for (int t = 0; t < n && t < LRB_MAX_SAMPLE_TABLES; ++t) {
+        if (!compact_tables[t]) return lrb_set_error(LRB_EINVAL, "%s: null table %d", who, t);
+        ids[t] = (uint64_t)(uintptr_t)compact_tables[t];
+    }
+    uint32_t W = 0;
+    const int rc = lrb_check_table_settings(who, n, ids, bin_sizes, bins, &W);
+    if (rc) return rc;
+    if (!part->has_rids) return lrb_set_error(LRB_EINVAL, "%s: partition was built without read ids", who);
+    if (part->key_lo & ((1u << part->shift) - 1u))
+        return lrb_set_error(LRB_EINVAL, "%s: the partition's key range must start at a bucket boundary (key_lo %u)", who, part->key_lo);
+    if (bucket_lo < 0) bucket_lo = 0;
+    if (bucket_hi > part->n_buckets) bucket_hi = part->n_buckets;
+    if (part->n_chunks == 0) return LRB_OK;
+    cudaStream_t st = (cudaStream_t)stream;
+    const PartMeta* meta = reinterpret_cast<const PartMeta*>(part->small);
+    const ChunkList L = chunk_list(part);
+    const StepTables T = step_tables(part->steps, part->step_capacity);
+    const int shift = part->shift;
+    const uint32_t cbase0 = (part->key_lo + ((uint32_t)bucket_lo << shift)) >> 1;
+    if (bucket_hi > bucket_lo) {
+        const dim3 gs(search_grid(L, part->n_chunks), (unsigned)(bucket_hi - bucket_lo));
+        for (int t0 = 0, off = 0; t0 < n;) {
+            const int g = std::min(group, n - t0);
+            SampleGroup S = {};
+            S.W = W;
+            for (int j = 0; j < g; ++j) {
+                S.table[j] = compact_tables[t0 + j];
+                S.S32[j] = bin_sizes[t0 + j] > 0xFFFFFFFFl ? 0xFFFFFFFFu : (uint32_t)bin_sizes[t0 + j];
+                S.magic[j] = coverage_magic(S.S32[j]);
+                S.B[j] = (uint32_t)bins[t0 + j];
+                S.off[j] = (uint32_t)off;
+                off += bins[t0 + j];
+            }
+            if (g == 2)
+                LRB_LAUNCH("k_search_samples", st, k_search_samples<8, 2><<<gs, 256, 0, st>>>(part->keys, meta, bucket_lo, part->n_chunks, L, T,
+                                                                                             cbase0, shift, S, hist));
+            else
+                LRB_LAUNCH("k_search_samples", st, k_search_samples<8, 1><<<gs, 256, 0, st>>>(part->keys, meta, bucket_lo, part->n_chunks, L, T,
+                                                                                             cbase0, shift, S, hist));
+            t0 += g;
+        }
+    }
+    if (part->n_reads && bucket_hi == part->n_buckets)
+        LRB_LAUNCH("k_row_sums", st, k_row_sums<<<(unsigned)((part->n_reads + 255) / 256), 256, 0, st>>>(hist, sums, part->n_reads, (uint32_t)bins[0], W));
+    LRB_CUDA(cudaGetLastError());
+    return LRB_OK;
+}
+
+extern "C" int lrb_dev_partition_search_samples(const lrb_partition* part, int bucket_lo, int bucket_hi, const uint32_t* const* compact_tables,
+                                                int n, const long* bin_sizes, const int* bins, uint32_t* hist, uint32_t* sums, void* stream) {
+    return lrb_dev_partition_search_samples_grouped(part, bucket_lo, bucket_hi, compact_tables, n, bin_sizes, bins, hist, sums, 0, stream);
 }

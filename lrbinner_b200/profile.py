@@ -11,6 +11,7 @@
 The arithmetic lives in the CUDA kernels; nothing here computes profiles on the CPU.
 """
 import ctypes as C
+import os
 
 import numpy as np
 
@@ -191,19 +192,29 @@ class Context:
         self.device = device
 
     def profile(self, reads, k=None, bin_size=None, bins=None, want_table=False, use_loaded_table=False, out=None,
-                keep_table=False, add_to_table=False, coverage=None):
+                keep_table=False, add_to_table=False, coverage=None, samples=None):
         """Returns dict(comp=[N,P] u32, hist=[N,bins] u32, sums=[N] u32, table=[2^30] u32) for the requested parts.
         `out` may carry preallocated (ideally page-locked) arrays under the same keys.  add_to_table: count these reads
         INTO the context's complete table (from an earlier count or table_load) instead of from zero; on failure the
         context holds no table.
         coverage=[(bin_size, bins), ...] (instead of bin_size / bins): up to 8 settings searched in one pass over the table
         (lrb_profile_host_settings).  hist is then [N, W], W = the sum of the bins, with each setting's columns after those of
-        the settings before it; hists[m] is the [N, bins_m] view of setting m, and sums are the same for every setting."""
+        the settings before it; hists[m] is the [N, bins_m] view of setting m, and sums are the same for every setting.
+        samples=[(slot, bin_size, bins), ...] (instead of coverage / bin_size / bins): coverage against up to 8 sample slots
+        (sample_table_load / sample_table_keep) instead of the context's table (lrb_profile_host_samples); hist [N, W] holds
+        table 0's bins, then table 1's, ..., hists[t] is table t's view and sums are shared."""
         if coverage is not None and (bin_size is not None or bins is not None):
             raise _lib.LrbError(_lib.LRB_EINVAL, "coverage=[(bin_size, bins), ...] replaces bin_size / bins: give one or the other")
+        if samples is not None and (coverage is not None or bin_size is not None or bins is not None):
+            raise _lib.LrbError(_lib.LRB_EINVAL, "samples=[(slot, bin_size, bins), ...] replaces coverage / bin_size / bins: give one or the other")
         n = reads.n_reads
         out = dict(out or {})
         comp = hist = sums = table = hists = None
+        slots = None
+        if samples is not None:
+            samples = [(int(t), int(s_), int(b)) for t, s_, b in samples]
+            slots = np.array([t for t, _, _ in samples], dtype=np.int32)
+            coverage = [(s_, b) for _, s_, b in samples]
         set_bs, set_bins = _settings_arrays(coverage if coverage is not None else
                                             [(bin_size if bin_size is not None else 1, bins if bins is not None else 1)])
         if k is not None:
@@ -222,13 +233,16 @@ class Context:
             table = out.get("table")
             if table is None:
                 table = np.empty(_lib.TABLE_ENTRIES, dtype=np.uint32)
-        check(lib.lrb_profile_host_settings(self._h, reads._h, int(k) if k is not None else 0, len(set_bs), _ptr(set_bs),
-                                            _ptr(set_bins), _ptr(comp) if comp is not None else None,
-                                            _ptr(hist) if hist is not None else None, _ptr(sums) if sums is not None else None,
-                                            _ptr(table) if table is not None else None,
-                                            (_lib.PROFILE_USE_LOADED_TABLE if use_loaded_table else 0) |
-                                            (_lib.PROFILE_KEEP_TABLE if keep_table else 0) |
-                                            (_lib.PROFILE_ADD_TO_TABLE if add_to_table else 0)))
+        flags = ((_lib.PROFILE_USE_LOADED_TABLE if use_loaded_table else 0) | (_lib.PROFILE_KEEP_TABLE if keep_table else 0) |
+                 (_lib.PROFILE_ADD_TO_TABLE if add_to_table else 0))
+        parts = (_ptr(comp) if comp is not None else None, _ptr(hist) if hist is not None else None,
+                 _ptr(sums) if sums is not None else None, _ptr(table) if table is not None else None)
+        if slots is not None:
+            check(lib.lrb_profile_host_samples(self._h, reads._h, int(k) if k is not None else 0, len(set_bs), _ptr(slots),
+                                               _ptr(set_bs), _ptr(set_bins), *parts, flags))
+        else:
+            check(lib.lrb_profile_host_settings(self._h, reads._h, int(k) if k is not None else 0, len(set_bs), _ptr(set_bs),
+                                                _ptr(set_bins), *parts, flags))
         if coverage is not None:
             offs = np.concatenate([[0], np.cumsum(set_bins)])
             hists = [hist[:, offs[m]:offs[m + 1]] for m in range(len(set_bins))]
@@ -252,6 +266,17 @@ class Context:
 
     def table_save(self, path):
         check(lib.lrb_ctx_table_save(self._h, str(path).encode()))
+
+    def sample_table_load(self, slot, path):
+        """Load the canonical rows of a 15mers-counts file into sample slot `slot` on every device (2 GiB each)."""
+        check(lib.lrb_ctx_sample_table_load(self._h, int(slot), os.fsencode(path)))
+
+    def sample_table_keep(self, slot):
+        """Copy the context's own complete table, in compact form, into sample slot `slot` on every device."""
+        check(lib.lrb_ctx_sample_table_keep(self._h, int(slot)))
+
+    def sample_table_free(self, slot):
+        check(lib.lrb_ctx_sample_table_free(self._h, int(slot)))
 
     def table_spectrum(self, max_count=65536):
         """Abundance spectrum of the context's table: u64[max_count + 3] = n_c for c < max_count (canonical 15-mers
@@ -482,6 +507,32 @@ class PartitionWorkspace:
         check(lib.lrb_dev_partition_search_settings(C.byref(self.part), bucket_lo, 64 if bucket_hi is None else bucket_hi,
                                                     C.c_void_p(table.data_ptr()), len(bs), _ptr(bs), _ptr(bc),
                                                     C.c_void_p(hist.data_ptr()), C.c_void_p(sums.data_ptr()), _stream()))
+
+    def search_samples(self, tables, settings, hist, sums, bucket_lo=0, bucket_hi=None, group=0):
+        """Search against several compact sample tables (dev_table_compact) at once (lrb_dev_partition_search_samples):
+        tables[t] is binned with settings[t] = (bin_size, bins) into its column block of hist [N, W]; hist and sums zeroed
+        by the caller as for apply(search=True).  group: tables per walk over the lists (0: the library's choice)."""
+        bs, bc = _settings_arrays(settings)
+        ptrs = (C.c_void_p * max(len(tables), 1))(*[t.data_ptr() for t in tables])
+        check(lib.lrb_dev_partition_search_samples_grouped(C.byref(self.part), bucket_lo, 64 if bucket_hi is None else bucket_hi,
+                                                           ptrs, len(tables), _ptr(bs), _ptr(bc), C.c_void_p(hist.data_ptr()),
+                                                           C.c_void_p(sums.data_ptr()), int(group), _stream()))
+
+
+def dev_table_compact(table, out=None):
+    """Compact form of a full-layout table (a 2^30-entry device tensor): its canonical rows, 2^29 entries
+    (lrb_dev_table_compact).  Returns `out` (allocated on the table's device when None)."""
+    if out is None:
+        out = table.new_empty(_lib.COMPACT_ENTRIES)
+    check(lib.lrb_dev_table_compact(C.c_void_p(table.data_ptr()), C.c_void_p(out.data_ptr()), _stream()))
+    return out
+
+
+def read_table_canonical(path, row_lo=0, row_hi=_lib.TABLE_ENTRIES >> 16):
+    """Canonical rows [row_lo, row_hi) of a 15mers-counts file as u32[(row_hi - row_lo) * 2^15] (host; no device)."""
+    out = np.empty((int(row_hi) - int(row_lo)) << 15, dtype=np.uint32)
+    check(lib.lrb_table_read_canonical(os.fsencode(path), int(row_lo), int(row_hi), _ptr(out)))
+    return out
 
 
 def _settings_arrays(settings):

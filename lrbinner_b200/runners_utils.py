@@ -72,6 +72,26 @@ def run_15mer_vecs_settings(reads_path, output, settings, threads, write_npy=Fal
     check_proc(o, "Counting 15-mer profiles for several settings")
 
 
+def run_15mer_vecs_samples(reads_path, output, table_paths, bin_size, bin_count, threads, write_npy=False):
+    """Differential coverage: the reads against several 15mers-counts tables (typically other samples'
+    {out}/profiles/15mers-counts) in one call (lrb_search_15mers_samples): each table is loaded once and the reads are
+    parsed once.  Writes {output}/profiles/cov_profs_samples (and .npy with write_npy): per read, table 0's -bc values, then
+    table 1's, ..., each block byte for byte the cov_profs line run_15mer_vecs writes against that table.  One (bin_size,
+    bin_count) for every table, as LRBinner has one -bs / -bc.  cov_profs itself is never touched (INTEGRATION.md).  No
+    reference counterpart."""
+    if not os.path.isdir(f"{output}/profiles"):
+        os.makedirs(f"{output}/profiles")
+    n = len(table_paths)
+    out = f"{output}/profiles/cov_profs_samples"
+    paths = (C.c_char_p * max(n, 1))(*[os.fsencode(p) for p in table_paths])
+    bs = (C.c_long * max(n, 1))(*[int(bin_size)] * n)
+    bc = (C.c_int * max(n, 1))(*[int(bin_count)] * n)
+    logger.debug(f"LIB::lrb_search_15mers_samples {list(table_paths)} \"{reads_path}\" \"{out}\" {bin_size} {bin_count} {threads}")
+    o = _lib.lib.lrb_search_15mers_samples(paths, n, bs, bc, os.fsencode(reads_path), os.fsencode(out),
+                                           os.fsencode(out + ".npy") if write_npy else None, int(threads))
+    check_proc(o, "Counting 15-mer profiles against several samples")
+
+
 def run_15mer_histo(output, threads, max_count=65536):
     """Abundance spectrum of {output}/profiles/15mers-counts as {output}/profiles/15mers-histo (jellyfish `histo`
     layout: "count n_kmers" lines of canonical 15-mers), to choose -bs / -bc from (INTEGRATION.md).  No reference
