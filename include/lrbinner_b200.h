@@ -256,16 +256,11 @@ int lrb_dev_partition_search_settings(const lrb_partition* part, int bucket_lo, 
  * single-table search with that table's full layout, for every table that is symmetric (T[x] == T[revcomp x], as every
  * counted table is): like every partitioned search, only the bit-15-clear member of each {x, revcomp x} pair is read.
  * sums[r] (the read's valid windows, the same for every table) is rewritten by the call that includes the last bucket.
- * One walk over the lists per group of tables (the group size is measured, DESIGN.md section 4).  LRB_EINVAL unless
- * 1 <= n <= LRB_MAX_SAMPLE_TABLES, every bin_size >= 1, every bins in [1, LRB_MAX_BINS], W <= LRB_MAX_BINS, no
- * (table pointer, bin_size, bins) repeats, the partition has read ids and starts at a bucket boundary. */
+ * One walk over the lists per table.  LRB_EINVAL unless 1 <= n <= LRB_MAX_SAMPLE_TABLES, every bin_size >= 1, every
+ * bins in [1, LRB_MAX_BINS], W <= LRB_MAX_BINS, no (table pointer, bin_size, bins) repeats, the partition has read ids
+ * and starts at a bucket boundary. */
 int lrb_dev_partition_search_samples(const lrb_partition* part, int bucket_lo, int bucket_hi, const uint32_t* const* compact_tables,
                                      int n, const long* bin_sizes, const int* bins, uint32_t* hist, uint32_t* sums, void* stream);
-/* The same with the group size given: 1 (one walk per table) or 2 (two tables per walk); 0 is the default of
- * lrb_dev_partition_search_samples.  For measuring the two against each other. */
-int lrb_dev_partition_search_samples_grouped(const lrb_partition* part, int bucket_lo, int bucket_hi,
-                                             const uint32_t* const* compact_tables, int n, const long* bin_sizes, const int* bins,
-                                             uint32_t* hist, uint32_t* sums, int group, void* stream);
 
 /* Pack ASCII on the device: bases[] (device, concatenated) -> codes/valid of `dev` (layout prebuilt). */
 int lrb_dev_pack_ascii(const lrb_reads_view* dev, const char* bases, const uint64_t* offsets, void* stream);
@@ -338,8 +333,7 @@ int lrb_profile_host(lrb_ctx* ctx, const lrb_reads* reads, int k, long bin_size,
  * W = sum of bins[m], holds for every read setting 0's bins, then setting 1's, ...; cov_sums[N] is shared by all settings.
  * Every flag and part of lrb_profile_host works alongside (composition, count, KEEP / ADD_TO / USE_LOADED_TABLE, batches,
  * several devices); lrb_profile_host is its n = 1 case.  The settings are checked as in lrb_dev_partition_search_settings
- * when coverage is asked for, before any device work; n > 1 under LRB_TABLE_PATH=direct is refused (LRB_EINVAL).  The
- * experiment switches LRB_SEARCH_LUT and LRB_SEARCH_HINT act on single-setting calls only. */
+ * when coverage is asked for, before any device work; n > 1 under LRB_TABLE_PATH=direct is refused (LRB_EINVAL). */
 int lrb_profile_host_settings(lrb_ctx* ctx, const lrb_reads* reads, int k, int n, const long* bin_sizes, const int* bins,
                               uint32_t* comp_counts, uint32_t* cov_hist, uint32_t* cov_sums, uint32_t* table_host, int flags);
 /* Sample slots: a context holds up to LRB_MAX_SAMPLE_TABLES sample tables beside its own table, each in compact form

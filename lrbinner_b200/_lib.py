@@ -106,7 +106,6 @@ _SIG = {
     "lrb_dev_partition_apply_range": (C.c_int, [_P, C.c_int, C.c_int, C.c_int, _P, C.c_long, C.c_int, _P, _P, _P]),
     "lrb_dev_partition_search_settings": (C.c_int, [_P, C.c_int, C.c_int, _P, C.c_int, _P, _P, _P, _P, _P]),
     "lrb_dev_partition_search_samples": (C.c_int, [_P, C.c_int, C.c_int, _P, C.c_int, _P, _P, _P, _P, _P]),
-    "lrb_dev_partition_search_samples_grouped": (C.c_int, [_P, C.c_int, C.c_int, _P, C.c_int, _P, _P, _P, _P, C.c_int, _P]),
     "lrb_dev_table_compact": (C.c_int, [_P, _P, _P]),
     "lrb_dev_pack_ascii": (C.c_int, [C.POINTER(ReadsView), _P, _P, _P]),
     "lrb_dev_format_composition": (C.c_int, [_P, _P, C.c_uint64, C.c_int, _P, _P]),

@@ -88,7 +88,6 @@ struct lrb_ctx {
     cudaEvent_t ev[8] = {};
     cudaEvent_t sync_ev[LRB_PART_MAX_CHUNKS + 2] = {};  // [0] index arrays, [1..] H2D chunks, [last] composition D2H
     cudaEvent_t counted = nullptr;                       // this device's private counts are complete
-    cudaEvent_t mirrored = nullptr;                      // the mirror pass (on the exchange stream, beside the search) is done
     cudaEvent_t sum_ev[kMaxRounds] = {}, round_ev[kMaxRounds] = {};  // exchange: my piece of round k is summed / round k has arrived here
     cudaEvent_t xev[2] = {};                             // exchange start / end (timed)
     DevBuf codes, valid, read_len, read_blk, tile_read, tile_blk;
@@ -120,11 +119,10 @@ struct lrb_ctx {
 
 // The exchange stream runs at the highest priority: its small kernels (lrb_dev_add_planes, the mirror) then get SM slots
 // ahead of the queued CTAs of the search they hide behind, instead of being stretched over the whole search
-// (measured at N = 2: k_add_planes 2.2 ms per 16 MiB piece at default priority).  LRB_XCHG_PRIO=0 turns it off.
+// (measured at N = 2: k_add_planes 2.2 ms per 16 MiB piece at default priority).
 static cudaError_t create_xchg_stream(cudaStream_t* s) {
     int lo = 0, hi = 0;
-    const char* e = getenv("LRB_XCHG_PRIO");
-    if ((e && atoi(e) == 0) || cudaDeviceGetStreamPriorityRange(&lo, &hi) != cudaSuccess) return cudaStreamCreateWithFlags(s, cudaStreamNonBlocking);
+    if (cudaDeviceGetStreamPriorityRange(&lo, &hi) != cudaSuccess) return cudaStreamCreateWithFlags(s, cudaStreamNonBlocking);
     return cudaStreamCreateWithPriority(s, cudaStreamNonBlocking, hi);
 }
 
@@ -144,7 +142,6 @@ static int ctx_create_one(int device, lrb_ctx** out) {
     for (auto& ev : c->xev) cudaEventCreate(&ev);
     for (auto& ev : c->sync_ev) cudaEventCreateWithFlags(&ev, cudaEventDisableTiming);
     cudaEventCreateWithFlags(&c->counted, cudaEventDisableTiming);
-    cudaEventCreateWithFlags(&c->mirrored, cudaEventDisableTiming);
     for (auto& ev : c->sum_ev) cudaEventCreateWithFlags(&ev, cudaEventDisableTiming);
     for (auto& ev : c->round_ev) cudaEventCreateWithFlags(&ev, cudaEventDisableTiming);
     *out = c;
@@ -214,7 +211,6 @@ extern "C" void lrb_ctx_destroy(lrb_ctx* c) {
     for (auto& ev : c->sum_ev) if (ev) cudaEventDestroy(ev);
     for (auto& ev : c->round_ev) if (ev) cudaEventDestroy(ev);
     if (c->counted) cudaEventDestroy(c->counted);
-    if (c->mirrored) cudaEventDestroy(c->mirrored);
     if (c->copy_in) cudaStreamDestroy(c->copy_in);
     if (c->copy_out) cudaStreamDestroy(c->copy_out);
     if (c->xchg) cudaStreamDestroy(c->xchg);
@@ -252,7 +248,7 @@ struct Job {
     uint32_t *comp = nullptr, *hist = nullptr, *sums = nullptr, *table_host = nullptr;
     bool do_comp = false, do_search = false, do_count = false, use_loaded = false, add_to_table = false;
     bool use_part = true, want_smem_env = false, force_l2 = false, comp_pinned = false;
-    int bucket_shift = 24, h2d_chunks = 16;
+    int bucket_shift = 24;
     bool force_ship_valid = false;
 };
 
@@ -422,7 +418,7 @@ int stage_front(lrb_ctx* c, const lrb_reads* r, const Job& J, uint64_t row0, boo
         cudaGetLastError();
         if ((rc = reserve_batch(c, r, J, J.do_count))) return rc;
     }
-    const ChunkPlan ch = plan_chunks(r, J.h2d_chunks);
+    const ChunkPlan ch = plan_chunks(r, 16);
     if (timed) CTX_CUDA(cudaEventRecord(c->ev[0], st));
     else CTX_CUDA(cudaEventRecord(c->sync_ev[LRB_PART_MAX_CHUNKS + 1], st));
     CTX_CUDA(cudaStreamWaitEvent(sin, timed ? c->ev[0] : c->sync_ev[LRB_PART_MAX_CHUNKS + 1], 0));   // earlier work is done with the buffers
@@ -434,12 +430,9 @@ int stage_front(lrb_ctx* c, const lrb_reads* r, const Job& J, uint64_t row0, boo
     // compute stream: zero the outputs while the first chunk is in flight.  The table is zeroed only when counts will be
     // ADDED to it (several batches, or no lists): a device's only batch WRITES its table slices (apply mode bit 3).
     const bool count_writes = J.do_count && lists && only_batch && !add_into_table;
-    // experiment (LRB_COMP_BESIDE=1): the composition does not ride along with the chunks but runs on the copy_out stream
-    // beside the search, once the count is enqueued (it needs nothing but the packed stream)
-    const bool comp_beside = J.do_comp && n && only_batch && lists && J.do_count && J.do_search && env_int("LRB_COMP_BESIDE", 0) > 0;
     if (J.do_count && first_batch && !count_writes && !add_into_table)
         CTX_CUDA(cudaMemsetAsync(c->table.p, 0, sizeof(uint32_t) * (size_t)kTableEntries, st));
-    if (J.do_comp && n && !comp_beside) CTX_CUDA(cudaMemsetAsync(c->comp.p, 0, sizeof(uint32_t) * n * J.P, st));
+    if (J.do_comp && n) CTX_CUDA(cudaMemsetAsync(c->comp.p, 0, sizeof(uint32_t) * n * J.P, st));
     CTX_CUDA(cudaStreamWaitEvent(st, c->sync_ev[0], 0));  // index arrays (and validity exceptions) are on the device
     if (!ship_valid && (rc = lrb_dev_fill_valid(&v, (const uint32_t*)c->exc_blk.p, (const uint32_t*)c->exc_valid.p, r->n_exc, st))) return rc;
     if (lists) {
@@ -448,7 +441,7 @@ int stage_front(lrb_ctx* c, const lrb_reads* r, const Job& J, uint64_t row0, boo
     }
     for (int i = 0; i < ch.n; ++i) {
         CTX_CUDA(cudaStreamWaitEvent(st, c->sync_ev[1 + i], 0));
-        if (J.do_comp && n && !comp_beside && (rc = lrb_dev_composition(&v, J.k, (uint32_t*)c->comp.p, ch.ct[i], ch.ct[i + 1], st))) return rc;
+        if (J.do_comp && n && (rc = lrb_dev_composition(&v, J.k, (uint32_t*)c->comp.p, ch.ct[i], ch.ct[i + 1], st))) return rc;
         if (lists) {
             if ((rc = lrb_dev_partition_add(&v, (const uint32_t*)c->blk_read.p, ch.cb[i], ch.cb[i + 1], &c->part, st))) return rc;
         } else if (J.do_count && !J.use_part) {
@@ -457,7 +450,7 @@ int stage_front(lrb_ctx* c, const lrb_reads* r, const Job& J, uint64_t row0, boo
     }
     if (timed) CTX_CUDA(cudaEventRecord(c->ev[2], st));  // composition (+ partition) of every chunk done
     c->comp_late_dst = nullptr;
-    if (J.do_comp && n && !comp_beside) {
+    if (J.do_comp && n) {
         uint32_t* dst = J.comp + (size_t)row0 * J.P;
         const size_t bytes = sizeof(uint32_t) * n * J.P;
         if (defer_comp) {                          // pageable destination: goes home at the end of the call
@@ -474,17 +467,6 @@ int stage_front(lrb_ctx* c, const lrb_reads* r, const Job& J, uint64_t row0, boo
         // ONE launch over all buckets when the second-level lists exist (no per-bucket tails), else RED.ADD per bucket
         const int mode = (c->part.sub ? (1 | 4) : 1) | (count_writes ? 8 : 0);
         if ((rc = lrb_dev_partition_apply(&c->part, mode, (uint32_t*)c->table.p, J.bin_size, J.bins, nullptr, nullptr, st))) return rc;
-    }
-    if (comp_beside) {
-        uint32_t* dst = J.comp + (size_t)row0 * J.P;
-        const size_t bytes = sizeof(uint32_t) * n * J.P;
-        CTX_CUDA(cudaEventRecord(c->mirrored, st));   // (event free at this point: the mirror comes after the search)
-        CTX_CUDA(cudaStreamWaitEvent(sout, c->mirrored, 0));
-        CTX_CUDA(cudaMemsetAsync(c->comp.p, 0, bytes, sout));
-        if ((rc = lrb_dev_composition(&v, J.k, (uint32_t*)c->comp.p, 0, r->n_tiles, sout))) return rc;
-        if (defer_comp) { c->comp_late_dst = dst; c->comp_late_bytes = bytes; }
-        else CTX_CUDA(cudaMemcpyAsync(dst, c->comp.p, bytes, cudaMemcpyDeviceToHost, sout));
-        CTX_CUDA(cudaEventRecord(c->sync_ev[LRB_PART_MAX_CHUNKS + 1], sout));
     }
     return LRB_OK;
 }
@@ -717,8 +699,6 @@ static int profile_host(lrb_ctx* c, const lrb_reads* r, int k, int n_set, const 
         J.force_l2 = e && !strcmp(e, "l2");
         const int bl = env_int("LRB_BUCKET_LOG2", 24);
         if (bl >= 24 && bl <= 25) J.bucket_shift = bl;
-        const int hc = env_int("LRB_H2D_CHUNKS", 16);
-        if (hc > 0) J.h2d_chunks = hc;
         J.force_ship_valid = env_int("LRB_SHIP_VALID", 0) > 0;
     }
     J.comp_pinned = host_ptr_is_pinned(comp_counts);
@@ -880,20 +860,10 @@ static int profile_host(lrb_ctx* c, const lrb_reads* r, int k, int n_set, const 
         };
         if (single) {
             const uint64_t nr = p.kept->n_reads;
-            // The mirror writes only the half of the table the list-driven search never reads, so it COULD run beside the
-            // search (LRB_MIRROR_OVERLAP=1: on the exchange stream, after the count resp. the last exchange round).  Measured
-            // and rejected as the default (profiles/r02_exp1_variants.jsonl): the 4 GiB it streams through L2 evict the
-            // search's resident table slice — the search goes from 20.5 to 26.2 ms to hide a 1.26 ms pass.
+            // The mirror writes only the half of the table the list-driven search never reads, yet it runs after the search:
+            // beside it (measured, profiles/r02_exp1_variants.jsonl) the 4 GiB it streams through L2 evict the search's
+            // resident table slice — the search goes from 20.5 to 26.2 ms to hide a 1.26 ms pass.
             const bool mirror_here = J.do_count && (x == c || !J.use_part);
-            const bool mirror_beside = mirror_here && J.use_part && J.do_search && nr && p.kept->n_blocks && env_int("LRB_MIRROR_OVERLAP", 0) > 0;
-            if (mirror_beside) {
-                if (!exchanged) {
-                    CTX_CUDA(cudaEventRecord(x->counted, st));
-                    CTX_CUDA(cudaStreamWaitEvent(x->xchg, x->counted, 0));
-                }
-                if ((rc2 = lrb_dev_mirror((uint32_t*)x->table.p, x->xchg))) return rc2;
-                CTX_CUDA(cudaEventRecord(x->mirrored, x->xchg));
-            }
             if (J.do_search && nr) {
                 CTX_CUDA(cudaMemsetAsync(x->hist.p, 0, sizeof(uint32_t) * nr * (size_t)J.bins, st));
                 CTX_CUDA(cudaMemsetAsync(x->sums.p, 0, sizeof(uint32_t) * nr, st));
@@ -913,8 +883,7 @@ static int profile_host(lrb_ctx* c, const lrb_reads* r, int k, int n_set, const 
             if (rc2) return rc2;
             if (x == c) CTX_CUDA(cudaEventRecord(c->ev[3], st));  // table passes done
             // the full table (both strands) is needed on device 0 (lrb_ctx_table_save, table_host) and by the direct search
-            if (mirror_beside) CTX_CUDA(cudaStreamWaitEvent(st, x->mirrored, 0));
-            else if (mirror_here && (rc2 = lrb_dev_mirror((uint32_t*)x->table.p, st))) return rc2;
+            if (mirror_here && (rc2 = lrb_dev_mirror((uint32_t*)x->table.p, st))) return rc2;
             if (x == c) CTX_CUDA(cudaEventRecord(c->ev[4], st));
             if (!J.use_part && J.do_search && nr &&
                 (rc2 = lrb_dev_search(&x->dview, (const uint32_t*)x->table.p, J.bin_size, J.bins, (uint32_t*)x->hist.p, (uint32_t*)x->sums.p, 0,

@@ -119,19 +119,9 @@ k_count15(const uint32_t* __restrict__ codes, const uint32_t* __restrict__ valid
 
 // mirror: T[x] = T[rc(x)] for all x with bit 15 set — a 64x64 tiled "transpose" whose index algebra
 // (mirror_dst_index / mirror_src_index) lives in lane_core.cuh.  Reads touch only bit-15-clear entries,
-// writes only bit-15-set ones, so the pass is race-free in place; both sides move 256 B rows.
+// writes only bit-15-set ones, so the pass is race-free in place; both sides move 256 B rows.  Global accesses are
+// 16 bytes wide: a source row of the tile is 64 contiguous entries = 16 uint4, and so is a destination row.
 __global__ void __launch_bounds__(256) k_mirror(uint32_t* __restrict__ table) {
-    __shared__ uint32_t tile[64][65];
-    const uint32_t t = blockIdx.x;
-    const uint32_t tx = threadIdx.x & 63u, ty = threadIdx.x >> 6;  // 64 x 4
-    for (uint32_t sb = ty; sb < 64; sb += 4) tile[sb][tx] = table[mirror_src_index(t, sb, tx)];
-    __syncthreads();
-    for (uint32_t a = ty; a < 64; a += 4) table[mirror_dst_index(t, a, tx)] = tile[rc_small(tx, 3)][rc_small(a, 3)];
-}
-
-// the same with 16-byte global accesses: a source row of the tile is 64 contiguous entries = 16 uint4, and so is a
-// destination row; a quarter of the LDG / STG instructions for the same bytes
-__global__ void __launch_bounds__(256) k_mirror_v4(uint32_t* __restrict__ table) {
     __shared__ uint32_t tile[64][65];
     const uint32_t t = blockIdx.x;
     const uint32_t c4 = (threadIdx.x & 15u) * 4u, r = threadIdx.x >> 4;  // 16 uint4 columns x 16 rows per pass
@@ -485,9 +475,7 @@ extern "C" int lrb_dev_count(const lrb_reads_view* dev, uint32_t* table, uint64_
 
 extern "C" int lrb_dev_mirror(uint32_t* table, void* stream) {
     if (!table) return lrb_set_error(LRB_EINVAL, "lrb_dev_mirror: null table");
-    static const bool scalar = getenv("LRB_MIRROR_SCALAR") && atoi(getenv("LRB_MIRROR_SCALAR")) > 0;   // round-1 kernel, for A/B timing
-    if (scalar) LRB_LAUNCH("k_mirror", (cudaStream_t)stream, k_mirror<<<1u << 17, 256, 0, (cudaStream_t)stream>>>(table));
-    else LRB_LAUNCH("k_mirror", (cudaStream_t)stream, k_mirror_v4<<<1u << 17, 256, 0, (cudaStream_t)stream>>>(table));
+    LRB_LAUNCH("k_mirror", (cudaStream_t)stream, k_mirror<<<1u << 17, 256, 0, (cudaStream_t)stream>>>(table));
     LRB_CUDA(cudaGetLastError());
     return LRB_OK;
 }

@@ -254,20 +254,12 @@ __device__ void chunk_scan_warp(PartMeta* __restrict__ m, int c, int nb, ull cap
 // copies whole runs, contiguous on both sides.  The next step's block and prelude are fetched while the current one
 // is copied out; two barriers per step.  The kernel is bound by shared-memory wavefronts (the scattered staging
 // store and the ranking atomic), so nothing else is staged.
-// BULK (experiment, LRB_PART_BULK=1): the run copy-out goes through the bulk-copy engine (cp.async.bulk shared -> global,
-// SASS UBLKCP) instead of LDS + STG: every staged run starts at the same offset modulo 16 bytes as its destination, so all
-// but <= 3 entries at either end of a run move as one 16-byte-aligned bulk copy issued by one lane.
-__device__ __forceinline__ void bulk_s2g(void* gdst, const void* ssrc, uint32_t bytes) {
-    asm volatile("cp.async.bulk.global.shared::cta.bulk_group [%0], [%1], %2;" ::"l"(gdst), "r"((uint32_t)__cvta_generic_to_shared(ssrc)), "r"(bytes)
-                 : "memory");
-}
-
-template <bool WITH_RID, bool FULL, bool BULK = false>
+template <bool WITH_RID, bool FULL>
 __global__ void __launch_bounds__(kPartThreads)
 k_partition(const uint32_t* __restrict__ codes, const uint32_t* __restrict__ valid, const uint32_t* __restrict__ blk_read,
             uint64_t blk_lo, uint64_t blk_hi, uint32_t key_lo, uint32_t key_hi, int shift, int nb, uint32_t n_steps, uint32_t G,
             uint32_t step0, StepTables T, const PartMeta* __restrict__ meta, int c, uint32_t* __restrict__ ent_out) {
-    __shared__ __align__(16) uint32_t s_ent[kStepSlots + (BULK ? 6 * kMaxBuckets : 0)];  // staged entries, grouped by bucket
+    __shared__ uint32_t s_ent[kStepSlots];                          // staged entries, grouped by bucket
     __shared__ uint32_t s_cur[2][kMaxBuckets];                      // staging cursor of each bucket
     __shared__ uint32_t s_beg[2][kMaxBuckets], s_n[2][kMaxBuckets]; // staged run of each bucket
     __shared__ uint32_t* s_dst[2][kMaxBuckets];                     // where the run goes in ent_out
@@ -287,17 +279,14 @@ k_partition(const uint32_t* __restrict__ codes, const uint32_t* __restrict__ val
         const uint16_t* cs = T.cnt + (size_t)(step0 + s) * kMaxBuckets;
         const uint32_t c0 = (lane < nb) ? cs[lane] : 0u;
         const uint32_t c1 = (lane + 32 < nb) ? cs[lane + 32] : 0u;
-        // BULK: a staged run starts at its destination's offset modulo 4 entries and occupies a whole number of 16 B units
-        const uint32_t m0 = BULK ? (uint32_t)((reg0 + run0) & 3ull) : 0u, m1 = BULK ? (uint32_t)((reg1 + run1) & 3ull) : 0u;
-        const uint32_t p0 = BULK ? ((m0 + c0 + 3u) & ~3u) : c0, p1 = BULK ? ((m1 + c1 + 3u) & ~3u) : c1;
-        uint32_t x0 = p0, x1 = p1;
+        uint32_t x0 = c0, x1 = c1;
 #pragma unroll
         for (int d = 1; d < 32; d <<= 1) {
             const uint32_t y0 = __shfl_up_sync(0xFFFFFFFFu, x0, d), y1 = __shfl_up_sync(0xFFFFFFFFu, x1, d);
             if (lane >= d) { x0 += y0; x1 += y1; }
         }
         const uint32_t tot0 = __shfl_sync(0xFFFFFFFFu, x0, 31);
-        const uint32_t e0 = x0 - p0 + m0, e1 = tot0 + x1 - p1 + m1;  // exclusive staging offsets
+        const uint32_t e0 = x0 - c0, e1 = tot0 + x1 - c1;  // exclusive staging offsets
         s_cur[buf][lane] = s_beg[buf][lane] = e0;
         s_cur[buf][lane + 32] = s_beg[buf][lane + 32] = e1;
         s_n[buf][lane] = c0;
@@ -344,29 +333,12 @@ k_partition(const uint32_t* __restrict__ codes, const uint32_t* __restrict__ val
             fetch(s + 1, v, pv, b, rd, r0v);
             if (warp == 0) prelude(s + 1, buf ^ 1);
         }
-        if (BULK) {
-            if (lane == 0) asm volatile("fence.proxy.async.shared::cta;" ::: "memory");  // the staged entries were written by generic-proxy stores
-            for (int bk = warp; bk < nb; bk += kPartThreads / 32) {
-                const uint32_t n = s_n[buf][bk], sb = s_beg[buf][bk];
-                const uint32_t* src = s_ent + sb;
-                uint32_t* dst = s_dst[buf][bk];
-                const uint32_t head = min(n, (4u - (sb & 3u)) & 3u), body = (n - head) & ~3u, tail = n - head - body;
-                if (lane < head) __stcs(dst + lane, src[lane]);
-                if (lane < tail) __stcs(dst + head + body + lane, src[head + body + lane]);
-                if (lane == 0 && body) bulk_s2g(dst + head, src + head, body * 4u);
-            }
-            if (lane == 0) {  // the staging area is rewritten in the next step: wait until the engine has read it
-                asm volatile("cp.async.bulk.commit_group;" ::: "memory");
-                asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory");
-            }
-        } else {
-            for (int bk = warp; bk < nb; bk += kPartThreads / 32) {  // each warp copies whole runs: contiguous both sides
-                const uint32_t n = s_n[buf][bk];
-                const uint32_t* src = s_ent + s_beg[buf][bk];
-                uint32_t* dst = s_dst[buf][bk];
+        for (int bk = warp; bk < nb; bk += kPartThreads / 32) {  // each warp copies whole runs: contiguous both sides
+            const uint32_t n = s_n[buf][bk];
+            const uint32_t* src = s_ent + s_beg[buf][bk];
+            uint32_t* dst = s_dst[buf][bk];
 #pragma unroll 2
-                for (uint32_t i = lane; i < n; i += 32) __stcs(dst + i, src[i]);
-            }
+            for (uint32_t i = lane; i < n; i += 32) __stcs(dst + i, src[i]);
         }
         __syncthreads();
     }
@@ -454,7 +426,6 @@ constexpr int kL2CtasPerSm = 2;   // measured: a third CTA per SM (fits: 40 regi
 
 struct L2Layout {
     uint32_t nsub, n_cta, C3, nb;   // sub-slices per bucket, CTAs of k2_partition, UNIFORM entries per segment (small inputs), buckets
-    uint32_t strided;               // k2_partition row ownership (fill rows are permuted to match)
     // position of a sub-slice's counter in a fill row: the sub-slices warp + 16 j that one k2_partition warp owns sit next to
     // each other, so its lanes read and write one 64-byte stretch instead of 16 sectors
     __host__ __device__ uint32_t fill_pos(uint32_t sub) const { return (sub & 15u) * (nsub >> 4) + (sub >> 4); }
@@ -466,12 +437,11 @@ struct L2Layout {
     // capacity and leaned on the fallback / spill area).  Too small a sample -> the uniform C3.
     uint64_t seg0, seg_units;       // first segment; u16 units available for segments
     // cell table (u16 offset cells0): uint2 info[ncell] = {offset in octets, capacity}, u32 hist[ncell], u32 run_len[nb].
-    // info of cell (b, sub) sits at b * nsub + cell_pos(sub): the permutation of the fill rows, so that the 16 rows a
+    // info of cell (b, sub) sits at b * nsub + fill_pos(sub): the permutation of the fill rows, so that the 16 rows a
     // k2_partition warp owns are one 128-byte load (in natural order they are 16 sectors: +25 % l1tex wavefronts per tile)
     uint64_t cells0;
     uint64_t windows_est;           // upper estimate of the windows the whole partition will hold (its list capacity)
     __host__ __device__ uint32_t ncell() const { return nb * nsub; }
-    __host__ __device__ uint32_t cell_pos(uint32_t sub) const { return strided ? fill_pos(sub) : sub; }
     __device__ const uint2* cell_info(const uint16_t* ws) const { return reinterpret_cast<const uint2*>(ws + cells0); }
     __device__ uint32_t* cell_hist(uint16_t* ws) const { return reinterpret_cast<uint32_t*>(ws + cells0) + 2 * ncell(); }
     // tiles of bucket b a k2_partition CTA takes per visit (<= kL2Run; shorter for small buckets, so that every CTA still
@@ -518,7 +488,7 @@ __global__ void __launch_bounds__(1024) k_plan_cells(uint16_t* __restrict__ ws, 
     const uint32_t tid = threadIdx.x, ncell = Y.ncell();
     uint2* info = const_cast<uint2*>(Y.cell_info(ws));
     uint32_t* rl = const_cast<uint32_t*>(Y.run_len(ws));
-    auto slot = [&](uint32_t c) { return (c / Y.nsub) * Y.nsub + Y.cell_pos(c % Y.nsub); };
+    auto slot = [&](uint32_t c) { return (c / Y.nsub) * Y.nsub + Y.fill_pos(c % Y.nsub); };
     const uint32_t* hist = Y.cell_hist(ws);
     if (tid < (uint32_t)kMaxBuckets) s_bsum[tid] = 0;
     __syncthreads();
@@ -586,7 +556,7 @@ __global__ void __launch_bounds__(1024) k_plan_cells(uint16_t* __restrict__ ws, 
     }
 }
 
-template <int LOG2_NSUB, bool STRIDED>
+template <int LOG2_NSUB>
 __global__ void __launch_bounds__(kL2Threads, kL2CtasPerSm)
 k2_partition(const uint32_t* __restrict__ ents, PartMeta* __restrict__ meta, int c, uint16_t* __restrict__ ws, L2Layout Y) {
     extern __shared__ uint32_t s_dyn[];
@@ -691,10 +661,10 @@ k2_partition(const uint32_t* __restrict__ ents, PartMeta* __restrict__ meta, int
         }
         for (uint32_t i = lane; i < n; i += 32) spill_keys[base + i] = key_at(i);
     };
-    // lane j < spw of a warp looks after row / fill counter j of the warp's sub-slices.  STRIDED (default): the warp owns
-    // sub-slices warp + 16 j — measured 2 ms faster per step than the blocked ownership 16 warp + j (LRB_K2_ROWS=block)
-    const uint32_t my_sub = STRIDED ? warp + (uint32_t)kL2Warps * lane : warp * spw + lane;
-    const uint32_t my_pos = STRIDED ? Y.fill_pos(my_sub) : my_sub;   // its counter in the fill row
+    // lane j < spw of a warp looks after row / fill counter j of the warp's sub-slices.  The warp owns sub-slices
+    // warp + 16 j — measured 2 ms faster per step than the blocked ownership 16 warp + j
+    const uint32_t my_sub = warp + (uint32_t)kL2Warps * lane;
+    const uint32_t my_pos = Y.fill_pos(my_sub);   // its counter in the fill row
     uint32_t e[kL2PerThread];
     uint32_t n_cur = 0, n_next = 0, b_cur = 0, b_next = 0;
     bool have = seek();
@@ -794,7 +764,7 @@ k2_partition(const uint32_t* __restrict__ ents, PartMeta* __restrict__ meta, int
         for (uint32_t rest = full_rows; rest; rest &= rest - 1u) {
             const uint32_t jj = (uint32_t)__ffs(rest) - 1u;
             const uint32_t n = __shfl_sync(0xFFFFFFFFu, n_my, jj);
-            const uint32_t sub = (STRIDED ? warp + (uint32_t)kL2Warps * jj : warp * spw + jj);
+            const uint32_t sub = warp + (uint32_t)kL2Warps * jj;
             const uint16_t* src = s_stage + (sub << cap_shift);
             const uint32_t bkt = b_cur;
             spill_warp(min(n, cap), bkt, [&](uint32_t i) { return Y.key_of(bkt, sub, src[(i + 2u * sub) & (cap - 1u)] & 0x7FFFu); });
@@ -822,7 +792,7 @@ k2_partition(const uint32_t* __restrict__ ents, PartMeta* __restrict__ meta, int
         for (uint32_t jj = 0; jj < spw; ++jj) {
             const uint32_t ns = __shfl_sync(0xFFFFFFFFu, ns_my, jj);
             const uint32_t off = __shfl_sync(0xFFFFFFFFu, off_my, jj) + lane;
-            const uint32_t sub = (STRIDED ? warp + (uint32_t)kL2Warps * jj : warp * spw + jj);
+            const uint32_t sub = warp + (uint32_t)kL2Warps * jj;
             const uint16_t* src = s_stage + (sub << cap_shift);
             const uint32_t p0 = (lane + 2u * sub) & cm, p1 = (lane + 32u + 2u * sub) & cm;
             if (lane < ns) lists[off] = src[p0];
@@ -831,7 +801,7 @@ k2_partition(const uint32_t* __restrict__ ents, PartMeta* __restrict__ meta, int
         for (uint32_t rest = big; rest; rest &= rest - 1u) {  // rare: long rows, rows that spilled into the overflow list
             const uint32_t jj = (uint32_t)__ffs(rest) - 1u;
             const uint32_t ns = __shfl_sync(0xFFFFFFFFu, ns_my, jj), n = __shfl_sync(0xFFFFFFFFu, n_my, jj);
-            const uint32_t sub = (STRIDED ? warp + (uint32_t)kL2Warps * jj : warp * spw + jj);
+            const uint32_t sub = warp + (uint32_t)kL2Warps * jj;
             uint16_t* __restrict__ dst = lists + __shfl_sync(0xFFFFFFFFu, off_my, jj);
             const uint16_t* src = s_stage + (sub << cap_shift);
             for (uint32_t j = lane + 64u; j < ns; j += 32) dst[j] = src[(j + 2u * sub) & cm];
@@ -898,9 +868,9 @@ k_count_smem(const uint16_t* __restrict__ ws, const PartMeta* __restrict__ meta,
         }
         return;
     }
-    const uint32_t* __restrict__ fill = reinterpret_cast<const uint32_t*>(ws) + (size_t)bucket * Y.nsub + (Y.strided ? Y.fill_pos(sub) : sub);  // + cta * nb * nsub
+    const uint32_t* __restrict__ fill = reinterpret_cast<const uint32_t*>(ws) + (size_t)bucket * Y.nsub + Y.fill_pos(sub);  // + cta * nb * nsub
     const size_t fill_stride = (size_t)Y.nb * Y.nsub;
-    const uint2 ci = __ldg(Y.cell_info(ws) + (uint32_t)bucket * Y.nsub + Y.cell_pos(sub));
+    const uint2 ci = __ldg(Y.cell_info(ws) + (uint32_t)bucket * Y.nsub + Y.fill_pos(sub));
     const uint32_t seg_cap = ci.y;
     const uint16_t* __restrict__ lists = ws + Y.seg0 + 8ull * ci.x;   // this cell's n_cta segments
     uint4* tab4 = reinterpret_cast<uint4*>(s_tab);
@@ -970,21 +940,7 @@ k_count_smem(const uint16_t* __restrict__ ws, const PartMeta* __restrict__ meta,
 // its entries.  Equal (read, bin) entries of a warp share one RED.  Tasks are numbered across all chunks
 // (L.task0 = prefix of tasks per chunk) so small chunks still fill the machine.
 constexpr uint32_t kTaskRuns = 16;
-constexpr uint32_t kBinLut = 2048;  // counts below this go through a shared-memory bin table when (B+1)*S fits
-
-// L2 eviction-priority hints (PTX createpolicy / ld.global.L2::cache_hint): HINT = 1 marks the table gathers evict_last
-// (the 32 MiB slice of the current bucket should outlive the 312 MB entry stream and the histogram REDs that pass
-// through L2 beside it); the entry stream is already evict-first (__ldcs).  Kept or rejected on measured DRAM bytes.
-__device__ __forceinline__ uint64_t l2_policy_evict_last() {
-    uint64_t p;
-    asm("createpolicy.fractional.L2::evict_last.b64 %0, 1.0;" : "=l"(p));
-    return p;
-}
-__device__ __forceinline__ uint32_t ldg_hint(const uint32_t* a, uint64_t pol) {
-    uint32_t v;
-    asm("ld.global.L2::cache_hint.u32 %0, [%1], %2;" : "=r"(v) : "l"(a), "l"(pol));
-    return v;
-}
+constexpr int kSearchUnroll = 8;   // gathers in flight per lane in the walk's full steps: 8 (22.3 ms at config #2) beats 4 (23.7 ms)
 
 // The walk over the entries of one bucket, shared by the single-setting search, the multi-setting one and the multi-table
 // one: load(e) gathers what entry e needs from the table(s) (a count, or one count per table); put(hbase, cnt,
@@ -993,7 +949,7 @@ __device__ __forceinline__ uint32_t ldg_hint(const uint32_t* a, uint64_t pol) {
 // every lane of the warp together, so it may use warp-wide primitives.  One launch may cover several buckets (gridDim.y):
 // CTAs are dispatched x-fastest, so the buckets are still worked on one after the other (their slices take turns in L2)
 // but the tail of one overlaps the head of the next.
-template <int U, class Load, class Put>
+template <class Load, class Put>
 __device__ __forceinline__ void search_keys_body(const uint32_t* __restrict__ ents, const PartMeta* __restrict__ meta, int bucket,
                                                  int n_chunks, const ChunkList& L, const StepTables& T, int shift,
                                                  uint32_t* __restrict__ hist, uint32_t pitch, uint32_t (*s_bnd)[kTaskRuns + 1],
@@ -1028,6 +984,7 @@ __device__ __forceinline__ void search_keys_body(const uint32_t* __restrict__ en
             put(hbase, cnt, act, lane, seek, row);
         };
         uint32_t i0 = span_beg;
+        constexpr int U = kSearchUnroll;
         constexpr uint32_t kStep = 32u * U;
         if (i0 + kStep <= span_end) {  // full steps: no predicates; the entries of step t+1 are fetched while step t gathers
             uint32_t e[U], nx[U];
@@ -1052,7 +1009,7 @@ __device__ __forceinline__ void search_keys_body(const uint32_t* __restrict__ en
                 for (int u = 0; u < U; ++u) e[u] = nx[u];
             }
         }
-        for (; i0 + 128u <= span_end; i0 += 128u) {  // (U > 4) full 128-entry steps that are left
+        for (; i0 + 128u <= span_end; i0 += 128u) {  // full 128-entry steps that are left
             const uint32_t* src = region + i0 + lane;
             const uint32_t e0 = __ldcs(src), e1 = __ldcs(src + 32), e2 = __ldcs(src + 64), e3 = __ldcs(src + 96);
             const Count c0 = load(e0), c1 = load(e1), c2 = load(e2), c3 = load(e3);
@@ -1082,18 +1039,12 @@ __device__ __forceinline__ void search_keys_body(const uint32_t* __restrict__ en
     }
 }
 
-// load functor of the walk for the full-layout table: the count of the entry's key (HINT = 1: gathers marked evict_last)
-template <int HINT>
+// load functor of the walk for the full-layout table: the count of the entry's key
 __device__ __forceinline__ auto table_load(const uint32_t* __restrict__ table, uint32_t bucket_base, uint32_t hi_mask2) {
-    const uint64_t pol = HINT ? l2_policy_evict_last() : 0ull;
-    return [=](uint32_t e) {
-        const uint32_t key = entry_key(e, bucket_base, hi_mask2);
-        return HINT ? ldg_hint(table + key, pol) : table[key];
-    };
+    return [=](uint32_t e) { return table[entry_key(e, bucket_base, hi_mask2)]; };
 }
 
 // hist[read][bin(table[key])] += 1 for one (bin size, bin count): rows of B bins
-template <bool USE_LUT, int U, int HINT = 0>
 __global__ void __launch_bounds__(256)
 k_search_keys(const uint32_t* __restrict__ ents, const PartMeta* __restrict__ meta, int bucket0, int n_chunks, ChunkList L,
               StepTables T, uint32_t bucket_base0, uint32_t hi_mask2, int shift, const uint32_t* __restrict__ table, uint32_t S32,
@@ -1102,20 +1053,13 @@ k_search_keys(const uint32_t* __restrict__ ents, const PartMeta* __restrict__ me
     const uint32_t bucket_base = bucket_base0 + ((uint32_t)blockIdx.y << shift);
     __shared__ uint32_t s_bnd[8][kTaskRuns + 1];  // per warp: start of each run of the span, [kTaskRuns] = end of the span
     __shared__ uint32_t s_r0[8][kTaskRuns];       // per warp: read index of each run's step relative to the span's first
-    __shared__ uint16_t s_lut[USE_LUT ? kBinLut : 2];
     if (meta->overflow) return;
-    // every count >= (B+1)*S lands in the last bin (pos >= B), so the table covers the whole rule
-    const uint32_t lut_top = USE_LUT ? (B + 1u) * S32 : 0u;
-    if (USE_LUT) {
-        for (uint32_t i = threadIdx.x; i <= lut_top; i += blockDim.x) s_lut[i] = (uint16_t)coverage_bin(i, S32, magic, B);
-        __syncthreads();
-    }
-    search_keys_body<U>(ents, meta, bucket, n_chunks, L, T, shift, hist, B, s_bnd, s_r0, table_load<HINT>(table, bucket_base, hi_mask2),
+    search_keys_body(ents, meta, bucket, n_chunks, L, T, shift, hist, B, s_bnd, s_r0, table_load(table, bucket_base, hi_mask2),
                               [&](uint32_t* hbase, uint32_t cnt, bool act, uint32_t lane, auto seek, auto row) {
                                   uint32_t cell = 0xFFFFFFFFu;
                                   if (act) {
                                       seek();
-                                      const uint32_t bin = USE_LUT ? s_lut[min(cnt, lut_top)] : coverage_bin(cnt, S32, magic, B);
+                                      const uint32_t bin = coverage_bin(cnt, S32, magic, B);
                                       cell = row() * B + bin;
                                   }
                                   const uint32_t peers = __match_any_sync(0xFFFFFFFFu, cell);
@@ -1132,7 +1076,6 @@ struct CovSettings {
     uint32_t n, W;
 };
 
-template <int U>
 __global__ void __launch_bounds__(256)
 k_search_settings(const uint32_t* __restrict__ ents, const PartMeta* __restrict__ meta, int bucket0, int n_chunks, ChunkList L,
                   StepTables T, uint32_t bucket_base0, uint32_t hi_mask2, int shift, const uint32_t* __restrict__ table,
@@ -1142,7 +1085,7 @@ k_search_settings(const uint32_t* __restrict__ ents, const PartMeta* __restrict_
     __shared__ uint32_t s_bnd[8][kTaskRuns + 1];
     __shared__ uint32_t s_r0[8][kTaskRuns];
     if (meta->overflow) return;
-    search_keys_body<U>(ents, meta, bucket, n_chunks, L, T, shift, hist, C.W, s_bnd, s_r0, table_load<0>(table, bucket_base, hi_mask2),
+    search_keys_body(ents, meta, bucket, n_chunks, L, T, shift, hist, C.W, s_bnd, s_r0, table_load(table, bucket_base, hi_mask2),
                            [&](uint32_t* hbase, uint32_t cnt, bool act, uint32_t lane, auto seek, auto row) {
                                uint32_t base = 0;
                                if (act) {
@@ -1158,30 +1101,23 @@ k_search_settings(const uint32_t* __restrict__ ents, const PartMeta* __restrict_
                            });
 }
 
-// Several sample tables in one walk over the lists.  A sample table is held compact (lrb_dev_table_compact): only its
-// bit-15-clear keys, entry i = T[((i >> 15) << 16) | (i & 0x7FFF)].  A list entry keeps its key inside the bucket with bit
-// 15 dropped in its low shift - 1 bits, so the entry's compact index is (bucket_base >> 1) | (e & (2^(shift-1) - 1)) and a
-// bucket's slice of a compact table is one contiguous 2^(shift-1)-entry range.  k_search_samples gathers each entry's
-// count from the G tables of a group and bins it with that table's setting into that table's column block, one
-// __match_any_sync and aggregated REDs per block as k_search_settings does per setting.  The host runs one walk per group.
+// Several sample tables, one walk over the lists per table.  A sample table is held compact (lrb_dev_table_compact): only
+// its bit-15-clear keys, entry i = T[((i >> 15) << 16) | (i & 0x7FFF)].  A list entry keeps its key inside the bucket with
+// bit 15 dropped in its low shift - 1 bits, so the entry's compact index is (bucket_base >> 1) | (e & (2^(shift-1) - 1))
+// and a bucket's slice of a compact table is one contiguous 2^(shift-1)-entry range.  k_search_samples gathers each
+// entry's count from one table and bins it with that table's setting into that table's column block.  Walking two tables
+// at once saves one read of the lists per pair but measured 1.28-1.30x slower on config #2 (DESIGN.md section 4).
+// The fields sit at the offsets of the former two-table layout (the pad words): packed back to back, nvcc schedules
+// k_search_samples differently and it measured 0.5 % slower (22.36 against 22.23 ms over the 64 buckets of config #2,
+// NVIDIA B200 at a 1000 W limit).
 struct SampleGroup {
-    const uint32_t* table[2];  // compact tables of the group
-    uint64_t magic[2];
-    uint32_t S32[2], B[2], off[2];
+    const uint32_t* table;     // compact table
+    const uint32_t* pad0;
+    uint64_t magic, pad1;
+    uint32_t S32, pad2, B, pad3, off, pad4;
     uint32_t W;                // row pitch: the bins of every table of the call
 };
 
-// Tables per walk: one.  Two compact slices of a 2^24-key bucket (64 MiB) would fit the 126 MB L2 beside the list stream
-// and the histogram lines, and fusing them saves one read of the lists per pair; measured on config #2 it is 1.28-1.30x
-// slower than one walk per table for 2, 4 and 8 tables (profiles/r06_samples_bench.jsonl, DESIGN.md section 4).
-constexpr int kSampleGroup = 1;
-
-template <int G>
-struct SampleCounts {
-    uint32_t c[G];
-};
-
-template <int U, int G>
 __global__ void __launch_bounds__(256)
 k_search_samples(const uint32_t* __restrict__ ents, const PartMeta* __restrict__ meta, int bucket0, int n_chunks, ChunkList L,
                  StepTables T, uint32_t cbase0, int shift, const __grid_constant__ SampleGroup S, uint32_t* __restrict__ hist) {
@@ -1191,30 +1127,20 @@ k_search_samples(const uint32_t* __restrict__ ents, const PartMeta* __restrict__
     __shared__ uint32_t s_bnd[8][kTaskRuns + 1];
     __shared__ uint32_t s_r0[8][kTaskRuns];
     if (meta->overflow) return;
-    const uint32_t* slice[G];  // the bucket's slice of each table
-#pragma unroll
-    for (int g = 0; g < G; ++g) slice[g] = S.table[g] + cbase;
-    search_keys_body<U>(ents, meta, bucket, n_chunks, L, T, shift, hist, S.W, s_bnd, s_r0,
-                        [&](uint32_t e) {
-                            SampleCounts<G> r;
-#pragma unroll
-                            for (int g = 0; g < G; ++g) r.c[g] = __ldg(slice[g] + (e & emask));
-                            return r;
-                        },
-                        [&](uint32_t* hbase, const SampleCounts<G>& cnt, bool act, uint32_t lane, auto seek, auto row) {
-                            uint32_t base = 0;
-                            if (act) {
-                                seek();
-                                base = row() * S.W;
-                            }
-#pragma unroll
-                            for (int g = 0; g < G; ++g) {
-                                uint32_t cell = 0xFFFFFFFFu;
-                                if (act) cell = base + S.off[g] + coverage_bin(cnt.c[g], S.S32[g], S.magic[g], S.B[g]);
-                                const uint32_t peers = __match_any_sync(0xFFFFFFFFu, cell);
-                                if (act && (uint32_t)__ffs(peers) - 1u == lane) atomicAdd(hbase + cell, (uint32_t)__popc(peers));
-                            }
-                        });
+    const uint32_t* slice = S.table + cbase;  // the bucket's slice of the table
+    search_keys_body(ents, meta, bucket, n_chunks, L, T, shift, hist, S.W, s_bnd, s_r0,
+                     [&](uint32_t e) { return __ldg(slice + (e & emask)); },
+                     [&](uint32_t* hbase, uint32_t cnt, bool act, uint32_t lane, auto seek, auto row) {
+                         uint32_t base = 0;
+                         if (act) {
+                             seek();
+                             base = row() * S.W;
+                         }
+                         uint32_t cell = 0xFFFFFFFFu;
+                         if (act) cell = base + S.off + coverage_bin(cnt, S.S32, S.magic, S.B);
+                         const uint32_t peers = __match_any_sync(0xFFFFFFFFu, cell);
+                         if (act && (uint32_t)__ffs(peers) - 1u == lane) atomicAdd(hbase + cell, (uint32_t)__popc(peers));
+                     });
 }
 
 // sums[r] = number of windows of read r that were bucketed so far = sum of the B bins that start its histogram row (every
@@ -1239,11 +1165,6 @@ ChunkList chunk_list(const lrb_partition* part) {
         L.task0[c + 1] = L.task0[c] + (L.nsteps[c] + kTaskRuns - 1) / kTaskRuns;
     }
     return L;
-}
-
-uint32_t l2_strided() {  // which rows a k2_partition warp sweeps: "strided" (warp + 16 j, default: 2 ms faster) or "block" (16 warp + j)
-    const char* e = getenv("LRB_K2_ROWS");
-    return (e && e[0] == 'b') ? 0u : 1u;
 }
 
 int sms() {
@@ -1366,26 +1287,21 @@ static int add_chunk(const lrb_reads_view* dev, const uint32_t* blk_read, uint64
     else
         LRB_LAUNCH("k_step_hist", st, k_step_hist<false><<<n_groups, kPartThreads, 0, st>>>(dev->codes, dev->valid, br, blk_lo, blk_hi, part->key_lo, part->key_hi, shift, n_steps, G, step0, T));
     LRB_LAUNCH("k_group_scan", st, k_group_scan<<<nb, 256, 0, st>>>(T, n_groups, meta, c, nb, (ull)part->capacity));
-#define LRB_LAUNCH_PART(RID, FULLK, ...)                                                                                              \
-    LRB_LAUNCH("k_partition", st, k_partition<RID, FULLK, ##__VA_ARGS__><<<n_groups, kPartThreads, 0, st>>>(dev->codes, dev->valid, br, blk_lo, blk_hi, part->key_lo, part->key_hi, \
+#define LRB_LAUNCH_PART(RID, FULLK)                                                                                              \
+    LRB_LAUNCH("k_partition", st, k_partition<RID, FULLK><<<n_groups, kPartThreads, 0, st>>>(dev->codes, dev->valid, br, blk_lo, blk_hi, part->key_lo, part->key_hi, \
                                                                shift, nb, n_steps, G, step0, T, meta, c, part->keys))
-    static const bool bulk = getenv("LRB_PART_BULK") && atoi(getenv("LRB_PART_BULK")) > 0;   // experiment: copy-out by cp.async.bulk
-    if (bulk && full && part->has_rids) LRB_LAUNCH_PART(true, true, true);
-    else if (bulk && full) LRB_LAUNCH_PART(false, true, true);
-    else if (part->has_rids) { if (full) LRB_LAUNCH_PART(true, true); else LRB_LAUNCH_PART(true, false); }
+    if (part->has_rids) { if (full) LRB_LAUNCH_PART(true, true); else LRB_LAUNCH_PART(true, false); }
     else { if (full) LRB_LAUNCH_PART(false, true); else LRB_LAUNCH_PART(false, false); }
 #undef LRB_LAUNCH_PART
     if (part->l2_enabled) {
         L2Layout Y;
-        Y.nsub = 1u << (shift - 16); Y.n_cta = part->l2_ncta; Y.C3 = part->l2_C3; Y.nb = (uint32_t)nb; Y.strided = l2_strided();
+        Y.nsub = 1u << (shift - 16); Y.n_cta = part->l2_ncta; Y.C3 = part->l2_C3; Y.nb = (uint32_t)nb;
         Y.seg0 = part->l2_seg0; Y.seg_units = part->l2_span; Y.cells0 = part->l2_cells0; Y.windows_est = part->capacity;
         Y.spill0 = part->l2_spill0; Y.spill_cap = part->l2_spill_cap; Y.key_lo = part->key_lo; Y.shift = shift;
         if (c == 0) {   // segment capacities from the key distribution of a sample of the first chunk (see L2Layout)
             const uint64_t stride = std::max<uint64_t>(1, nblk >> 18);   // <= 2^18 blocks = 8 M windows: ~500 per cell, 0.1 ms
             const uint64_t n_samp = (nblk + stride - 1) / stride;
-            static const bool uniform_caps = getenv("LRB_K2_UNIFORM") && atoi(getenv("LRB_K2_UNIFORM")) > 0;   // experiment: no sample -> one capacity for all cells
-            if (uniform_caps) {
-            } else if (full)
+            if (full)
                 LRB_LAUNCH("k_sample_cells", st, k_sample_cells<true><<<(unsigned)((n_samp + 255) / 256), 256, 0, st>>>(dev->codes, dev->valid, blk_lo, blk_hi, stride, part->key_lo, part->key_hi, part->sub, Y));
             else
                 LRB_LAUNCH("k_sample_cells", st, k_sample_cells<false><<<(unsigned)((n_samp + 255) / 256), 256, 0, st>>>(dev->codes, dev->valid, blk_lo, blk_hi, stride, part->key_lo, part->key_hi, part->sub, Y));
@@ -1394,15 +1310,9 @@ static int add_chunk(const lrb_reads_view* dev, const uint32_t* blk_read, uint64
         constexpr int kSmemL2 = kL2Stage * (int)sizeof(uint16_t);
 #define LRB_LAUNCH_K2(LG)                                                                                               \
     case LG:                                                                                                            \
-        if (strided) {                                                                                                  \
-            LRB_CUDA(cudaFuncSetAttribute(k2_partition<LG, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemL2)); \
-            LRB_LAUNCH("k2_partition", st, k2_partition<LG, true><<<Y.n_cta, kL2Threads, kSmemL2, st>>>(part->keys, meta, c, part->sub, Y));            \
-        } else {                                                                                                        \
-            LRB_CUDA(cudaFuncSetAttribute(k2_partition<LG, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemL2)); \
-            LRB_LAUNCH("k2_partition", st, k2_partition<LG, false><<<Y.n_cta, kL2Threads, kSmemL2, st>>>(part->keys, meta, c, part->sub, Y));           \
-        }                                                                                                               \
+        LRB_CUDA(cudaFuncSetAttribute(k2_partition<LG>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemL2));         \
+        LRB_LAUNCH("k2_partition", st, k2_partition<LG><<<Y.n_cta, kL2Threads, kSmemL2, st>>>(part->keys, meta, c, part->sub, Y)); \
         break
-        const bool strided = Y.strided != 0;
         switch (shift - 16) {  // log2 of the sub-slices per bucket (shift is 20..25)
             LRB_LAUNCH_K2(4); LRB_LAUNCH_K2(5); LRB_LAUNCH_K2(6); LRB_LAUNCH_K2(7); LRB_LAUNCH_K2(8); LRB_LAUNCH_K2(9);
             default: return lrb_set_error(LRB_EINVAL, "second-level lists need log2_bucket_keys in [20, 25]");
@@ -1468,7 +1378,7 @@ extern "C" int lrb_dev_partition_apply_range(const lrb_partition* part, int mode
     const bool overwrite = do_count && (mode & 8);   // the caller did not zero the slices of the applied buckets
     L2Layout Y = {};
     if (smem_count) {
-        Y.nsub = 1u << (part->shift - 16); Y.n_cta = part->l2_ncta; Y.C3 = part->l2_C3; Y.nb = (uint32_t)part->n_buckets; Y.strided = l2_strided();
+        Y.nsub = 1u << (part->shift - 16); Y.n_cta = part->l2_ncta; Y.C3 = part->l2_C3; Y.nb = (uint32_t)part->n_buckets;
         Y.seg0 = part->l2_seg0; Y.seg_units = part->l2_span; Y.cells0 = part->l2_cells0; Y.windows_est = part->capacity;
         Y.spill0 = part->l2_spill0; Y.spill_cap = part->l2_spill_cap; Y.key_lo = part->key_lo; Y.shift = part->shift;
     }
@@ -1489,14 +1399,6 @@ extern "C" int lrb_dev_partition_apply_range(const lrb_partition* part, int mode
     const uint32_t hi_mask2 = ((1u << shift) - 1u) & ~0xFFFFu;
     const unsigned grid = (unsigned)sms() * 8;
     const unsigned sgrid = search_grid(L, part->n_chunks);
-    // bin rule through a shared-memory table instead of arithmetic: measured slower on B200 (the extra LDS competes with
-    // the gathers for the memory pipe), kept behind LRB_SEARCH_LUT=1 for experiments
-    const char* lut_env = getenv("LRB_SEARCH_LUT");
-    const bool use_lut = lut_env && atoi(lut_env) > 0 && ((uint64_t)bins + 1) * S32 < kBinLut;
-    const char* hint_env = getenv("LRB_SEARCH_HINT");   // 1: evict_last on the table gathers (experiment, see k_search_keys)
-    const bool hint = hint_env && atoi(hint_env) > 0;
-    const char* un_env = getenv("LRB_SEARCH_UNROLL");  // gathers in flight per lane: 8 (default, 22.3 ms at config #2) or 4 (23.7 ms)
-    const bool unroll8 = !(un_env && atoi(un_env) == 4);
     constexpr int kSmemTable = (1 << kSubBits) * (int)sizeof(uint32_t);
     if (smem_count) {
         LRB_CUDA(cudaFuncSetAttribute(k_count_smem<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemTable));
@@ -1517,14 +1419,8 @@ extern "C" int lrb_dev_partition_apply_range(const lrb_partition* part, int mode
     if (search_batched) {
         const uint32_t base0 = part->key_lo + ((uint32_t)bucket_lo << shift);
         const dim3 gs(sgrid, (unsigned)(bucket_hi - bucket_lo));
-#define LRB_LAUNCH_SEARCH(LUT, UN, ...)                                                                                                \
-    LRB_LAUNCH("k_search_keys", st, k_search_keys<LUT, UN, ##__VA_ARGS__><<<gs, 256, 0, st>>>(part->keys, meta, bucket_lo, part->n_chunks, L, T, base0, hi_mask2, shift, table, S32, magic, \
-                                               (uint32_t)bins, hist))
-        if (use_lut) LRB_LAUNCH_SEARCH(true, 4);
-        else if (unroll8 && hint) LRB_LAUNCH_SEARCH(false, 8, 1);
-        else if (unroll8) LRB_LAUNCH_SEARCH(false, 8);
-        else LRB_LAUNCH_SEARCH(false, 4);
-#undef LRB_LAUNCH_SEARCH
+        LRB_LAUNCH("k_search_keys", st, k_search_keys<<<gs, 256, 0, st>>>(part->keys, meta, bucket_lo, part->n_chunks, L, T, base0, hi_mask2, shift,
+                                                                         table, S32, magic, (uint32_t)bins, hist));
     }
     for (int b = bucket_lo; b < bucket_hi && !count_batched && !search_batched; ++b) {
         const uint32_t bucket_base = part->key_lo + ((uint32_t)b << shift);
@@ -1532,16 +1428,9 @@ extern "C" int lrb_dev_partition_apply_range(const lrb_partition* part, int mode
         else if (smem_count) LRB_LAUNCH("k_count_smem", st, k_count_smem<false><<<Y.nsub, 1024, kSmemTable, st>>>(part->sub, meta, b, Y, bucket_base, shift, table));
         if (do_count) LRB_LAUNCH("k_count_keys", st, k_count_keys<<<grid, 256, 0, st>>>(part->keys, meta, b, part->n_chunks, bucket_base, shift, hi_mask2, table, smem_count ? 1 : 0));
         if (smem_count) LRB_LAUNCH("k_count_spill", st, k_count_spill<<<grid, 256, 0, st>>>(part->sub, meta, Y, b, b + 1, table));
-        if (do_search) {
-#define LRB_LAUNCH_SEARCH(LUT, UN, ...)                                                                                                \
-    LRB_LAUNCH("k_search_keys", st, k_search_keys<LUT, UN, ##__VA_ARGS__><<<sgrid, 256, 0, st>>>(part->keys, meta, b, part->n_chunks, L, T, bucket_base, hi_mask2, shift, table, S32, magic, \
-                                                  (uint32_t)bins, hist))
-            if (use_lut) LRB_LAUNCH_SEARCH(true, 4);
-            else if (unroll8 && hint) LRB_LAUNCH_SEARCH(false, 8, 1);
-            else if (unroll8) LRB_LAUNCH_SEARCH(false, 8);
-            else LRB_LAUNCH_SEARCH(false, 4);
-#undef LRB_LAUNCH_SEARCH
-        }
+        if (do_search)
+            LRB_LAUNCH("k_search_keys", st, k_search_keys<<<sgrid, 256, 0, st>>>(part->keys, meta, b, part->n_chunks, L, T, bucket_base, hi_mask2, shift,
+                                                                                table, S32, magic, (uint32_t)bins, hist));
     }
     if (do_search && part->n_reads && bucket_hi == part->n_buckets)
         LRB_LAUNCH("k_row_sums", st, k_row_sums<<<(unsigned)((part->n_reads + 255) / 256), 256, 0, st>>>(hist, sums, part->n_reads, (uint32_t)bins, (uint32_t)bins));
@@ -1551,7 +1440,7 @@ extern "C" int lrb_dev_partition_apply_range(const lrb_partition* part, int mode
 
 // Several coverage settings in one search (k_search_settings): hist rows of W = sum of bins[m] words, setting m's bins at
 // column sum_{j<m} bins[j]; sums are rewritten by the call that includes the last bucket.  n = 1 is mode 2 of
-// lrb_dev_partition_apply_range (where the experiment switches LRB_SEARCH_LUT / _HINT / _UNROLL apply).
+// lrb_dev_partition_apply_range.
 extern "C" int lrb_dev_partition_search_settings(const lrb_partition* part, int bucket_lo, int bucket_hi, const uint32_t* table, int n,
                                                  const long* bin_sizes, const int* bins, uint32_t* hist, uint32_t* sums, void* stream) {
     if (!part || !table || !hist || !sums) return lrb_set_error(LRB_EINVAL, "lrb_dev_partition_search_settings: null argument");
@@ -1580,10 +1469,10 @@ extern "C" int lrb_dev_partition_search_settings(const lrb_partition* part, int 
     const uint32_t hi_mask2 = ((1u << shift) - 1u) & ~0xFFFFu;
     if (bucket_hi > bucket_lo) {
         const dim3 gs(search_grid(L, part->n_chunks), (unsigned)(bucket_hi - bucket_lo));
-        LRB_LAUNCH("k_search_settings", st, k_search_settings<8><<<gs, 256, 0, st>>>(part->keys, meta, bucket_lo, part->n_chunks, L,
-                                                                                     step_tables(part->steps, part->step_capacity),
-                                                                                     part->key_lo + ((uint32_t)bucket_lo << shift),
-                                                                                     hi_mask2, shift, table, C, hist));
+        LRB_LAUNCH("k_search_settings", st, k_search_settings<<<gs, 256, 0, st>>>(part->keys, meta, bucket_lo, part->n_chunks, L,
+                                                                                  step_tables(part->steps, part->step_capacity),
+                                                                                  part->key_lo + ((uint32_t)bucket_lo << shift),
+                                                                                  hi_mask2, shift, table, C, hist));
     }
     if (part->n_reads && bucket_hi == part->n_buckets)
         LRB_LAUNCH("k_row_sums", st, k_row_sums<<<(unsigned)((part->n_reads + 255) / 256), 256, 0, st>>>(hist, sums, part->n_reads, (uint32_t)bins[0], W));
@@ -1592,15 +1481,11 @@ extern "C" int lrb_dev_partition_search_settings(const lrb_partition* part, int 
 }
 
 // Several compact sample tables in one search (k_search_samples): hist rows of W = sum of bins[t] words, table t's bins at
-// column sum_{j<t} bins[j]; one walk over the lists per group of `group` tables; sums are rewritten by the call that
-// includes the last bucket.
-extern "C" int lrb_dev_partition_search_samples_grouped(const lrb_partition* part, int bucket_lo, int bucket_hi,
-                                                        const uint32_t* const* compact_tables, int n, const long* bin_sizes,
-                                                        const int* bins, uint32_t* hist, uint32_t* sums, int group, void* stream) {
+// column sum_{j<t} bins[j]; one walk over the lists per table; sums are rewritten by the call that includes the last bucket.
+extern "C" int lrb_dev_partition_search_samples(const lrb_partition* part, int bucket_lo, int bucket_hi, const uint32_t* const* compact_tables,
+                                                int n, const long* bin_sizes, const int* bins, uint32_t* hist, uint32_t* sums, void* stream) {
     static const char* who = "lrb_dev_partition_search_samples";
     if (!part || !compact_tables || !hist || !sums) return lrb_set_error(LRB_EINVAL, "%s: null argument", who);
-    if (group < 0 || group > 2) return lrb_set_error(LRB_EINVAL, "%s: group must be 0 (the default), 1 or 2 (got %d)", who, group);
-    if (group == 0) group = kSampleGroup;
     uint64_t ids[LRB_MAX_SAMPLE_TABLES] = {};
     for (int t = 0; t < n && t < LRB_MAX_SAMPLE_TABLES; ++t) {
         if (!compact_tables[t]) return lrb_set_error(LRB_EINVAL, "%s: null table %d", who, t);
@@ -1623,34 +1508,20 @@ extern "C" int lrb_dev_partition_search_samples_grouped(const lrb_partition* par
     const uint32_t cbase0 = (part->key_lo + ((uint32_t)bucket_lo << shift)) >> 1;
     if (bucket_hi > bucket_lo) {
         const dim3 gs(search_grid(L, part->n_chunks), (unsigned)(bucket_hi - bucket_lo));
-        for (int t0 = 0, off = 0; t0 < n;) {
-            const int g = std::min(group, n - t0);
+        for (int t = 0, off = 0; t < n; off += bins[t], ++t) {
             SampleGroup S = {};
             S.W = W;
-            for (int j = 0; j < g; ++j) {
-                S.table[j] = compact_tables[t0 + j];
-                S.S32[j] = bin_sizes[t0 + j] > 0xFFFFFFFFl ? 0xFFFFFFFFu : (uint32_t)bin_sizes[t0 + j];
-                S.magic[j] = coverage_magic(S.S32[j]);
-                S.B[j] = (uint32_t)bins[t0 + j];
-                S.off[j] = (uint32_t)off;
-                off += bins[t0 + j];
-            }
-            if (g == 2)
-                LRB_LAUNCH("k_search_samples", st, k_search_samples<8, 2><<<gs, 256, 0, st>>>(part->keys, meta, bucket_lo, part->n_chunks, L, T,
-                                                                                             cbase0, shift, S, hist));
-            else
-                LRB_LAUNCH("k_search_samples", st, k_search_samples<8, 1><<<gs, 256, 0, st>>>(part->keys, meta, bucket_lo, part->n_chunks, L, T,
-                                                                                             cbase0, shift, S, hist));
-            t0 += g;
+            S.table = compact_tables[t];
+            S.S32 = bin_sizes[t] > 0xFFFFFFFFl ? 0xFFFFFFFFu : (uint32_t)bin_sizes[t];
+            S.magic = coverage_magic(S.S32);
+            S.B = (uint32_t)bins[t];
+            S.off = (uint32_t)off;
+            LRB_LAUNCH("k_search_samples", st, k_search_samples<<<gs, 256, 0, st>>>(part->keys, meta, bucket_lo, part->n_chunks, L, T,
+                                                                                   cbase0, shift, S, hist));
         }
     }
     if (part->n_reads && bucket_hi == part->n_buckets)
         LRB_LAUNCH("k_row_sums", st, k_row_sums<<<(unsigned)((part->n_reads + 255) / 256), 256, 0, st>>>(hist, sums, part->n_reads, (uint32_t)bins[0], W));
     LRB_CUDA(cudaGetLastError());
     return LRB_OK;
-}
-
-extern "C" int lrb_dev_partition_search_samples(const lrb_partition* part, int bucket_lo, int bucket_hi, const uint32_t* const* compact_tables,
-                                                int n, const long* bin_sizes, const int* bins, uint32_t* hist, uint32_t* sums, void* stream) {
-    return lrb_dev_partition_search_samples_grouped(part, bucket_lo, bucket_hi, compact_tables, n, bin_sizes, bins, hist, sums, 0, stream);
 }

@@ -157,10 +157,6 @@ class CudaEngine:
     def mirror(self, table):
         self.p.dev_mirror(table)
 
-    def mirror_on(self, table, stream):
-        with self.torch.cuda.stream(stream):
-            self.p.dev_mirror(table)
-
     def search(self, table, bin_size, bins, hist, sums, read_lo, read_hi, key_lo, key_hi):
         self._partition(read_lo, read_hi, key_lo, key_hi, count=False)   # re-used from count() when the rectangle is the same
         self.ws.apply(table, count=False, search=True, bin_size=bin_size, bins=bins, hist=hist, sums=sums)
@@ -266,8 +262,8 @@ class PeerExchange:
     of the node).  A side stream moves rows of the canonical half between the tables with pitched device-to-device
     copies (lrb_dev_copy2d: the copy engines carry them through NVSwitch), orders the ranks with device-side barriers
     and adds pulled rows with lrb_dev_add_planes (see run()).  The main stream only waits for a round's event and
-    searches its buckets, so the exchange runs ahead of the search and hides behind it; the mirror pass (it writes
-    only the non-canonical half, which the search never reads) follows the last round on the side stream.
+    searches its buckets, so the exchange runs ahead of the search and hides behind it; the mirror pass follows the
+    search on the main stream.
     NCCL's all-reduce moves the same bytes with SM-resident kernels; pipelining it slice by slice hid only 2 of its
     6.4 ms at N = 2 and left 13 ms exposed at N = 8 (profiles/r01_bench_n2_*.json, r01_bench_n8_*.json)."""
 
@@ -287,9 +283,7 @@ class PeerExchange:
         self.stage = None
         # highest priority: k_add_planes / the mirror get SM slots ahead of the queued CTAs of the search they hide behind
         # (at default priority every 16 MiB add took 2.2 ms at N = 2, stretching the exchange over the whole search)
-        self.mirror_beside = os.environ.get("LRB_MIRROR_OVERLAP", "0") != "0"
-        prio = -1 if os.environ.get("LRB_XCHG_PRIO", "1") != "0" else 0
-        self.comm = torch.cuda.Stream(device=device, priority=prio)
+        self.comm = torch.cuda.Stream(device=device, priority=-1)
 
     def timings(self):
         """Of the last run(), after a synchronize: ms from "count done" to the first round's rows being final on this rank
@@ -352,8 +346,6 @@ class PeerExchange:
                 ev = torch.cuda.Event(enable_timing=True)
                 ev.record(comm)
                 events.append(ev)
-            if self.mirror_beside:
-                engine.mirror_on(table, comm)                 # non-canonical half: never read by the search
             self.hdl.barrier()                                # (the next step refills the tables only after everybody is here)
         for k, ev in enumerate(events):
             main.wait_event(ev)
@@ -361,10 +353,9 @@ class PeerExchange:
                 engine.search_slice(table, bin_size, bins, hist_all, sums_all, lo, hi, pieces[rounds[k][0][0]][0], pieces[rounds[k][-1][0]][1])
         main.wait_stream(comm)
         self.last_events = (ready, events[0], events[-1]) if events else None   # timings(): after a synchronize
-        if not self.mirror_beside:
-            # after the search, not beside it: the mirror streams 4 GiB through L2 and evicts the search's resident table
-            # slice (single GPU, profiles/r02_exp1_variants.jsonl: search 20.5 -> 26.2 ms with the mirror beside it)
-            engine.mirror(table)
+        # after the search, not beside it: the mirror streams 4 GiB through L2 and evicts the search's resident table
+        # slice (single GPU, profiles/r02_exp1_variants.jsonl: search 20.5 -> 26.2 ms with the mirror beside it)
+        engine.mirror(table)
 
 
 _SIDE = {}

@@ -508,15 +508,15 @@ class PartitionWorkspace:
                                                     C.c_void_p(table.data_ptr()), len(bs), _ptr(bs), _ptr(bc),
                                                     C.c_void_p(hist.data_ptr()), C.c_void_p(sums.data_ptr()), _stream()))
 
-    def search_samples(self, tables, settings, hist, sums, bucket_lo=0, bucket_hi=None, group=0):
+    def search_samples(self, tables, settings, hist, sums, bucket_lo=0, bucket_hi=None):
         """Search against several compact sample tables (dev_table_compact) at once (lrb_dev_partition_search_samples):
         tables[t] is binned with settings[t] = (bin_size, bins) into its column block of hist [N, W]; hist and sums zeroed
-        by the caller as for apply(search=True).  group: tables per walk over the lists (0: the library's choice)."""
+        by the caller as for apply(search=True)."""
         bs, bc = _settings_arrays(settings)
         ptrs = (C.c_void_p * max(len(tables), 1))(*[t.data_ptr() for t in tables])
-        check(lib.lrb_dev_partition_search_samples_grouped(C.byref(self.part), bucket_lo, 64 if bucket_hi is None else bucket_hi,
-                                                           ptrs, len(tables), _ptr(bs), _ptr(bc), C.c_void_p(hist.data_ptr()),
-                                                           C.c_void_p(sums.data_ptr()), int(group), _stream()))
+        check(lib.lrb_dev_partition_search_samples(C.byref(self.part), bucket_lo, 64 if bucket_hi is None else bucket_hi,
+                                                   ptrs, len(tables), _ptr(bs), _ptr(bc), C.c_void_p(hist.data_ptr()),
+                                                   C.c_void_p(sums.data_ptr()), _stream()))
 
 
 def dev_table_compact(table, out=None):

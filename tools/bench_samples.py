@@ -4,11 +4,11 @@ Usage: bench_samples.py [--out FILE] [--reps N] [--file-reps N] [--parent-tree D
 
 (a) Config #2 (1 M ONT reads, 5 Gbases) resident on the device, against n = 1, 2, 4, 8 sample tables (the reads' own table
     and tables counted from other synthetic communities), all with -bs 10 -bc 32: CUDA-event time of
-    lrb_dev_partition_search_samples_grouped over all 64 buckets with one table per walk (G = 1) and two (G = 2), and of
-    n single-table searches (lrb_dev_partition_apply_range mode 2 against the full-layout tables) over the same lists;
-    the three are timed alternately, rep by rep, with the rows zeroed outside the timed window.  The tables (2 GiB compact,
-    4 GiB full) and the 312 MB entry stream are larger than the 126 MB L2.  Every rep's blocks are checked against the
-    single searches.
+    lrb_dev_partition_search_samples over all 64 buckets (one walk per table, G = 1) and of n single-table searches
+    (lrb_dev_partition_apply_range mode 2 against the full-layout tables) over the same lists; the two are timed
+    alternately, rep by rep, with the rows zeroed outside the timed window.  The tables (2 GiB compact, 4 GiB full) and the
+    312 MB entry stream are larger than the 126 MB L2.  Every rep's blocks are checked against the single searches.
+    (Two tables per walk, G = 2, was measured 1.28-1.30x slower than G = 1: profiles/r06_samples_bench.jsonl.)
 (b) Loading a page-cached table file: lrb_ctx_sample_table_load (canonical rows, 2 GiB read) against lrb_ctx_table_load
     (4 GiB), alternately.
 (c) Config #1 (100 k reads, 0.5 Gbases) as a FASTA file against 3 tables: one lrb_search_15mers_samples call against
@@ -78,40 +78,36 @@ def device_resident(emit, reps):
     n = spec.n_reads
     for nt in (1, 2, 4, 8):
         S = [(BS, BC)] * nt
-        hist = {g: torch.zeros((n, BC * nt), dtype=torch.int32, device=DEV) for g in (1, 2)}
-        sums = {g: torch.zeros(n, dtype=torch.int32, device=DEV) for g in (1, 2)}
+        hist = torch.zeros((n, BC * nt), dtype=torch.int32, device=DEV)
+        sums = torch.zeros(n, dtype=torch.int32, device=DEV)
         singles = [torch.zeros((n, BC), dtype=torch.int32, device=DEV) for _ in range(nt)]
         s1 = torch.zeros(n, dtype=torch.int32, device=DEV)
 
-        def run_group(g):
-            return lambda: ws.search_samples(compact[:nt], S, hist[g], sums[g], group=g)
+        def run_samples():
+            ws.search_samples(compact[:nt], S, hist, sums)
 
         def run_singles():
             for t, h in enumerate(singles):
                 ws.apply(full[t], count=False, search=True, bin_size=BS, bins=BC, hist=h, sums=s1)
 
-        t = {1: [], 2: [], "single": []}
+        t = {1: [], "single": []}
         for rep in range(reps + 2):                   # two warm-up reps
-            for g in (1, 2):
-                hist[g].zero_()
-                sums[g].zero_()
+            hist.zero_()
+            sums.zero_()
             for h in singles:
                 h.zero_()
             s1.zero_()
             torch.cuda.synchronize()
-            ms = {1: event_ms(run_group(1)), 2: event_ms(run_group(2)), "single": event_ms(run_singles)}
+            ms = {1: event_ms(run_samples), "single": event_ms(run_singles)}
             if rep >= 2:
                 for k, v in ms.items():
                     t[k].append(v)
-        for g in (1, 2):
-            for i, h in enumerate(singles):
-                assert torch.equal(hist[g][:, i * BC:(i + 1) * BC], h), (nt, g, i)
-            assert torch.equal(sums[g], s1)
+        for i, h in enumerate(singles):
+            assert torch.equal(hist[:, i * BC:(i + 1) * BC], h), (nt, i)
+        assert torch.equal(sums, s1)
         emit({"what": "samples_search_device", "config": "cfg2_1M_5kb_ont_k4", "n_tables": nt, "W": BC * nt, "setting": [BS, BC],
-              "reps": reps, "G1": stats(t[1]), "G2": stats(t[2]), "single_calls": stats(t["single"]),
-              "G2_over_G1": float(np.median(t[2]) / np.median(t[1])),
-              "single_calls_over_G1": float(np.median(t["single"]) / np.median(t[1])),
-              "single_calls_over_G2": float(np.median(t["single"]) / np.median(t[2])), "results_equal": True})
+              "reps": reps, "G1": stats(t[1]), "single_calls": stats(t["single"]),
+              "single_calls_over_G1": float(np.median(t["single"]) / np.median(t[1])), "results_equal": True})
         del hist, sums, singles, s1
         torch.cuda.empty_cache()
     del ws, full, compact, dr
