@@ -261,6 +261,14 @@ int lrb_dev_partition_search_settings(const lrb_partition* part, int bucket_lo, 
  * and starts at a bucket boundary. */
 int lrb_dev_partition_search_samples(const lrb_partition* part, int bucket_lo, int bucket_hi, const uint32_t* const* compact_tables,
                                      int n, const long* bin_sizes, const int* bins, uint32_t* hist, uint32_t* sums, void* stream);
+/* Search with coverage bins given by count edges (no reference counterpart): edges is a HOST array of n_edges strictly
+ * increasing thresholds t_0 < ... < t_{n-1}, t_0 >= 2, and a window whose 15-mer is counted c times goes to bin
+ * #{i : t_i <= c} (searchsorted(edges, c, side="right")) of rows of B = n_edges + 1 words.  Counts 0 and 1 always go to
+ * bin 0, as in the reference's rule; edges {2, 3, ..., B} equal -bs 1 -bc B and no edges equal -bc 1.  Bucket range and
+ * sums as in lrb_dev_partition_search_settings.  LRB_EINVAL unless 0 <= n_edges <= LRB_MAX_BINS - 1, edges is non-NULL
+ * when n_edges > 0, the edges are strictly increasing and t_0 >= 2, and the partition has read ids. */
+int lrb_dev_partition_search_edges(const lrb_partition* part, int bucket_lo, int bucket_hi, const uint32_t* table,
+                                   const uint32_t* edges, int n_edges, uint32_t* hist, uint32_t* sums, void* stream);
 
 /* Pack ASCII on the device: bases[] (device, concatenated) -> codes/valid of `dev` (layout prebuilt). */
 int lrb_dev_pack_ascii(const lrb_reads_view* dev, const char* bases, const uint64_t* offsets, void* stream);
@@ -358,6 +366,12 @@ int lrb_table_read_canonical(const char* path, uint32_t row_lo, uint32_t row_hi,
 int lrb_profile_host_samples(lrb_ctx* ctx, const lrb_reads* reads, int k, int n, const int* slots, const long* bin_sizes,
                              const int* bins, uint32_t* comp_counts, uint32_t* cov_hist, uint32_t* cov_sums, uint32_t* table_host,
                              int flags);
+/* lrb_profile_host with coverage bins given by count edges (lrb_dev_partition_search_edges): cov_hist[N*(n_edges + 1)].
+ * Every flag and part of lrb_profile_host works alongside (composition, count, KEEP / ADD_TO / USE_LOADED_TABLE, batches,
+ * several devices).  The edges are checked as in lrb_dev_partition_search_edges when coverage is asked for, before any
+ * device work; LRB_TABLE_PATH=direct is refused (LRB_EINVAL). */
+int lrb_profile_host_edges(lrb_ctx* ctx, const lrb_reads* reads, int k, const uint32_t* edges, int n_edges, uint32_t* comp_counts,
+                           uint32_t* cov_hist, uint32_t* cov_sums, uint32_t* table_host, int flags);
 /* How the last lrb_profile_host call ran. */
 typedef struct {
     int n_devices;            /* GPUs that took part */
@@ -432,6 +446,11 @@ int lrb_table_read_file(const char* path, uint32_t* table);
  * bin_size < 1 or bins outside [1, LRB_MAX_BINS], and when keys at or above max_count exist but
  * max_count < bin_size * (bins + 1): their bin is then not determined by the spectrum.  No reference counterpart. */
 int lrb_spectrum_bin_mass(const uint64_t* spectrum, uint32_t max_count, long bin_size, int bins, uint64_t* mass);
+/* The same for coverage bins given by count edges (lrb_dev_partition_search_edges): mass[n_edges + 1], mass[b] = sum over c
+ * of c * n_c * [#{i : edges[i] <= c} == b].  Keys at or above max_count add their sum to the last bin.  LRB_EINVAL for
+ * edges lrb_dev_partition_search_edges refuses, and when keys at or above max_count exist but max_count is below the last
+ * edge: their bin is then not determined by the spectrum.  No reference counterpart. */
+int lrb_spectrum_edge_mass(const uint64_t* spectrum, uint32_t max_count, const uint32_t* edges, int n_edges, uint64_t* mass);
 /* jellyfish `histo` text of a spectrum: "c n_c\n" for every c in [1, max_count) with n_c > 0, ascending, then
  * "max_count n_over\n" when keys at or above max_count exist.  Counts are of canonical 15-mers (each {x, revcomp(x)}
  * pair once).  No reference counterpart. */
@@ -463,6 +482,13 @@ int lrb_search_15mers_settings(const char* table_path, const char* reads_path, i
  * bins) twice).  No reference counterpart. */
 int lrb_search_15mers_samples(const char* const* table_paths, int n, const long* bin_sizes, const int* bins, const char* reads_path,
                               const char* out_txt, const char* out_npy, int threads);
+/* lrb_search_15mers with coverage bins given by count edges (lrb_dev_partition_search_edges): one table load and one parse;
+ * out_txt gets rows of n_edges + 1 values written exactly as lrb_search_15mers writes its rows (edges {2, ..., B} give its
+ * -bs 1 -bc B file byte for byte), out_npy (may be NULL) the [N, n_edges + 1] float rows.  Input larger than one segment
+ * is read segment by segment and the rows are appended in file order.  The arguments are checked before any file or
+ * device is touched (LRB_EINVAL as for lrb_profile_host_edges; a NULL path too).  No reference counterpart. */
+int lrb_search_15mers_edges(const char* table_path, const char* reads_path, const uint32_t* edges, int n_edges, const char* out_txt,
+                            const char* out_npy, int threads);
 /* Abundance spectrum of a 15mers-counts file as lrb_write_spectrum_txt text (loaded on device LRB_DEVICE).  Missing or
  * malformed table file: LRB_EIO / LRB_EFORMAT; no device: LRB_ECUDA.  No reference counterpart. */
 int lrb_table_spectrum(const char* table_path, const char* out_txt, uint32_t max_count);

@@ -106,6 +106,7 @@ _SIG = {
     "lrb_dev_partition_apply_range": (C.c_int, [_P, C.c_int, C.c_int, C.c_int, _P, C.c_long, C.c_int, _P, _P, _P]),
     "lrb_dev_partition_search_settings": (C.c_int, [_P, C.c_int, C.c_int, _P, C.c_int, _P, _P, _P, _P, _P]),
     "lrb_dev_partition_search_samples": (C.c_int, [_P, C.c_int, C.c_int, _P, C.c_int, _P, _P, _P, _P, _P]),
+    "lrb_dev_partition_search_edges": (C.c_int, [_P, C.c_int, C.c_int, _P, _P, C.c_int, _P, _P, _P]),
     "lrb_dev_table_compact": (C.c_int, [_P, _P, _P]),
     "lrb_dev_pack_ascii": (C.c_int, [C.POINTER(ReadsView), _P, _P, _P]),
     "lrb_dev_format_composition": (C.c_int, [_P, _P, C.c_uint64, C.c_int, _P, _P]),
@@ -121,6 +122,7 @@ _SIG = {
     "lrb_profile_host": (C.c_int, [_P, _P, C.c_int, C.c_long, C.c_int, _P, _P, _P, _P, C.c_int]),
     "lrb_profile_host_settings": (C.c_int, [_P, _P, C.c_int, C.c_int, _P, _P, _P, _P, _P, _P, C.c_int]),
     "lrb_profile_host_samples": (C.c_int, [_P, _P, C.c_int, C.c_int, _P, _P, _P, _P, _P, _P, _P, C.c_int]),
+    "lrb_profile_host_edges": (C.c_int, [_P, _P, C.c_int, _P, C.c_int, _P, _P, _P, _P, C.c_int]),
     "lrb_ctx_sample_table_load": (C.c_int, [_P, C.c_int, C.c_char_p]),
     "lrb_ctx_sample_table_keep": (C.c_int, [_P, C.c_int]),
     "lrb_ctx_sample_table_free": (C.c_int, [_P, C.c_int]),
@@ -146,6 +148,7 @@ _SIG = {
     "lrb_table_write_file": (C.c_int, [C.c_char_p, _P]),
     "lrb_table_read_file": (C.c_int, [C.c_char_p, _P]),
     "lrb_spectrum_bin_mass": (C.c_int, [_P, C.c_uint32, C.c_long, C.c_int, _P]),
+    "lrb_spectrum_edge_mass": (C.c_int, [_P, C.c_uint32, _P, C.c_int, _P]),
     "lrb_write_spectrum_txt": (C.c_int, [C.c_char_p, _P, C.c_uint32]),
     "lrb_kmer_lut": (C.c_int, [C.c_int, _P]),
     "lrb_count_kmers": (C.c_int, [C.c_char_p, C.c_char_p, C.c_int, C.c_int]),
@@ -153,6 +156,7 @@ _SIG = {
     "lrb_search_15mers": (C.c_int, [C.c_char_p, C.c_char_p, C.c_char_p, C.c_long, C.c_int, C.c_int]),
     "lrb_search_15mers_settings": (C.c_int, [C.c_char_p, C.c_char_p, C.c_int, _P, _P, _P, _P, C.c_int]),
     "lrb_search_15mers_samples": (C.c_int, [_P, C.c_int, _P, _P, C.c_char_p, C.c_char_p, C.c_char_p, C.c_int]),
+    "lrb_search_15mers_edges": (C.c_int, [C.c_char_p, C.c_char_p, _P, C.c_int, C.c_char_p, C.c_char_p, C.c_int]),
     "lrb_table_spectrum": (C.c_int, [C.c_char_p, C.c_char_p, C.c_uint32]),
     "lrb_profile": (C.c_int, [C.c_char_p, C.c_char_p, C.c_int, C.c_long, C.c_int, C.c_int, C.c_int, C.c_int]),
     "lrb_profile_multi": (C.c_int, [C.c_char_p, C.c_char_p, C.c_int, C.c_long, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int]),

@@ -245,6 +245,9 @@ struct Job {
     int set_bins[LRB_MAX_COV_SETTINGS] = {1};
     int n_samp = 0;                   // > 0: coverage against these sample slots (lrb_profile_host_samples), setting t each
     int samp_slot[LRB_MAX_SAMPLE_TABLES] = {};
+    bool by_edges = false;            // bins given by count edges (lrb_profile_host_edges): bins = n_edges + 1
+    const uint32_t* edges = nullptr;  // the caller's host array, alive for the call
+    int n_edges = 0;
     uint32_t *comp = nullptr, *hist = nullptr, *sums = nullptr, *table_host = nullptr;
     bool do_comp = false, do_search = false, do_count = false, use_loaded = false, add_to_table = false;
     bool use_part = true, want_smem_env = false, force_l2 = false, comp_pinned = false;
@@ -474,6 +477,9 @@ int stage_front(lrb_ctx* c, const lrb_reads* r, const Job& J, uint64_t row0, boo
 // Pass 2: coverage rows of the batch's reads against the device's (finished) table, buckets [b_lo, b_hi) of the lists.
 int search_lists(lrb_ctx* c, const Job& J, uint64_t n, int b_lo, int b_hi) {
     if (!n) return LRB_OK;
+    if (J.by_edges)
+        return lrb_dev_partition_search_edges(&c->part, b_lo, b_hi, (const uint32_t*)c->table.p, J.edges, J.n_edges, (uint32_t*)c->hist.p,
+                                              (uint32_t*)c->sums.p, c->stream);
     if (J.n_samp) {
         const uint32_t* tabs[LRB_MAX_SAMPLE_TABLES];
         for (int t = 0; t < J.n_samp; ++t) tabs[t] = (const uint32_t*)c->sample[J.samp_slot[t]].p;
@@ -654,9 +660,17 @@ static int check_sample_slots(int n, const int* slots, const long* bin_sizes, co
     return lrb_check_table_settings("lrb_profile_host_samples", n, ids, bin_sizes, bins, W);
 }
 
-// slots: NULL, or the sample slot of each of the n_set settings (coverage against those instead of the context's table)
+// Bins given by count edges instead of (bin size, bin count) settings (lrb_profile_host_edges).
+struct EdgeBins {
+    const uint32_t* edges;
+    int n;
+};
+
+// slots: NULL, or the sample slot of each of the n_set settings (coverage against those instead of the context's table);
+// eb: NULL, or the count edges that bin the coverage instead of the settings (n_set, bin_sizes and bins are then unused)
 static int profile_host(lrb_ctx* c, const lrb_reads* r, int k, int n_set, const long* bin_sizes, const int* bins, const int* slots,
-                        uint32_t* comp_counts, uint32_t* cov_hist, uint32_t* cov_sums, uint32_t* table_host, int flags) {
+                        uint32_t* comp_counts, uint32_t* cov_hist, uint32_t* cov_sums, uint32_t* table_host, int flags,
+                        const EdgeBins* eb = nullptr) {
     Job J;
     J.reads = r; J.k = k; J.P = comp_width(k);
     J.comp = comp_counts; J.hist = cov_hist; J.sums = cov_sums; J.table_host = table_host;
@@ -676,15 +690,25 @@ static int profile_host(lrb_ctx* c, const lrb_reads* r, int k, int n_set, const 
                 return lrb_set_error(LRB_EINVAL, "lrb_profile_host_samples: LRB_TABLE_PATH=direct reads only the full-layout table, not sample slots");
             J.n_samp = n_set;
             std::copy(slots, slots + n_set, J.samp_slot);
+        } else if (eb) {
+            if ((rc = lrb_check_cov_edges("lrb_profile_host_edges", eb->edges, eb->n))) return rc;
+            if (direct_table_path())
+                return lrb_set_error(LRB_EINVAL, "lrb_profile_host_edges: LRB_TABLE_PATH=direct bins by bin size and count only, not by edges");
+            J.by_edges = true;
+            J.edges = eb->edges;
+            J.n_edges = eb->n;
+            W = (uint32_t)eb->n + 1u;
         } else if ((rc = lrb_check_cov_settings("lrb_profile_host", n_set, bin_sizes, bins, &W))) {
             return rc;
         }
-        if (n_set > 1 && direct_table_path())
-            return lrb_set_error(LRB_EINVAL, "LRB_TABLE_PATH=direct searches one coverage setting per call (%d settings asked for)", n_set);
-        J.n_set = n_set;
-        std::copy(bin_sizes, bin_sizes + n_set, J.set_bs);
-        std::copy(bins, bins + n_set, J.set_bins);
-        J.bin_size = bin_sizes[0];
+        if (!eb) {
+            if (n_set > 1 && direct_table_path())
+                return lrb_set_error(LRB_EINVAL, "LRB_TABLE_PATH=direct searches one coverage setting per call (%d settings asked for)", n_set);
+            J.n_set = n_set;
+            std::copy(bin_sizes, bin_sizes + n_set, J.set_bs);
+            std::copy(bins, bins + n_set, J.set_bins);
+            J.bin_size = bin_sizes[0];
+        }
         J.bins = (int)W;
     }
     J.use_loaded = (flags & LRB_PROFILE_USE_LOADED_TABLE) != 0;
@@ -961,6 +985,18 @@ extern "C" int lrb_profile_host_samples(lrb_ctx* c, const lrb_reads* r, int k, i
     if (rc) return rc;
     if (!c) return lrb_set_error(LRB_EINVAL, "lrb_profile_host_samples: null context");
     rc = profile_host(c, r, k, n, bin_sizes, bins, slots, comp_counts, cov_hist, cov_sums, table_host, flags);
+    if (rc && (flags & LRB_PROFILE_ADD_TO_TABLE)) c->table_ready = false;
+    return rc;
+}
+
+extern "C" int lrb_profile_host_edges(lrb_ctx* c, const lrb_reads* r, int k, const uint32_t* edges, int n_edges, uint32_t* comp_counts,
+                                      uint32_t* cov_hist, uint32_t* cov_sums, uint32_t* table_host, int flags) {
+    if (!r) return lrb_set_error(LRB_EINVAL, "lrb_profile_host_edges: null argument");
+    int rc = lrb_check_cov_edges("lrb_profile_host_edges", edges, n_edges);   // before the context: no device needed to refuse
+    if (rc) return rc;
+    if (!c) return lrb_set_error(LRB_EINVAL, "lrb_profile_host_edges: null context");
+    const EdgeBins eb{edges, n_edges};
+    rc = profile_host(c, r, k, 1, nullptr, nullptr, nullptr, comp_counts, cov_hist, cov_sums, table_host, flags, &eb);
     if (rc && (flags & LRB_PROFILE_ADD_TO_TABLE)) c->table_ready = false;
     return rc;
 }
@@ -1548,6 +1584,34 @@ extern "C" int lrb_search_15mers_samples(const char* const* table_paths, int n, 
         int rc2 = lrb_profile_host_samples(cg.c, s, 0, n, slots, bin_sizes, bins, nullptr, hist.data(), sums.data(), nullptr, 0);
         if (!rc2) rc2 = lrb_append_coverage_txt(out_txt, hist.data(), sums.data(), nr, (int)W, threads, row0);
         if (!rc2 && out_npy) rc2 = lrb_append_coverage_npy(out_npy, hist.data(), sums.data(), nr, (int)W, threads, row0);
+        return rc2;
+    };
+    if (in.whole) return search(in.whole, 0);
+    if ((rc = each_segment(in, false, search))) return rc;
+    segments_notice(in, 1);
+    return LRB_OK;
+}
+
+extern "C" int lrb_search_15mers_edges(const char* table_path, const char* reads_path, const uint32_t* edges, int n_edges,
+                                       const char* out_txt, const char* out_npy, int threads) {
+    static const char* who = "lrb_search_15mers_edges";
+    if (!table_path || !reads_path || !out_txt) return lrb_set_error(LRB_EINVAL, "%s: null path", who);
+    int rc = lrb_check_cov_edges(who, edges, n_edges);
+    if (rc) return rc;
+    if (direct_table_path()) return lrb_set_error(LRB_EINVAL, "%s: LRB_TABLE_PATH=direct bins by bin size and count only, not by edges", who);
+    const int B = n_edges + 1;
+    CtxGuard cg;
+    if ((rc = create_ctx(0, &cg.c))) return rc;
+    if ((rc = lrb_ctx_table_load(cg.c, table_path))) return rc;
+    if ((rc = truncate_file(out_txt))) return rc;
+    Input in;
+    if ((rc = open_input(reads_path, threads, 4ull * ((uint64_t)B + 1), in))) return rc;
+    auto search = [&](const lrb_reads* s, uint64_t row0) -> int {
+        const uint64_t n = s->n_reads;
+        std::vector<uint32_t> hist((size_t)n * B + 1), sums(n + 1);
+        int rc2 = lrb_profile_host_edges(cg.c, s, 0, edges, n_edges, nullptr, hist.data(), sums.data(), nullptr, LRB_PROFILE_USE_LOADED_TABLE);
+        if (!rc2) rc2 = lrb_append_coverage_txt(out_txt, hist.data(), sums.data(), n, B, threads, row0);
+        if (!rc2 && out_npy) rc2 = lrb_append_coverage_npy(out_npy, hist.data(), sums.data(), n, B, threads, row0);
         return rc2;
     };
     if (in.whole) return search(in.whole, 0);

@@ -69,3 +69,7 @@ int lrb_check_cov_settings(const char* who, int n, const long* bin_sizes, const 
 // The same for n sample tables with one setting each (LRB_MAX_SAMPLE_TABLES at most): ids[t] says which table t is, and only
 // the same (table, bin_size, bins) twice is refused.
 int lrb_check_table_settings(const char* who, int n, const uint64_t* ids, const long* bin_sizes, const int* bins, uint32_t* width);
+
+// Coverage bins given by n count edges: 0 <= n <= LRB_MAX_BINS - 1, edges non-NULL when n > 0, strictly increasing, the
+// first >= 2 (counts 0 and 1 stay in bin 0, as in the reference's rule).  LRB_EINVAL naming `who` and the bad value.
+int lrb_check_cov_edges(const char* who, const uint32_t* edges, int n);

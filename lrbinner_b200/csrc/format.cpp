@@ -300,6 +300,17 @@ int lrb_check_table_settings(const char* who, int n, const uint64_t* ids, const 
     return check_settings(who, n, ids, bin_sizes, bins, width);
 }
 
+int lrb_check_cov_edges(const char* who, const uint32_t* edges, int n) {
+    if (n < 0 || n > LRB_MAX_BINS - 1) return lrb_set_error(LRB_EINVAL, "%s: the number of edges must be in [0, %d] (got %d)", who, LRB_MAX_BINS - 1, n);
+    if (n > 0 && !edges) return lrb_set_error(LRB_EINVAL, "%s: null edges (%d edges)", who, n);
+    if (n > 0 && edges[0] < 2)
+        return lrb_set_error(LRB_EINVAL, "%s: the first edge must be >= 2, so that counts 0 and 1 stay in bin 0 (got %u)", who, edges[0]);
+    for (int i = 1; i < n; ++i)
+        if (edges[i] <= edges[i - 1])
+            return lrb_set_error(LRB_EINVAL, "%s: edges must be strictly increasing (edge %d = %u after edge %d = %u)", who, i, edges[i], i - 1, edges[i - 1]);
+    return LRB_OK;
+}
+
 // ---- abundance spectrum of the table (lrb_dev_table_spectrum layout: n_c for c < M, then n_over, sum_over, max) ----
 extern "C" int lrb_spectrum_bin_mass(const uint64_t* spectrum, uint32_t max_count, long bin_size, int bins, uint64_t* mass) {
     if (!spectrum || !mass) return lrb_set_error(LRB_EINVAL, "lrb_spectrum_bin_mass: null argument");
@@ -317,6 +328,26 @@ extern "C" int lrb_spectrum_bin_mass(const uint64_t* spectrum, uint32_t max_coun
     for (uint64_t c = 0; c < M; ++c)
         if (spectrum[c]) mass[lrb::coverage_bin((uint32_t)c, S32, magic, (uint32_t)bins)] += c * spectrum[c];
     mass[bins - 1] += spectrum[M + 1];
+    return LRB_OK;
+}
+
+extern "C" int lrb_spectrum_edge_mass(const uint64_t* spectrum, uint32_t max_count, const uint32_t* edges, int n_edges, uint64_t* mass) {
+    static const char* who = "lrb_spectrum_edge_mass";
+    if (!spectrum || !mass) return lrb_set_error(LRB_EINVAL, "%s: null argument", who);
+    const int rc = lrb_check_cov_edges(who, edges, n_edges);
+    if (rc) return rc;
+    const uint64_t M = max_count;
+    // every count >= the last edge lands in the last bin; below it the spectrum must resolve the count itself
+    if (spectrum[M] > 0 && n_edges > 0 && M < edges[n_edges - 1])
+        return lrb_set_error(LRB_EINVAL, "%s: %llu keys counted >= max_count %u, which is below the last edge %u", who,
+                             (unsigned long long)spectrum[M], max_count, edges[n_edges - 1]);
+    std::fill(mass, mass + n_edges + 1, 0ull);
+    int b = 0;   // bin of count c: the edges are increasing, so it only moves forward
+    for (uint64_t c = 0; c < M; ++c) {
+        while (b < n_edges && edges[b] <= c) ++b;
+        mass[b] += c * spectrum[c];
+    }
+    mass[n_edges] += spectrum[M + 1];
     return LRB_OK;
 }
 

@@ -29,6 +29,8 @@
 //                   row of their concatenated bins (lrb_dev_partition_search_settings)
 //   k_search_samples  the same walk over compact sample tables, one or two per launch: each table's count binned by
 //                   its own setting into its column block of one row (lrb_dev_partition_search_samples)
+//   k_search_edges  the same walk, the gathered count binned by caller-given count edges: bin = #{i : t_i <= count}
+//                   (lrb_dev_partition_search_edges)
 //   k_row_sums      sums[read] = sum of hist[read][*]  (every window lands in exactly one bin of each setting)
 //
 // The stream can be added in several chunks (lrb_dev_partition_add), each with its own regions, so the
@@ -1143,6 +1145,45 @@ k_search_samples(const uint32_t* __restrict__ ents, const PartMeta* __restrict__
                      });
 }
 
+// Bins given by count edges t_0 < ... < t_{n-1} (t_0 >= 2, checked on the host): a count c goes to bin #{i : t_i <= c},
+// rows of B = n + 1 bins.  The edges reach the kernel by value (16 380 bytes at most, within the parameter limit) and
+// are copied once per CTA into shared memory, padded to P - 1 words (P = the least power of two >= B) with 0xFFFFFFFF.
+// The bin is then found by log2(P) warp-uniform halving steps, each one LDS; a padding word compares <= c only when
+// c = 0xFFFFFFFF, where every edge does too, so min(pos, n) is exact.  For B <= 32 the edges of one step sit in distinct
+// banks.
+struct CovEdges {
+    uint32_t n, P;                  // edges, the padded search size
+    uint32_t t[LRB_MAX_BINS - 1];
+};
+
+__global__ void __launch_bounds__(256)
+k_search_edges(const uint32_t* __restrict__ ents, const PartMeta* __restrict__ meta, int bucket0, int n_chunks, ChunkList L,
+               StepTables T, uint32_t bucket_base0, uint32_t hi_mask2, int shift, const uint32_t* __restrict__ table,
+               const __grid_constant__ CovEdges E, uint32_t* __restrict__ hist) {
+    const int bucket = bucket0 + (int)blockIdx.y;
+    const uint32_t bucket_base = bucket_base0 + ((uint32_t)blockIdx.y << shift);
+    __shared__ uint32_t s_bnd[8][kTaskRuns + 1];
+    __shared__ uint32_t s_r0[8][kTaskRuns];
+    extern __shared__ uint32_t s_edge[];          // P - 1 words (dynamic)
+    if (meta->overflow) return;
+    for (uint32_t i = threadIdx.x; i + 1u < E.P; i += blockDim.x) s_edge[i] = i < E.n ? E.t[i] : 0xFFFFFFFFu;
+    __syncthreads();
+    const uint32_t B = E.n + 1u;
+    search_keys_body(ents, meta, bucket, n_chunks, L, T, shift, hist, B, s_bnd, s_r0, table_load(table, bucket_base, hi_mask2),
+                     [&](uint32_t* hbase, uint32_t cnt, bool act, uint32_t lane, auto seek, auto row) {
+                         uint32_t cell = 0xFFFFFFFFu;
+                         if (act) {
+                             seek();
+                             uint32_t pos = 0;
+                             for (uint32_t step = E.P >> 1; step; step >>= 1)
+                                 pos += s_edge[pos + step - 1u] <= cnt ? step : 0u;
+                             cell = row() * B + min(pos, E.n);
+                         }
+                         const uint32_t peers = __match_any_sync(0xFFFFFFFFu, cell);
+                         if (act && (uint32_t)__ffs(peers) - 1u == lane) atomicAdd(hbase + cell, (uint32_t)__popc(peers));
+                     });
+}
+
 // sums[r] = number of windows of read r that were bucketed so far = sum of the B bins that start its histogram row (every
 // setting of a row counts each window once, so the first one does)
 __global__ void __launch_bounds__(256) k_row_sums(const uint32_t* __restrict__ hist, uint32_t* __restrict__ sums, uint64_t n_reads, uint32_t B,
@@ -1522,6 +1563,44 @@ extern "C" int lrb_dev_partition_search_samples(const lrb_partition* part, int b
     }
     if (part->n_reads && bucket_hi == part->n_buckets)
         LRB_LAUNCH("k_row_sums", st, k_row_sums<<<(unsigned)((part->n_reads + 255) / 256), 256, 0, st>>>(hist, sums, part->n_reads, (uint32_t)bins[0], W));
+    LRB_CUDA(cudaGetLastError());
+    return LRB_OK;
+}
+
+// Coverage bins given by count edges (k_search_edges): hist rows of n_edges + 1 words; edges is a HOST array, checked by
+// lrb_check_cov_edges; sums are rewritten by the call that includes the last bucket.
+extern "C" int lrb_dev_partition_search_edges(const lrb_partition* part, int bucket_lo, int bucket_hi, const uint32_t* table,
+                                              const uint32_t* edges, int n_edges, uint32_t* hist, uint32_t* sums, void* stream) {
+    static const char* who = "lrb_dev_partition_search_edges";
+    if (!part || !table || !hist || !sums) return lrb_set_error(LRB_EINVAL, "%s: null argument", who);
+    const int rc = lrb_check_cov_edges(who, edges, n_edges);
+    if (rc) return rc;
+    if (!part->has_rids) return lrb_set_error(LRB_EINVAL, "%s: partition was built without read ids", who);
+    if (bucket_lo < 0) bucket_lo = 0;
+    if (bucket_hi > part->n_buckets) bucket_hi = part->n_buckets;
+    if (part->n_chunks == 0) return LRB_OK;
+    cudaStream_t st = (cudaStream_t)stream;
+    CovEdges E;
+    E.n = (uint32_t)n_edges;
+    E.P = 1;
+    while (E.P < E.n + 1u) E.P <<= 1;
+    std::copy(edges, edges + n_edges, E.t);
+    std::fill(E.t + n_edges, E.t + (LRB_MAX_BINS - 1), 0xFFFFFFFFu);
+    const uint32_t B = E.n + 1u;
+    const PartMeta* meta = reinterpret_cast<const PartMeta*>(part->small);
+    const ChunkList L = chunk_list(part);
+    const int shift = part->shift;
+    const uint32_t hi_mask2 = ((1u << shift) - 1u) & ~0xFFFFu;
+    if (bucket_hi > bucket_lo) {
+        const dim3 gs(search_grid(L, part->n_chunks), (unsigned)(bucket_hi - bucket_lo));
+        const size_t smem = sizeof(uint32_t) * (E.P - 1u);   // at most 16 380 bytes: no opt-in needed
+        LRB_LAUNCH("k_search_edges", st, k_search_edges<<<gs, 256, smem, st>>>(part->keys, meta, bucket_lo, part->n_chunks, L,
+                                                                               step_tables(part->steps, part->step_capacity),
+                                                                               part->key_lo + ((uint32_t)bucket_lo << shift),
+                                                                               hi_mask2, shift, table, E, hist));
+    }
+    if (part->n_reads && bucket_hi == part->n_buckets)
+        LRB_LAUNCH("k_row_sums", st, k_row_sums<<<(unsigned)((part->n_reads + 255) / 256), 256, 0, st>>>(hist, sums, part->n_reads, B, B));
     LRB_CUDA(cudaGetLastError());
     return LRB_OK;
 }

@@ -192,7 +192,7 @@ class Context:
         self.device = device
 
     def profile(self, reads, k=None, bin_size=None, bins=None, want_table=False, use_loaded_table=False, out=None,
-                keep_table=False, add_to_table=False, coverage=None, samples=None):
+                keep_table=False, add_to_table=False, coverage=None, samples=None, edges=None):
         """Returns dict(comp=[N,P] u32, hist=[N,bins] u32, sums=[N] u32, table=[2^30] u32) for the requested parts.
         `out` may carry preallocated (ideally page-locked) arrays under the same keys.  add_to_table: count these reads
         INTO the context's complete table (from an earlier count or table_load) instead of from zero; on failure the
@@ -202,11 +202,19 @@ class Context:
         the settings before it; hists[m] is the [N, bins_m] view of setting m, and sums are the same for every setting.
         samples=[(slot, bin_size, bins), ...] (instead of coverage / bin_size / bins): coverage against up to 8 sample slots
         (sample_table_load / sample_table_keep) instead of the context's table (lrb_profile_host_samples); hist [N, W] holds
-        table 0's bins, then table 1's, ..., hists[t] is table t's view and sums are shared."""
+        table 0's bins, then table 1's, ..., hists[t] is table t's view and sums are shared.
+        edges=[t_1, ..., t_{B-1}] (instead of every other coverage argument): bins given by strictly increasing count edges,
+        t_1 >= 2; a window whose 15-mer is counted c times goes to bin searchsorted(edges, c, side="right") of hist [N, B]
+        (lrb_profile_host_edges)."""
         if coverage is not None and (bin_size is not None or bins is not None):
             raise _lib.LrbError(_lib.LRB_EINVAL, "coverage=[(bin_size, bins), ...] replaces bin_size / bins: give one or the other")
         if samples is not None and (coverage is not None or bin_size is not None or bins is not None):
             raise _lib.LrbError(_lib.LRB_EINVAL, "samples=[(slot, bin_size, bins), ...] replaces coverage / bin_size / bins: give one or the other")
+        if edges is not None:
+            if samples is not None or coverage is not None or bin_size is not None or bins is not None:
+                raise _lib.LrbError(_lib.LRB_EINVAL, "edges=[...] replaces samples / coverage / bin_size / bins: give one or the other")
+            edges = _edges_array(edges)   # refused here, before a context is needed
+            return self._profile_edges(reads, k, edges, want_table, use_loaded_table, out, keep_table, add_to_table)
         n = reads.n_reads
         out = dict(out or {})
         comp = hist = sums = table = hists = None
@@ -247,6 +255,31 @@ class Context:
             offs = np.concatenate([[0], np.cumsum(set_bins)])
             hists = [hist[:, offs[m]:offs[m + 1]] for m in range(len(set_bins))]
         return {"comp": comp, "hist": hist, "hists": hists, "sums": sums, "table": table}
+
+    def _profile_edges(self, reads, k, edges, want_table, use_loaded_table, out, keep_table, add_to_table):
+        n = reads.n_reads
+        out = dict(out or {})
+        comp = table = None
+        if k is not None:
+            comp = out.get("comp")
+            if comp is None:
+                comp = np.zeros((n, COMP_WIDTH[k]), dtype=np.uint32)
+        hist = out.get("hist")
+        if hist is None:
+            hist = np.zeros((n, edges.size + 1), dtype=np.uint32)
+        sums = out.get("sums")
+        if sums is None:
+            sums = np.zeros(n, dtype=np.uint32)
+        if want_table:
+            table = out.get("table")
+            if table is None:
+                table = np.empty(_lib.TABLE_ENTRIES, dtype=np.uint32)
+        flags = ((_lib.PROFILE_USE_LOADED_TABLE if use_loaded_table else 0) | (_lib.PROFILE_KEEP_TABLE if keep_table else 0) |
+                 (_lib.PROFILE_ADD_TO_TABLE if add_to_table else 0))
+        check(lib.lrb_profile_host_edges(self._h, reads._h, int(k) if k is not None else 0, _ptr(edges), int(edges.size),
+                                         _ptr(comp) if comp is not None else None, _ptr(hist), _ptr(sums),
+                                         _ptr(table) if table is not None else None, flags))
+        return {"comp": comp, "hist": hist, "hists": None, "sums": sums, "table": table}
 
     def info(self):
         """How the last profile() ran: devices, batches, table path, wall / exchange milliseconds."""
@@ -418,6 +451,52 @@ def spectrum_bin_mass(spectrum, bin_size, bins):
     return mass
 
 
+def spectrum_edge_mass(spectrum, edges):
+    """Windows per coverage bin implied by a spectrum for bins given by count edges (lrb_spectrum_edge_mass): equals
+    hist.sum(0) of Context.profile(edges=edges) over the reads the table was counted from."""
+    spec = np.ascontiguousarray(spectrum, dtype=np.uint64)
+    if spec.size < 3:
+        raise _lib.LrbError(_lib.LRB_EINVAL, "a spectrum has max_count + 3 words")
+    e = _edges_array(edges)
+    mass = np.zeros(e.size + 1, dtype=np.uint64)
+    check(lib.lrb_spectrum_edge_mass(_ptr(spec), spec.size - 3, _ptr(e), int(e.size), _ptr(mass)))
+    return mass
+
+
+def spectrum_quantile_edges(spectrum, bins):
+    """Count edges that split the windows of a spectrum (lrb_dev_table_spectrum layout) into `bins` bins of about equal
+    mass, the most information per column: with M = max_count, mass(c) = c * n_c for c < M and Total = the sum of the
+    masses plus the overflow keys' sum, t_i (i = 1 .. bins - 1) is the smallest c in [2, M] with
+    bins * sum_{c' < c} mass(c') >= i * Total, in exact integers.  The walk stops at the first i without such a c, and
+    repeated edges are dropped, so the result has at most bins - 1 strictly increasing edges: a single count holding more
+    than 1 / bins of the mass (or the mass above M) gives fewer bins than asked for."""
+    spec = np.ascontiguousarray(spectrum, dtype=np.uint64)
+    if spec.size < 3:
+        raise _lib.LrbError(_lib.LRB_EINVAL, "a spectrum has max_count + 3 words")
+    B = int(bins)
+    if not 1 <= B <= _lib.MAX_BINS:
+        raise _lib.LrbError(_lib.LRB_EINVAL, f"bins must be in [1, {_lib.MAX_BINS}] (got {B})")
+    M = spec.size - 3
+    nz = [int(c) for c in np.flatnonzero(spec[:M])]
+    total = sum(c * int(spec[c]) for c in nz) + int(spec[M + 1])
+    # prefix(c) = sum_{c' < c} mass(c') only grows just after a counted c0, so the candidates are 2 and every c0 + 1 > 2
+    steps = [(2, sum(c * int(spec[c]) for c in nz if c < 2))]
+    run = steps[0][1]
+    for c0 in nz:
+        if c0 >= 2:
+            run += c0 * int(spec[c0])
+            steps.append((c0 + 1, run))
+    edges, j = [], 0
+    for i in range(1, B):
+        while j < len(steps) and B * steps[j][1] < i * total:
+            j += 1
+        if j == len(steps):
+            break
+        if not edges or edges[-1] != steps[j][0]:
+            edges.append(steps[j][0])
+    return edges
+
+
 def dev_search(dr, table, bin_size, bins, hist, sums, tile_lo=0, tile_hi=None, key_lo=0, key_hi=_lib.TABLE_ENTRIES):
     check(lib.lrb_dev_search(C.byref(dr.view), C.c_void_p(table.data_ptr()), bin_size, bins, C.c_void_p(hist.data_ptr()),
                              C.c_void_p(sums.data_ptr()), tile_lo, dr.n_tiles if tile_hi is None else tile_hi, key_lo,
@@ -517,6 +596,30 @@ class PartitionWorkspace:
         check(lib.lrb_dev_partition_search_samples(C.byref(self.part), bucket_lo, 64 if bucket_hi is None else bucket_hi,
                                                    ptrs, len(tables), _ptr(bs), _ptr(bc), C.c_void_p(hist.data_ptr()),
                                                    C.c_void_p(sums.data_ptr()), _stream()))
+
+    def search_edges(self, table, edges, hist, sums, bucket_lo=0, bucket_hi=None):
+        """Search with bins given by count edges (lrb_dev_partition_search_edges): hist is [N, len(edges) + 1], hist and
+        sums zeroed by the caller as for apply(search=True)."""
+        e = _edges_array(edges)
+        check(lib.lrb_dev_partition_search_edges(C.byref(self.part), bucket_lo, 64 if bucket_hi is None else bucket_hi,
+                                                 C.c_void_p(table.data_ptr()), _ptr(e), int(e.size), C.c_void_p(hist.data_ptr()),
+                                                 C.c_void_p(sums.data_ptr()), _stream()))
+
+
+def _edges_array(edges):
+    """Count edges as a u32 array, refused (LRB_EINVAL) as the library refuses them: at most MAX_BINS - 1 values, strictly
+    increasing, the first >= 2."""
+    e = [int(x) for x in edges]
+    if len(e) > _lib.MAX_BINS - 1:
+        raise _lib.LrbError(_lib.LRB_EINVAL, f"the number of edges must be in [0, {_lib.MAX_BINS - 1}] (got {len(e)})")
+    if e and e[0] < 2:
+        raise _lib.LrbError(_lib.LRB_EINVAL, f"the first edge must be >= 2, so that counts 0 and 1 stay in bin 0 (got {e[0]})")
+    for i in range(1, len(e)):
+        if e[i] <= e[i - 1]:
+            raise _lib.LrbError(_lib.LRB_EINVAL, f"edges must be strictly increasing (edge {i} = {e[i]} after edge {i - 1} = {e[i - 1]})")
+    if e and e[-1] > 0xFFFFFFFF:
+        raise _lib.LrbError(_lib.LRB_EINVAL, f"edges are u32 counts (got {e[-1]})")
+    return np.array(e, dtype=np.uint32)
 
 
 def dev_table_compact(table, out=None):

@@ -92,6 +92,31 @@ def run_15mer_vecs_samples(reads_path, output, table_paths, bin_size, bin_count,
     check_proc(o, "Counting 15-mer profiles against several samples")
 
 
+def run_15mer_vecs_edges(reads_path, output, edges, threads, write_npy=False):
+    """Coverage profiles with bins given by count edges (lrb_search_15mers_edges): a window whose 15-mer is counted c times
+    in {output}/profiles/15mers-counts goes to bin searchsorted(edges, c, side="right"), for strictly increasing edges
+    with the first >= 2 (geometric edges, or profile.spectrum_quantile_edges of the table's spectrum).  Writes
+    {output}/profiles/cov_profs_edges (and .npy with write_npy), len(edges) + 1 values per read in the cov_profs format,
+    and the edges as one line to cov_profs_edges.edges.  cov_profs itself is never touched: copy the file to cov_profs
+    and resume from stage 3_1 (INTEGRATION.md).  No reference counterpart."""
+    from .profile import _edges_array
+    try:
+        e = _edges_array(edges)
+    except _lib.LrbError as err:   # refused like a library call: nothing written, the exit code of the refusal
+        logger.error(f"Error in step: Counting 15-mer profiles by edges ({err})")
+        sys.exit(err.code)
+    if not os.path.isdir(f"{output}/profiles"):
+        os.makedirs(f"{output}/profiles")
+    out = f"{output}/profiles/cov_profs_edges"
+    logger.debug(f"LIB::lrb_search_15mers_edges \"{output}/profiles/15mers-counts\" \"{reads_path}\" \"{out}\" {e.tolist()} {threads}")
+    o = _lib.lib.lrb_search_15mers_edges(os.fsencode(f"{output}/profiles/15mers-counts"), os.fsencode(reads_path),
+                                         e.ctypes.data_as(C.c_void_p), int(e.size), os.fsencode(out),
+                                         os.fsencode(out + ".npy") if write_npy else None, int(threads))
+    check_proc(o, "Counting 15-mer profiles by edges")
+    with open(out + ".edges", "w") as f:
+        f.write(" ".join(str(x) for x in e.tolist()) + "\n")
+
+
 def run_15mer_histo(output, threads, max_count=65536):
     """Abundance spectrum of {output}/profiles/15mers-counts as {output}/profiles/15mers-histo (jellyfish `histo`
     layout: "count n_kmers" lines of canonical 15-mers), to choose -bs / -bc from (INTEGRATION.md).  No reference
