@@ -238,16 +238,8 @@ namespace {
 
 struct Job {
     const lrb_reads* reads = nullptr;
-    int k = 0, P = 0, bins = 1;       // bins: width of a coverage row, the sum of the settings' bin counts
-    long bin_size = 1;                // setting 0's (the only one the direct search takes)
-    int n_set = 1;                    // coverage settings binned in one search (lrb_profile_host_settings)
-    long set_bs[LRB_MAX_COV_SETTINGS] = {1};
-    int set_bins[LRB_MAX_COV_SETTINGS] = {1};
-    int n_samp = 0;                   // > 0: coverage against these sample slots (lrb_profile_host_samples), setting t each
-    int samp_slot[LRB_MAX_SAMPLE_TABLES] = {};
-    bool by_edges = false;            // bins given by count edges (lrb_profile_host_edges): bins = n_edges + 1
-    const uint32_t* edges = nullptr;  // the caller's host array, alive for the call
-    int n_edges = 0;
+    int k = 0, P = 0;
+    CovLayout cov;                    // the coverage row (checked); compact blocks read sample slots b[m].table
     uint32_t *comp = nullptr, *hist = nullptr, *sums = nullptr, *table_host = nullptr;
     bool do_comp = false, do_search = false, do_count = false, use_loaded = false, add_to_table = false;
     bool use_part = true, want_smem_env = false, force_l2 = false, comp_pinned = false;
@@ -285,7 +277,7 @@ uint64_t batch_bytes(const Job& J, uint64_t blocks, uint64_t reads, uint64_t til
     uint64_t b = blocks * 12 + 64;                                        // codes + valid
     b += reads * 8 + tiles * 8 + 64;                                      // read_len, read_blk, tiles
     if (J.do_comp) b += reads * 4ull * J.P;
-    if (J.do_search) b += reads * 4ull * (J.bins + 1);
+    if (J.do_search) b += reads * 4ull * (J.cov.W + 1);
     if (J.use_part && (J.do_count || J.do_search)) {
         b += blocks * 128 + blocks * 4;                                   // 4 B per slot of list entries, blk_read
         b += 4ull * lrb_partition_steps_words(lrb_partition_step_capacity(blocks, LRB_PART_MAX_CHUNKS));
@@ -305,7 +297,7 @@ int reserve_batch(lrb_ctx* c, const lrb_reads* r, const Job& J, bool want_count_
     if ((rc = c->tile_blk.reserve(sizeof(uint32_t) * (nt + 1)))) return rc;
     if (J.do_comp && (rc = c->comp.reserve(std::max<size_t>(16, sizeof(uint32_t) * n * J.P)))) return rc;
     if (J.do_search) {
-        if ((rc = c->hist.reserve(std::max<size_t>(16, sizeof(uint32_t) * n * (size_t)J.bins)))) return rc;
+        if ((rc = c->hist.reserve(std::max<size_t>(16, sizeof(uint32_t) * n * (size_t)J.cov.W)))) return rc;
         if ((rc = c->sums.reserve(std::max<size_t>(16, sizeof(uint32_t) * n)))) return rc;
     }
     if ((rc = c->exc_blk.reserve(sizeof(uint32_t) * (r->n_exc + 1)))) return rc;
@@ -469,7 +461,7 @@ int stage_front(lrb_ctx* c, const lrb_reads* r, const Job& J, uint64_t row0, boo
     if (J.do_count && lists) {
         // ONE launch over all buckets when the second-level lists exist (no per-bucket tails), else RED.ADD per bucket
         const int mode = (c->part.sub ? (1 | 4) : 1) | (count_writes ? 8 : 0);
-        if ((rc = lrb_dev_partition_apply(&c->part, mode, (uint32_t*)c->table.p, J.bin_size, J.bins, nullptr, nullptr, st))) return rc;
+        if ((rc = lrb_dev_partition_apply(&c->part, mode, (uint32_t*)c->table.p, 1, 1, nullptr, nullptr, st))) return rc;
     }
     return LRB_OK;
 }
@@ -477,26 +469,16 @@ int stage_front(lrb_ctx* c, const lrb_reads* r, const Job& J, uint64_t row0, boo
 // Pass 2: coverage rows of the batch's reads against the device's (finished) table, buckets [b_lo, b_hi) of the lists.
 int search_lists(lrb_ctx* c, const Job& J, uint64_t n, int b_lo, int b_hi) {
     if (!n) return LRB_OK;
-    if (J.by_edges)
-        return lrb_dev_partition_search_edges(&c->part, b_lo, b_hi, (const uint32_t*)c->table.p, J.edges, J.n_edges, (uint32_t*)c->hist.p,
-                                              (uint32_t*)c->sums.p, c->stream);
-    if (J.n_samp) {
-        const uint32_t* tabs[LRB_MAX_SAMPLE_TABLES];
-        for (int t = 0; t < J.n_samp; ++t) tabs[t] = (const uint32_t*)c->sample[J.samp_slot[t]].p;
-        return lrb_dev_partition_search_samples(&c->part, b_lo, b_hi, tabs, J.n_samp, J.set_bs, J.set_bins, (uint32_t*)c->hist.p,
-                                                (uint32_t*)c->sums.p, c->stream);
-    }
-    if (J.n_set > 1)
-        return lrb_dev_partition_search_settings(&c->part, b_lo, b_hi, (const uint32_t*)c->table.p, J.n_set, J.set_bs, J.set_bins,
-                                                 (uint32_t*)c->hist.p, (uint32_t*)c->sums.p, c->stream);
-    return lrb_dev_partition_apply_range(&c->part, 2, b_lo, b_hi, (uint32_t*)c->table.p, J.bin_size, J.bins, (uint32_t*)c->hist.p,
-                                         (uint32_t*)c->sums.p, c->stream);
+    const uint32_t* slots[LRB_MAX_SAMPLE_TABLES];
+    for (int t = 0; t < LRB_MAX_SAMPLE_TABLES; ++t) slots[t] = (const uint32_t*)c->sample[t].p;
+    return lrb_partition_search("lrb_profile_host", &c->part, b_lo, b_hi, (const uint32_t*)c->table.p, slots, J.cov, (uint32_t*)c->hist.p,
+                                (uint32_t*)c->sums.p, c->stream);
 }
 
 int rows_home(lrb_ctx* c, const Job& J, uint64_t n, uint64_t row0) {
     cudaStream_t st = c->stream;
     if (J.do_search && n) {
-        CTX_CUDA(cudaMemcpyAsync(J.hist + (size_t)row0 * J.bins, c->hist.p, sizeof(uint32_t) * n * (size_t)J.bins, cudaMemcpyDeviceToHost, st));
+        CTX_CUDA(cudaMemcpyAsync(J.hist + (size_t)row0 * J.cov.W, c->hist.p, sizeof(uint32_t) * n * (size_t)J.cov.W, cudaMemcpyDeviceToHost, st));
         CTX_CUDA(cudaMemcpyAsync(J.sums + row0, c->sums.p, sizeof(uint32_t) * n, cudaMemcpyDeviceToHost, st));
     }
     CTX_CUDA(cudaStreamWaitEvent(st, c->sync_ev[LRB_PART_MAX_CHUNKS + 1], 0));  // join the copy_out stream (early composition D2H)
@@ -649,73 +631,38 @@ static bool direct_table_path() {   // one random HBM access per window (kernels
     return e && !strcmp(e, "direct");
 }
 
-// slot numbers in range, then the settings of the tables, the same slot with the same setting twice refused
-static int check_sample_slots(int n, const int* slots, const long* bin_sizes, const int* bins, uint32_t* W) {
-    uint64_t ids[LRB_MAX_SAMPLE_TABLES] = {};
-    for (int t = 0; t < n && t < LRB_MAX_SAMPLE_TABLES; ++t) {
-        if (slots[t] < 0 || slots[t] >= LRB_MAX_SAMPLE_TABLES)
-            return lrb_set_error(LRB_EINVAL, "lrb_profile_host_samples: slot must be in [0, %d) (table %d: got %d)", LRB_MAX_SAMPLE_TABLES, t, slots[t]);
-        ids[t] = (uint64_t)slots[t];
-    }
-    return lrb_check_table_settings("lrb_profile_host_samples", n, ids, bin_sizes, bins, W);
+// The direct search takes one (bin_size, bins) block of the full-layout table.
+static int refuse_direct(const char* who, const CovLayout& cov) {
+    if (cov.single() || !direct_table_path()) return LRB_OK;
+    char what[32];
+    if (cov.compact) snprintf(what, sizeof what, "sample tables");
+    else if (cov.b[0].by_edges) snprintf(what, sizeof what, "count edges");
+    else snprintf(what, sizeof what, "%d settings", cov.n);
+    return lrb_set_error(LRB_EINVAL, "%s: LRB_TABLE_PATH=direct searches the full-layout table with one (bin_size, bins) setting per call, not %s",
+                         who, what);
 }
 
-// Bins given by count edges instead of (bin size, bin count) settings (lrb_profile_host_edges).
-struct EdgeBins {
-    const uint32_t* edges;
-    int n;
-};
-
-// slots: NULL, or the sample slot of each of the n_set settings (coverage against those instead of the context's table);
-// eb: NULL, or the count edges that bin the coverage instead of the settings (n_set, bin_sizes and bins are then unused)
-static int profile_host(lrb_ctx* c, const lrb_reads* r, int k, int n_set, const long* bin_sizes, const int* bins, const int* slots,
-                        uint32_t* comp_counts, uint32_t* cov_hist, uint32_t* cov_sums, uint32_t* table_host, int flags,
-                        const EdgeBins* eb = nullptr) {
+// cov: checked (lrb_check_cov_layout); a compact layout searches the sample slots b[t].table instead of the context's table
+static int profile_host(const char* who, lrb_ctx* c, const lrb_reads* r, int k, const CovLayout& cov, uint32_t* comp_counts,
+                        uint32_t* cov_hist, uint32_t* cov_sums, uint32_t* table_host, int flags) {
     Job J;
     J.reads = r; J.k = k; J.P = comp_width(k);
     J.comp = comp_counts; J.hist = cov_hist; J.sums = cov_sums; J.table_host = table_host;
+    J.cov = cov;
     J.do_comp = comp_counts != nullptr;
     if (J.do_comp && !J.P) return lrb_set_error(LRB_EINVAL, "k must be 3, 4 or 5 (got %d)", k);
     J.do_search = cov_hist || cov_sums;
     if (J.do_search && (!cov_hist || !cov_sums)) return lrb_set_error(LRB_EINVAL, "cov_hist and cov_sums go together");
-    if (slots && !J.do_search) return lrb_set_error(LRB_EINVAL, "lrb_profile_host_samples: sample tables need cov_hist and cov_sums");
-    if (J.do_search) {
-        uint32_t W = 0;
-        int rc;
-        if (slots) {
-            if ((rc = check_sample_slots(n_set, slots, bin_sizes, bins, &W))) return rc;
-            for (int t = 0; t < n_set; ++t)
-                if (!c->sample_ready[slots[t]]) return lrb_set_error(LRB_EINVAL, "lrb_profile_host_samples: sample slot %d is empty (table %d)", slots[t], t);
-            if (direct_table_path())
-                return lrb_set_error(LRB_EINVAL, "lrb_profile_host_samples: LRB_TABLE_PATH=direct reads only the full-layout table, not sample slots");
-            J.n_samp = n_set;
-            std::copy(slots, slots + n_set, J.samp_slot);
-        } else if (eb) {
-            if ((rc = lrb_check_cov_edges("lrb_profile_host_edges", eb->edges, eb->n))) return rc;
-            if (direct_table_path())
-                return lrb_set_error(LRB_EINVAL, "lrb_profile_host_edges: LRB_TABLE_PATH=direct bins by bin size and count only, not by edges");
-            J.by_edges = true;
-            J.edges = eb->edges;
-            J.n_edges = eb->n;
-            W = (uint32_t)eb->n + 1u;
-        } else if ((rc = lrb_check_cov_settings("lrb_profile_host", n_set, bin_sizes, bins, &W))) {
-            return rc;
-        }
-        if (!eb) {
-            if (n_set > 1 && direct_table_path())
-                return lrb_set_error(LRB_EINVAL, "LRB_TABLE_PATH=direct searches one coverage setting per call (%d settings asked for)", n_set);
-            J.n_set = n_set;
-            std::copy(bin_sizes, bin_sizes + n_set, J.set_bs);
-            std::copy(bins, bins + n_set, J.set_bins);
-            J.bin_size = bin_sizes[0];
-        }
-        J.bins = (int)W;
-    }
+    if (cov.compact && !J.do_search) return lrb_set_error(LRB_EINVAL, "%s: sample tables need cov_hist and cov_sums", who);
+    for (int t = 0; cov.compact && t < cov.n; ++t)
+        if (!c->sample_ready[cov.b[t].table]) return lrb_set_error(LRB_EINVAL, "%s: sample slot %d is empty (table %d)", who, cov.b[t].table, t);
+    int rc;
+    if (J.do_search && (rc = refuse_direct(who, cov))) return rc;
     J.use_loaded = (flags & LRB_PROFILE_USE_LOADED_TABLE) != 0;
     J.add_to_table = (flags & LRB_PROFILE_ADD_TO_TABLE) != 0;
     if (J.use_loaded && J.add_to_table) return lrb_set_error(LRB_EINVAL, "LRB_PROFILE_USE_LOADED_TABLE and LRB_PROFILE_ADD_TO_TABLE exclude each other");
     if ((J.use_loaded || J.add_to_table) && !c->table_ready) return lrb_set_error(LRB_EINVAL, "no table loaded in this context");
-    J.do_count = !J.use_loaded && ((J.do_search && !J.n_samp) || table_host || (flags & (LRB_PROFILE_KEEP_TABLE | LRB_PROFILE_ADD_TO_TABLE)));
+    J.do_count = !J.use_loaded && ((J.do_search && !cov.compact) || table_host || (flags & (LRB_PROFILE_KEEP_TABLE | LRB_PROFILE_ADD_TO_TABLE)));
     {
         if (direct_table_path()) J.use_part = false;
         const char* e = getenv("LRB_COUNT_PATH");
@@ -728,7 +675,7 @@ static int profile_host(lrb_ctx* c, const lrb_reads* r, int k, int n_set, const 
     J.comp_pinned = host_ptr_is_pinned(comp_counts);
     const auto wall0 = std::chrono::steady_clock::now();
     const uint64_t n = r->n_reads, nb = r->n_blocks;
-    const bool need_table = J.do_count || (J.do_search && !J.n_samp);   // sample slots are allocated already
+    const bool need_table = J.do_count || (J.do_search && !cov.compact);   // sample slots are allocated already
 
     // ---- devices and their read ranges (contiguous, balanced by blocks) ------------------------------------------
     std::vector<DevPlan> plans;
@@ -758,7 +705,7 @@ static int profile_host(lrb_ctx* c, const lrb_reads* r, int k, int n_set, const 
     const bool multi = D > 1;
 
     // ---- tables first, then size the batches against what is left --------------------------------------------------
-    int rc = on_devices(plans, [&](DevPlan& p) -> int {
+    rc = on_devices(plans, [&](DevPlan& p) -> int {
         CTX_CUDA(cudaSetDevice(p.c->device));
         int rc2;
         if (need_table && (rc2 = p.c->table.reserve(sizeof(uint32_t) * (size_t)kTableEntries))) return rc2;
@@ -825,7 +772,7 @@ static int profile_host(lrb_ctx* c, const lrb_reads* r, int k, int n_set, const 
     // Adding to the table: device 0 counts into its complete table, every other device into a private table from zero, so
     // that after the exchange  sum over devices of the canonical halves = previous table + this read set;  the mirror then
     // rebuilds the other half on device 0 as for any count.
-    c->table_ready = (J.use_loaded || (J.n_samp && !J.do_count)) ? c->table_ready : false;   // a search of sample slots leaves it
+    c->table_ready = (J.use_loaded || (cov.compact && !J.do_count)) ? c->table_ready : false;   // a search of sample slots leaves it
     if (J.use_loaded && multi) {   // the loaded table lives on device 0: hand it to the others
         CTX_CUDA(cudaSetDevice(c->device));
         CTX_CUDA(cudaEventRecord(c->counted, c->stream));
@@ -889,7 +836,7 @@ static int profile_host(lrb_ctx* c, const lrb_reads* r, int k, int n_set, const 
             // resident table slice — the search goes from 20.5 to 26.2 ms to hide a 1.26 ms pass.
             const bool mirror_here = J.do_count && (x == c || !J.use_part);
             if (J.do_search && nr) {
-                CTX_CUDA(cudaMemsetAsync(x->hist.p, 0, sizeof(uint32_t) * nr * (size_t)J.bins, st));
+                CTX_CUDA(cudaMemsetAsync(x->hist.p, 0, sizeof(uint32_t) * nr * (size_t)J.cov.W, st));
                 CTX_CUDA(cudaMemsetAsync(x->sums.p, 0, sizeof(uint32_t) * nr, st));
             }
             if (J.do_search && J.use_part && p.kept->n_blocks) {
@@ -910,7 +857,7 @@ static int profile_host(lrb_ctx* c, const lrb_reads* r, int k, int n_set, const 
             if (mirror_here && (rc2 = lrb_dev_mirror((uint32_t*)x->table.p, st))) return rc2;
             if (x == c) CTX_CUDA(cudaEventRecord(c->ev[4], st));
             if (!J.use_part && J.do_search && nr &&
-                (rc2 = lrb_dev_search(&x->dview, (const uint32_t*)x->table.p, J.bin_size, J.bins, (uint32_t*)x->hist.p, (uint32_t*)x->sums.p, 0,
+                (rc2 = lrb_dev_search(&x->dview, (const uint32_t*)x->table.p, J.cov.b[0].bin_size, J.cov.W, (uint32_t*)x->hist.p, (uint32_t*)x->sums.p, 0,
                                       p.kept->n_tiles, 0, kTableEntries, st)))
                 return rc2;
             if (x == c) CTX_CUDA(cudaEventRecord(c->ev[5], st));
@@ -930,11 +877,11 @@ static int profile_host(lrb_ctx* c, const lrb_reads* r, int k, int n_set, const 
                 const uint64_t nr = s->n_reads;
                 rc2 = stage_front(x, s, S, b.r0, /*with_rids=*/true, false, false);
                 if (!rc2 && nr) {
-                    cudaMemsetAsync(x->hist.p, 0, sizeof(uint32_t) * nr * (size_t)J.bins, st);
+                    cudaMemsetAsync(x->hist.p, 0, sizeof(uint32_t) * nr * (size_t)J.cov.W, st);
                     cudaMemsetAsync(x->sums.p, 0, sizeof(uint32_t) * nr, st);
                     if (J.use_part && s->n_blocks) rc2 = search_lists(x, J, nr, 0, n_buckets);
                     else if (!J.use_part)
-                        rc2 = lrb_dev_search(&x->dview, (const uint32_t*)x->table.p, J.bin_size, J.bins, (uint32_t*)x->hist.p, (uint32_t*)x->sums.p, 0,
+                        rc2 = lrb_dev_search(&x->dview, (const uint32_t*)x->table.p, J.cov.b[0].bin_size, J.cov.W, (uint32_t*)x->hist.p, (uint32_t*)x->sums.p, 0,
                                              s->n_tiles, 0, kTableEntries, st);
                 }
                 if (!rc2) rc2 = rows_home(x, J, nr, b.r0) || sync_ctx(x);
@@ -969,36 +916,36 @@ static int profile_host(lrb_ctx* c, const lrb_reads* r, int k, int n_set, const 
     return LRB_OK;
 }
 
+// The public profile calls: the coverage layout is checked before the context, so that no device is needed to refuse it,
+// and a failed LRB_PROFILE_ADD_TO_TABLE call leaves the context without a table (it may hold part of the read set).
+static int profile_call(const char* who, lrb_ctx* c, const lrb_reads* r, int k, CovLayout cov, uint32_t* comp_counts, uint32_t* cov_hist,
+                        uint32_t* cov_sums, uint32_t* table_host, int flags) {
+    if (!r) return lrb_set_error(LRB_EINVAL, "%s: null argument", who);
+    int rc = lrb_check_cov_layout(who, &cov);
+    if (!rc && !c) return lrb_set_error(LRB_EINVAL, "%s: null context", who);
+    if (!rc) rc = profile_host(who, c, r, k, cov, comp_counts, cov_hist, cov_sums, table_host, flags);
+    if (rc && c && (flags & LRB_PROFILE_ADD_TO_TABLE)) c->table_ready = false;
+    return rc;
+}
+
 extern "C" int lrb_profile_host_settings(lrb_ctx* c, const lrb_reads* r, int k, int n, const long* bin_sizes, const int* bins,
                                          uint32_t* comp_counts, uint32_t* cov_hist, uint32_t* cov_sums, uint32_t* table_host, int flags) {
-    if (!c || !r) return lrb_set_error(LRB_EINVAL, "lrb_profile_host: null argument");
-    const int rc = profile_host(c, r, k, n, bin_sizes, bins, nullptr, comp_counts, cov_hist, cov_sums, table_host, flags);
-    if (rc && (flags & LRB_PROFILE_ADD_TO_TABLE)) c->table_ready = false;   // the table may hold part of this read set
-    return rc;
+    // without coverage rows the settings are not used, and not checked
+    const CovLayout cov = cov_hist || cov_sums ? lrb_cov_settings(n, bin_sizes, bins) : CovLayout{};
+    return profile_call("lrb_profile_host", c, r, k, cov, comp_counts, cov_hist, cov_sums, table_host, flags);
 }
 
 extern "C" int lrb_profile_host_samples(lrb_ctx* c, const lrb_reads* r, int k, int n, const int* slots, const long* bin_sizes,
                                         const int* bins, uint32_t* comp_counts, uint32_t* cov_hist, uint32_t* cov_sums, uint32_t* table_host,
                                         int flags) {
-    if (!r || !slots) return lrb_set_error(LRB_EINVAL, "lrb_profile_host_samples: null argument");
-    int rc = check_sample_slots(n, slots, bin_sizes, bins, nullptr);   // before the context: no device needed to refuse
-    if (rc) return rc;
-    if (!c) return lrb_set_error(LRB_EINVAL, "lrb_profile_host_samples: null context");
-    rc = profile_host(c, r, k, n, bin_sizes, bins, slots, comp_counts, cov_hist, cov_sums, table_host, flags);
-    if (rc && (flags & LRB_PROFILE_ADD_TO_TABLE)) c->table_ready = false;
-    return rc;
+    if (!slots) return lrb_set_error(LRB_EINVAL, "lrb_profile_host_samples: null argument");
+    return profile_call("lrb_profile_host_samples", c, r, k, lrb_cov_settings(n, bin_sizes, bins, slots), comp_counts, cov_hist, cov_sums,
+                        table_host, flags);
 }
 
 extern "C" int lrb_profile_host_edges(lrb_ctx* c, const lrb_reads* r, int k, const uint32_t* edges, int n_edges, uint32_t* comp_counts,
                                       uint32_t* cov_hist, uint32_t* cov_sums, uint32_t* table_host, int flags) {
-    if (!r) return lrb_set_error(LRB_EINVAL, "lrb_profile_host_edges: null argument");
-    int rc = lrb_check_cov_edges("lrb_profile_host_edges", edges, n_edges);   // before the context: no device needed to refuse
-    if (rc) return rc;
-    if (!c) return lrb_set_error(LRB_EINVAL, "lrb_profile_host_edges: null context");
-    const EdgeBins eb{edges, n_edges};
-    rc = profile_host(c, r, k, 1, nullptr, nullptr, nullptr, comp_counts, cov_hist, cov_sums, table_host, flags, &eb);
-    if (rc && (flags & LRB_PROFILE_ADD_TO_TABLE)) c->table_ready = false;
-    return rc;
+    return profile_call("lrb_profile_host_edges", c, r, k, lrb_cov_edges(edges, n_edges), comp_counts, cov_hist, cov_sums, table_host, flags);
 }
 
 extern "C" int lrb_profile_host(lrb_ctx* c, const lrb_reads* r, int k, long bin_size, int bins, uint32_t* comp_counts,
@@ -1490,23 +1437,27 @@ extern "C" int lrb_count_15mers(const char* reads_path, const char* out_table, i
     return lrb_ctx_table_save(cg.c, out_table);
 }
 
-extern "C" int lrb_search_15mers(const char* table_path, const char* reads_path, const char* out_txt, long bin_size,
-                                 int bins, int threads) {
-    if (!table_path || !reads_path || !out_txt) return lrb_set_error(LRB_EINVAL, "lrb_search_15mers: null path");
-    if (bin_size <= 0) return lrb_set_error(LRB_EINVAL, "bin_size must be >= 1 (the reference divides by it)");
-    if (bins <= 0 || bins > LRB_MAX_BINS) return lrb_set_error(LRB_EINVAL, "bins must be in [1, %d]", LRB_MAX_BINS);
-    int rc;
+namespace {
+
+// The file-level searches: the coverage rows of every read of reads_path against the table(s) load(context) brings into a
+// new context, segment by segment; write(hist, sums, n_reads, row0) appends a segment's rows to the outputs, the n_outs
+// files of outs truncated first.  cov is checked; its compact blocks read the sample slots load() fills.
+template <class Load, class Write>
+int search_file(const char* who, const CovLayout& cov, const char* reads_path, const char* const* outs, int n_outs, int threads, Load load,
+                Write write) {
+    int rc = refuse_direct(who, cov);   // before any file or device work
+    if (rc) return rc;
     CtxGuard cg;
-    if ((rc = create_ctx(0, &cg.c))) return rc;
-    if ((rc = lrb_ctx_table_load(cg.c, table_path))) return rc;
-    if ((rc = truncate_file(out_txt))) return rc;
+    if ((rc = create_ctx(0, &cg.c)) || (rc = load(cg.c))) return rc;
+    for (int i = 0; i < n_outs; ++i)
+        if ((rc = truncate_file(outs[i]))) return rc;
     Input in;
-    if ((rc = open_input(reads_path, threads, 4ull * ((uint64_t)bins + 1), in))) return rc;
+    if ((rc = open_input(reads_path, threads, 4ull * ((uint64_t)cov.W + 1), in))) return rc;
     auto search = [&](const lrb_reads* s, uint64_t row0) -> int {
         const uint64_t n = s->n_reads;
-        std::vector<uint32_t> hist((size_t)n * bins + 1), sums(n + 1);
-        const int rc2 = lrb_profile_host(cg.c, s, 0, bin_size, bins, nullptr, hist.data(), sums.data(), nullptr, LRB_PROFILE_USE_LOADED_TABLE);
-        return rc2 ? rc2 : lrb_append_coverage_txt(out_txt, hist.data(), sums.data(), n, bins, threads, row0);
+        std::vector<uint32_t> hist((size_t)n * cov.W + 1), sums(n + 1);
+        const int rc2 = profile_call(who, cg.c, s, 0, cov, nullptr, hist.data(), sums.data(), nullptr, cov.compact ? 0 : LRB_PROFILE_USE_LOADED_TABLE);
+        return rc2 ? rc2 : write(hist.data(), sums.data(), n, row0);
     };
     if (in.whole) return search(in.whole, 0);
     if ((rc = each_segment(in, false, search))) return rc;
@@ -1514,110 +1465,90 @@ extern "C" int lrb_search_15mers(const char* table_path, const char* reads_path,
     return LRB_OK;
 }
 
+// writer of search_file: rows whole, as "%f" text and, when out_npy is given, .npy
+auto whole_rows(const char* out_txt, const char* out_npy, uint32_t W, int threads) {
+    return [=](const uint32_t* hist, const uint32_t* sums, uint64_t n, uint64_t row0) -> int {
+        int rc = lrb_append_coverage_txt(out_txt, hist, sums, n, (int)W, threads, row0);
+        if (!rc && out_npy) rc = lrb_append_coverage_npy(out_npy, hist, sums, n, (int)W, threads, row0);
+        return rc;
+    };
+}
+
+}  // namespace
+
+extern "C" int lrb_search_15mers(const char* table_path, const char* reads_path, const char* out_txt, long bin_size,
+                                 int bins, int threads) {
+    static const char* who = "lrb_search_15mers";
+    if (!table_path || !reads_path || !out_txt) return lrb_set_error(LRB_EINVAL, "%s: null path", who);
+    CovLayout cov = lrb_cov_settings(1, &bin_size, &bins);
+    const int rc = lrb_check_cov_layout(who, &cov);
+    if (rc) return rc;
+    return search_file(who, cov, reads_path, &out_txt, 1, threads, [&](lrb_ctx* c) { return lrb_ctx_table_load(c, table_path); },
+                       whole_rows(out_txt, nullptr, cov.W, threads));
+}
+
 extern "C" int lrb_search_15mers_settings(const char* table_path, const char* reads_path, int n, const long* bin_sizes, const int* bins,
                                           const char* const* out_txts, const char* const* out_npys, int threads) {
-    if (!table_path || !reads_path || !out_txts) return lrb_set_error(LRB_EINVAL, "lrb_search_15mers_settings: null path");
-    uint32_t W = 0;
-    int rc = lrb_check_cov_settings("lrb_search_15mers_settings", n, bin_sizes, bins, &W);
+    static const char* who = "lrb_search_15mers_settings";
+    if (!table_path || !reads_path || !out_txts) return lrb_set_error(LRB_EINVAL, "%s: null path", who);
+    CovLayout cov = lrb_cov_settings(n, bin_sizes, bins);
+    const int rc = lrb_check_cov_layout(who, &cov);
     if (rc) return rc;
     for (int m = 0; m < n; ++m)
-        if (!out_txts[m]) return lrb_set_error(LRB_EINVAL, "lrb_search_15mers_settings: null output path (setting %d)", m);
-    if (n > 1 && direct_table_path())
-        return lrb_set_error(LRB_EINVAL, "LRB_TABLE_PATH=direct searches one coverage setting per call (%d settings asked for)", n);
-    CtxGuard cg;
-    if ((rc = create_ctx(0, &cg.c))) return rc;
-    if ((rc = lrb_ctx_table_load(cg.c, table_path))) return rc;
-    for (int m = 0; m < n; ++m)
-        if ((rc = truncate_file(out_txts[m]))) return rc;
-    Input in;
-    if ((rc = open_input(reads_path, threads, 4ull * ((uint64_t)W + 1), in))) return rc;
+        if (!out_txts[m]) return lrb_set_error(LRB_EINVAL, "%s: null output path (setting %d)", who, m);
     // rows of W words come back; each file gets its setting's columns, so the writers are those of lrb_search_15mers
-    auto search = [&](const lrb_reads* s, uint64_t row0) -> int {
-        const uint64_t nr = s->n_reads;
-        std::vector<uint32_t> hist((size_t)nr * W + 1), sums(nr + 1), one;
-        int rc2 = lrb_profile_host_settings(cg.c, s, 0, n, bin_sizes, bins, nullptr, hist.data(), sums.data(), nullptr, LRB_PROFILE_USE_LOADED_TABLE);
+    std::vector<uint32_t> one;
+    auto split = [&](const uint32_t* hist, const uint32_t* sums, uint64_t nr, uint64_t row0) -> int {
+        int rc2 = LRB_OK;
         for (int m = 0, off = 0; m < n && !rc2; off += bins[m], ++m) {
             const size_t B = (size_t)bins[m];
             one.resize(nr * B + 1);
-            for (uint64_t r = 0; r < nr; ++r) std::copy_n(hist.data() + r * W + off, B, one.data() + r * B);
-            rc2 = lrb_append_coverage_txt(out_txts[m], one.data(), sums.data(), nr, bins[m], threads, row0);
-            if (!rc2 && out_npys && out_npys[m]) rc2 = lrb_append_coverage_npy(out_npys[m], one.data(), sums.data(), nr, bins[m], threads, row0);
+            for (uint64_t r = 0; r < nr; ++r) std::copy_n(hist + r * cov.W + off, B, one.data() + r * B);
+            rc2 = lrb_append_coverage_txt(out_txts[m], one.data(), sums, nr, bins[m], threads, row0);
+            if (!rc2 && out_npys && out_npys[m]) rc2 = lrb_append_coverage_npy(out_npys[m], one.data(), sums, nr, bins[m], threads, row0);
         }
         return rc2;
     };
-    if (in.whole) return search(in.whole, 0);
-    if ((rc = each_segment(in, false, search))) return rc;
-    segments_notice(in, 1);
-    return LRB_OK;
+    return search_file(who, cov, reads_path, out_txts, n, threads, [&](lrb_ctx* c) { return lrb_ctx_table_load(c, table_path); }, split);
 }
 
 extern "C" int lrb_search_15mers_samples(const char* const* table_paths, int n, const long* bin_sizes, const int* bins, const char* reads_path,
                                          const char* out_txt, const char* out_npy, int threads) {
     static const char* who = "lrb_search_15mers_samples";
     if (!table_paths || !reads_path || !out_txt) return lrb_set_error(LRB_EINVAL, "%s: null path", who);
-    // slot of each table: the first entry with the same path string (a table listed twice is loaded once)
-    uint64_t ids[LRB_MAX_SAMPLE_TABLES] = {};
+    // slot of each table, numbered in order of first appearance: a table listed twice (the same path string) is loaded once
     int slots[LRB_MAX_SAMPLE_TABLES] = {}, n_slots = 0;
     for (int t = 0; t < n && t < LRB_MAX_SAMPLE_TABLES; ++t) {
         if (!table_paths[t]) return lrb_set_error(LRB_EINVAL, "%s: null table path (table %d)", who, t);
         int j = 0;
         while (j < t && strcmp(table_paths[j], table_paths[t])) ++j;
-        ids[t] = (uint64_t)j;
         slots[t] = j == t ? n_slots++ : slots[j];
     }
-    uint32_t W = 0;
-    int rc = lrb_check_table_settings(who, n, ids, bin_sizes, bins, &W);
+    CovLayout cov = lrb_cov_settings(n, bin_sizes, bins, slots);
+    const int rc = lrb_check_cov_layout(who, &cov);
     if (rc) return rc;
-    if (direct_table_path()) return lrb_set_error(LRB_EINVAL, "%s: LRB_TABLE_PATH=direct reads only the full-layout table, not sample slots", who);
-    CtxGuard cg;
-    if ((rc = create_ctx(0, &cg.c))) return rc;
-    for (int t = 0; t < n; ++t)
-        if (ids[t] == (uint64_t)t && (rc = lrb_ctx_sample_table_load(cg.c, slots[t], table_paths[t]))) return rc;
-    if ((rc = truncate_file(out_txt))) return rc;
-    Input in;
-    if ((rc = open_input(reads_path, threads, 4ull * ((uint64_t)W + 1), in))) return rc;
+    auto load = [&](lrb_ctx* c) -> int {
+        for (int t = 0, next = 0; t < n; ++t)
+            if (slots[t] == next) {
+                const int rc2 = lrb_ctx_sample_table_load(c, next++, table_paths[t]);
+                if (rc2) return rc2;
+            }
+        return LRB_OK;
+    };
     // every block of a row is normalised by the same sums (the read's valid windows), so the writers of one table apply at
     // width W and the line is the n single-table lines joined by one space
-    auto search = [&](const lrb_reads* s, uint64_t row0) -> int {
-        const uint64_t nr = s->n_reads;
-        std::vector<uint32_t> hist((size_t)nr * W + 1), sums(nr + 1);
-        int rc2 = lrb_profile_host_samples(cg.c, s, 0, n, slots, bin_sizes, bins, nullptr, hist.data(), sums.data(), nullptr, 0);
-        if (!rc2) rc2 = lrb_append_coverage_txt(out_txt, hist.data(), sums.data(), nr, (int)W, threads, row0);
-        if (!rc2 && out_npy) rc2 = lrb_append_coverage_npy(out_npy, hist.data(), sums.data(), nr, (int)W, threads, row0);
-        return rc2;
-    };
-    if (in.whole) return search(in.whole, 0);
-    if ((rc = each_segment(in, false, search))) return rc;
-    segments_notice(in, 1);
-    return LRB_OK;
+    return search_file(who, cov, reads_path, &out_txt, 1, threads, load, whole_rows(out_txt, out_npy, cov.W, threads));
 }
 
 extern "C" int lrb_search_15mers_edges(const char* table_path, const char* reads_path, const uint32_t* edges, int n_edges,
                                        const char* out_txt, const char* out_npy, int threads) {
     static const char* who = "lrb_search_15mers_edges";
     if (!table_path || !reads_path || !out_txt) return lrb_set_error(LRB_EINVAL, "%s: null path", who);
-    int rc = lrb_check_cov_edges(who, edges, n_edges);
+    CovLayout cov = lrb_cov_edges(edges, n_edges);
+    const int rc = lrb_check_cov_layout(who, &cov);
     if (rc) return rc;
-    if (direct_table_path()) return lrb_set_error(LRB_EINVAL, "%s: LRB_TABLE_PATH=direct bins by bin size and count only, not by edges", who);
-    const int B = n_edges + 1;
-    CtxGuard cg;
-    if ((rc = create_ctx(0, &cg.c))) return rc;
-    if ((rc = lrb_ctx_table_load(cg.c, table_path))) return rc;
-    if ((rc = truncate_file(out_txt))) return rc;
-    Input in;
-    if ((rc = open_input(reads_path, threads, 4ull * ((uint64_t)B + 1), in))) return rc;
-    auto search = [&](const lrb_reads* s, uint64_t row0) -> int {
-        const uint64_t n = s->n_reads;
-        std::vector<uint32_t> hist((size_t)n * B + 1), sums(n + 1);
-        int rc2 = lrb_profile_host_edges(cg.c, s, 0, edges, n_edges, nullptr, hist.data(), sums.data(), nullptr, LRB_PROFILE_USE_LOADED_TABLE);
-        if (!rc2) rc2 = lrb_append_coverage_txt(out_txt, hist.data(), sums.data(), n, B, threads, row0);
-        if (!rc2 && out_npy) rc2 = lrb_append_coverage_npy(out_npy, hist.data(), sums.data(), n, B, threads, row0);
-        return rc2;
-    };
-    if (in.whole) return search(in.whole, 0);
-    if ((rc = each_segment(in, false, search))) return rc;
-    segments_notice(in, 1);
-    return LRB_OK;
+    return search_file(who, cov, reads_path, &out_txt, 1, threads, [&](lrb_ctx* c) { return lrb_ctx_table_load(c, table_path); },
+                       whole_rows(out_txt, out_npy, cov.W, threads));
 }
 
 extern "C" int lrb_table_spectrum(const char* table_path, const char* out_txt, uint32_t max_count) {

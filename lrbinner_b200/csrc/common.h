@@ -62,14 +62,44 @@ void lrb_host_free(void* p, bool pinned);
 // bases per segment of the segment reader for result rows of `row_bytes_per_read` (lrb_reader_open: segment_bases = 0)
 uint64_t lrb_segment_budget(uint64_t row_bytes_per_read);
 
-// n coverage settings (bin_sizes[m], bins[m]) of one search: 1 <= n <= LRB_MAX_COV_SETTINGS, bin_size >= 1, bins in
-// [1, LRB_MAX_BINS], no pair twice, row width W = sum of bins <= LRB_MAX_BINS (into *width).  LRB_EINVAL naming `who`.
-int lrb_check_cov_settings(const char* who, int n, const long* bin_sizes, const int* bins, uint32_t* width);
+// ---- the coverage row of one search --------------------------------------------------------------------------------
+// A row is up to 8 column blocks side by side.  Each block bins the count of one table, the full-layout table or compact
+// table (sample slot) `table`, either by (bin_size, bins) or by count edges.  The public calls build three shapes: n
+// (bin_size, bins) blocks on the full table, n such blocks on compact tables, one edge block on the full table.
+static_assert(LRB_MAX_COV_SETTINGS == LRB_MAX_SAMPLE_TABLES, "one block per setting or per sample table");
 
-// The same for n sample tables with one setting each (LRB_MAX_SAMPLE_TABLES at most): ids[t] says which table t is, and only
-// the same (table, bin_size, bins) twice is refused.
-int lrb_check_table_settings(const char* who, int n, const uint64_t* ids, const long* bin_sizes, const int* bins, uint32_t* width);
+struct CovBlock {
+    int table = -1;                    // -1: the full-layout table; t >= 0: compact table t
+    long bin_size = 1;                 // bins by (bin_size, bins), unless by_edges:
+    int bins = 1;
+    bool by_edges = false;             // bins by edges[n_edges] (the caller's array): a count c goes to #{i : edges[i] <= c}
+    const uint32_t* edges = nullptr;
+    int n_edges = 0;
+    uint32_t width() const { return by_edges ? (uint32_t)n_edges + 1u : (uint32_t)bins; }
+};
 
-// Coverage bins given by n count edges: 0 <= n <= LRB_MAX_BINS - 1, edges non-NULL when n > 0, strictly increasing, the
-// first >= 2 (counts 0 and 1 stay in bin 0, as in the reference's rule).  LRB_EINVAL naming `who` and the bad value.
-int lrb_check_cov_edges(const char* who, const uint32_t* edges, int n);
+struct CovLayout {
+    int n = 1;                         // blocks as asked for: lrb_check_cov_layout refuses n outside [1, 8]
+    bool compact = false;              // the blocks read compact tables (sample tables)
+    bool null_settings = false;        // bin_sizes or bins was NULL: the blocks were left unset
+    CovBlock b[LRB_MAX_COV_SETTINGS];
+    uint32_t W = 1;                    // row width, the blocks' bins together (lrb_check_cov_layout)
+    bool single() const { return n == 1 && !compact && !b[0].by_edges; }   // what the direct search and k_search_keys take
+};
+
+// n (bin_sizes[m], bins[m]) blocks, on the full table (slots NULL) or on compact table slots[m].  Reads the arrays only as
+// far as lrb_check_cov_layout can then refuse them: not when one is NULL, never past LRB_MAX_COV_SETTINGS blocks.
+CovLayout lrb_cov_settings(int n, const long* bin_sizes, const int* bins, const int* slots = nullptr);
+// one block on the full table binned by count edges (the array is kept, not copied)
+CovLayout lrb_cov_edges(const uint32_t* edges, int n_edges);
+
+// Checks a layout and fills L->W; LRB_EINVAL naming `who` and the bad value.  Blocks: 1 <= n <= 8, compact tables in
+// [0, 8), bin_size >= 1, bins in [1, LRB_MAX_BINS], no (table, bin_size, bins) twice; edges: at most LRB_MAX_BINS - 1,
+// non-NULL when there are any, strictly increasing, the first >= 2 (counts 0 and 1 stay in bin 0, as in the reference's
+// rule); the row at most LRB_MAX_BINS wide.
+int lrb_check_cov_layout(const char* who, CovLayout* L);
+
+// The partitioned search of the buckets [bucket_lo, bucket_hi) for a checked layout: block m reads `table`, or
+// compact[b[m].table] on a compact layout.  sums are rewritten by the call that includes the last bucket (partition.cu).
+int lrb_partition_search(const char* who, const lrb_partition* part, int bucket_lo, int bucket_hi, const uint32_t* table,
+                         const uint32_t* const* compact, const CovLayout& L, uint32_t* hist, uint32_t* sums, void* stream);

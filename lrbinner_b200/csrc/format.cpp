@@ -270,37 +270,29 @@ extern "C" int lrb_table_read_file(const char* path, uint32_t* table) {
     return LRB_OK;
 }
 
-// ids == nullptr: n settings of one table; else n sample tables, ids[t] telling which table t is (equal ids, same table)
-static int check_settings(const char* who, int n, const uint64_t* ids, const long* bin_sizes, const int* bins, uint32_t* width) {
-    const char* what = ids ? "table" : "setting";
-    const int most = ids ? LRB_MAX_SAMPLE_TABLES : LRB_MAX_COV_SETTINGS;
-    if (n < 1 || n > most) return lrb_set_error(LRB_EINVAL, "%s: the number of %ss must be in [1, %d] (got %d)", who, ids ? "sample table" : "setting", most, n);
-    if (!bin_sizes || !bins) return lrb_set_error(LRB_EINVAL, "%s: null bin_sizes / bins", who);
-    uint64_t W = 0;
-    for (int m = 0; m < n; ++m) {
-        if (bin_sizes[m] < 1) return lrb_set_error(LRB_EINVAL, "%s: bin_size must be >= 1 (%s %d: got %ld)", who, what, m, bin_sizes[m]);
-        if (bins[m] < 1 || bins[m] > LRB_MAX_BINS) return lrb_set_error(LRB_EINVAL, "%s: bins must be in [1, %d] (%s %d: got %d)", who, LRB_MAX_BINS, what, m, bins[m]);
-        for (int j = 0; j < m; ++j)
-            if (bin_sizes[j] == bin_sizes[m] && bins[j] == bins[m] && (!ids || ids[j] == ids[m]))
-                return lrb_set_error(LRB_EINVAL, "%s: %s %d repeats %s %d (%sbin_size %ld, bins %d)", who, what, m, what, j, ids ? "same table, " : "",
-                                     bin_sizes[m], bins[m]);
-        W += (uint64_t)bins[m];
+// ---- the coverage row of a search (common.h) ---------------------------------------------------------------------
+CovLayout lrb_cov_settings(int n, const long* bin_sizes, const int* bins, const int* slots) {
+    CovLayout L;
+    L.n = n;
+    L.compact = slots != nullptr;
+    L.null_settings = !bin_sizes || !bins;
+    for (int m = 0; m < n && m < LRB_MAX_COV_SETTINGS && !L.null_settings; ++m) {
+        L.b[m].table = slots ? slots[m] : -1;
+        L.b[m].bin_size = bin_sizes[m];
+        L.b[m].bins = bins[m];
     }
-    if (W > LRB_MAX_BINS) return lrb_set_error(LRB_EINVAL, "%s: the %ss' bins add up to %llu, more than %d", who, what, (unsigned long long)W, LRB_MAX_BINS);
-    if (width) *width = (uint32_t)W;
-    return LRB_OK;
+    return L;
 }
 
-int lrb_check_cov_settings(const char* who, int n, const long* bin_sizes, const int* bins, uint32_t* width) {
-    return check_settings(who, n, nullptr, bin_sizes, bins, width);
+CovLayout lrb_cov_edges(const uint32_t* edges, int n_edges) {
+    CovLayout L;
+    L.b[0].by_edges = true;
+    L.b[0].edges = edges;
+    L.b[0].n_edges = n_edges;
+    return L;
 }
 
-int lrb_check_table_settings(const char* who, int n, const uint64_t* ids, const long* bin_sizes, const int* bins, uint32_t* width) {
-    if (!ids) return lrb_set_error(LRB_EINVAL, "%s: null table ids", who);
-    return check_settings(who, n, ids, bin_sizes, bins, width);
-}
-
-int lrb_check_cov_edges(const char* who, const uint32_t* edges, int n) {
+static int check_edges(const char* who, const uint32_t* edges, int n) {
     if (n < 0 || n > LRB_MAX_BINS - 1) return lrb_set_error(LRB_EINVAL, "%s: the number of edges must be in [0, %d] (got %d)", who, LRB_MAX_BINS - 1, n);
     if (n > 0 && !edges) return lrb_set_error(LRB_EINVAL, "%s: null edges (%d edges)", who, n);
     if (n > 0 && edges[0] < 2)
@@ -308,6 +300,36 @@ int lrb_check_cov_edges(const char* who, const uint32_t* edges, int n) {
     for (int i = 1; i < n; ++i)
         if (edges[i] <= edges[i - 1])
             return lrb_set_error(LRB_EINVAL, "%s: edges must be strictly increasing (edge %d = %u after edge %d = %u)", who, i, edges[i], i - 1, edges[i - 1]);
+    return LRB_OK;
+}
+
+int lrb_check_cov_layout(const char* who, CovLayout* L) {
+    const char* what = L->compact ? "table" : "setting";
+    if (L->n < 1 || L->n > LRB_MAX_COV_SETTINGS)
+        return lrb_set_error(LRB_EINVAL, "%s: the number of %ss must be in [1, %d] (got %d)", who, L->compact ? "sample table" : "setting",
+                             LRB_MAX_COV_SETTINGS, L->n);
+    if (L->null_settings) return lrb_set_error(LRB_EINVAL, "%s: null bin_sizes / bins", who);
+    uint64_t W = 0;
+    for (int m = 0; m < L->n; ++m) {
+        const CovBlock& b = L->b[m];
+        if (b.by_edges) {
+            const int rc = check_edges(who, b.edges, b.n_edges);
+            if (rc) return rc;
+            W += b.width();
+            continue;
+        }
+        if (L->compact && (b.table < 0 || b.table >= LRB_MAX_SAMPLE_TABLES))
+            return lrb_set_error(LRB_EINVAL, "%s: slot must be in [0, %d) (table %d: got %d)", who, LRB_MAX_SAMPLE_TABLES, m, b.table);
+        if (b.bin_size < 1) return lrb_set_error(LRB_EINVAL, "%s: bin_size must be >= 1 (%s %d: got %ld)", who, what, m, b.bin_size);
+        if (b.bins < 1 || b.bins > LRB_MAX_BINS) return lrb_set_error(LRB_EINVAL, "%s: bins must be in [1, %d] (%s %d: got %d)", who, LRB_MAX_BINS, what, m, b.bins);
+        for (int j = 0; j < m; ++j)
+            if (L->b[j].table == b.table && L->b[j].bin_size == b.bin_size && L->b[j].bins == b.bins)
+                return lrb_set_error(LRB_EINVAL, "%s: %s %d repeats %s %d (%sbin_size %ld, bins %d)", who, what, m, what, j,
+                                     L->compact ? "same table, " : "", b.bin_size, b.bins);
+        W += b.width();
+    }
+    if (W > LRB_MAX_BINS) return lrb_set_error(LRB_EINVAL, "%s: the %ss' bins add up to %llu, more than %d", who, what, (unsigned long long)W, LRB_MAX_BINS);
+    L->W = (uint32_t)W;
     return LRB_OK;
 }
 
@@ -334,7 +356,8 @@ extern "C" int lrb_spectrum_bin_mass(const uint64_t* spectrum, uint32_t max_coun
 extern "C" int lrb_spectrum_edge_mass(const uint64_t* spectrum, uint32_t max_count, const uint32_t* edges, int n_edges, uint64_t* mass) {
     static const char* who = "lrb_spectrum_edge_mass";
     if (!spectrum || !mass) return lrb_set_error(LRB_EINVAL, "%s: null argument", who);
-    const int rc = lrb_check_cov_edges(who, edges, n_edges);
+    CovLayout L = lrb_cov_edges(edges, n_edges);
+    const int rc = lrb_check_cov_layout(who, &L);
     if (rc) return rc;
     const uint64_t M = max_count;
     // every count >= the last edge lands in the last bin; below it the spectrum must resolve the count itself

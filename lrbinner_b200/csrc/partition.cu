@@ -1479,64 +1479,16 @@ extern "C" int lrb_dev_partition_apply_range(const lrb_partition* part, int mode
     return LRB_OK;
 }
 
-// Several coverage settings in one search (k_search_settings): hist rows of W = sum of bins[m] words, setting m's bins at
-// column sum_{j<m} bins[j]; sums are rewritten by the call that includes the last bucket.  n = 1 is mode 2 of
-// lrb_dev_partition_apply_range.
-extern "C" int lrb_dev_partition_search_settings(const lrb_partition* part, int bucket_lo, int bucket_hi, const uint32_t* table, int n,
-                                                 const long* bin_sizes, const int* bins, uint32_t* hist, uint32_t* sums, void* stream) {
-    if (!part || !table || !hist || !sums) return lrb_set_error(LRB_EINVAL, "lrb_dev_partition_search_settings: null argument");
-    uint32_t W = 0;
-    const int rc = lrb_check_cov_settings("lrb_dev_partition_search_settings", n, bin_sizes, bins, &W);
-    if (rc) return rc;
-    if (n == 1)
-        return lrb_dev_partition_apply_range(part, 2, bucket_lo, bucket_hi, const_cast<uint32_t*>(table), bin_sizes[0], bins[0], hist, sums, stream);
-    if (!part->has_rids) return lrb_set_error(LRB_EINVAL, "lrb_dev_partition_search_settings: partition was built without read ids");
-    if (bucket_lo < 0) bucket_lo = 0;
-    if (bucket_hi > part->n_buckets) bucket_hi = part->n_buckets;
-    if (part->n_chunks == 0) return LRB_OK;
-    cudaStream_t st = (cudaStream_t)stream;
-    CovSettings C = {};
-    C.n = (uint32_t)n;
-    C.W = W;
-    for (int m = 0, off = 0; m < n; off += bins[m], ++m) {
-        C.S32[m] = bin_sizes[m] > 0xFFFFFFFFl ? 0xFFFFFFFFu : (uint32_t)bin_sizes[m];
-        C.magic[m] = coverage_magic(C.S32[m]);
-        C.B[m] = (uint32_t)bins[m];
-        C.off[m] = (uint32_t)off;
-    }
-    const PartMeta* meta = reinterpret_cast<const PartMeta*>(part->small);
-    const ChunkList L = chunk_list(part);
-    const int shift = part->shift;
-    const uint32_t hi_mask2 = ((1u << shift) - 1u) & ~0xFFFFu;
-    if (bucket_hi > bucket_lo) {
-        const dim3 gs(search_grid(L, part->n_chunks), (unsigned)(bucket_hi - bucket_lo));
-        LRB_LAUNCH("k_search_settings", st, k_search_settings<<<gs, 256, 0, st>>>(part->keys, meta, bucket_lo, part->n_chunks, L,
-                                                                                  step_tables(part->steps, part->step_capacity),
-                                                                                  part->key_lo + ((uint32_t)bucket_lo << shift),
-                                                                                  hi_mask2, shift, table, C, hist));
-    }
-    if (part->n_reads && bucket_hi == part->n_buckets)
-        LRB_LAUNCH("k_row_sums", st, k_row_sums<<<(unsigned)((part->n_reads + 255) / 256), 256, 0, st>>>(hist, sums, part->n_reads, (uint32_t)bins[0], W));
-    LRB_CUDA(cudaGetLastError());
-    return LRB_OK;
-}
-
-// Several compact sample tables in one search (k_search_samples): hist rows of W = sum of bins[t] words, table t's bins at
-// column sum_{j<t} bins[j]; one walk over the lists per table; sums are rewritten by the call that includes the last bucket.
-extern "C" int lrb_dev_partition_search_samples(const lrb_partition* part, int bucket_lo, int bucket_hi, const uint32_t* const* compact_tables,
-                                                int n, const long* bin_sizes, const int* bins, uint32_t* hist, uint32_t* sums, void* stream) {
-    static const char* who = "lrb_dev_partition_search_samples";
-    if (!part || !compact_tables || !hist || !sums) return lrb_set_error(LRB_EINVAL, "%s: null argument", who);
-    uint64_t ids[LRB_MAX_SAMPLE_TABLES] = {};
-    for (int t = 0; t < n && t < LRB_MAX_SAMPLE_TABLES; ++t) {
-        if (!compact_tables[t]) return lrb_set_error(LRB_EINVAL, "%s: null table %d", who, t);
-        ids[t] = (uint64_t)(uintptr_t)compact_tables[t];
-    }
-    uint32_t W = 0;
-    const int rc = lrb_check_table_settings(who, n, ids, bin_sizes, bins, &W);
-    if (rc) return rc;
+// The search of one coverage layout (common.h).  A single (bin_size, bins) block on the full table is mode 2 of
+// lrb_dev_partition_apply_range (k_search_keys); otherwise one launch of k_search_settings for several such blocks, one of
+// k_search_edges for an edge block, or one of k_search_samples per compact block, then k_row_sums.
+int lrb_partition_search(const char* who, const lrb_partition* part, int bucket_lo, int bucket_hi, const uint32_t* table,
+                         const uint32_t* const* compact, const CovLayout& cov, uint32_t* hist, uint32_t* sums, void* stream) {
+    if (cov.single())
+        return lrb_dev_partition_apply_range(part, 2, bucket_lo, bucket_hi, const_cast<uint32_t*>(table), cov.b[0].bin_size, cov.b[0].bins, hist,
+                                             sums, stream);
     if (!part->has_rids) return lrb_set_error(LRB_EINVAL, "%s: partition was built without read ids", who);
-    if (part->key_lo & ((1u << part->shift) - 1u))
+    if (cov.compact && (part->key_lo & ((1u << part->shift) - 1u)))
         return lrb_set_error(LRB_EINVAL, "%s: the partition's key range must start at a bucket boundary (key_lo %u)", who, part->key_lo);
     if (bucket_lo < 0) bucket_lo = 0;
     if (bucket_hi > part->n_buckets) bucket_hi = part->n_buckets;
@@ -1546,61 +1498,88 @@ extern "C" int lrb_dev_partition_search_samples(const lrb_partition* part, int b
     const ChunkList L = chunk_list(part);
     const StepTables T = step_tables(part->steps, part->step_capacity);
     const int shift = part->shift;
-    const uint32_t cbase0 = (part->key_lo + ((uint32_t)bucket_lo << shift)) >> 1;
+    const uint32_t hi_mask2 = ((1u << shift) - 1u) & ~0xFFFFu;
+    const uint32_t base0 = part->key_lo + ((uint32_t)bucket_lo << shift);
     if (bucket_hi > bucket_lo) {
         const dim3 gs(search_grid(L, part->n_chunks), (unsigned)(bucket_hi - bucket_lo));
-        for (int t = 0, off = 0; t < n; off += bins[t], ++t) {
-            SampleGroup S = {};
-            S.W = W;
-            S.table = compact_tables[t];
-            S.S32 = bin_sizes[t] > 0xFFFFFFFFl ? 0xFFFFFFFFu : (uint32_t)bin_sizes[t];
-            S.magic = coverage_magic(S.S32);
-            S.B = (uint32_t)bins[t];
-            S.off = (uint32_t)off;
-            LRB_LAUNCH("k_search_samples", st, k_search_samples<<<gs, 256, 0, st>>>(part->keys, meta, bucket_lo, part->n_chunks, L, T,
-                                                                                   cbase0, shift, S, hist));
+        if (cov.b[0].by_edges) {
+            const CovBlock& b = cov.b[0];
+            CovEdges E;
+            E.n = (uint32_t)b.n_edges;
+            E.P = 1;
+            while (E.P < E.n + 1u) E.P <<= 1;
+            std::copy(b.edges, b.edges + b.n_edges, E.t);
+            std::fill(E.t + b.n_edges, E.t + (LRB_MAX_BINS - 1), 0xFFFFFFFFu);
+            const size_t smem = sizeof(uint32_t) * (E.P - 1u);   // at most 16 380 bytes: no opt-in needed
+            LRB_LAUNCH("k_search_edges", st, k_search_edges<<<gs, 256, smem, st>>>(part->keys, meta, bucket_lo, part->n_chunks, L, T, base0,
+                                                                                   hi_mask2, shift, table, E, hist));
+        } else if (cov.compact) {
+            for (int t = 0, off = 0; t < cov.n; off += cov.b[t].bins, ++t) {
+                SampleGroup S = {};
+                S.W = cov.W;
+                S.table = compact[cov.b[t].table];
+                S.S32 = cov.b[t].bin_size > 0xFFFFFFFFl ? 0xFFFFFFFFu : (uint32_t)cov.b[t].bin_size;
+                S.magic = coverage_magic(S.S32);
+                S.B = (uint32_t)cov.b[t].bins;
+                S.off = (uint32_t)off;
+                LRB_LAUNCH("k_search_samples", st, k_search_samples<<<gs, 256, 0, st>>>(part->keys, meta, bucket_lo, part->n_chunks, L, T,
+                                                                                       base0 >> 1, shift, S, hist));
+            }
+        } else {
+            CovSettings C = {};
+            C.n = (uint32_t)cov.n;
+            C.W = cov.W;
+            for (int m = 0, off = 0; m < cov.n; off += cov.b[m].bins, ++m) {
+                C.S32[m] = cov.b[m].bin_size > 0xFFFFFFFFl ? 0xFFFFFFFFu : (uint32_t)cov.b[m].bin_size;
+                C.magic[m] = coverage_magic(C.S32[m]);
+                C.B[m] = (uint32_t)cov.b[m].bins;
+                C.off[m] = (uint32_t)off;
+            }
+            LRB_LAUNCH("k_search_settings", st, k_search_settings<<<gs, 256, 0, st>>>(part->keys, meta, bucket_lo, part->n_chunks, L, T, base0,
+                                                                                      hi_mask2, shift, table, C, hist));
         }
     }
     if (part->n_reads && bucket_hi == part->n_buckets)
-        LRB_LAUNCH("k_row_sums", st, k_row_sums<<<(unsigned)((part->n_reads + 255) / 256), 256, 0, st>>>(hist, sums, part->n_reads, (uint32_t)bins[0], W));
+        LRB_LAUNCH("k_row_sums", st, k_row_sums<<<(unsigned)((part->n_reads + 255) / 256), 256, 0, st>>>(hist, sums, part->n_reads, cov.b[0].width(), cov.W));
     LRB_CUDA(cudaGetLastError());
     return LRB_OK;
 }
 
+// Several coverage settings in one search (k_search_settings): hist rows of W = sum of bins[m] words, setting m's bins at
+// column sum_{j<m} bins[j]; sums are rewritten by the call that includes the last bucket.  n = 1 is mode 2 of
+// lrb_dev_partition_apply_range.
+extern "C" int lrb_dev_partition_search_settings(const lrb_partition* part, int bucket_lo, int bucket_hi, const uint32_t* table, int n,
+                                                 const long* bin_sizes, const int* bins, uint32_t* hist, uint32_t* sums, void* stream) {
+    static const char* who = "lrb_dev_partition_search_settings";
+    if (!part || !table || !hist || !sums) return lrb_set_error(LRB_EINVAL, "%s: null argument", who);
+    CovLayout L = lrb_cov_settings(n, bin_sizes, bins);
+    const int rc = lrb_check_cov_layout(who, &L);
+    return rc ? rc : lrb_partition_search(who, part, bucket_lo, bucket_hi, table, nullptr, L, hist, sums, stream);
+}
+
+// Several compact sample tables in one search (k_search_samples): hist rows of W = sum of bins[t] words, table t's bins at
+// column sum_{j<t} bins[j]; one walk over the lists per table; sums are rewritten by the call that includes the last bucket.
+extern "C" int lrb_dev_partition_search_samples(const lrb_partition* part, int bucket_lo, int bucket_hi, const uint32_t* const* compact_tables,
+                                                int n, const long* bin_sizes, const int* bins, uint32_t* hist, uint32_t* sums, void* stream) {
+    static const char* who = "lrb_dev_partition_search_samples";
+    if (!part || !compact_tables || !hist || !sums) return lrb_set_error(LRB_EINVAL, "%s: null argument", who);
+    int slots[LRB_MAX_SAMPLE_TABLES] = {};   // block t reads compact_tables[slots[t]], the first entry with its pointer
+    for (int t = 0; t < n && t < LRB_MAX_SAMPLE_TABLES; ++t) {
+        if (!compact_tables[t]) return lrb_set_error(LRB_EINVAL, "%s: null table %d", who, t);
+        while (compact_tables[slots[t]] != compact_tables[t]) ++slots[t];
+    }
+    CovLayout L = lrb_cov_settings(n, bin_sizes, bins, slots);
+    const int rc = lrb_check_cov_layout(who, &L);
+    return rc ? rc : lrb_partition_search(who, part, bucket_lo, bucket_hi, nullptr, compact_tables, L, hist, sums, stream);
+}
+
 // Coverage bins given by count edges (k_search_edges): hist rows of n_edges + 1 words; edges is a HOST array, checked by
-// lrb_check_cov_edges; sums are rewritten by the call that includes the last bucket.
+// lrb_check_cov_layout; sums are rewritten by the call that includes the last bucket.
 extern "C" int lrb_dev_partition_search_edges(const lrb_partition* part, int bucket_lo, int bucket_hi, const uint32_t* table,
                                               const uint32_t* edges, int n_edges, uint32_t* hist, uint32_t* sums, void* stream) {
     static const char* who = "lrb_dev_partition_search_edges";
     if (!part || !table || !hist || !sums) return lrb_set_error(LRB_EINVAL, "%s: null argument", who);
-    const int rc = lrb_check_cov_edges(who, edges, n_edges);
-    if (rc) return rc;
-    if (!part->has_rids) return lrb_set_error(LRB_EINVAL, "%s: partition was built without read ids", who);
-    if (bucket_lo < 0) bucket_lo = 0;
-    if (bucket_hi > part->n_buckets) bucket_hi = part->n_buckets;
-    if (part->n_chunks == 0) return LRB_OK;
-    cudaStream_t st = (cudaStream_t)stream;
-    CovEdges E;
-    E.n = (uint32_t)n_edges;
-    E.P = 1;
-    while (E.P < E.n + 1u) E.P <<= 1;
-    std::copy(edges, edges + n_edges, E.t);
-    std::fill(E.t + n_edges, E.t + (LRB_MAX_BINS - 1), 0xFFFFFFFFu);
-    const uint32_t B = E.n + 1u;
-    const PartMeta* meta = reinterpret_cast<const PartMeta*>(part->small);
-    const ChunkList L = chunk_list(part);
-    const int shift = part->shift;
-    const uint32_t hi_mask2 = ((1u << shift) - 1u) & ~0xFFFFu;
-    if (bucket_hi > bucket_lo) {
-        const dim3 gs(search_grid(L, part->n_chunks), (unsigned)(bucket_hi - bucket_lo));
-        const size_t smem = sizeof(uint32_t) * (E.P - 1u);   // at most 16 380 bytes: no opt-in needed
-        LRB_LAUNCH("k_search_edges", st, k_search_edges<<<gs, 256, smem, st>>>(part->keys, meta, bucket_lo, part->n_chunks, L,
-                                                                               step_tables(part->steps, part->step_capacity),
-                                                                               part->key_lo + ((uint32_t)bucket_lo << shift),
-                                                                               hi_mask2, shift, table, E, hist));
-    }
-    if (part->n_reads && bucket_hi == part->n_buckets)
-        LRB_LAUNCH("k_row_sums", st, k_row_sums<<<(unsigned)((part->n_reads + 255) / 256), 256, 0, st>>>(hist, sums, part->n_reads, B, B));
-    LRB_CUDA(cudaGetLastError());
-    return LRB_OK;
+    CovLayout L = lrb_cov_edges(edges, n_edges);
+    const int rc = lrb_check_cov_layout(who, &L);
+    return rc ? rc : lrb_partition_search(who, part, bucket_lo, bucket_hi, table, nullptr, L, hist, sums, stream);
 }

@@ -206,34 +206,35 @@ class Context:
         edges=[t_1, ..., t_{B-1}] (instead of every other coverage argument): bins given by strictly increasing count edges,
         t_1 >= 2; a window whose 15-mer is counted c times goes to bin searchsorted(edges, c, side="right") of hist [N, B]
         (lrb_profile_host_edges)."""
-        if coverage is not None and (bin_size is not None or bins is not None):
-            raise _lib.LrbError(_lib.LRB_EINVAL, "coverage=[(bin_size, bins), ...] replaces bin_size / bins: give one or the other")
-        if samples is not None and (coverage is not None or bin_size is not None or bins is not None):
-            raise _lib.LrbError(_lib.LRB_EINVAL, "samples=[(slot, bin_size, bins), ...] replaces coverage / bin_size / bins: give one or the other")
-        if edges is not None:
-            if samples is not None or coverage is not None or bin_size is not None or bins is not None:
-                raise _lib.LrbError(_lib.LRB_EINVAL, "edges=[...] replaces samples / coverage / bin_size / bins: give one or the other")
-            edges = _edges_array(edges)   # refused here, before a context is needed
-            return self._profile_edges(reads, k, edges, want_table, use_loaded_table, out, keep_table, add_to_table)
+        given = [arg for arg, v in (("edges=[...]", edges), ("samples=[(slot, bin_size, bins), ...]", samples),
+                                    ("coverage=[(bin_size, bins), ...]", coverage)) if v is not None]
+        if given and len(given) + (bin_size is not None or bins is not None) > 1:
+            raise _lib.LrbError(_lib.LRB_EINVAL, f"{given[0]} replaces the other coverage arguments (bin_size / bins, coverage, samples, "
+                                                 "edges): give one of them")
         n = reads.n_reads
         out = dict(out or {})
-        comp = hist = sums = table = hists = None
-        slots = None
+        comp = hist = sums = table = hists = slots = width = None
+        if edges is not None:
+            edges = _edges_array(edges)   # refused here, before a context is needed
+            width = edges.size + 1
         if samples is not None:
             samples = [(int(t), int(s_), int(b)) for t, s_, b in samples]
             slots = np.array([t for t, _, _ in samples], dtype=np.int32)
             coverage = [(s_, b) for _, s_, b in samples]
         set_bs, set_bins = _settings_arrays(coverage if coverage is not None else
                                             [(bin_size if bin_size is not None else 1, bins if bins is not None else 1)])
+        if bins is not None or coverage is not None:
+            width = max(int(np.clip(set_bins, 1, None).sum()), 1)
+            if coverage is not None and width > _lib.MAX_BINS:   # refused by the library before any work: no real buffer
+                width = 1
         if k is not None:
             comp = out.get("comp")
             if comp is None:
                 comp = np.zeros((n, COMP_WIDTH[k]), dtype=np.uint32)
-        if bins is not None or coverage is not None:
-            width = max(int(np.clip(set_bins, 1, None).sum()), 1)
+        if width is not None:
             hist = out.get("hist")
-            if hist is None:   # a width the library refuses (it checks the settings before any work) gets no real buffer
-                hist = np.zeros((n, width if coverage is None or width <= _lib.MAX_BINS else 1), dtype=np.uint32)
+            if hist is None:
+                hist = np.zeros((n, width), dtype=np.uint32)
             sums = out.get("sums")
             if sums is None:
                 sums = np.zeros(n, dtype=np.uint32)
@@ -243,43 +244,19 @@ class Context:
                 table = np.empty(_lib.TABLE_ENTRIES, dtype=np.uint32)
         flags = ((_lib.PROFILE_USE_LOADED_TABLE if use_loaded_table else 0) | (_lib.PROFILE_KEEP_TABLE if keep_table else 0) |
                  (_lib.PROFILE_ADD_TO_TABLE if add_to_table else 0))
+        k = int(k) if k is not None else 0
         parts = (_ptr(comp) if comp is not None else None, _ptr(hist) if hist is not None else None,
                  _ptr(sums) if sums is not None else None, _ptr(table) if table is not None else None)
-        if slots is not None:
-            check(lib.lrb_profile_host_samples(self._h, reads._h, int(k) if k is not None else 0, len(set_bs), _ptr(slots),
-                                               _ptr(set_bs), _ptr(set_bins), *parts, flags))
+        if edges is not None:
+            check(lib.lrb_profile_host_edges(self._h, reads._h, k, _ptr(edges), int(edges.size), *parts, flags))
+        elif slots is not None:
+            check(lib.lrb_profile_host_samples(self._h, reads._h, k, len(set_bs), _ptr(slots), _ptr(set_bs), _ptr(set_bins), *parts, flags))
         else:
-            check(lib.lrb_profile_host_settings(self._h, reads._h, int(k) if k is not None else 0, len(set_bs), _ptr(set_bs),
-                                                _ptr(set_bins), *parts, flags))
+            check(lib.lrb_profile_host_settings(self._h, reads._h, k, len(set_bs), _ptr(set_bs), _ptr(set_bins), *parts, flags))
         if coverage is not None:
             offs = np.concatenate([[0], np.cumsum(set_bins)])
             hists = [hist[:, offs[m]:offs[m + 1]] for m in range(len(set_bins))]
         return {"comp": comp, "hist": hist, "hists": hists, "sums": sums, "table": table}
-
-    def _profile_edges(self, reads, k, edges, want_table, use_loaded_table, out, keep_table, add_to_table):
-        n = reads.n_reads
-        out = dict(out or {})
-        comp = table = None
-        if k is not None:
-            comp = out.get("comp")
-            if comp is None:
-                comp = np.zeros((n, COMP_WIDTH[k]), dtype=np.uint32)
-        hist = out.get("hist")
-        if hist is None:
-            hist = np.zeros((n, edges.size + 1), dtype=np.uint32)
-        sums = out.get("sums")
-        if sums is None:
-            sums = np.zeros(n, dtype=np.uint32)
-        if want_table:
-            table = out.get("table")
-            if table is None:
-                table = np.empty(_lib.TABLE_ENTRIES, dtype=np.uint32)
-        flags = ((_lib.PROFILE_USE_LOADED_TABLE if use_loaded_table else 0) | (_lib.PROFILE_KEEP_TABLE if keep_table else 0) |
-                 (_lib.PROFILE_ADD_TO_TABLE if add_to_table else 0))
-        check(lib.lrb_profile_host_edges(self._h, reads._h, int(k) if k is not None else 0, _ptr(edges), int(edges.size),
-                                         _ptr(comp) if comp is not None else None, _ptr(hist), _ptr(sums),
-                                         _ptr(table) if table is not None else None, flags))
-        return {"comp": comp, "hist": hist, "hists": None, "sums": sums, "table": table}
 
     def info(self):
         """How the last profile() ran: devices, batches, table path, wall / exchange milliseconds."""
