@@ -146,6 +146,10 @@ int lrb_dev_table_spectrum(const uint32_t* table, uint32_t key_lo, uint32_t key_
  * takes them in this form.  `table` is a full-layout 2^30-entry table (the other half need not be mirrored). */
 #define LRB_COMPACT_ENTRIES (1ull << 29)
 int lrb_dev_table_compact(const uint32_t* table, uint32_t* compact, void* stream);
+/* lrb_dev_table_spectrum of a whole compact table (lrb_dev_table_compact): entry i of the compact table is read where the
+ * full form reads canonical key i, so the spectrum equals that of the full-layout table it was taken from.  Same layout,
+ * accumulate-into contract and max_count range as lrb_dev_table_spectrum; `compact` must be 16-byte aligned. */
+int lrb_dev_compact_spectrum(const uint32_t* compact, uint32_t max_count, uint64_t* spectrum, void* stream);
 
 /* Multi-GPU table exchange helpers (the reference has no counterpart: it is single-process; SURVEY.md 8e).
  * lrb_dev_copy2d: pitched device-to-device copy on the copy engines; src may be a peer GPU's table mapped into this
@@ -269,6 +273,32 @@ int lrb_dev_partition_search_samples(const lrb_partition* part, int bucket_lo, i
  * when n_edges > 0, the edges are strictly increasing and t_0 >= 2, and the partition has read ids. */
 int lrb_dev_partition_search_edges(const lrb_partition* part, int bucket_lo, int bucket_hi, const uint32_t* table,
                                    const uint32_t* edges, int n_edges, uint32_t* hist, uint32_t* sums, void* stream);
+/* One block of a mixed coverage row: the table it reads and how it bins the count.  table -1 is the full-layout table
+ * (the context's own table); 0..7 is compact table / sample slot t (at the file level: table_paths[t]).  by_edges 0 bins by
+ * (bin_size, bins) as -bs / -bc do; by_edges 1 bins by edges[n_edges] as lrb_dev_partition_search_edges does (n_edges = 0
+ * is one bin). */
+typedef struct {
+    int table;
+    int by_edges;
+    long bin_size;
+    int bins;
+    const uint32_t* edges;
+    int n_edges;
+} lrb_cov_block;
+/* Search with a mixed coverage row (no reference counterpart): up to LRB_MAX_COV_SETTINGS blocks, each on the full-layout
+ * `table` or on compact_tables[t] (a HOST array of LRB_MAX_SAMPLE_TABLES device pointers, NULL where unused; may be NULL
+ * when no block reads a slot), each binned by (bin_size, bins) or by edges (HOST arrays).  Rows of W = the blocks' bins
+ * together, block 0's bins first, in the caller's order; block m of row r equals row r of the single-block search of its
+ * table and binning (for compact tables: of every symmetric table, as in lrb_dev_partition_search_samples).  The lists are
+ * walked once per distinct table, and every block of that table is binned from the one gather.  A layout the settings,
+ * samples or edges search could take runs exactly as that search does.  Bucket range and sums as in
+ * lrb_dev_partition_search_settings.  LRB_EINVAL unless 1 <= n <= LRB_MAX_COV_SETTINGS, every table is -1 or in
+ * [0, LRB_MAX_SAMPLE_TABLES), every block passes the checks of its binning, W <= LRB_MAX_BINS, no block repeats (same table
+ * and binning), the tables the blocks read are non-NULL, the partition has read ids and, when a block reads a compact
+ * table, starts at a bucket boundary. */
+int lrb_dev_partition_search_layout(const lrb_partition* part, int bucket_lo, int bucket_hi, const uint32_t* table,
+                                    const uint32_t* const* compact_tables, const lrb_cov_block* blocks, int n, uint32_t* hist,
+                                    uint32_t* sums, void* stream);
 
 /* Pack ASCII on the device: bases[] (device, concatenated) -> codes/valid of `dev` (layout prebuilt). */
 int lrb_dev_pack_ascii(const lrb_reads_view* dev, const char* bases, const uint64_t* offsets, void* stream);
@@ -372,6 +402,15 @@ int lrb_profile_host_samples(lrb_ctx* ctx, const lrb_reads* reads, int k, int n,
  * device work; LRB_TABLE_PATH=direct is refused (LRB_EINVAL). */
 int lrb_profile_host_edges(lrb_ctx* ctx, const lrb_reads* reads, int k, const uint32_t* edges, int n_edges, uint32_t* comp_counts,
                            uint32_t* cov_hist, uint32_t* cov_sums, uint32_t* table_host, int flags);
+/* lrb_profile_host with a mixed coverage row (lrb_dev_partition_search_layout): cov_hist[N*W], block 0's bins first; a
+ * block reads the context's own table (table -1) or sample slot t.  A block on the context's table needs it counted from
+ * these reads, or loaded (USE_LOADED_TABLE / ADD_TO_TABLE), as lrb_profile_host does; a layout of slots alone searches no
+ * count and leaves the context's table as it was.  Every flag and part works alongside (composition, count, KEEP / ADD_TO /
+ * USE_LOADED_TABLE, batches, several devices).  The blocks are checked as in lrb_dev_partition_search_layout before any
+ * device work; an empty slot, a slot block without cov_hist / cov_sums and LRB_TABLE_PATH=direct (unless the layout is one
+ * (bin_size, bins) block on the context's table) are refused with LRB_EINVAL. */
+int lrb_profile_host_layout(lrb_ctx* ctx, const lrb_reads* reads, int k, const lrb_cov_block* blocks, int n, uint32_t* comp_counts,
+                            uint32_t* cov_hist, uint32_t* cov_sums, uint32_t* table_host, int flags);
 /* How the last lrb_profile_host call ran. */
 typedef struct {
     int n_devices;            /* GPUs that took part */
@@ -399,6 +438,9 @@ int lrb_ctx_table_save(lrb_ctx* ctx, const char* path);          /* HBM -> write
  * multi-device call included, or lrb_ctx_table_load) into spectrum_host[max_count + 3]; synchronous.  LRB_EINVAL when the
  * context holds no table.  The table is left as it is.  No reference counterpart. */
 int lrb_ctx_table_spectrum(lrb_ctx* ctx, uint32_t max_count, uint64_t* spectrum_host);
+/* The same for sample slot `slot` of the context (lrb_dev_compact_spectrum on the primary device).  LRB_EINVAL for a slot
+ * outside [0, LRB_MAX_SAMPLE_TABLES) or an empty slot.  No reference counterpart. */
+int lrb_ctx_sample_table_spectrum(lrb_ctx* ctx, int slot, uint32_t max_count, uint64_t* spectrum_host);
 
 /* Launch accounting (csrc/prof.cu).  lrb_prof_launches: kernels this library has launched since it was loaded (always
  * counted; bench.py's gpu_launches).  lrb_prof_enable(1) additionally brackets every launch with CUDA events on the stream
@@ -489,6 +531,16 @@ int lrb_search_15mers_samples(const char* const* table_paths, int n, const long*
  * device is touched (LRB_EINVAL as for lrb_profile_host_edges; a NULL path too).  No reference counterpart. */
 int lrb_search_15mers_edges(const char* table_path, const char* reads_path, const uint32_t* edges, int n_edges, const char* out_txt,
                             const char* out_npy, int threads);
+/* Mixed coverage rows from files: the reads against n_tables 15mers-counts files (1 <= n_tables <= LRB_MAX_SAMPLE_TABLES),
+ * each loaded once into a sample slot (canonical rows only; a path listed twice is loaded once), the reads parsed once.
+ * Block m reads table_paths[blocks[m].table] (table -1 is refused: there is no context table here) and line r of out_txt
+ * is, block after block joined by one space, the line the single-block call (lrb_search_15mers, or
+ * lrb_search_15mers_edges) writes for that table and binning, for every symmetric (counted) table.  out_npy (may be NULL)
+ * gets the [N, W] float rows.  Input larger than one segment is read segment by segment.  LRB_GPUS is honoured.  Arguments
+ * are checked before any file or device work (LRB_EINVAL: a NULL path, n_tables, a table index, the checks of
+ * lrb_dev_partition_search_layout, the same (path, binning) twice).  No reference counterpart. */
+int lrb_search_15mers_layout(const char* const* table_paths, int n_tables, const char* reads_path, const lrb_cov_block* blocks, int n,
+                             const char* out_txt, const char* out_npy, int threads);
 /* Abundance spectrum of a 15mers-counts file as lrb_write_spectrum_txt text (loaded on device LRB_DEVICE).  Missing or
  * malformed table file: LRB_EIO / LRB_EFORMAT; no device: LRB_ECUDA.  No reference counterpart. */
 int lrb_table_spectrum(const char* table_path, const char* out_txt, uint32_t max_count);

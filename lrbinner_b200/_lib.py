@@ -56,6 +56,12 @@ class RunInfo(C.Structure):
 PROFILE_USE_LOADED_TABLE, PROFILE_KEEP_TABLE, PROFILE_ADD_TO_TABLE = 1, 2, 4
 
 
+class CovBlockC(C.Structure):
+    """lrb_cov_block: one block of a mixed coverage row (table -1 = the context's table, 0..7 = a sample slot)."""
+    _fields_ = [("table", C.c_int), ("by_edges", C.c_int), ("bin_size", C.c_long), ("bins", C.c_int), ("edges", C.c_void_p),
+                ("n_edges", C.c_int)]
+
+
 class SynthParams(C.Structure):
     _fields_ = [("seed", C.c_uint64), ("n_genomes", C.c_uint32), ("sub_thr", C.c_uint32), ("ins_thr", C.c_uint32),
                 ("del_thr", C.c_uint32), ("n_thr", C.c_uint32), ("read_base", C.c_uint64)]
@@ -91,6 +97,7 @@ _SIG = {
     "lrb_dev_count": (C.c_int, [C.POINTER(ReadsView), _P, C.c_uint64, C.c_uint64, C.c_uint32, C.c_uint32, _P]),
     "lrb_dev_mirror": (C.c_int, [_P, _P]),
     "lrb_dev_table_spectrum": (C.c_int, [_P, C.c_uint32, C.c_uint32, C.c_uint32, _P, _P]),
+    "lrb_dev_compact_spectrum": (C.c_int, [_P, C.c_uint32, _P, _P]),
     "lrb_dev_copy2d": (C.c_int, [_P, C.c_uint64, _P, C.c_uint64, C.c_uint64, C.c_uint64, _P]),
     "lrb_dev_add_planes": (C.c_int, [_P, C.c_uint64, _P, C.c_uint64, C.c_int, C.c_uint32, C.c_uint32, _P]),
     "lrb_dev_search": (C.c_int, [C.POINTER(ReadsView), _P, C.c_long, C.c_int, _P, _P, C.c_uint64, C.c_uint64,
@@ -107,6 +114,7 @@ _SIG = {
     "lrb_dev_partition_search_settings": (C.c_int, [_P, C.c_int, C.c_int, _P, C.c_int, _P, _P, _P, _P, _P]),
     "lrb_dev_partition_search_samples": (C.c_int, [_P, C.c_int, C.c_int, _P, C.c_int, _P, _P, _P, _P, _P]),
     "lrb_dev_partition_search_edges": (C.c_int, [_P, C.c_int, C.c_int, _P, _P, C.c_int, _P, _P, _P]),
+    "lrb_dev_partition_search_layout": (C.c_int, [_P, C.c_int, C.c_int, _P, _P, _P, C.c_int, _P, _P, _P]),
     "lrb_dev_table_compact": (C.c_int, [_P, _P, _P]),
     "lrb_dev_pack_ascii": (C.c_int, [C.POINTER(ReadsView), _P, _P, _P]),
     "lrb_dev_format_composition": (C.c_int, [_P, _P, C.c_uint64, C.c_int, _P, _P]),
@@ -123,6 +131,7 @@ _SIG = {
     "lrb_profile_host_settings": (C.c_int, [_P, _P, C.c_int, C.c_int, _P, _P, _P, _P, _P, _P, C.c_int]),
     "lrb_profile_host_samples": (C.c_int, [_P, _P, C.c_int, C.c_int, _P, _P, _P, _P, _P, _P, _P, C.c_int]),
     "lrb_profile_host_edges": (C.c_int, [_P, _P, C.c_int, _P, C.c_int, _P, _P, _P, _P, C.c_int]),
+    "lrb_profile_host_layout": (C.c_int, [_P, _P, C.c_int, _P, C.c_int, _P, _P, _P, _P, C.c_int]),
     "lrb_ctx_sample_table_load": (C.c_int, [_P, C.c_int, C.c_char_p]),
     "lrb_ctx_sample_table_keep": (C.c_int, [_P, C.c_int]),
     "lrb_ctx_sample_table_free": (C.c_int, [_P, C.c_int]),
@@ -133,6 +142,7 @@ _SIG = {
     "lrb_ctx_table_load": (C.c_int, [_P, C.c_char_p]),
     "lrb_ctx_table_save": (C.c_int, [_P, C.c_char_p]),
     "lrb_ctx_table_spectrum": (C.c_int, [_P, C.c_uint32, _P]),
+    "lrb_ctx_sample_table_spectrum": (C.c_int, [_P, C.c_int, C.c_uint32, _P]),
     "lrb_prof_launches": (C.c_uint64, []),
     "lrb_prof_enable": (C.c_int, [C.c_int]),
     "lrb_prof_report": (C.c_int, [_P, C.c_size_t]),
@@ -157,6 +167,7 @@ _SIG = {
     "lrb_search_15mers_settings": (C.c_int, [C.c_char_p, C.c_char_p, C.c_int, _P, _P, _P, _P, C.c_int]),
     "lrb_search_15mers_samples": (C.c_int, [_P, C.c_int, _P, _P, C.c_char_p, C.c_char_p, C.c_char_p, C.c_int]),
     "lrb_search_15mers_edges": (C.c_int, [C.c_char_p, C.c_char_p, _P, C.c_int, C.c_char_p, C.c_char_p, C.c_int]),
+    "lrb_search_15mers_layout": (C.c_int, [_P, C.c_int, C.c_char_p, _P, C.c_int, C.c_char_p, C.c_char_p, C.c_int]),
     "lrb_table_spectrum": (C.c_int, [C.c_char_p, C.c_char_p, C.c_uint32]),
     "lrb_profile": (C.c_int, [C.c_char_p, C.c_char_p, C.c_int, C.c_long, C.c_int, C.c_int, C.c_int, C.c_int]),
     "lrb_profile_multi": (C.c_int, [C.c_char_p, C.c_char_p, C.c_int, C.c_long, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int]),

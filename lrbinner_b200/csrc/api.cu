@@ -239,7 +239,7 @@ namespace {
 struct Job {
     const lrb_reads* reads = nullptr;
     int k = 0, P = 0;
-    CovLayout cov;                    // the coverage row (checked); compact blocks read sample slots b[m].table
+    CovLayout cov;                    // the coverage row (checked); a block with b[m].table >= 0 reads that sample slot
     uint32_t *comp = nullptr, *hist = nullptr, *sums = nullptr, *table_host = nullptr;
     bool do_comp = false, do_search = false, do_count = false, use_loaded = false, add_to_table = false;
     bool use_part = true, want_smem_env = false, force_l2 = false, comp_pinned = false;
@@ -635,14 +635,15 @@ static bool direct_table_path() {   // one random HBM access per window (kernels
 static int refuse_direct(const char* who, const CovLayout& cov) {
     if (cov.single() || !direct_table_path()) return LRB_OK;
     char what[32];
-    if (cov.compact) snprintf(what, sizeof what, "sample tables");
+    if (cov.kind == CovKind::blocks) snprintf(what, sizeof what, "a layout of %d blocks", cov.n);
+    else if (cov.kind == CovKind::samples) snprintf(what, sizeof what, "sample tables");
     else if (cov.b[0].by_edges) snprintf(what, sizeof what, "count edges");
     else snprintf(what, sizeof what, "%d settings", cov.n);
     return lrb_set_error(LRB_EINVAL, "%s: LRB_TABLE_PATH=direct searches the full-layout table with one (bin_size, bins) setting per call, not %s",
                          who, what);
 }
 
-// cov: checked (lrb_check_cov_layout); a compact layout searches the sample slots b[t].table instead of the context's table
+// cov: checked (lrb_check_cov_layout); a block with b[m].table >= 0 searches that sample slot instead of the context's table
 static int profile_host(const char* who, lrb_ctx* c, const lrb_reads* r, int k, const CovLayout& cov, uint32_t* comp_counts,
                         uint32_t* cov_hist, uint32_t* cov_sums, uint32_t* table_host, int flags) {
     Job J;
@@ -653,16 +654,17 @@ static int profile_host(const char* who, lrb_ctx* c, const lrb_reads* r, int k, 
     if (J.do_comp && !J.P) return lrb_set_error(LRB_EINVAL, "k must be 3, 4 or 5 (got %d)", k);
     J.do_search = cov_hist || cov_sums;
     if (J.do_search && (!cov_hist || !cov_sums)) return lrb_set_error(LRB_EINVAL, "cov_hist and cov_sums go together");
-    if (cov.compact && !J.do_search) return lrb_set_error(LRB_EINVAL, "%s: sample tables need cov_hist and cov_sums", who);
-    for (int t = 0; cov.compact && t < cov.n; ++t)
-        if (!c->sample_ready[cov.b[t].table]) return lrb_set_error(LRB_EINVAL, "%s: sample slot %d is empty (table %d)", who, cov.b[t].table, t);
+    if (cov.reads_slots() && !J.do_search) return lrb_set_error(LRB_EINVAL, "%s: sample tables need cov_hist and cov_sums", who);
+    for (int t = 0; t < cov.n; ++t)
+        if (cov.b[t].table >= 0 && !c->sample_ready[cov.b[t].table])
+            return lrb_set_error(LRB_EINVAL, "%s: sample slot %d is empty (%s %d)", who, cov.b[t].table, cov.kind == CovKind::blocks ? "block" : "table", t);
     int rc;
     if (J.do_search && (rc = refuse_direct(who, cov))) return rc;
     J.use_loaded = (flags & LRB_PROFILE_USE_LOADED_TABLE) != 0;
     J.add_to_table = (flags & LRB_PROFILE_ADD_TO_TABLE) != 0;
     if (J.use_loaded && J.add_to_table) return lrb_set_error(LRB_EINVAL, "LRB_PROFILE_USE_LOADED_TABLE and LRB_PROFILE_ADD_TO_TABLE exclude each other");
     if ((J.use_loaded || J.add_to_table) && !c->table_ready) return lrb_set_error(LRB_EINVAL, "no table loaded in this context");
-    J.do_count = !J.use_loaded && ((J.do_search && !cov.compact) || table_host || (flags & (LRB_PROFILE_KEEP_TABLE | LRB_PROFILE_ADD_TO_TABLE)));
+    J.do_count = !J.use_loaded && ((J.do_search && cov.reads_full()) || table_host || (flags & (LRB_PROFILE_KEEP_TABLE | LRB_PROFILE_ADD_TO_TABLE)));
     {
         if (direct_table_path()) J.use_part = false;
         const char* e = getenv("LRB_COUNT_PATH");
@@ -675,7 +677,7 @@ static int profile_host(const char* who, lrb_ctx* c, const lrb_reads* r, int k, 
     J.comp_pinned = host_ptr_is_pinned(comp_counts);
     const auto wall0 = std::chrono::steady_clock::now();
     const uint64_t n = r->n_reads, nb = r->n_blocks;
-    const bool need_table = J.do_count || (J.do_search && !cov.compact);   // sample slots are allocated already
+    const bool need_table = J.do_count || (J.do_search && cov.reads_full());   // sample slots are allocated already
 
     // ---- devices and their read ranges (contiguous, balanced by blocks) ------------------------------------------
     std::vector<DevPlan> plans;
@@ -772,7 +774,7 @@ static int profile_host(const char* who, lrb_ctx* c, const lrb_reads* r, int k, 
     // Adding to the table: device 0 counts into its complete table, every other device into a private table from zero, so
     // that after the exchange  sum over devices of the canonical halves = previous table + this read set;  the mirror then
     // rebuilds the other half on device 0 as for any count.
-    c->table_ready = (J.use_loaded || (cov.compact && !J.do_count)) ? c->table_ready : false;   // a search of sample slots leaves it
+    c->table_ready = (J.use_loaded || (!cov.reads_full() && !J.do_count)) ? c->table_ready : false;   // a search of sample slots leaves it
     if (J.use_loaded && multi) {   // the loaded table lives on device 0: hand it to the others
         CTX_CUDA(cudaSetDevice(c->device));
         CTX_CUDA(cudaEventRecord(c->counted, c->stream));
@@ -946,6 +948,11 @@ extern "C" int lrb_profile_host_samples(lrb_ctx* c, const lrb_reads* r, int k, i
 extern "C" int lrb_profile_host_edges(lrb_ctx* c, const lrb_reads* r, int k, const uint32_t* edges, int n_edges, uint32_t* comp_counts,
                                       uint32_t* cov_hist, uint32_t* cov_sums, uint32_t* table_host, int flags) {
     return profile_call("lrb_profile_host_edges", c, r, k, lrb_cov_edges(edges, n_edges), comp_counts, cov_hist, cov_sums, table_host, flags);
+}
+
+extern "C" int lrb_profile_host_layout(lrb_ctx* c, const lrb_reads* r, int k, const lrb_cov_block* blocks, int n, uint32_t* comp_counts,
+                                       uint32_t* cov_hist, uint32_t* cov_sums, uint32_t* table_host, int flags) {
+    return profile_call("lrb_profile_host_layout", c, r, k, lrb_cov_layout(blocks, n), comp_counts, cov_hist, cov_sums, table_host, flags);
 }
 
 extern "C" int lrb_profile_host(lrb_ctx* c, const lrb_reads* r, int k, long bin_size, int bins, uint32_t* comp_counts,
@@ -1243,6 +1250,26 @@ extern "C" int lrb_ctx_table_spectrum(lrb_ctx* c, uint32_t max_count, uint64_t* 
     return rc;
 }
 
+extern "C" int lrb_ctx_sample_table_spectrum(lrb_ctx* c, int slot, uint32_t max_count, uint64_t* spectrum_host) {
+    static const char* who = "lrb_ctx_sample_table_spectrum";
+    int rc;
+    if ((rc = check_slot(c, slot, who))) return rc;
+    if (!spectrum_host) return lrb_set_error(LRB_EINVAL, "%s: null argument", who);
+    if (max_count < 2 || max_count > LRB_SPECTRUM_MAX_COUNT)
+        return lrb_set_error(LRB_EINVAL, "%s: max_count must be in [2, %u] (got %u)", who, LRB_SPECTRUM_MAX_COUNT, max_count);
+    if (!c->sample_ready[slot]) return lrb_set_error(LRB_EINVAL, "%s: sample slot %d is empty", who, slot);
+    CTX_CUDA(cudaSetDevice(c->device));
+    const size_t bytes = sizeof(uint64_t) * ((size_t)max_count + 3);
+    DevBuf spec;
+    rc = spec.reserve(bytes);
+    if (!rc && cudaMemsetAsync(spec.p, 0, bytes, c->stream) != cudaSuccess) rc = lrb_set_error(LRB_ECUDA, "cudaMemsetAsync failed");
+    if (!rc) rc = lrb_dev_compact_spectrum((const uint32_t*)c->sample[slot].p, max_count, (uint64_t*)spec.p, c->stream);
+    if (!rc && cudaMemcpyAsync(spectrum_host, spec.p, bytes, cudaMemcpyDeviceToHost, c->stream) != cudaSuccess) rc = lrb_set_error(LRB_ECUDA, "D2H failed");
+    if (cudaStreamSynchronize(c->stream) != cudaSuccess && !rc) rc = lrb_set_error(LRB_ECUDA, "spectrum failed: %s", cudaGetErrorString(cudaGetLastError()));
+    spec.release();
+    return rc;
+}
+
 // ---- synthetic reads ---------------------------------------------------------------------------
 namespace {
 
@@ -1441,7 +1468,7 @@ namespace {
 
 // The file-level searches: the coverage rows of every read of reads_path against the table(s) load(context) brings into a
 // new context, segment by segment; write(hist, sums, n_reads, row0) appends a segment's rows to the outputs, the n_outs
-// files of outs truncated first.  cov is checked; its compact blocks read the sample slots load() fills.
+// files of outs truncated first.  cov is checked; its blocks on slots read the sample slots load() fills.
 template <class Load, class Write>
 int search_file(const char* who, const CovLayout& cov, const char* reads_path, const char* const* outs, int n_outs, int threads, Load load,
                 Write write) {
@@ -1456,7 +1483,7 @@ int search_file(const char* who, const CovLayout& cov, const char* reads_path, c
     auto search = [&](const lrb_reads* s, uint64_t row0) -> int {
         const uint64_t n = s->n_reads;
         std::vector<uint32_t> hist((size_t)n * cov.W + 1), sums(n + 1);
-        const int rc2 = profile_call(who, cg.c, s, 0, cov, nullptr, hist.data(), sums.data(), nullptr, cov.compact ? 0 : LRB_PROFILE_USE_LOADED_TABLE);
+        const int rc2 = profile_call(who, cg.c, s, 0, cov, nullptr, hist.data(), sums.data(), nullptr, cov.reads_full() ? LRB_PROFILE_USE_LOADED_TABLE : 0);
         return rc2 ? rc2 : write(hist.data(), sums.data(), n, row0);
     };
     if (in.whole) return search(in.whole, 0);
@@ -1549,6 +1576,47 @@ extern "C" int lrb_search_15mers_edges(const char* table_path, const char* reads
     if (rc) return rc;
     return search_file(who, cov, reads_path, &out_txt, 1, threads, [&](lrb_ctx* c) { return lrb_ctx_table_load(c, table_path); },
                        whole_rows(out_txt, out_npy, cov.W, threads));
+}
+
+extern "C" int lrb_search_15mers_layout(const char* const* table_paths, int n_tables, const char* reads_path, const lrb_cov_block* blocks, int n,
+                                        const char* out_txt, const char* out_npy, int threads) {
+    static const char* who = "lrb_search_15mers_layout";
+    if (!table_paths || !reads_path || !out_txt) return lrb_set_error(LRB_EINVAL, "%s: null path", who);
+    if (n_tables < 1 || n_tables > LRB_MAX_SAMPLE_TABLES)
+        return lrb_set_error(LRB_EINVAL, "%s: the number of tables must be in [1, %d] (got %d)", who, LRB_MAX_SAMPLE_TABLES, n_tables);
+    CovLayout cov = lrb_cov_layout(blocks, n);
+    int rc = lrb_check_cov_layout(who, &cov);
+    if (rc) return rc;
+    // slot of each table, numbered in order of first appearance: a path listed twice (the same string) is loaded once
+    int slot_of[LRB_MAX_SAMPLE_TABLES] = {}, n_slots = 0;
+    const char* slot_path[LRB_MAX_SAMPLE_TABLES] = {};
+    for (int t = 0; t < n_tables; ++t) {
+        if (!table_paths[t]) return lrb_set_error(LRB_EINVAL, "%s: null table path (table %d)", who, t);
+        int j = 0;
+        while (j < t && strcmp(table_paths[j], table_paths[t])) ++j;
+        slot_of[t] = j == t ? n_slots++ : slot_of[j];
+        slot_path[slot_of[t]] = table_paths[j];
+    }
+    for (int m = 0; m < cov.n; ++m) {
+        const int t = cov.b[m].table;
+        if (t < 0 || t >= n_tables)
+            return lrb_set_error(LRB_EINVAL, "%s: block %d reads table %d; a block of a file-level layout names its table by its index in [0, %d) "
+                                 "of table_paths", who, m, t, n_tables);
+        cov.b[m].table = slot_of[t];
+    }
+    if ((rc = lrb_check_cov_layout(who, &cov))) return rc;   // the same path and binning twice
+    bool used[LRB_MAX_SAMPLE_TABLES] = {};
+    for (int m = 0; m < cov.n; ++m) used[cov.b[m].table] = true;
+    auto load = [&](lrb_ctx* c) -> int {   // the tables some block reads
+        for (int t = 0; t < n_slots; ++t) {
+            const int rc2 = used[t] ? lrb_ctx_sample_table_load(c, t, slot_path[t]) : LRB_OK;
+            if (rc2) return rc2;
+        }
+        return LRB_OK;
+    };
+    // every block of a row is normalised by the same sums (the read's valid windows), so the writers of one block apply at
+    // width W and the line is the n single-block lines joined by one space
+    return search_file(who, cov, reads_path, &out_txt, 1, threads, load, whole_rows(out_txt, out_npy, cov.W, threads));
 }
 
 extern "C" int lrb_table_spectrum(const char* table_path, const char* out_txt, uint32_t max_count) {

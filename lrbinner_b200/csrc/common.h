@@ -64,8 +64,9 @@ uint64_t lrb_segment_budget(uint64_t row_bytes_per_read);
 
 // ---- the coverage row of one search --------------------------------------------------------------------------------
 // A row is up to 8 column blocks side by side.  Each block bins the count of one table, the full-layout table or compact
-// table (sample slot) `table`, either by (bin_size, bins) or by count edges.  The public calls build three shapes: n
-// (bin_size, bins) blocks on the full table, n such blocks on compact tables, one edge block on the full table.
+// table (sample slot) `table`, either by (bin_size, bins) or by count edges.  The settings, samples and edges calls build
+// three shapes (n (bin_size, bins) blocks on the full table, n such blocks on compact tables, one edge block on the full
+// table); the layout calls take any blocks (lrb_cov_block).
 static_assert(LRB_MAX_COV_SETTINGS == LRB_MAX_SAMPLE_TABLES, "one block per setting or per sample table");
 
 struct CovBlock {
@@ -78,13 +79,19 @@ struct CovBlock {
     uint32_t width() const { return by_edges ? (uint32_t)n_edges + 1u : (uint32_t)bins; }
 };
 
+// which public call built a layout: the words its refusals use ("setting", "sample table", "block")
+enum class CovKind { settings, samples, edges, blocks };
+
 struct CovLayout {
     int n = 1;                         // blocks as asked for: lrb_check_cov_layout refuses n outside [1, 8]
-    bool compact = false;              // the blocks read compact tables (sample tables)
-    bool null_settings = false;        // bin_sizes or bins was NULL: the blocks were left unset
+    CovKind kind = CovKind::settings;
+    bool null_settings = false;        // bin_sizes / bins (or the blocks) were NULL: the blocks were left unset
     CovBlock b[LRB_MAX_COV_SETTINGS];
     uint32_t W = 1;                    // row width, the blocks' bins together (lrb_check_cov_layout)
-    bool single() const { return n == 1 && !compact && !b[0].by_edges; }   // what the direct search and k_search_keys take
+    bool single() const { return n == 1 && b[0].table < 0 && !b[0].by_edges; }   // what the direct search and k_search_keys take
+    // some block reads the full-layout table (it must be counted or loaded, on every device) / some block reads a slot
+    bool reads_full() const { for (int m = 0; m < n && m < LRB_MAX_COV_SETTINGS; ++m) if (b[m].table < 0) return true; return false; }
+    bool reads_slots() const { for (int m = 0; m < n && m < LRB_MAX_COV_SETTINGS; ++m) if (b[m].table >= 0) return true; return false; }
 };
 
 // n (bin_sizes[m], bins[m]) blocks, on the full table (slots NULL) or on compact table slots[m].  Reads the arrays only as
@@ -92,14 +99,16 @@ struct CovLayout {
 CovLayout lrb_cov_settings(int n, const long* bin_sizes, const int* bins, const int* slots = nullptr);
 // one block on the full table binned by count edges (the array is kept, not copied)
 CovLayout lrb_cov_edges(const uint32_t* edges, int n_edges);
+// the n public blocks as they are (edge arrays kept, not copied); read as far as lrb_cov_settings reads its arrays
+CovLayout lrb_cov_layout(const lrb_cov_block* blocks, int n);
 
 // Checks a layout and fills L->W; LRB_EINVAL naming `who` and the bad value.  Blocks: 1 <= n <= 8, compact tables in
-// [0, 8), bin_size >= 1, bins in [1, LRB_MAX_BINS], no (table, bin_size, bins) twice; edges: at most LRB_MAX_BINS - 1,
-// non-NULL when there are any, strictly increasing, the first >= 2 (counts 0 and 1 stay in bin 0, as in the reference's
-// rule); the row at most LRB_MAX_BINS wide.
+// [0, 8) (and -1, the full table, in a layout of lrb_cov_block), bin_size >= 1, bins in [1, LRB_MAX_BINS]; edges: at most
+// LRB_MAX_BINS - 1, non-NULL when there are any, strictly increasing, the first >= 2 (counts 0 and 1 stay in bin 0, as in
+// the reference's rule); no block twice (same table, same binning); the row at most LRB_MAX_BINS wide.
 int lrb_check_cov_layout(const char* who, CovLayout* L);
 
-// The partitioned search of the buckets [bucket_lo, bucket_hi) for a checked layout: block m reads `table`, or
-// compact[b[m].table] on a compact layout.  sums are rewritten by the call that includes the last bucket (partition.cu).
+// The partitioned search of the buckets [bucket_lo, bucket_hi) for a checked layout: a block reads `table`, or
+// compact[b[m].table] when b[m].table >= 0.  sums are rewritten by the call that includes the last bucket (partition.cu).
 int lrb_partition_search(const char* who, const lrb_partition* part, int bucket_lo, int bucket_hi, const uint32_t* table,
                          const uint32_t* const* compact, const CovLayout& L, uint32_t* hist, uint32_t* sums, void* stream);

@@ -274,7 +274,7 @@ extern "C" int lrb_table_read_file(const char* path, uint32_t* table) {
 CovLayout lrb_cov_settings(int n, const long* bin_sizes, const int* bins, const int* slots) {
     CovLayout L;
     L.n = n;
-    L.compact = slots != nullptr;
+    L.kind = slots ? CovKind::samples : CovKind::settings;
     L.null_settings = !bin_sizes || !bins;
     for (int m = 0; m < n && m < LRB_MAX_COV_SETTINGS && !L.null_settings; ++m) {
         L.b[m].table = slots ? slots[m] : -1;
@@ -286,9 +286,27 @@ CovLayout lrb_cov_settings(int n, const long* bin_sizes, const int* bins, const 
 
 CovLayout lrb_cov_edges(const uint32_t* edges, int n_edges) {
     CovLayout L;
+    L.kind = CovKind::edges;
     L.b[0].by_edges = true;
     L.b[0].edges = edges;
     L.b[0].n_edges = n_edges;
+    return L;
+}
+
+CovLayout lrb_cov_layout(const lrb_cov_block* blocks, int n) {
+    CovLayout L;
+    L.n = n;
+    L.kind = CovKind::blocks;
+    L.null_settings = !blocks;
+    for (int m = 0; m < n && m < LRB_MAX_COV_SETTINGS && blocks; ++m) {
+        CovBlock& b = L.b[m];
+        b.table = blocks[m].table;
+        b.by_edges = blocks[m].by_edges != 0;
+        b.bin_size = b.by_edges ? 1 : blocks[m].bin_size;
+        b.bins = b.by_edges ? 1 : blocks[m].bins;
+        b.edges = b.by_edges ? blocks[m].edges : nullptr;
+        b.n_edges = b.by_edges ? blocks[m].n_edges : 0;
+    }
     return L;
 }
 
@@ -303,29 +321,43 @@ static int check_edges(const char* who, const uint32_t* edges, int n) {
     return LRB_OK;
 }
 
+static bool same_binning(const CovBlock& a, const CovBlock& b) {
+    if (a.table != b.table || a.by_edges != b.by_edges) return false;
+    if (!a.by_edges) return a.bin_size == b.bin_size && a.bins == b.bins;
+    return a.n_edges == b.n_edges && std::equal(a.edges, a.edges + a.n_edges, b.edges);
+}
+
 int lrb_check_cov_layout(const char* who, CovLayout* L) {
-    const char* what = L->compact ? "table" : "setting";
+    const bool samples = L->kind == CovKind::samples, blocks = L->kind == CovKind::blocks;
+    const char* what = blocks ? "block" : samples ? "table" : "setting";
     if (L->n < 1 || L->n > LRB_MAX_COV_SETTINGS)
-        return lrb_set_error(LRB_EINVAL, "%s: the number of %ss must be in [1, %d] (got %d)", who, L->compact ? "sample table" : "setting",
+        return lrb_set_error(LRB_EINVAL, "%s: the number of %ss must be in [1, %d] (got %d)", who, blocks ? "block" : samples ? "sample table" : "setting",
                              LRB_MAX_COV_SETTINGS, L->n);
-    if (L->null_settings) return lrb_set_error(LRB_EINVAL, "%s: null bin_sizes / bins", who);
+    if (L->null_settings) return lrb_set_error(LRB_EINVAL, blocks ? "%s: null blocks" : "%s: null bin_sizes / bins", who);
     uint64_t W = 0;
     for (int m = 0; m < L->n; ++m) {
         const CovBlock& b = L->b[m];
+        if (blocks && (b.table < -1 || b.table >= LRB_MAX_SAMPLE_TABLES))
+            return lrb_set_error(LRB_EINVAL, "%s: table must be -1 (the full-layout table) or a slot in [0, %d) (block %d: got %d)", who,
+                                 LRB_MAX_SAMPLE_TABLES, m, b.table);
         if (b.by_edges) {
-            const int rc = check_edges(who, b.edges, b.n_edges);
+            char at[160];   // a block of a layout is named in the message
+            if (blocks) snprintf(at, sizeof at, "%s: block %d", who, m);
+            const int rc = check_edges(blocks ? at : who, b.edges, b.n_edges);
             if (rc) return rc;
-            W += b.width();
-            continue;
+        } else {
+            if (samples && (b.table < 0 || b.table >= LRB_MAX_SAMPLE_TABLES))
+                return lrb_set_error(LRB_EINVAL, "%s: slot must be in [0, %d) (table %d: got %d)", who, LRB_MAX_SAMPLE_TABLES, m, b.table);
+            if (b.bin_size < 1) return lrb_set_error(LRB_EINVAL, "%s: bin_size must be >= 1 (%s %d: got %ld)", who, what, m, b.bin_size);
+            if (b.bins < 1 || b.bins > LRB_MAX_BINS) return lrb_set_error(LRB_EINVAL, "%s: bins must be in [1, %d] (%s %d: got %d)", who, LRB_MAX_BINS, what, m, b.bins);
         }
-        if (L->compact && (b.table < 0 || b.table >= LRB_MAX_SAMPLE_TABLES))
-            return lrb_set_error(LRB_EINVAL, "%s: slot must be in [0, %d) (table %d: got %d)", who, LRB_MAX_SAMPLE_TABLES, m, b.table);
-        if (b.bin_size < 1) return lrb_set_error(LRB_EINVAL, "%s: bin_size must be >= 1 (%s %d: got %ld)", who, what, m, b.bin_size);
-        if (b.bins < 1 || b.bins > LRB_MAX_BINS) return lrb_set_error(LRB_EINVAL, "%s: bins must be in [1, %d] (%s %d: got %d)", who, LRB_MAX_BINS, what, m, b.bins);
-        for (int j = 0; j < m; ++j)
-            if (L->b[j].table == b.table && L->b[j].bin_size == b.bin_size && L->b[j].bins == b.bins)
-                return lrb_set_error(LRB_EINVAL, "%s: %s %d repeats %s %d (%sbin_size %ld, bins %d)", who, what, m, what, j,
-                                     L->compact ? "same table, " : "", b.bin_size, b.bins);
+        for (int j = 0; j < m; ++j) {
+            if (!same_binning(L->b[j], b)) continue;
+            if (b.by_edges)
+                return lrb_set_error(LRB_EINVAL, "%s: block %d repeats block %d (same table, the same %d edges)", who, m, j, b.n_edges);
+            return lrb_set_error(LRB_EINVAL, "%s: %s %d repeats %s %d (%sbin_size %ld, bins %d)", who, what, m, what, j,
+                                 samples || blocks ? "same table, " : "", b.bin_size, b.bins);
+        }
         W += b.width();
     }
     if (W > LRB_MAX_BINS) return lrb_set_error(LRB_EINVAL, "%s: the %ss' bins add up to %llu, more than %d", who, what, (unsigned long long)W, LRB_MAX_BINS);

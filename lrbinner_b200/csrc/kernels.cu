@@ -183,6 +183,12 @@ __device__ __forceinline__ void spec_add(uint32_t* s_hist, uint32_t* my_lane, un
     a.vmax = max(a.vmax, v);
 }
 
+// FULL: canonical index ci is the table word canon_word(ci); else the table is compact (lrb_dev_table_compact) and ci is
+// its entry ci
+template <bool FULL>
+__device__ __forceinline__ uint64_t spec_word(uint64_t ci) { return FULL ? canon_word(ci) : ci; }
+
+template <bool FULL>
 __global__ void __launch_bounds__(kSpecThreads)
 k_table_spectrum(const uint32_t* __restrict__ table, uint64_t u_beg, uint64_t u_end, uint64_t e0_lo, uint64_t e0_hi,
                  uint64_t e1_lo, uint64_t e1_hi, uint32_t M, unsigned long long* __restrict__ spec) {
@@ -202,7 +208,7 @@ k_table_spectrum(const uint32_t* __restrict__ table, uint64_t u_beg, uint64_t u_
 #pragma unroll
         for (int k = 0; k < kSpecUnroll; ++k) {   // a warp reads 4 x 512 contiguous bytes
             const uint64_t u = base + (uint64_t)k * 32 + lane;
-            if (u < n_units) q[k] = __ldcs(reinterpret_cast<const uint4*>(table + canon_word((u_beg + u) * 4)));
+            if (u < n_units) q[k] = __ldcs(reinterpret_cast<const uint4*>(table + spec_word<FULL>((u_beg + u) * 4)));
         }
 #pragma unroll
         for (int k = 0; k < kSpecUnroll; ++k) {
@@ -220,7 +226,7 @@ k_table_spectrum(const uint32_t* __restrict__ table, uint64_t u_beg, uint64_t u_
     // the < 8 entries before the first / after the last whole unit (key ranges not aligned to 4)
     if (blockIdx.x == 0 && threadIdx.x < 16) {
         const uint64_t ci = threadIdx.x < 8 ? e0_lo + threadIdx.x : e1_lo + (threadIdx.x - 8);
-        if (ci < (threadIdx.x < 8 ? e0_hi : e1_hi)) spec_add(s_hist, my_lane, spec, M, __ldg(table + canon_word(ci)), 1u, a);
+        if (ci < (threadIdx.x < 8 ? e0_hi : e1_hi)) spec_add(s_hist, my_lane, spec, M, __ldg(table + spec_word<FULL>(ci)), 1u, a);
     }
 
     a.n_over = __reduce_add_sync(0xFFFFFFFFu, a.n_over);
@@ -491,6 +497,24 @@ extern "C" int lrb_dev_table_compact(const uint32_t* table, uint32_t* compact, v
 // canonical (bit-15-clear) keys below `key` (key <= 2^30): 2^15 per complete 2^16-entry row, then the clear half of its row
 static uint64_t canon_rank(uint64_t key) { return ((key >> 16) << 15) + std::min<uint64_t>(key & 0xFFFFu, 0x8000u); }
 
+// the spectrum of canonical indices [ci_lo, ci_hi): whole 4-entry units [u_beg, u_end); the entries outside them are the
+// edges e0 (head) and e1 (tail), < 8 in all
+template <bool FULL>
+static int launch_spectrum(const char* name, const uint32_t* table, uint64_t ci_lo, uint64_t ci_hi, uint32_t max_count, uint64_t* spectrum,
+                           cudaStream_t st) {
+    uint64_t u_beg = (ci_lo + 3) / 4, u_end = ci_hi / 4;
+    uint64_t e0_lo = ci_lo, e0_hi = u_beg * 4, e1_lo = u_end * 4, e1_hi = ci_hi;
+    if (u_beg >= u_end) { u_end = u_beg; e0_hi = ci_hi; e1_lo = e1_hi = 0; }
+    const uint64_t per_cta = (uint64_t)kSpecThreads * kSpecUnroll;
+    const uint64_t want = std::max<uint64_t>(1, (u_end - u_beg + per_cta - 1) / per_cta);
+    const unsigned grid = (unsigned)std::min<uint64_t>(want, (uint64_t)sm_count() * 3);  // 3 x 64 KiB per SM
+    LRB_CUDA(cudaFuncSetAttribute(k_table_spectrum<FULL>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSpecSmem));
+    LRB_LAUNCH(name, st, k_table_spectrum<FULL><<<grid, kSpecThreads, kSpecSmem, st>>>(table, u_beg, u_end, e0_lo, e0_hi, e1_lo, e1_hi,
+                                                                                      max_count, reinterpret_cast<unsigned long long*>(spectrum)));
+    LRB_CUDA(cudaGetLastError());
+    return LRB_OK;
+}
+
 extern "C" int lrb_dev_table_spectrum(const uint32_t* table, uint32_t key_lo, uint32_t key_hi, uint32_t max_count,
                                       uint64_t* spectrum, void* stream) {
     if (!table || !spectrum) return lrb_set_error(LRB_EINVAL, "lrb_dev_table_spectrum: null argument");
@@ -501,19 +525,15 @@ extern "C" int lrb_dev_table_spectrum(const uint32_t* table, uint32_t key_lo, ui
     if (key_lo >= hi) return LRB_OK;
     const uint64_t ci_lo = canon_rank(key_lo), ci_hi = canon_rank(hi);
     if (ci_lo >= ci_hi) return LRB_OK;
-    // whole 4-entry units [u_beg, u_end); the entries outside them are the edges e0 (head) and e1 (tail), < 8 in all
-    uint64_t u_beg = (ci_lo + 3) / 4, u_end = ci_hi / 4;
-    uint64_t e0_lo = ci_lo, e0_hi = u_beg * 4, e1_lo = u_end * 4, e1_hi = ci_hi;
-    if (u_beg >= u_end) { u_end = u_beg; e0_hi = ci_hi; e1_lo = e1_hi = 0; }
-    const uint64_t per_cta = (uint64_t)kSpecThreads * kSpecUnroll;
-    const uint64_t want = std::max<uint64_t>(1, (u_end - u_beg + per_cta - 1) / per_cta);
-    const unsigned grid = (unsigned)std::min<uint64_t>(want, (uint64_t)sm_count() * 3);  // 3 x 64 KiB per SM
-    cudaStream_t st = (cudaStream_t)stream;
-    LRB_CUDA(cudaFuncSetAttribute(k_table_spectrum, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSpecSmem));
-    LRB_LAUNCH("k_table_spectrum", st, k_table_spectrum<<<grid, kSpecThreads, kSpecSmem, st>>>(table, u_beg, u_end, e0_lo, e0_hi, e1_lo, e1_hi,
-                                                                                  max_count, reinterpret_cast<unsigned long long*>(spectrum)));
-    LRB_CUDA(cudaGetLastError());
-    return LRB_OK;
+    return launch_spectrum<true>("k_table_spectrum", table, ci_lo, ci_hi, max_count, spectrum, (cudaStream_t)stream);
+}
+
+extern "C" int lrb_dev_compact_spectrum(const uint32_t* compact, uint32_t max_count, uint64_t* spectrum, void* stream) {
+    if (!compact || !spectrum) return lrb_set_error(LRB_EINVAL, "lrb_dev_compact_spectrum: null argument");
+    if ((uintptr_t)compact & 15u) return lrb_set_error(LRB_EINVAL, "lrb_dev_compact_spectrum: the table must be 16-byte aligned");
+    if (max_count < 2 || max_count > LRB_SPECTRUM_MAX_COUNT)
+        return lrb_set_error(LRB_EINVAL, "lrb_dev_compact_spectrum: max_count must be in [2, %u] (got %u)", LRB_SPECTRUM_MAX_COUNT, max_count);
+    return launch_spectrum<false>("k_table_spectrum_compact", compact, 0, LRB_COMPACT_ENTRIES, max_count, spectrum, (cudaStream_t)stream);
 }
 
 // ---- multi-GPU table exchange helpers (lrbinner_b200/dist.py: PeerExchange) -----------------------------------------

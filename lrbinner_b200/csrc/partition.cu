@@ -31,6 +31,8 @@
 //                   its own setting into its column block of one row (lrb_dev_partition_search_samples)
 //   k_search_edges  the same walk, the gathered count binned by caller-given count edges: bin = #{i : t_i <= count}
 //                   (lrb_dev_partition_search_edges)
+//   k_search_layout  the same walk, once per distinct table of a mixed row: the gathered count binned by every block of
+//                   that table, (bin size, bin count) or count edges, into the block's columns (lrb_dev_partition_search_layout)
 //   k_row_sums      sums[read] = sum of hist[read][*]  (every window lands in exactly one bin of each setting)
 //
 // The stream can be added in several chunks (lrb_dev_partition_add), each with its own regions, so the
@@ -1184,6 +1186,75 @@ k_search_edges(const uint32_t* __restrict__ ents, const PartMeta* __restrict__ m
                      });
 }
 
+// A mixed row (lrb_dev_partition_search_layout): the blocks of one table, each binned by (bin size, bin count) as in
+// k_search_settings or by count edges as in k_search_edges, into its own columns of rows of W words.  One walk per distinct
+// table: the gather happens once and every block of that table bins it (several binnings of one gather measured 1.09-1.65x
+// faster than separate searches, k_search_settings), while two tables in one walk measured 1.28-1.30x slower (k_search_samples
+// with two tables, DESIGN.md section 4).  The edges of the walk's edge blocks sit back to back in t[]; each edge block's are
+// copied into its own P - 1 words of dynamic shared memory (P = the least power of two >= its bins, padding 0xFFFFFFFF),
+// searched as in k_search_edges.  COMPACT: the table is compact (as in k_search_samples), else full-layout.  Five CTAs
+// per SM, as k_search_edges runs: left to itself ptxas gives the compact form 61 registers (4 CTAs) and spills the
+// full-layout form at 48; at (256, 5) both take 48 without spills.
+struct CovWalk {
+    const uint32_t* table;
+    uint32_t n, W;                                  // blocks of this walk, row pitch
+    uint64_t magic[LRB_MAX_COV_SETTINGS];
+    uint32_t by_edges[LRB_MAX_COV_SETTINGS];        // kind: 0 (bin size, bin count), 1 edges
+    uint32_t S32[LRB_MAX_COV_SETTINGS], B[LRB_MAX_COV_SETTINGS], off[LRB_MAX_COV_SETTINGS];   // B: the block's bins
+    uint32_t eoff[LRB_MAX_COV_SETTINGS];            // edge blocks: first edge in t[], first word in shared memory
+    uint32_t soff[LRB_MAX_COV_SETTINGS], P[LRB_MAX_COV_SETTINGS];
+    uint32_t t[LRB_MAX_BINS - 1];                   // a row has at most LRB_MAX_BINS - 1 edges in all
+};
+
+template <bool COMPACT>
+__global__ void __launch_bounds__(256, 5)
+k_search_layout(const uint32_t* __restrict__ ents, const PartMeta* __restrict__ meta, int bucket0, int n_chunks, ChunkList L,
+                StepTables T, uint32_t base0, uint32_t hi_mask2, int shift, const __grid_constant__ CovWalk C, uint32_t* __restrict__ hist) {
+    const int bucket = bucket0 + (int)blockIdx.y;
+    __shared__ uint32_t s_bnd[8][kTaskRuns + 1];
+    __shared__ uint32_t s_r0[8][kTaskRuns];
+    extern __shared__ uint32_t s_edge[];          // sum of P - 1 words over the edge blocks (dynamic)
+    if (meta->overflow) return;
+    for (uint32_t m = 0; m < C.n; ++m)
+        if (C.by_edges[m])
+            for (uint32_t i = threadIdx.x; i + 1u < C.P[m]; i += blockDim.x)
+                s_edge[C.soff[m] + i] = i + 1u < C.B[m] ? C.t[C.eoff[m] + i] : 0xFFFFFFFFu;
+    __syncthreads();
+    auto put = [&](uint32_t* hbase, uint32_t cnt, bool act, uint32_t lane, auto seek, auto row) {
+        uint32_t base = 0;
+        if (act) {
+            seek();
+            base = row() * C.W;
+        }
+        for (uint32_t m = 0; m < C.n; ++m) {
+            uint32_t cell = 0xFFFFFFFFu;
+            if (act) {
+                uint32_t bin;
+                if (C.by_edges[m]) {   // warp-uniform
+                    const uint32_t* se = s_edge + C.soff[m];
+                    uint32_t pos = 0;
+                    for (uint32_t step = C.P[m] >> 1; step; step >>= 1) pos += se[pos + step - 1u] <= cnt ? step : 0u;
+                    bin = min(pos, C.B[m] - 1u);
+                } else {
+                    bin = coverage_bin(cnt, C.S32[m], C.magic[m], C.B[m]);
+                }
+                cell = base + C.off[m] + bin;
+            }
+            const uint32_t peers = __match_any_sync(0xFFFFFFFFu, cell);
+            if (act && (uint32_t)__ffs(peers) - 1u == lane) atomicAdd(hbase + cell, (uint32_t)__popc(peers));
+        }
+    };
+    if (COMPACT) {
+        const uint32_t* slice = C.table + (base0 >> 1) + ((uint32_t)blockIdx.y << (shift - 1));   // the bucket's slice
+        const uint32_t emask = (1u << (shift - 1)) - 1u;
+        search_keys_body(ents, meta, bucket, n_chunks, L, T, shift, hist, C.W, s_bnd, s_r0,
+                         [&](uint32_t e) { return __ldg(slice + (e & emask)); }, put);
+    } else {
+        const uint32_t bucket_base = base0 + ((uint32_t)blockIdx.y << shift);
+        search_keys_body(ents, meta, bucket, n_chunks, L, T, shift, hist, C.W, s_bnd, s_r0, table_load(C.table, bucket_base, hi_mask2), put);
+    }
+}
+
 // sums[r] = number of windows of read r that were bucketed so far = sum of the B bins that start its histogram row (every
 // setting of a row counts each window once, so the first one does)
 __global__ void __launch_bounds__(256) k_row_sums(const uint32_t* __restrict__ hist, uint32_t* __restrict__ sums, uint64_t n_reads, uint32_t B,
@@ -1479,20 +1550,26 @@ extern "C" int lrb_dev_partition_apply_range(const lrb_partition* part, int mode
     return LRB_OK;
 }
 
-// The search of one coverage layout (common.h).  A single (bin_size, bins) block on the full table is mode 2 of
-// lrb_dev_partition_apply_range (k_search_keys); otherwise one launch of k_search_settings for several such blocks, one of
-// k_search_edges for an edge block, or one of k_search_samples per compact block, then k_row_sums.
+// The search of one coverage layout (common.h).  A layout of one of the three shapes runs the kernel tuned for it: a single
+// (bin_size, bins) block on the full table is mode 2 of lrb_dev_partition_apply_range (k_search_keys); several such blocks
+// are one launch of k_search_settings; (bin_size, bins) blocks on compact tables one launch of k_search_samples each; one
+// edge block on the full table one launch of k_search_edges.  Any other layout is one launch of k_search_layout per
+// distinct table, in order of first appearance.  Then k_row_sums.
 int lrb_partition_search(const char* who, const lrb_partition* part, int bucket_lo, int bucket_hi, const uint32_t* table,
                          const uint32_t* const* compact, const CovLayout& cov, uint32_t* hist, uint32_t* sums, void* stream) {
     if (cov.single())
         return lrb_dev_partition_apply_range(part, 2, bucket_lo, bucket_hi, const_cast<uint32_t*>(table), cov.b[0].bin_size, cov.b[0].bins, hist,
                                              sums, stream);
     if (!part->has_rids) return lrb_set_error(LRB_EINVAL, "%s: partition was built without read ids", who);
-    if (cov.compact && (part->key_lo & ((1u << part->shift) - 1u)))
+    if (cov.reads_slots() && (part->key_lo & ((1u << part->shift) - 1u)))
         return lrb_set_error(LRB_EINVAL, "%s: the partition's key range must start at a bucket boundary (key_lo %u)", who, part->key_lo);
     if (bucket_lo < 0) bucket_lo = 0;
     if (bucket_hi > part->n_buckets) bucket_hi = part->n_buckets;
     if (part->n_chunks == 0) return LRB_OK;
+    bool any_edges = false;
+    for (int m = 0; m < cov.n; ++m) any_edges = any_edges || cov.b[m].by_edges;
+    const bool settings = !any_edges && !cov.reads_slots(), samples = !any_edges && !cov.reads_full();
+    const bool edges = cov.n == 1 && cov.b[0].by_edges && cov.b[0].table < 0;
     cudaStream_t st = (cudaStream_t)stream;
     const PartMeta* meta = reinterpret_cast<const PartMeta*>(part->small);
     const ChunkList L = chunk_list(part);
@@ -1500,9 +1577,10 @@ int lrb_partition_search(const char* who, const lrb_partition* part, int bucket_
     const int shift = part->shift;
     const uint32_t hi_mask2 = ((1u << shift) - 1u) & ~0xFFFFu;
     const uint32_t base0 = part->key_lo + ((uint32_t)bucket_lo << shift);
+    auto s32 = [](long bin_size) { return bin_size > 0xFFFFFFFFl ? 0xFFFFFFFFu : (uint32_t)bin_size; };
     if (bucket_hi > bucket_lo) {
         const dim3 gs(search_grid(L, part->n_chunks), (unsigned)(bucket_hi - bucket_lo));
-        if (cov.b[0].by_edges) {
+        if (edges) {
             const CovBlock& b = cov.b[0];
             CovEdges E;
             E.n = (uint32_t)b.n_edges;
@@ -1513,30 +1591,72 @@ int lrb_partition_search(const char* who, const lrb_partition* part, int bucket_
             const size_t smem = sizeof(uint32_t) * (E.P - 1u);   // at most 16 380 bytes: no opt-in needed
             LRB_LAUNCH("k_search_edges", st, k_search_edges<<<gs, 256, smem, st>>>(part->keys, meta, bucket_lo, part->n_chunks, L, T, base0,
                                                                                    hi_mask2, shift, table, E, hist));
-        } else if (cov.compact) {
+        } else if (samples) {
             for (int t = 0, off = 0; t < cov.n; off += cov.b[t].bins, ++t) {
                 SampleGroup S = {};
                 S.W = cov.W;
                 S.table = compact[cov.b[t].table];
-                S.S32 = cov.b[t].bin_size > 0xFFFFFFFFl ? 0xFFFFFFFFu : (uint32_t)cov.b[t].bin_size;
+                S.S32 = s32(cov.b[t].bin_size);
                 S.magic = coverage_magic(S.S32);
                 S.B = (uint32_t)cov.b[t].bins;
                 S.off = (uint32_t)off;
                 LRB_LAUNCH("k_search_samples", st, k_search_samples<<<gs, 256, 0, st>>>(part->keys, meta, bucket_lo, part->n_chunks, L, T,
                                                                                        base0 >> 1, shift, S, hist));
             }
-        } else {
+        } else if (settings) {
             CovSettings C = {};
             C.n = (uint32_t)cov.n;
             C.W = cov.W;
             for (int m = 0, off = 0; m < cov.n; off += cov.b[m].bins, ++m) {
-                C.S32[m] = cov.b[m].bin_size > 0xFFFFFFFFl ? 0xFFFFFFFFu : (uint32_t)cov.b[m].bin_size;
+                C.S32[m] = s32(cov.b[m].bin_size);
                 C.magic[m] = coverage_magic(C.S32[m]);
                 C.B[m] = (uint32_t)cov.b[m].bins;
                 C.off[m] = (uint32_t)off;
             }
             LRB_LAUNCH("k_search_settings", st, k_search_settings<<<gs, 256, 0, st>>>(part->keys, meta, bucket_lo, part->n_chunks, L, T, base0,
                                                                                       hi_mask2, shift, table, C, hist));
+        } else {
+            uint32_t col[LRB_MAX_COV_SETTINGS];   // first column of each block
+            for (int m = 0, off = 0; m < cov.n; off += (int)cov.b[m].width(), ++m) col[m] = (uint32_t)off;
+            bool done[LRB_MAX_COV_SETTINGS] = {};
+            for (int first = 0; first < cov.n; ++first) {
+                if (done[first]) continue;
+                const int tab = cov.b[first].table;
+                CovWalk C;
+                C.table = tab < 0 ? table : compact[tab];
+                C.n = 0;
+                C.W = cov.W;
+                uint32_t n_t = 0, smem_words = 0;
+                for (int m = first; m < cov.n; ++m) {
+                    const CovBlock& b = cov.b[m];
+                    if (b.table != tab) continue;
+                    done[m] = true;
+                    const uint32_t j = C.n++;
+                    C.by_edges[j] = b.by_edges;
+                    C.B[j] = b.width();
+                    C.off[j] = col[m];
+                    C.S32[j] = b.by_edges ? 1u : s32(b.bin_size);
+                    C.magic[j] = coverage_magic(C.S32[j]);
+                    C.eoff[j] = n_t;
+                    C.soff[j] = smem_words;
+                    C.P[j] = 1;
+                    if (b.by_edges) {
+                        while (C.P[j] < C.B[j]) C.P[j] <<= 1;
+                        std::copy(b.edges, b.edges + b.n_edges, C.t + n_t);
+                        n_t += (uint32_t)b.n_edges;
+                        smem_words += C.P[j] - 1u;
+                    }
+                }
+                std::fill(C.t + n_t, C.t + (LRB_MAX_BINS - 1), 0xFFFFFFFFu);
+                // each edge block pads to less than twice its bins: at most 2 x 4096 words in all, no opt-in needed
+                const size_t smem = sizeof(uint32_t) * smem_words;
+                if (tab < 0)
+                    LRB_LAUNCH("k_search_layout", st, k_search_layout<false><<<gs, 256, smem, st>>>(part->keys, meta, bucket_lo, part->n_chunks, L,
+                                                                                                   T, base0, hi_mask2, shift, C, hist));
+                else
+                    LRB_LAUNCH("k_search_layout", st, k_search_layout<true><<<gs, 256, smem, st>>>(part->keys, meta, bucket_lo, part->n_chunks, L,
+                                                                                                  T, base0, hi_mask2, shift, C, hist));
+            }
         }
     }
     if (part->n_reads && bucket_hi == part->n_buckets)
@@ -1582,4 +1702,23 @@ extern "C" int lrb_dev_partition_search_edges(const lrb_partition* part, int buc
     CovLayout L = lrb_cov_edges(edges, n_edges);
     const int rc = lrb_check_cov_layout(who, &L);
     return rc ? rc : lrb_partition_search(who, part, bucket_lo, bucket_hi, table, nullptr, L, hist, sums, stream);
+}
+
+// A mixed coverage row (k_search_layout, or the kernel of the shape the layout has): blocks is a HOST array, checked by
+// lrb_check_cov_layout; block m reads `table` (table -1) or compact_tables[t]; sums are rewritten by the call that includes
+// the last bucket.
+extern "C" int lrb_dev_partition_search_layout(const lrb_partition* part, int bucket_lo, int bucket_hi, const uint32_t* table,
+                                               const uint32_t* const* compact_tables, const lrb_cov_block* blocks, int n, uint32_t* hist,
+                                               uint32_t* sums, void* stream) {
+    static const char* who = "lrb_dev_partition_search_layout";
+    if (!part || !hist || !sums) return lrb_set_error(LRB_EINVAL, "%s: null argument", who);
+    CovLayout L = lrb_cov_layout(blocks, n);
+    const int rc = lrb_check_cov_layout(who, &L);
+    if (rc) return rc;
+    for (int m = 0; m < L.n; ++m) {
+        const int t = L.b[m].table;
+        if (t < 0 && !table) return lrb_set_error(LRB_EINVAL, "%s: null table (block %d reads the full-layout table)", who, m);
+        if (t >= 0 && (!compact_tables || !compact_tables[t])) return lrb_set_error(LRB_EINVAL, "%s: null compact table %d (block %d)", who, t, m);
+    }
+    return lrb_partition_search(who, part, bucket_lo, bucket_hi, table, compact_tables, L, hist, sums, stream);
 }

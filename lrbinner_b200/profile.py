@@ -10,6 +10,7 @@
 
 The arithmetic lives in the CUDA kernels; nothing here computes profiles on the CPU.
 """
+import collections
 import ctypes as C
 import os
 
@@ -192,7 +193,7 @@ class Context:
         self.device = device
 
     def profile(self, reads, k=None, bin_size=None, bins=None, want_table=False, use_loaded_table=False, out=None,
-                keep_table=False, add_to_table=False, coverage=None, samples=None, edges=None):
+                keep_table=False, add_to_table=False, coverage=None, samples=None, edges=None, layout=None):
         """Returns dict(comp=[N,P] u32, hist=[N,bins] u32, sums=[N] u32, table=[2^30] u32) for the requested parts.
         `out` may carry preallocated (ideally page-locked) arrays under the same keys.  add_to_table: count these reads
         INTO the context's complete table (from an earlier count or table_load) instead of from zero; on failure the
@@ -205,18 +206,26 @@ class Context:
         table 0's bins, then table 1's, ..., hists[t] is table t's view and sums are shared.
         edges=[t_1, ..., t_{B-1}] (instead of every other coverage argument): bins given by strictly increasing count edges,
         t_1 >= 2; a window whose 15-mer is counted c times goes to bin searchsorted(edges, c, side="right") of hist [N, B]
-        (lrb_profile_host_edges)."""
-        given = [arg for arg, v in (("edges=[...]", edges), ("samples=[(slot, bin_size, bins), ...]", samples),
+        (lrb_profile_host_edges).
+        layout=[CovBlock, ...] (instead of every other coverage argument): a mixed row of up to 8 blocks, each on the
+        context's table (table=None) or a sample slot, each binned by (bin_size, bins) or by edges (lrb_profile_host_layout);
+        hist [N, W] holds block 0's bins, then block 1's, ..., hists[m] is block m's view and sums are shared.  A block on
+        the context's table counts it from these reads unless use_loaded_table / add_to_table; a layout of slots alone
+        leaves the context's table as it was."""
+        given = [arg for arg, v in (("layout=[CovBlock, ...]", layout), ("edges=[...]", edges), ("samples=[(slot, bin_size, bins), ...]", samples),
                                     ("coverage=[(bin_size, bins), ...]", coverage)) if v is not None]
         if given and len(given) + (bin_size is not None or bins is not None) > 1:
             raise _lib.LrbError(_lib.LRB_EINVAL, f"{given[0]} replaces the other coverage arguments (bin_size / bins, coverage, samples, "
-                                                 "edges): give one of them")
+                                                 "edges, layout): give one of them")
         n = reads.n_reads
         out = dict(out or {})
         comp = hist = sums = table = hists = slots = width = None
         if edges is not None:
             edges = _edges_array(edges)   # refused here, before a context is needed
             width = edges.size + 1
+        if layout is not None:
+            blocks, keep, widths = _layout_blocks(layout)   # refused here, before a context is needed
+            width = sum(widths)
         if samples is not None:
             samples = [(int(t), int(s_), int(b)) for t, s_, b in samples]
             slots = np.array([t for t, _, _ in samples], dtype=np.int32)
@@ -247,7 +256,11 @@ class Context:
         k = int(k) if k is not None else 0
         parts = (_ptr(comp) if comp is not None else None, _ptr(hist) if hist is not None else None,
                  _ptr(sums) if sums is not None else None, _ptr(table) if table is not None else None)
-        if edges is not None:
+        if layout is not None:
+            check(lib.lrb_profile_host_layout(self._h, reads._h, k, blocks, len(widths), *parts, flags))
+            offs = np.concatenate([[0], np.cumsum(widths)])
+            hists = [hist[:, offs[m]:offs[m + 1]] for m in range(len(widths))]
+        elif edges is not None:
             check(lib.lrb_profile_host_edges(self._h, reads._h, k, _ptr(edges), int(edges.size), *parts, flags))
         elif slots is not None:
             check(lib.lrb_profile_host_samples(self._h, reads._h, k, len(set_bs), _ptr(slots), _ptr(set_bs), _ptr(set_bins), *parts, flags))
@@ -293,6 +306,13 @@ class Context:
         counted c times), then keys counted >= max_count, their sum, and the largest count (lrb_dev_table_spectrum)."""
         spec = np.zeros(_spectrum_len(max_count), dtype=np.uint64)
         check(lib.lrb_ctx_table_spectrum(self._h, int(max_count), _ptr(spec)))
+        return spec
+
+    def sample_table_spectrum(self, slot, max_count=65536):
+        """table_spectrum() of sample slot `slot` (lrb_ctx_sample_table_spectrum): what table_spectrum() gave for the table
+        the slot was loaded from or kept, so each sample's equal-mass edges (spectrum_quantile_edges) come from its slot."""
+        spec = np.zeros(_spectrum_len(max_count), dtype=np.uint64)
+        check(lib.lrb_ctx_sample_table_spectrum(self._h, int(slot), int(max_count), _ptr(spec)))
         return spec
 
     def close(self):
@@ -414,6 +434,19 @@ def dev_table_spectrum(table, max_count, key_lo=0, key_hi=_lib.TABLE_ENTRIES, ou
         raise _lib.LrbError(_lib.LRB_EINVAL, f"spectrum buffer must be {n} contiguous 8-byte words")
     check(lib.lrb_dev_table_spectrum(C.c_void_p(table.data_ptr()), int(key_lo), min(int(key_hi), _lib.TABLE_ENTRIES), int(max_count),
                                      C.c_void_p(out.data_ptr()), _stream()))
+    return out
+
+
+def dev_compact_spectrum(compact, max_count, out=None):
+    """dev_table_spectrum of a whole compact table (dev_table_compact; lrb_dev_compact_spectrum), accumulated into `out`
+    (zeroed here when not given) and returned."""
+    import torch
+    n = _spectrum_len(max_count)
+    if out is None:
+        out = torch.zeros(n, dtype=torch.int64, device=compact.device)
+    elif out.numel() < n or out.element_size() != 8 or not out.is_contiguous():
+        raise _lib.LrbError(_lib.LRB_EINVAL, f"spectrum buffer must be {n} contiguous 8-byte words")
+    check(lib.lrb_dev_compact_spectrum(C.c_void_p(compact.data_ptr()), int(max_count), C.c_void_p(out.data_ptr()), _stream()))
     return out
 
 
@@ -581,6 +614,70 @@ class PartitionWorkspace:
         check(lib.lrb_dev_partition_search_edges(C.byref(self.part), bucket_lo, 64 if bucket_hi is None else bucket_hi,
                                                  C.c_void_p(table.data_ptr()), _ptr(e), int(e.size), C.c_void_p(hist.data_ptr()),
                                                  C.c_void_p(sums.data_ptr()), _stream()))
+
+
+    def search_layout(self, table, compact_tables, blocks, hist, sums, bucket_lo=0, bucket_hi=None):
+        """Search with a mixed row (lrb_dev_partition_search_layout): block m (a CovBlock) reads `table` (table=None) or
+        compact_tables[slot] (a list, up to 8 compact tables or None, indexed by slot) into its columns of hist [N, W];
+        hist and sums zeroed by the caller as for apply(search=True)."""
+        arr, keep, _ = _layout_blocks(blocks)
+        tables = list(compact_tables or [])
+        if len(tables) > _lib.MAX_SAMPLE_TABLES:
+            raise _lib.LrbError(_lib.LRB_EINVAL, f"at most {_lib.MAX_SAMPLE_TABLES} compact tables (got {len(tables)})")
+        ptrs = (C.c_void_p * _lib.MAX_SAMPLE_TABLES)(*[t.data_ptr() if t is not None else None for t in tables])
+        check(lib.lrb_dev_partition_search_layout(C.byref(self.part), bucket_lo, 64 if bucket_hi is None else bucket_hi,
+                                                  C.c_void_p(table.data_ptr()) if table is not None else None, ptrs, arr, len(keep),
+                                                  C.c_void_p(hist.data_ptr()), C.c_void_p(sums.data_ptr()), _stream()))
+
+
+class CovBlock(collections.namedtuple("CovBlock", "table bin_size bins edges", defaults=(None, None, None, None))):
+    """One block of a mixed coverage row: table=None reads the context's own table, table=t sample slot t (at the file
+    level, runners_utils.run_15mer_vecs_layout: table_paths[t]); binned by bin_size= and bins= (-bs / -bc) or by edges=
+    (strictly increasing counts, the first >= 2)."""
+    __slots__ = ()
+
+
+def _layout_blocks(layout):
+    """(lrb_cov_block array, the edge arrays it points into, the blocks' widths) of a list of CovBlock, refused (LRB_EINVAL) as
+    the library refuses it: 1 to 8 blocks, table None or a slot in [0, 8), edges or (bin_size >= 1, bins in [1, MAX_BINS]),
+    no block twice, the row at most MAX_BINS wide."""
+    blocks = list(layout)
+    if not 1 <= len(blocks) <= _lib.MAX_COV_SETTINGS:
+        raise _lib.LrbError(_lib.LRB_EINVAL, f"the number of blocks must be in [1, {_lib.MAX_COV_SETTINGS}] (got {len(blocks)})")
+    arr = (_lib.CovBlockC * len(blocks))()
+    keep, widths, seen = [], [], {}
+    for m, b in enumerate(blocks):
+        if not isinstance(b, CovBlock):
+            raise _lib.LrbError(_lib.LRB_EINVAL, f"block {m} is not a CovBlock (got {b!r})")
+        t = -1 if b.table is None else int(b.table)
+        if b.table is not None and not 0 <= t < _lib.MAX_SAMPLE_TABLES:
+            raise _lib.LrbError(_lib.LRB_EINVAL, f"table must be None (the context's table) or a slot in [0, {_lib.MAX_SAMPLE_TABLES}) "
+                                                 f"(block {m}: got {b.table})")
+        if b.edges is not None:
+            if b.bin_size is not None or b.bins is not None:
+                raise _lib.LrbError(_lib.LRB_EINVAL, f"block {m}: give edges or (bin_size, bins), not both")
+            e = _edges_array(b.edges)
+            keep.append(e)
+            arr[m] = _lib.CovBlockC(t, 1, 1, 1, e.ctypes.data if e.size else None, int(e.size))
+            key, width = (t, "edges", tuple(e.tolist())), int(e.size) + 1
+        else:
+            if b.bin_size is None or b.bins is None:
+                raise _lib.LrbError(_lib.LRB_EINVAL, f"block {m}: give edges or both bin_size and bins")
+            s_, n_ = int(b.bin_size), int(b.bins)
+            if not 1 <= s_ < 2 ** (8 * C.sizeof(C.c_long) - 1):
+                raise _lib.LrbError(_lib.LRB_EINVAL, f"bin_size must be >= 1 (block {m}: got {s_})")
+            if not 1 <= n_ <= _lib.MAX_BINS:
+                raise _lib.LrbError(_lib.LRB_EINVAL, f"bins must be in [1, {_lib.MAX_BINS}] (block {m}: got {n_})")
+            keep.append(None)
+            arr[m] = _lib.CovBlockC(t, 0, s_, n_, None, 0)
+            key, width = (t, s_, n_), n_
+        if key in seen:
+            raise _lib.LrbError(_lib.LRB_EINVAL, f"block {m} repeats block {seen[key]} (same table, same binning)")
+        seen[key] = m
+        widths.append(width)
+    if sum(widths) > _lib.MAX_BINS:
+        raise _lib.LrbError(_lib.LRB_EINVAL, f"the blocks' bins add up to {sum(widths)}, more than {_lib.MAX_BINS}")
+    return arr, keep, widths
 
 
 def _edges_array(edges):

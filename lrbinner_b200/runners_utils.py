@@ -117,6 +117,48 @@ def run_15mer_vecs_edges(reads_path, output, edges, threads, write_npy=False):
         f.write(" ".join(str(x) for x in e.tolist()) + "\n")
 
 
+def layout_lines(table_paths, blocks):
+    """The lines of cov_profs_layout.layout: one per block, "<table path>\tbs <S> bc <B>" or "<table path>\tedges <t1> <t2> ..."."""
+    lines = []
+    for b in blocks:
+        how = f"bs {int(b.bin_size)} bc {int(b.bins)}" if b.edges is None else " ".join(["edges"] + [str(int(x)) for x in b.edges])
+        lines.append(f"{table_paths[b.table]}\t{how}\n")
+    return lines
+
+
+def run_15mer_vecs_layout(reads_path, output, table_paths, blocks, threads, write_npy=False):
+    """Mixed coverage rows (lrb_search_15mers_layout): up to 8 blocks (profile.CovBlock), block m reading the 15mers-counts
+    file table_paths[blocks[m].table] and binned by its (bin_size, bins) or its edges, in one call: each table is loaded
+    once and the reads are parsed once.  Writes {output}/profiles/cov_profs_layout (and .npy with write_npy): per read,
+    block 0's values, then block 1's, ..., each block byte for byte the line the single-block runner (run_15mer_vecs,
+    run_15mer_vecs_edges) writes against that table; and cov_profs_layout.layout, one line per block saying how it was
+    made.  cov_profs itself is never touched (INTEGRATION.md).  No reference counterpart."""
+    from .profile import _layout_blocks
+    paths = [os.fspath(p) for p in table_paths]
+    try:
+        arr, _keep, _ = _layout_blocks(blocks)
+        for m, b in enumerate(blocks):
+            if b.table is None or not 0 <= int(b.table) < len(paths):
+                raise _lib.LrbError(_lib.LRB_EINVAL, f"block {m} reads table {b.table}: a block here names its table by its index in "
+                                                     f"[0, {len(paths)}) of table_paths")
+        if not 1 <= len(paths) <= _lib.MAX_SAMPLE_TABLES:
+            raise _lib.LrbError(_lib.LRB_EINVAL, f"the number of tables must be in [1, {_lib.MAX_SAMPLE_TABLES}] (got {len(paths)})")
+    except _lib.LrbError as err:   # refused like a library call: nothing written, the exit code of the refusal
+        logger.error(f"Error in step: Counting 15-mer profiles by layout ({err})")
+        sys.exit(err.code)
+    if not os.path.isdir(f"{output}/profiles"):
+        os.makedirs(f"{output}/profiles")
+    out = f"{output}/profiles/cov_profs_layout"
+    n = len(paths)
+    c_paths = (C.c_char_p * n)(*[os.fsencode(p) for p in paths])
+    logger.debug(f"LIB::lrb_search_15mers_layout {paths} \"{reads_path}\" \"{out}\" {list(blocks)} {threads}")
+    o = _lib.lib.lrb_search_15mers_layout(c_paths, n, os.fsencode(reads_path), arr, len(blocks), os.fsencode(out),
+                                          os.fsencode(out + ".npy") if write_npy else None, int(threads))
+    check_proc(o, "Counting 15-mer profiles by layout")
+    with open(out + ".layout", "w") as f:
+        f.writelines(layout_lines(paths, blocks))
+
+
 def run_15mer_histo(output, threads, max_count=65536):
     """Abundance spectrum of {output}/profiles/15mers-counts as {output}/profiles/15mers-histo (jellyfish `histo`
     layout: "count n_kmers" lines of canonical 15-mers), to choose -bs / -bc from (INTEGRATION.md).  No reference

@@ -4,9 +4,12 @@ Usage: launch_counts.py [--tree DIR] [--parent-tree DIR] [--out FILE]
 
 For every call (lrb_profile_host, lrb_profile_host_settings with 3 settings, lrb_profile_host_samples with 2 slots,
 lrb_profile_host_edges, and each lrb_dev_partition_search_*) the library's launch profiler (lrb_prof_enable) reports the
-kernel names and launch counts, and the rows and sums are hashed.  --tree imports the package of another built checkout
-instead of this one.  --parent-tree runs this script against that tree too and exits non-zero unless both trees launch the
-same kernels the same number of times and return the same rows.  Needs one CUDA device.
+kernel names and launch counts, and the rows and sums are hashed.  Where the package has mixed coverage rows (CovBlock), a
+mixed layout goes through lrb_profile_host_layout and lrb_dev_partition_search_layout, and the 3 settings and the 2 slots are
+given once more as layouts: those must launch and return exactly what the settings and samples calls did.  --tree imports
+the package of another built checkout instead of this one.  --parent-tree runs this script against that tree too and exits
+non-zero unless both trees launch the same kernels the same number of times and return the same rows for every call the
+other tree has, and the layouts of existing shapes match their calls.  Needs one CUDA device.
 """
 import argparse
 import hashlib
@@ -24,6 +27,10 @@ def measure():
     from lrbinner_b200 import _lib
     from lrbinner_b200.profile import (Context, PartitionWorkspace, dev_count, dev_mirror, dev_table_compact)
     from lrbinner_b200.synth import SynthSpec
+    try:
+        from lrbinner_b200.profile import CovBlock
+    except ImportError:                  # a tree without mixed coverage rows
+        CovBlock = None
 
     dev = "cuda:0"
     spec = SynthSpec(4000, seed=11, n_rate=1e-3, lowercase_frac=0.02, edge_lengths=True, scale=0.01)
@@ -56,6 +63,13 @@ def measure():
     ctx.sample_table_keep(0)
     ctx.sample_table_keep(3)
     record("lrb_profile_host_samples[2]", lambda: [(r := ctx.profile(reads, samples=[(0, 32, 10), (3, 8, 5)]))["hist"], r["sums"]])
+    if CovBlock:
+        record("layout as lrb_profile_host_settings[3]",
+               lambda: [(r := ctx.profile(reads, layout=[CovBlock(None, s_, b) for s_, b in settings]))["hist"], r["sums"]])
+        record("layout as lrb_profile_host_samples[2]",
+               lambda: [(r := ctx.profile(reads, layout=[CovBlock(0, 32, 10), CovBlock(3, 8, 5)]))["hist"], r["sums"]])
+        mixed = [CovBlock(3, edges=edges), CovBlock(None, 32, 10), CovBlock(0, 8, 5), CovBlock(3, 1, 16)]
+        record("lrb_profile_host_layout[4]", lambda: [(r := ctx.profile(reads, layout=mixed))["hist"], r["sums"]])
     ctx.close()
 
     dr, _ = spec.device_reads(dev)
@@ -78,7 +92,14 @@ def measure():
     record("lrb_dev_partition_search_settings[3]", lambda: search("search_settings", 31, table, settings))
     record("lrb_dev_partition_search_samples[2]", lambda: search("search_samples", 15, compact, [(32, 10), (8, 5)]))
     record("lrb_dev_partition_search_edges", lambda: search("search_edges", len(edges) + 1, table, edges))
+    if CovBlock:
+        record("lrb_dev_partition_search_layout[4]", lambda: search("search_layout", 39, table, [compact[0], None, None, compact[1]], mixed))
     return results
+
+
+# layouts of existing shapes and the calls whose launches and rows they must repeat
+SAME_AS = {"layout as lrb_profile_host_settings[3]": "lrb_profile_host_settings[3]",
+           "layout as lrb_profile_host_samples[2]": "lrb_profile_host_samples[2]"}
 
 
 def main():
@@ -94,10 +115,13 @@ def main():
             out = subprocess.run([sys.executable, os.path.abspath(__file__), "--tree", os.path.abspath(tree)], capture_output=True,
                                  text=True, check=True, cwd=os.path.abspath(tree)).stdout
             got[build] = json.loads(out.splitlines()[-1])
-        same = got["parent"] == got["branch"]
+        parent, branch = got["parent"], got["branch"]
+        ref = {name: parent.get(name, branch.get(SAME_AS.get(name))) for name in branch}   # what each call must equal
+        verdict = {name: "same" if ref[name] == branch[name] else "new" if ref[name] is None else "DIFFERENT" for name in branch}
+        same = all(name in branch for name in parent) and "DIFFERENT" not in verdict.values()
         report = {"same": same, **got}
-        for name in got["branch"]:
-            print(f"{name:40s} {'same' if got['parent'].get(name) == got['branch'][name] else 'DIFFERENT'} {json.dumps(got['branch'][name])}")
+        for name in branch:
+            print(f"{name:40s} {verdict[name]} {json.dumps(branch[name])}")
         if args.out:
             with open(args.out, "w") as f:
                 json.dump(report, f, indent=1)
