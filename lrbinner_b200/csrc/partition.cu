@@ -413,7 +413,8 @@ k_count_keys(const uint32_t* __restrict__ ents, const PartMeta* __restrict__ met
 // current ones are swept), takes the next slot of its sub-slice's staging row with one returning shared-memory atomic
 // and drops its low 15 key bits there (2-byte staging, kL2Stage slots = 4x the expected share per sub-slice, so no
 // count pass and no scan are needed); after one barrier each warp sweeps the rows of the sub-slices it owns into the
-// lists (contiguous 2-byte stores).  The few entries that find their row full go through a small overflow list that
+// lists (each row is staged at its destination's position modulo 8, so it is copied as 16-byte words after a short
+// head).  The few entries that find their row full go through a small overflow list that
 // the owning warp appends after the row.  Every CTA appends to its OWN segment of every (bucket, sub-slice) list
 // ([bucket][sub][cta][C3] entries; fill counters in a private global row, read and written only by the owning lane),
 // so there is no reservation between CTAs and no ordering; list order is irrelevant for counting.  Segments have a
@@ -669,29 +670,40 @@ k2_partition(const uint32_t* __restrict__ ents, PartMeta* __restrict__ meta, int
     // warp + 16 j — measured 2 ms faster per step than the blocked ownership 16 warp + j
     const uint32_t my_sub = warp + (uint32_t)kL2Warps * lane;
     const uint32_t my_pos = Y.fill_pos(my_sub);   // its counter in the fill row
+    constexpr uint32_t cm = cap - 1u;
+    // Staging rows are rings ALIGNED WITH THEIR DESTINATION: the entry bound for list position d (u16 units from the
+    // bucket's first segment) is staged in slot (d + 8 sub) mod cap of row sub.  Segments start on 16-byte boundaries and
+    // cap is a multiple of 8, so every aligned 8-entry word of a segment is one aligned 16-byte word of the row and the
+    // sweep copies rows as uint4.  The rank-0 slot moves with the row's fill, which spreads rows over the banks as the
+    // former fixed rotation by 2 sub did; + 8 sub keeps rows apart when their fills agree modulo 64 (first tiles).
+    // s_cnt[sub] = (slot of rank 0) << 16 | entries ranked so far: the returning atomic of the place phase yields both.
+    uint32_t f_my = 0, cap_my = 0, rel_my = 0, boff0 = 0;   // the lane's row in the current bucket (b_cur)
+    auto rank0 = [&]() { return ((rel_my + f_my + 8u * my_sub) & cm) << 16; };
     uint32_t e[kL2PerThread];
     uint32_t n_cur = 0, n_next = 0, b_cur = 0, b_next = 0;
     bool have = seek();
-    if (have) fetch(e, b_cur, n_cur);
+    if (have) {
+        fetch(e, b_cur, n_cur);
+        const uint32_t cell0 = b_cur * nsub;
+        const uint2 ci = lane < spw ? __ldg(c_info + cell0 + my_pos) : make_uint2(0u, 0u);
+        boff0 = __ldg(&c_info[cell0].x);
+        f_my = lane < spw ? fill[(size_t)cell0 + my_pos] : 0u;
+        cap_my = ci.y;
+        rel_my = (ci.x - boff0) * 8u + blockIdx.x * cap_my;
+        if (lane < spw) s_cnt[my_sub] = rank0();
+    }
+    __syncthreads();
     for (uint32_t it = 0; have; ++it) {
         const uint32_t par = it & 1u;
         uint32_t* frow = fill + (size_t)b_cur * nsub;
-        const uint32_t f_my = lane < spw ? frow[my_pos] : 0u;    // written only by this lane (previous tiles of this CTA)
-        // this row's segment: capacity and position relative to the bucket's first segment
-        const uint32_t cell0 = b_cur * nsub;
-        const uint2 ci_my = lane < spw ? __ldg(c_info + cell0 + my_pos) : make_uint2(0u, 0u);   // the warp's rows: one 128-byte stretch
-        const uint32_t boff0 = __ldg(&c_info[cell0].x);
-        const uint32_t cap_my = ci_my.y;
-        const uint32_t rel_my = (ci_my.x - boff0) * 8u + blockIdx.x * cap_my;
         // place: one returning atomic + one predicated 2-byte store per entry (the staged half-word keeps entry bit 15, a
         // sub-slice bit: k_count_smem masks it off); entries that find their row full are remembered in a bit mask and go
         // to the overflow list afterwards
         uint32_t spill = 0;
         auto place = [&](int j) {
             const uint32_t sub = (e[j] >> kSubBits) & sub_mask;
-            const uint32_t idx = atomicAdd(&s_cnt[sub], 1u);
-            // rows fill at the same pace: rotate each by its sub-slice so equal idx means different banks
-            if (idx < cap) s_stage[(sub << cap_shift) + ((idx + 2u * sub) & (cap - 1u))] = (uint16_t)e[j];
+            const uint32_t r = atomicAdd(&s_cnt[sub], 1u);
+            if ((r & 0xFFFFu) < cap) s_stage[(sub << cap_shift) + ((r + (r >> 16)) & cm)] = (uint16_t)e[j];
             else spill |= 1u << j;
         };
         if (n_cur == (uint32_t)kStepSlots) {
@@ -742,24 +754,31 @@ k2_partition(const uint32_t* __restrict__ ents, PartMeta* __restrict__ meta, int
         have = advance();
         if (have) fetch(e, b_next, n_next);
         __syncthreads();
+        // the next tile's bucket when it is another one: where the lane's row goes there (read now, used after the sweep)
+        const bool switch_b = have && b_next != b_cur;
+        uint2 ci_nx = make_uint2(0u, 0u);
+        uint32_t boff_nx = 0, f_nx = 0;
+        if (switch_b) {
+            const uint32_t cell0 = b_next * nsub;
+            if (lane < spw) { ci_nx = __ldg(c_info + cell0 + my_pos); f_nx = fill[(size_t)cell0 + my_pos]; }
+            boff_nx = __ldg(&c_info[cell0].x);
+        }
         // sweep: the rows of this warp's sub-slices go to this CTA's segments.  The owning lane works out where its row
-        // goes (a 32-bit position inside the bucket's span) and how much of it; the copy loop is then two predicated
-        // 2-byte copies per row (the expected row holds 8192 / nsub = cap / 4 entries)
+        // goes (a 32-bit position inside the bucket's span) and how much of it; the copy is then one 16-byte word per
+        // lane, eight lanes (one 128-byte shared-memory wavefront) per row, plus the entries in front of the row's first
+        // aligned word (the expected row holds 8192 / nsub = cap / 4 entries)
         const uint32_t novl_raw = s_novl[par];
-        uint32_t n_my = lane < spw ? s_cnt[my_sub] : 0u;   // entries of the tile ranked into this row ...
+        uint32_t n_my = lane < spw ? s_cnt[my_sub] & 0xFFFFu : 0u;   // entries of the tile ranked into this row ...
         if (novl_raw > (uint32_t)kL2Ovl && lane < spw) {   // ... minus those that left through the spill area (warp-uniform test)
             const uint32_t gone = s_sp2[my_sub];
             if (gone) { n_my -= gone; s_sp2[my_sub] = 0; }
         }
         const bool ok_my = f_my + n_my <= cap_my;   // a full segment takes nothing more: the row goes to the spill area
-        uint32_t ns_my = 0, off_my = 0;
-        if (lane < spw && n_my) {
-            s_cnt[my_sub] = 0;
-            if (ok_my) {
-                frow[my_pos] = f_my + n_my;
-                ns_my = min(n_my, cap);
-                off_my = rel_my + f_my;   // < 2^32 (k_plan_cells clamps the capacities)
-            }
+        const uint32_t off_my = rel_my + f_my;      // list position of the row's rank 0 (< 2^32: k_plan_cells clamps the capacities)
+        uint32_t ns_my = 0;
+        if (lane < spw && n_my && ok_my) {
+            frow[my_pos] = f_my + n_my;
+            ns_my = min(n_my, cap);
         }
         if (tid == 0) s_novl[par ^ 1u] = 0;  // the next tile's list; last read before the previous tile's closing barrier
         // rows whose segment is full (a hot sub-slice: more than C3 entries from this CTA): staged part and overflow-list
@@ -767,11 +786,11 @@ k2_partition(const uint32_t* __restrict__ ents, PartMeta* __restrict__ meta, int
         const uint32_t full_rows = __ballot_sync(0xFFFFFFFFu, lane < spw && n_my != 0u && !ok_my);
         for (uint32_t rest = full_rows; rest; rest &= rest - 1u) {
             const uint32_t jj = (uint32_t)__ffs(rest) - 1u;
-            const uint32_t n = __shfl_sync(0xFFFFFFFFu, n_my, jj);
+            const uint32_t n = __shfl_sync(0xFFFFFFFFu, n_my, jj), off = __shfl_sync(0xFFFFFFFFu, off_my, jj);
             const uint32_t sub = warp + (uint32_t)kL2Warps * jj;
             const uint16_t* src = s_stage + (sub << cap_shift);
             const uint32_t bkt = b_cur;
-            spill_warp(min(n, cap), bkt, [&](uint32_t i) { return Y.key_of(bkt, sub, src[(i + 2u * sub) & (cap - 1u)] & 0x7FFFu); });
+            spill_warp(min(n, cap), bkt, [&](uint32_t i) { return Y.key_of(bkt, sub, src[(off + i + 8u * sub) & cm] & 0x7FFFu); });
             if (n > cap) {
                 const uint32_t novl = min(novl_raw, (uint32_t)kL2Ovl);
                 for (uint32_t i0 = 0; i0 < novl; i0 += 32) {
@@ -790,39 +809,74 @@ k2_partition(const uint32_t* __restrict__ ents, PartMeta* __restrict__ meta, int
             }
         }
         uint16_t* __restrict__ lists = ws + Y.seg0 + 8ull * boff0;
-        constexpr uint32_t cm = cap - 1u;
-        const uint32_t big = __ballot_sync(0xFFFFFFFFu, ns_my > 64u || (ok_my && n_my > cap));  // rows the fast loop does not finish
+        // Row jj = g + lane / 8 of the warp, lane q = lane % 8 of its group.  Head: list positions [off, next multiple of
+        // 8), entry by entry.  Then the aligned words from there up to the word holding the last entry, whole: the entries
+        // of that word past the row are past the segment's fill (k_count_smem reads only up to the fill, and the next tile
+        // of this row overwrites them), and the word ends inside the segment (segments are whole words).  One word per
+        // lane covers rows of up to 64 entries; the groups are independent, so their loads and stores overlap.  Longer
+        // rows (the mean row is 8192 / nsub entries: rare from 256 sub-slices per bucket up) take more words in a second loop.
+        const uint32_t q = lane & 7u;
+        auto row_of = [&](uint32_t g, uint32_t& ns, uint32_t& off, uint32_t& sub) {
+            const uint32_t jj = g + (lane >> 3);
+            ns = __shfl_sync(0xFFFFFFFFu, ns_my, jj & 31u);
+            off = __shfl_sync(0xFFFFFFFFu, off_my, jj & 31u);
+            if (jj >= spw) ns = 0;
+            sub = warp + (uint32_t)kL2Warps * jj;
+        };
+        auto copy_word = [&](uint32_t sub, uint32_t dw) {   // list word at dw (a multiple of 8) from its ring word
+            const uint16_t* src = s_stage + (sub << cap_shift);
+            *reinterpret_cast<uint4*>(lists + dw) = *reinterpret_cast<const uint4*>(src + ((dw + 8u * sub) & cm));
+        };
+        bool longer = false;
 #pragma unroll
-        for (uint32_t jj = 0; jj < spw; ++jj) {
-            const uint32_t ns = __shfl_sync(0xFFFFFFFFu, ns_my, jj);
-            const uint32_t off = __shfl_sync(0xFFFFFFFFu, off_my, jj) + lane;
-            const uint32_t sub = warp + (uint32_t)kL2Warps * jj;
-            const uint16_t* src = s_stage + (sub << cap_shift);
-            const uint32_t p0 = (lane + 2u * sub) & cm, p1 = (lane + 32u + 2u * sub) & cm;
-            if (lane < ns) lists[off] = src[p0];
-            if (lane + 32u < ns) lists[off + 32u] = src[p1];
+        for (uint32_t g = 0; g < spw; g += 4) {
+            uint32_t ns, off, sub;
+            row_of(g, ns, off, sub);
+            const uint32_t w0 = (off + 7u) >> 3, w1 = (off + ns + 7u) >> 3;   // first whole word, end of the row's words
+            const uint32_t d = (off & ~7u) + q;
+            if (d >= off && d < off + ns && d < w0 * 8u) lists[d] = s_stage[(sub << cap_shift) + ((d + 8u * sub) & cm)];
+            const uint32_t nw = (ns && w1 > w0) ? w1 - w0 : 0u;
+            if (q < nw) copy_word(sub, (w0 + q) * 8u);
+            longer |= nw > 8u;
         }
-        for (uint32_t rest = big; rest; rest &= rest - 1u) {  // rare: long rows, rows that spilled into the overflow list
-            const uint32_t jj = (uint32_t)__ffs(rest) - 1u;
-            const uint32_t ns = __shfl_sync(0xFFFFFFFFu, ns_my, jj), n = __shfl_sync(0xFFFFFFFFu, n_my, jj);
-            const uint32_t sub = warp + (uint32_t)kL2Warps * jj;
-            uint16_t* __restrict__ dst = lists + __shfl_sync(0xFFFFFFFFu, off_my, jj);
-            const uint16_t* src = s_stage + (sub << cap_shift);
-            for (uint32_t j = lane + 64u; j < ns; j += 32) dst[j] = src[(j + 2u * sub) & cm];
-            if (n > cap) {
-                const uint32_t novl = min(novl_raw, (uint32_t)kL2Ovl);
-                uint32_t base = ns;
-                for (uint32_t i0 = 0; i0 < novl; i0 += 32) {
-                    const uint32_t i = i0 + lane;
-                    const uint32_t r = i < novl ? s_ovl[i] : 0xFFFFFFFFu;
-                    const bool mine = i < novl && (r >> kSubBits) == sub;
-                    const uint32_t bal = __ballot_sync(0xFFFFFFFFu, mine);
-                    const uint32_t at = base + (uint32_t)__popc(bal & ((1u << lane) - 1u));
-                    if (mine && at < n) dst[at] = (uint16_t)(r & 0x7FFFu);
-                    base += (uint32_t)__popc(bal);
-                }
+        if (__any_sync(0xFFFFFFFFu, longer)) {
+#pragma unroll 1
+            for (uint32_t g = 0; g < spw; g += 4) {
+                uint32_t ns, off, sub;
+                row_of(g, ns, off, sub);
+                const uint32_t w0 = (off + 7u) >> 3, w1 = (off + ns + 7u) >> 3;
+                const uint32_t nw = (ns && w1 > w0) ? w1 - w0 : 0u;
+                for (uint32_t i = q + 8u; i < nw; i += 8) copy_word(sub, (w0 + i) * 8u);
             }
         }
+        const uint32_t ovl_rows = __ballot_sync(0xFFFFFFFFu, ok_my && n_my > cap);
+        if (ovl_rows) __syncwarp();   // the overflow-list entries land after (and over the tail of) the row's last word
+        for (uint32_t rest = ovl_rows; rest; rest &= rest - 1u) {  // rare: rows that spilled into the overflow list
+            const uint32_t jj = (uint32_t)__ffs(rest) - 1u;
+            const uint32_t n = __shfl_sync(0xFFFFFFFFu, n_my, jj);
+            const uint32_t sub = warp + (uint32_t)kL2Warps * jj;
+            uint16_t* __restrict__ dst = lists + __shfl_sync(0xFFFFFFFFu, off_my, jj);
+            const uint32_t novl = min(novl_raw, (uint32_t)kL2Ovl);
+            uint32_t base = cap;
+            for (uint32_t i0 = 0; i0 < novl; i0 += 32) {
+                const uint32_t i = i0 + lane;
+                const uint32_t r = i < novl ? s_ovl[i] : 0xFFFFFFFFu;
+                const bool mine = i < novl && (r >> kSubBits) == sub;
+                const uint32_t bal = __ballot_sync(0xFFFFFFFFu, mine);
+                const uint32_t at = base + (uint32_t)__popc(bal & ((1u << lane) - 1u));
+                if (mine && at < n) dst[at] = (uint16_t)(r & 0x7FFFu);
+                base += (uint32_t)__popc(bal);
+            }
+        }
+        // the next tile's rows: rank counters reset, rank-0 slots where its entries will go
+        if (ok_my) f_my += n_my;
+        if (switch_b) {
+            boff0 = boff_nx;
+            f_my = f_nx;
+            cap_my = ci_nx.y;
+            rel_my = (ci_nx.x - boff0) * 8u + blockIdx.x * cap_my;
+        }
+        if (have && lane < spw) s_cnt[my_sub] = rank0();
         __syncthreads();
         n_cur = n_next;
         b_cur = b_next;

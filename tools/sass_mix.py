@@ -4,7 +4,7 @@
 
 One row per kernel instantiation: static instruction counts by class.  The columns that matter for this path:
 LDG/STG (global), LDS/STS/ATOMS (shared), RED/ATOMG (global atomics), MATCH/SHFL/VOTE (warp aggregation),
-SHF/LOP3/IADD (the key arithmetic), BAR, and the Blackwell data-movement mnemonics (UBLKCP = cp.async.bulk,
+SHF/LOP3/IADD (the key arithmetic), BAR, LDS.128/STG.128 (16-byte accesses, also counted in LDS/STG), and the Blackwell data-movement mnemonics (UBLKCP = cp.async.bulk,
 UTMALDG/UTMASTG = TMA tensor copies, LDGSTS = cp.async, SYNCS = mbarrier) so that their presence or absence is on record.
 """
 import collections
@@ -17,6 +17,8 @@ CLASSES = [("LDG", r"^LDG"), ("STG", r"^STG"), ("LDS", r"^LDS"), ("STS", r"^STS"
            ("SHF", r"^SHF"), ("LOP3", r"^LOP3|^ULOP3"), ("IADD", r"^IADD|^UIADD|^IMAD|^LEA"), ("ISETP", r"^ISETP|^UISETP"), ("SEL", r"^SEL|^USEL"),
            ("POPC/BREV/FLO", r"^POPC|^BREV|^FLO"), ("BAR", r"^BAR"), ("BRA", r"^BRA|^BSSY|^BSYNC|^EXIT"),
            ("UBLKCP", r"^UBLKCP"), ("UTMA", r"^UTMALDG|^UTMASTG|^UTMAPF"), ("LDGSTS", r"^LDGSTS"), ("SYNCS", r"^SYNCS"), ("TCGEN05", r"^UTC|^TCGEN")]
+# 16-byte accesses, counted a second time beside their class (LDS / STG)
+WIDE = [("LDS.128", r"^LDS\.128"), ("STG.128", r"^STG(\.E)?\.128")]
 
 
 def demangle(names):
@@ -46,8 +48,11 @@ def main(path="lrbinner_b200/liblrb200.so"):
                 if re.match(pat, op):
                     funcs[cur][name] += 1
                     break
+            for name, pat in WIDE:
+                if re.match(pat, op):
+                    funcs[cur][name] += 1
     names = demangle(list(funcs))
-    cols = ["total"] + [c for c, _ in CLASSES]
+    cols = ["total"] + [c for c, _ in CLASSES] + [c for c, _ in WIDE]
     print("kernel," + ",".join(cols))
     for nm, cnt in sorted(zip(names, funcs.values())):
         print(f'"{nm}",' + ",".join(str(cnt[c]) for c in cols))
